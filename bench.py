@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the AL query pass (THC + local-peak + WPU + fusion + core-set) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one complete query over a fixed synthetic pool.  `--config` picks BASELINE.json's
@@ -18,10 +18,13 @@ REFERENCE's pick list for the configuration (oracle/pin_scale.py) the run fails 
 picks differ.  `value` = frames of the pool / time of one query with the pool resident in HBM; `e2e` =
 the same query through the public API with the pool in pinned host memory (H2D copies of heat maps /
 boxes / flags / features and the D2H read of the picks inside the timed region).  ONE JSON line on rank 0.
+`--dump-outputs DIR` writes what the last timed step returned (picks, scores, keypoints; a seeded sample of rows
+where an array is large) as .npy files: the inputs are fixed by the arguments, so two builds can be compared.
 """
 from __future__ import annotations
 
 import argparse
+import dataclasses
 import hashlib
 import json
 import os
@@ -68,11 +71,51 @@ def parse():
     p.add_argument("--cpu-frames", type=int, default=4096, help="frames of the CPU scoring sample")
     p.add_argument("--cpu-greedy-steps", type=int, default=20, help="greedy steps of the CPU core-set sample")
     p.add_argument("--cpu-rows", type=int, default=200000, help="rows of the CPU core-set sample (cost per step is linear in rows)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last timed step computed as DIR/<name>.npy (rank 0; at most 64 MB in all)")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def sha_picks(picks) -> str:
     return hashlib.sha256(np.asarray(picks, dtype="<i8").tobytes()).hexdigest()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def result_arrays(res) -> dict:
+    """The arrays and numbers a caller receives in a result dataclass (run statistics left out)."""
+    return {f.name: getattr(res, f.name) for f in dataclasses.fields(res) if f.name not in ("stats", "extra")}
+
+
+def dump_outputs(out_dir: str, outputs: dict):
+    """Write each output as out_dir/<name>.npy: float32 stays float32, everything else becomes float64 (which holds
+    the integer indices exactly).  Every output gets an equal share of the 64 MB; one larger than its share is
+    replaced by a fixed sample of its rows (seed 0, ascending), whose indices go to <name>_rows.npy, so that two
+    builds run with the same arguments dump the same elements."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    for name, v in outputs.items():
+        if v is None:
+            continue
+        t = v.detach() if isinstance(v, torch.Tensor) else torch.as_tensor(np.asarray(v))
+        arrays[name] = t.reshape(1) if t.dim() == 0 else t
+    share = DUMP_BYTES // max(1, len(arrays))
+    for name, t in arrays.items():
+        t = t if t.dtype in (torch.float32, torch.float64) else t.to(torch.float64)
+        row_bytes = t.numel() // max(1, t.shape[0]) * t.element_size()
+        if t.shape[0] * row_bytes > share:
+            m = share // (row_bytes + 8)
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], m, replace=False))
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------ clocks
@@ -296,7 +339,7 @@ def main():
             return
         import torch  # noqa: F401
         vals, det = [], None
-        for _ in range(max(1, min(a.steps, 3))):
+        for _ in range(a.steps):
             v, det = cpu_reference_arm(a.config, n, k, moks, a.cpu_frames, a.cpu_greedy_steps, a.cpu_rows)
             vals.append(v)
         v = statistics.median(vals)
@@ -489,6 +532,8 @@ def full_query(a, n, n_lab, k, moks, config, rank, world, local, dev):
         td.all_reduce(ms, op=td.ReduceOp.MAX)
     ms_step = float(ms.item()) / a.steps
     launches = vatlq._lib.launch_count() - launches0
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, result_arrays(res))
     prune = ops.prune_stats(reset=True)
     streamed_frac = prune["streamed"] / prune["tiles"] if prune["tiles"] else 1.0
     dmma_peak = ops.measure_fp64_mma(dev)
@@ -832,6 +877,9 @@ def small_config(a, n, k, moks, config, rank, world, dev):
             times.append(e0.elapsed_time(e1))
     launches = vatlq._lib.launch_count() - launches0
     ms_step = sum(times) / len(times)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, result_arrays(out) if dataclasses.is_dataclass(out)
+                     else {{2: "wpu", 3: "picks"}[a.config]: out})
     if a.config == 3:
         prune = ops.prune_stats(reset=True)
         sf = prune["streamed"] / prune["tiles"] if prune["tiles"] else 1.0

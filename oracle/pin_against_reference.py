@@ -25,6 +25,8 @@ REF = os.environ.get("VATL_REFERENCE", "/root/reference")
 GOLD = os.path.join(ROOT, "tests", "golden")
 sys.path.insert(0, ROOT)
 
+from oracle import golden_inputs as GI  # noqa: E402  (the heat maps and features are rebuilt, not stored)
+
 
 def import_reference():
     sys.path[:0] = [REF, os.path.join(REF, "ALiPy")]
@@ -76,49 +78,13 @@ def ref_autoencoder(R, weights):
     return ae.eval()
 
 
-def edge_maps():
-    """(E,17,64,48) fp32 frames built to hit the edge cases of SURVEY.md §8a."""
-    rng = np.random.default_rng(99)
-    base = rng.normal(0, 0.02, (17, 64, 48)).astype(np.float32)
-    frames = []
-    f = base.copy()                                   # 0: plateaus {1,1}, 0.5 and 0.49
-    f[0] = 0; f[0, 10, 10] = 1; f[0, 10, 11] = 1; f[0, 30, 30] = .5; f[0, 40, 20] = .49
-    f[1] = -np.abs(f[1]) - 0.1                        # all-negative joint: no peak survives
-    f[2] = np.minimum(f[2], 0); f[2, 5, 5] = 0        # max == 0
-    f[3] = 0; f[3, 0, 0] = 2; f[3, 63, 47] = 2        # ties -> first index; corners (no 1/4 px)
-    f[4] = 0; f[4, 1, 1] = 1; f[4, 1, 2] = .5         # px==1: not strictly interior
-    f[5] = 0; f[5, 2, 2] = 1; f[5, 2, 3] = .5; f[5, 3, 2] = .7; f[5, 1, 2] = .7   # dy sign 0
-    f[6] = 0; f[6, 62, 46] = 1; f[6, 61, 46] = .2     # px==46,py==62: not interior
-    f[7] = 0; f[7, 61, 45] = 1; f[7, 61, 44] = .2; f[7, 60, 45] = .3              # last interior
-    f[8] = 0.25                                       # constant positive: interior is all plateau
-    f[9] = 0; f[9, 0, 10] = -1                        # zeros everywhere but one negative
-    f[10] = 0; f[10, 20, :] = 1                       # a full ridge row
-    f[11] = 0; f[11, 31, 23] = 3; f[11, 31, 24] = 3; f[11, 32, 23] = 3            # plateau argmax
-    frames.append(f)
-    g = -np.abs(base) - 1.0                           # 1: every joint negative -> NaN peak mean
-    frames.append(g.astype(np.float32))
-    z = np.zeros_like(base)                           # 2: all-zero frame
-    frames.append(z)
-    frames.append(base.copy())                        # 3: pure noise
-    return np.stack(frames).astype(np.float32)
-
-
 def pin_next_rows(R, O, synth):
     """SURVEY.md §8f rows: HP / TPC / Entropy (reference methods compute_tpc / compute_entropy
     called unbound; the HP expression of :330 evaluated as written), Influence / Diversity /
     top-k (the sklearn calls of :469-477, :527-540, :581-590 evaluated as written)."""
     from sklearn.neighbors import KNeighborsTransformer
-    rng = np.random.default_rng(21)
-    n = 14
-    ids, ip, inx = synth.track_flags(n, rng, mean_len=5.0)
-    H = synth.heatmaps(n, seed=21, track_ids=ids)
-    # make TPC discriminative: inside a track most joints stay put, a few move by whole pixels
-    for i in range(1, n):
-        if ip[i]:
-            H[i] = H[i - 1] + rng.normal(0, 1e-4, H[i].shape).astype(np.float32)
-            for j in rng.choice(17, size=int(rng.integers(0, 6)), replace=False):
-                H[i, j] = np.roll(H[i - 1, j], (int(rng.integers(-2, 3)), int(rng.integers(-2, 3))), axis=(0, 1))
-    boxes = synth.boxes_xyxy(n, seed=21)
+    H, ip, inx, boxes, rng = GI.next_inputs()
+    n = H.shape[0]
     fake = SimpleNamespace(heatmap_to_coord=R.heatmap_to_coord_simple, eval_joints=list(range(17)),
                            hm_size=[64, 48], norm_type=None)
     hp_ref, tpc_ref, ent_ref, ent_pos_ref = [], [], [], []
@@ -150,11 +116,11 @@ def pin_next_rows(R, O, synth):
     assert len(set(tpc_ref)) > 3, tpc_ref
 
     # Influence / Diversity / top-k on clustered and i.i.d. embeddings
-    out = dict(H=H, boxes=boxes, is_prev=ip, is_next=inx, hp=np.array(hp_ref), tpc=np.array(tpc_ref),
+    out = dict(boxes=boxes, is_prev=ip, is_next=inx, hp=np.array(hp_ref), tpc=np.array(tpc_ref),
                entropy_raw=np.array(ent_ref), entropy_pos=np.array(ent_pos_ref))
     for tag, clustered in (("clu", True), ("iid", False)):
         N, k = 400, 20
-        X32 = synth.embeddings(N, d=256, seed=31 + clustered, clustered=clustered)
+        X32 = GI.next_features(clustered)
         X = X32.astype(np.float64)
         lab = sorted(rng.choice(N, 60, replace=False).tolist())
         unl = [i for i in range(N) if i not in set(lab)]
@@ -179,7 +145,7 @@ def pin_next_rows(R, O, synth):
         dd = dict((int(idx), sc) for idx, sc in sorted(dd.items(), key=lambda x: x[1]))          # :587-588
         div_ref = list(dd.keys())[:k]                                                            # :589
         same(div_ref, O.diversity_select(X, unl, total, k), f"diversity {tag}")
-        out.update({f"{tag}_X": X32, f"{tag}_labeled": np.array(lab, np.int64), f"{tag}_unc": unc_score,
+        out.update({f"{tag}_labeled": np.array(lab, np.int64), f"{tag}_unc": unc_score,
                     f"{tag}_cw": np.float64(cw), f"{tag}_k": np.int64(k), f"{tag}_rowsum": rowsum_ref,
                     f"{tag}_influence": infl, f"{tag}_total": total, f"{tag}_topk": np.array(top_ref, np.int64),
                     f"{tag}_div_rowsum": div, f"{tag}_diversity": np.array(div_ref, np.int64)})
@@ -224,27 +190,13 @@ def pin_peaks(R, O, synth):
     the RESTATED peak_local_max standing in for skimage.feature.peak_local_max (scikit-image is not installed
     here: the restatement's parity with the library is unpinned; everything around it is the reference's code)."""
     sys.modules["active_learning.ActiveLearning"].peak_local_max = O.peak_local_max   # (the module, not the class)
-    rng = np.random.default_rng(33)
-    H = synth.heatmaps(6, seed=33)
-    e = np.zeros((2, 17, 64, 48), np.float32)
-    f = e[0]
-    f[0] = 0.25                                                   # constant map: trivial image, no peak
-    f[1, 20, 20] = 1; f[1, 20, 24] = 1; f[1, 20, 25] = 0.9          # equal peaks 4 apart: the second is rejected
-    f[2, 20, 20] = 1; f[2, 20, 25] = 1                              # equal peaks 5 apart: both kept, margin 0
-    f[3, 4, 10] = 2; f[3, 30, 4] = 2; f[3, 59, 10] = 2; f[3, 30, 30] = 0.5   # border peaks are excluded
-    f[4, 10:13, 10:13] = 0.7; f[4, 40, 30] = 0.7                    # plateau: every plateau pixel is a candidate
-    f[5] = rng.normal(0, 0.02, (64, 48)).astype(np.float32)         # pure noise: more than five candidates
-    f[6] = -np.abs(rng.normal(0, 0.02, (64, 48))).astype(np.float32) - 1    # all negative
-    f[7, 5, 5] = 1; f[7, 58, 42] = 0.5                              # first / last interior pixel
-    f[8, 30, 20] = 1                                                # a single peak: entropy(softmax([x])) = 0
-    e[1] = H[0] * 0 + rng.normal(0, 1e-3, (17, 64, 48)).astype(np.float32)
-    H = np.concatenate([H, e], axis=0)
+    H = GI.peaks_inputs()
     fake = SimpleNamespace()
     mpe = np.array([float(R.AL.compute_mpe(fake, H[i])) for i in range(len(H))])
     mar = np.array([float(R.AL.compute_margin(fake, H[i])) for i in range(len(H))])
     same(mpe, [O.mpe_item(H[i]) for i in range(len(H))], "MPE")
     same(mar, [O.margin_item(H[i]) for i in range(len(H))], "Margin")
-    np.savez_compressed(os.path.join(GOLD, "peaks.npz"), H=H, mpe=mpe, margin=mar)
+    np.savez_compressed(os.path.join(GOLD, "peaks.npz"), mpe=mpe, margin=mar)
     print("MPE / Margin pinned (peak_local_max restated):", mpe[:3], mar[:3])
 
 
@@ -349,17 +301,8 @@ def main():
     same(O.localpeak_values(kat), [4, 3], "KAT oracle")
 
     # ---------------- scan: coords / maxvals / THC / peak mean ------------------------
-    rng = np.random.default_rng(0)
-    n = 10
-    ids, ip, inx = synth.track_flags(n, rng, mean_len=4.0)
-    H = synth.heatmaps(n, seed=0, track_ids=ids)
-    E = edge_maps()
-    H = np.concatenate([H, E], axis=0)
-    ne = E.shape[0]
-    ip = np.r_[ip, np.array([0, 1, 1, 0][:ne], np.uint8)]
-    inx = np.r_[inx, np.array([1, 1, 0, 0][:ne], np.uint8)]
+    H, ip, inx, boxes = GI.scan_inputs()
     n = H.shape[0]
-    boxes = synth.boxes_xyxy(n, seed=0)
     ref = {"hm_xy": [], "img_xy": [], "maxv": [], "peak": [], "thc": [], "thc3": []}
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
@@ -389,7 +332,7 @@ def main():
             ref["thc"].append(float(thc))
     thc_or = O.thc_pool(H, ip, inx)
     same(ref["thc"], thc_or, "thc pool")
-    np.savez_compressed(os.path.join(GOLD, "scan.npz"), H=H, boxes=boxes, is_prev=ip, is_next=inx,
+    np.savez_compressed(os.path.join(GOLD, "scan.npz"), boxes=boxes, is_prev=ip, is_next=inx,
                         hm_xy=np.stack(ref["hm_xy"]), img_xy=np.stack(ref["img_xy"]),
                         maxv=np.stack(ref["maxv"]), peak=np.array(ref["peak"], np.float32),
                         thc=np.array(ref["thc"], np.float64))
@@ -459,12 +402,12 @@ def main():
             picks_ref = R.AL.coreset_selection(fake, X, unc.copy())
         picks_or, md = O.coreset_select(X, unc.copy(), labeled, k, moks, lam, rule)
         same(picks_ref, picks_or, f"coreset {tag}")
-        cases[tag] = dict(X=X32, unc=unc, labeled=np.array(list(labeled), np.int64), k=k, moks=moks,
+        cases[tag] = dict(unc=unc, labeled=np.array(list(labeled), np.int64), k=k, moks=moks,
                           lam=lam, rule=rule, picks=np.array(picks_ref, np.int64), min_d=md)
 
     rng = np.random.default_rng(3)
-    Xc = synth.embeddings(600, d=256, seed=2, clustered=True)
-    Xi = synth.embeddings(500, d=256, seed=4, clustered=False)
+    F = GI.coreset_features()
+    Xc, Xi, Xd = F["clustered_round0"], F["iid_round0_moks"], F["duplicates"]
     unc_c, unc_i = rng.uniform(0, 1, 600), rng.uniform(0, 1, 500)
     lab20 = sorted(rng.choice(600, 120, replace=False).tolist())
     run_coreset("clustered_round0", Xc, unc_c, [], 60, 0.0, 0.01)
@@ -472,11 +415,9 @@ def main():
     run_coreset("iid_round0_moks", Xi, unc_i, [], 50, 0.6, 0.01)
     run_coreset("iid_fixed_lambda", Xi, unc_i, [3, 77, 200], 40, 0.3, 0.01, rule="fixed_lambda", fixed=True)
     run_coreset("iid_dist_only", Xi, unc_i, [5, 9], 40, 0.3, 0.0, rule="dist")
-    Xd = Xi.copy(); Xd[100:110] = Xd[10:20]                      # duplicate rows
     run_coreset("duplicates", Xd, unc_i, [0], 60, 0.5, 0.01)
     run_coreset("zero_unc", Xc, np.zeros(600), [7], 40, 0.6, 0.01)
-    Xfull = synth.embeddings(160, d=2048, seed=6, clustered=True)     # full feature width
-    run_coreset("d2048", Xfull, rng.uniform(0, 1, 160), [], 30, 0.6, 0.01)
+    run_coreset("d2048", F["d2048"], rng.uniform(0, 1, 160), [], 30, 0.6, 0.01)
     flat = {}
     for tag, c in cases.items():
         for key, val in c.items():

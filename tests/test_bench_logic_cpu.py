@@ -34,3 +34,27 @@ def test_traffic_table_and_peaks():
     assert bench.ncu_traffic("scan", 170000) > 35e9 and bench.ncu_traffic("scan", 123) is None
     gbs, src = bench.peak_hbm()
     assert 3000 < gbs < 9000 and isinstance(src, str)
+
+
+def test_dump_outputs_budget_and_fixed_sample(tmp_path):
+    import torch
+    import bench
+    from vatlq.query import QueryResult
+    n = 1 << 20
+    res = QueryResult(picks=torch.arange(5000, 0, -1), thc=torch.rand(n), wpu=torch.rand(n), peak_mean=torch.rand(n),
+                      kpts=torch.rand(n, 17, 3), unc=torch.rand(n, dtype=torch.float64), combine_weight=0.25, stats=object())
+    out = bench.result_arrays(res)
+    assert sorted(out) == ["combine_weight", "kpts", "peak_mean", "picks", "thc", "unc", "wpu"]
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), out)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["combine_weight.npy", "kpts.npy", "kpts_rows.npy", "peak_mean.npy", "picks.npy", "thc.npy", "unc.npy", "wpu.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64 << 20
+    for f in files:
+        x, y = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert x.dtype in (np.float32, np.float64) and np.array_equal(x, y)
+    rows = np.load(tmp_path / "a" / "kpts_rows.npy").astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "a" / "kpts.npy"), res.kpts[torch.from_numpy(rows)].numpy())
+    assert np.array_equal(np.load(tmp_path / "a" / "picks.npy"), np.arange(5000, 0, -1, dtype=np.float64))
+    assert np.array_equal(np.load(tmp_path / "a" / "thc.npy"), res.thc.numpy())
+    assert np.load(tmp_path / "a" / "combine_weight.npy").tolist() == [0.25]

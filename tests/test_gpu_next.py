@@ -1,7 +1,6 @@
 """GPU parity of the SURVEY.md §8f rows — HP / TPC / Entropy uncertainties, Influence / Diversity
 scores and the top-k / Diversity selections — against the reference outputs in tests/golden/next.npz
 (written by oracle/pin_against_reference.py) and against the oracle on larger seeded pools."""
-import os
 import warnings
 from types import SimpleNamespace
 
@@ -225,7 +224,8 @@ def test_peak_uncertainties_match_oracle(built_lib, kind):
     through the REFERENCE's own methods with the restated peak_local_max (golden), plus edge maps: plateaus,
     constant maps (trivial image -> no peak), peaks on the excluded border, ties."""
     v = built_lib
-    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "peaks.npz"))
+    from conftest import load_golden
+    z = load_golden("peaks.npz")
     H = z["H"]
     got_mpe, got_mar = v.ops.peak_uncertainty(torch.from_numpy(H).cuda())
     got = (got_mpe if kind == "MPE" else got_mar).cpu().numpy()

@@ -78,12 +78,18 @@ def test_fusion_matches_reference(gold_fuse):
     assert O.fuse_scores(np.array([3.0])).tolist() == [0.0]
 
 
+# sklearn's distances are BLAS matrix products, whose last bits depend on the CPU's BLAS kernel and thread count:
+# the golden holds the bits of the machine that pinned it, so on another CPU the oracle's distances are compared
+# within the rounding of ||x||^2 + ||y||^2 - 2 x.y (d(c,c) ~ 1e-7 from cancellation) and the selections exactly.
+BLAS_RTOL, BLAS_ATOL = 1e-9, 1e-6
+
+
 def test_coreset_matches_reference(gold_coreset):
     for tag, c in gold_coreset.items():
         picks, md = O.coreset_select(c["X"].astype(np.float64), c["unc"].copy(), c["labeled"].tolist(), int(c["k"]),
                                      float(c["moks"]), float(c["lam"]), str(c["rule"]))
         assert picks == c["picks"].tolist(), tag
-        assert np.array_equal(md, c["min_d"]), tag
+        assert np.allclose(md, c["min_d"], rtol=BLAS_RTOL, atol=BLAS_ATOL), tag
 
 
 # ---- SURVEY.md §8f rows: HP / TPC / Entropy, Influence / Diversity / top-k ----------------
@@ -109,11 +115,11 @@ def test_influence_diversity_topk_match_reference(gold_next):
         lab = set(g[f"{tag}_labeled"].tolist())
         unl = [i for i in range(X.shape[0]) if i not in lab]
         k, cw = int(g[f"{tag}_k"]), float(g[f"{tag}_cw"])
-        assert np.array_equal(O.cosine_rowsum(X[unl]), g[f"{tag}_rowsum"])
+        assert np.allclose(O.cosine_rowsum(X[unl]), g[f"{tag}_rowsum"], rtol=1e-13, atol=0)       # (BLAS, see above)
         infl = O.influence_scores(X, unl)
-        assert np.array_equal(infl, g[f"{tag}_influence"])
+        assert np.allclose(infl, g[f"{tag}_influence"], rtol=0, atol=1e-13)
+        assert np.array_equal(O.total_score(g[f"{tag}_unc"], g[f"{tag}_influence"], cw), g[f"{tag}_total"])
         total = O.total_score(g[f"{tag}_unc"], infl, cw)
-        assert np.array_equal(total, g[f"{tag}_total"])
         assert O.topk_select(unl, total, k) == g[f"{tag}_topk"].tolist()
         assert O.diversity_select(X, unl, total, k) == g[f"{tag}_diversity"].tolist()
     assert O.influence_scores(np.zeros((3, 8)), [1]).tolist() == [0.0]
