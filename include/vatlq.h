@@ -37,6 +37,16 @@ extern "C" {
 
 typedef void* vatlq_stream_t; /* cudaStream_t */
 
+/* Heat-map element types of the *_dt entry points.  Every fp16 and bf16 value is exactly representable in fp32
+ * and the kernels convert at the load, so for H in fp16 or bf16 every output of a *_dt call equals, bit for bit,
+ * what the fp32 entry point returns for the exact upcast of H (NaN positions included).  Halos and prev / next
+ * tensors must share H's dtype.  16-bit heat maps must be 8-byte aligned wherever the fp32 form needs 16 bytes
+ * (the scan's H stays 16-byte aligned: its maps are fetched by TMA bulk copies).  An unknown dtype or a
+ * misaligned pointer returns VATLQ_EINVAL before any device work. */
+#define VATLQ_F32 0
+#define VATLQ_F16 1
+#define VATLQ_BF16 2
+
 int vatlq_abi_version(void);
 const char* vatlq_last_error(void);
 /* number of kernel launches issued by this library since load (bench.py's gpu_launches) */
@@ -51,7 +61,8 @@ uint64_t vatlq_launch_count(void);
  *   heatmap_to_coord_simple/get_max_pred  alphapose/utils/transforms.py:550-583,710-727
  *   transform_preds/get_affine_transform  alphapose/utils/transforms.py:704-708,753-792
  *
- * H          (n,J,h,w) fp32 contiguous heat maps; every frame is read from HBM once.
+ * H          (n,J,h,w) fp32 contiguous heat maps (vatlq_heatmap_scan_dt: fp16 / bf16 too); every frame is
+ *            read from HBM once.
  * is_prev/is_next  u8[n] track-adjacency flags (alphapose/datasets/posetrack21.py:148-178);
  *            the t-1 / t+1 maps are H[t-1] / H[t+1] (SURVEY.md §7.3-7).
  * halo_prev/halo_next  optional (J,h,w) frames that precede H[0] / follow H[n-1] when the
@@ -72,12 +83,26 @@ int vatlq_heatmap_scan(const float* H, const uint8_t* is_prev, const uint8_t* is
                        float* thc, float* peak_sum, int32_t* peak_cnt, float* peak_mean,
                        float* coords_hm, float* kpts,
                        void* ws, size_t ws_bytes, vatlq_stream_t stream);
+/* The same scan of H in any VATLQ_* dtype (vatlq_heatmap_scan is this call with VATLQ_F32).  In 16 bits the scan
+ * reads 104 448 B per 17 x 64 x 48 frame (half of fp32) and writes 212 B (thc, peak_sum / cnt / mean, coords_hm,
+ * kpts); halo_prev / halo_next are (J,h,w) frames of H's dtype.  Workspace as vatlq_heatmap_scan_workspace_bytes. */
+int vatlq_heatmap_scan_dt(const void* H, int dtype, const uint8_t* is_prev, const uint8_t* is_next,
+                          int64_t n, int J, int h, int w,
+                          const void* halo_prev, const void* halo_next,
+                          const float* bbox_xyxy,
+                          float* thc, float* peak_sum, int32_t* peak_cnt, float* peak_mean,
+                          float* coords_hm, float* kpts,
+                          void* ws, size_t ws_bytes, vatlq_stream_t stream);
 
 /* Strict three-tensor THC (cur, prev, next separately forwarded as the reference does,
  * ActiveLearning.py:293-297,345-363).  prev/next may be NULL when no flag needs them. */
 int vatlq_thc3(const float* cur, const float* prev, const float* next,
                const uint8_t* is_prev, const uint8_t* is_next,
                int64_t n, int J, int h, int w, float* thc, vatlq_stream_t stream);
+/* vatlq_thc3 with cur / prev / next in one VATLQ_* dtype */
+int vatlq_thc3_dt(const void* cur, const void* prev, const void* next, int dtype,
+                  const uint8_t* is_prev, const uint8_t* is_next,
+                  int64_t n, int J, int h, int w, float* thc, vatlq_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
  * WPU: hybrid feature + whole-body auto-encoder + reconstruction MSE.  Replaces
@@ -208,6 +233,9 @@ int vatlq_pose_unc(const float* coords_hm, const float* kpts, const float* bbox_
                    vatlq_stream_t stream);
 int vatlq_heatmap_entropy(const float* H, int64_t n, int J, int h, int w, float* entropy,
                           void* ws, size_t ws_bytes, vatlq_stream_t stream);
+/* vatlq_heatmap_entropy of H in any VATLQ_* dtype */
+int vatlq_heatmap_entropy_dt(const void* H, int dtype, int64_t n, int J, int h, int w, float* entropy,
+                             void* ws, size_t ws_bytes, vatlq_stream_t stream);
 
 /* Influence (ActiveLearning.py:467-477) and Diversity (:581-590): row sums of the cosine-distance
  * matrix that KNeighborsTransformer(mode='distance', metric='cosine', n_neighbors=m-1) builds
@@ -241,6 +269,9 @@ int vatlq_fuse_blend(const double* unc, const double* infl, const uint8_t* mask,
 size_t vatlq_peak_workspace_bytes(int64_t n, int J, int h, int w);
 int vatlq_peak_unc(const float* H, int64_t n, int J, int h, int w, float* mpe, float* margin,
                    void* ws, size_t ws_bytes, vatlq_stream_t stream);
+/* vatlq_peak_unc of H in any VATLQ_* dtype (same workspace) */
+int vatlq_peak_unc_dt(const void* H, int dtype, int64_t n, int J, int h, int w, float* mpe, float* margin,
+                      void* ws, size_t ws_bytes, vatlq_stream_t stream);
 
 /* Candidate ordering on the device (ActiveLearning.py:527-538, 587-589): out_idx[n] = row ids with mask != 0
  * (mask NULL: all) by descending (descending != 0) or ascending score, equal scores in ascending id order —

@@ -18,7 +18,10 @@ SIGNATURES = {
     "vatlq_heatmap_scan_workspace_bytes": (_sz, [_i64, _int]),
     "vatlq_heatmap_scan": (_int, [_vp, _vp, _vp, _i64, _int, _int, _int, _vp, _vp, _vp,
                                   _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "vatlq_heatmap_scan_dt": (_int, [_vp, _int, _vp, _vp, _i64, _int, _int, _int, _vp, _vp, _vp,
+                                     _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "vatlq_thc3": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _vp, _vp]),
+    "vatlq_thc3_dt": (_int, [_vp, _vp, _vp, _int, _vp, _vp, _i64, _int, _int, _int, _vp, _vp]),
     "vatlq_wpu_weight_count": (_sz, [_int, _int]),
     "vatlq_wpu": (_int, [_vp, _vp, _vp, _int, _int, _int, _vp, _vp, _vp, _i64, _vp]),
     "vatlq_fuse_stats": (_int, [_vp, _vp, _vp, _i64, _vp, _vp]),
@@ -35,6 +38,7 @@ SIGNATURES = {
     "vatlq_pairwise_dist": (_int, [_vp, _i64, _int, _vp, _i64, _vp, _vp, _sz, _vp]),
     "vatlq_pose_unc": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _vp, _vp, _vp, _vp, _vp]),
     "vatlq_heatmap_entropy": (_int, [_vp, _i64, _int, _int, _int, _vp, _vp, _sz, _vp]),
+    "vatlq_heatmap_entropy_dt": (_int, [_vp, _int, _i64, _int, _int, _int, _vp, _vp, _sz, _vp]),
     "vatlq_cosine_workspace_bytes": (_sz, [_int]),
     "vatlq_cosine_colsum": (_int, [_vp, _i64, _int, _vp, _i64, _vp, _vp, _sz, _vp]),
     "vatlq_cosine_rowsum": (_int, [_vp, _i64, _int, _vp, _i64, _vp, _dbl, _vp, _vp]),
@@ -42,6 +46,7 @@ SIGNATURES = {
     "vatlq_fuse_blend": (_int, [_vp, _vp, _vp, _i64, _dbl, _vp, _vp]),
     "vatlq_peak_workspace_bytes": (_sz, [_i64, _int, _int, _int]),
     "vatlq_peak_unc": (_int, [_vp, _i64, _int, _int, _int, _vp, _vp, _vp, _sz, _vp]),
+    "vatlq_peak_unc_dt": (_int, [_vp, _int, _i64, _int, _int, _int, _vp, _vp, _vp, _sz, _vp]),
     "vatlq_rank_workspace_bytes": (_sz, [_i64]),
     "vatlq_rank_scores": (_int, [_vp, _vp, _i64, _int, _vp, _vp, _sz, _vp]),
     "vatlq_kmeans_workspace_bytes": (_sz, [_i64, _int, _i64]),
@@ -67,6 +72,7 @@ SIGNATURES = {
 
 _lib = None
 EINVAL, ECOMM, ESTATE = -1, -3, -4     # VATLQ_E* of include/vatlq.h
+F32, F16, BF16 = 0, 1, 2               # VATLQ_F32 / VATLQ_F16 / VATLQ_BF16: heat-map element types of the *_dt entries
 
 
 class VatlqError(RuntimeError):

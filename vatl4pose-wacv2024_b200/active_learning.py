@@ -45,6 +45,12 @@ def _as_cuda(a, dtype=torch.float32):
     return t.to(device=_dev(), dtype=dtype).contiguous()
 
 
+def _heatmaps(out: torch.Tensor) -> torch.Tensor:
+    """The estimator's heat maps as the kernels read them: fp16 / bf16 (autocast or a .half() model) as they are —
+    the scores equal those of their exact fp32 upcast — every other dtype as `.float()` like the reference."""
+    return (out if out.dtype in (torch.float16, torch.bfloat16) else out.float()).contiguous()
+
+
 # ----------------------------------------------------------------------------------------
 # single-item shims with the reference's signatures (tests read like the reference's code)
 # ----------------------------------------------------------------------------------------
@@ -364,7 +370,7 @@ class ActiveLearning:
                 raise _lib.VatlqError("eval_loader must walk the id-sorted pool in order (shuffle=False)")
             cur = inps[:, 0].to(dev)
             out, emb = forward_with_embedding(m, cur, want_feat, fuse=bool(getattr(self.opt, "fuse_embedding", True)))
-            H = out[:, self.eval_joints].float().contiguous()             # (:277-281)
+            H = _heatmaps(out[:, self.eval_joints])                       # (:277-281)
             if want_feat:
                 X[pos:pos + b] = emb.float()                              # (:283-286)
             boxes = torch.as_tensor(np.asarray(bboxes_crop), dtype=torch.float32).reshape(b, 4).to(dev)
@@ -381,8 +387,8 @@ class ActiveLearning:
             else:
                 have_gt = False
             if strict:   # the reference's own three forwards (:293-297)
-                Hp = m(inps[:, 1].to(dev))[:, self.eval_joints].float().contiguous()
-                Hn = m(inps[:, 2].to(dev))[:, self.eval_joints].float().contiguous()
+                Hp = _heatmaps(m(inps[:, 1].to(dev))[:, self.eval_joints])
+                Hn = _heatmaps(m(inps[:, 2].to(dev))[:, self.eval_joints])
                 thc_strict[pos:pos + b] = ops.thc3(H, Hp, Hn, ip, inx)
             if self.eval_hook is not None:
                 self.eval_hook(self, batch, qp.kpts[pos:pos + b])

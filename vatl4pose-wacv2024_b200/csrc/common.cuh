@@ -1,9 +1,12 @@
 // Shared helpers for libvatlq (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <atomic>
+#include <type_traits>
 
 #include "../../include/vatlq.h"
 
@@ -59,6 +62,68 @@ __device__ __forceinline__ float4 ldg_stream(const float4* p) {
                : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w)
                : "l"(p));
   return r;
+}
+
+// ---------------------------------------------------------------- heat-map element types (VATLQ_F32 / F16 / BF16)
+// Every fp16 and bf16 value is exactly representable in fp32, so a 16-bit heat map is read through an exact
+// conversion at the load and everything after it is the fp32 arithmetic.  A "quad" is four consecutive pixels:
+// one float4 (16 B) in fp32, one uint2 (8 B) in 16 bits; a lane that owns quad q owns the same four pixels in
+// either form, so every accumulation chain sees the same values in the same order as on the fp32 upcast.
+__device__ __forceinline__ float to_f32(float x) { return x; }
+__device__ __forceinline__ float to_f32(__half x) { return __half2float(x); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 x) { return __bfloat162float(x); }
+
+template <typename T> struct QuadOf { using type = uint2; };
+template <> struct QuadOf<float> { using type = float4; };
+
+__device__ __forceinline__ float4 quad_f32(float4 v, const float*) { return v; }
+__device__ __forceinline__ float4 quad_f32(uint2 v, const __half*) {
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&v.x));
+  const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&v.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ float4 quad_f32(uint2 v, const __nv_bfloat16*) {   // bf16 = the top half of an fp32
+  return make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16),
+                     __uint_as_float(v.y & 0xffff0000u));
+}
+// quad q of p (shared or global memory, plain load)
+template <typename T>
+__device__ __forceinline__ float4 load_quad(const T* p, size_t q) {
+  return quad_f32(reinterpret_cast<const typename QuadOf<T>::type*>(p)[q], p);
+}
+// quad q of p through the read-only path (__ldg)
+template <typename T>
+__device__ __forceinline__ float4 ldg_quad(const T* p, size_t q) {
+  return quad_f32(__ldg(reinterpret_cast<const typename QuadOf<T>::type*>(p) + q), p);
+}
+__device__ __forceinline__ float ldg_f32(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ldg_f32(const __half* p) { return __half2float(__ldg(p)); }
+__device__ __forceinline__ float ldg_f32(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+
+__device__ __forceinline__ uint2 ldg_stream(const uint2* p) {
+  uint2 r;
+  asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
+  return r;
+}
+// quad q of p, streamed (read once: no L1 allocation)
+template <typename T>
+__device__ __forceinline__ float4 ldg_stream_quad(const T* p, size_t q) {
+  return quad_f32(ldg_stream(reinterpret_cast<const typename QuadOf<T>::type*>(p) + q), p);
+}
+
+// host side: element size of a VATLQ_* dtype code (0: unknown code)
+inline size_t dtype_size(int dtype) {
+  return dtype == VATLQ_F32 ? 4 : (dtype == VATLQ_F16 || dtype == VATLQ_BF16) ? 2 : 0;
+}
+// host side: p suits the quad loads of a dtype (16 B in fp32, 8 B in 16 bits)
+inline bool quad_aligned(const void* p, int dtype) { return ((uintptr_t)p & (4 * dtype_size(dtype) - 1)) == 0; }
+
+// call f(T*) with H cast to the element type of dtype (dtype already validated)
+template <typename F>
+inline int with_dtype(int dtype, F&& f) {
+  if (dtype == VATLQ_F16) return f((const __half*)nullptr);
+  if (dtype == VATLQ_BF16) return f((const __nv_bfloat16*)nullptr);
+  return f((const float*)nullptr);
 }
 
 __device__ __forceinline__ float warp_max(float v) {

@@ -111,27 +111,27 @@ __device__ __forceinline__ void peak_scores(const float (&peaks)[5], int npk, fl
   *margin_out = margin;
 }
 
-// CH / CW > 0: compile-time map shape (64 x 48: index arithmetic without runtime divisions), else the arguments
-template <int CH, int CW>
-__device__ __forceinline__ void peak_map_generic(const float* __restrict__ H, long long mi, int h_, int w_, float* __restrict__ mpe_map,
+// CH / CW > 0: compile-time map shape (64 x 48: index arithmetic without runtime divisions), else the arguments.
+// T: fp32, or a 16-bit type converted exactly while the map is staged into the fp32 image.
+template <int CH, int CW, typename T>
+__device__ __forceinline__ void peak_map_generic(const T* __restrict__ H, long long mi, int h_, int w_, float* __restrict__ mpe_map,
                                                  float* __restrict__ margin_map, float* img, int lane) {
   const int h = CH > 0 ? CH : h_, w = CW > 0 ? CW : w_;
   const int npx = h * w;
   float* aux = img + npx;                         // row maxima, then the peak mask (as 0 / 1); img: the map
-  const float* src = H + (size_t)mi * npx;
+  const T* src = H + (size_t)mi * npx;
   float vmin = INFINITY;
-  if (CH > 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0) {
-    const float4* s4 = reinterpret_cast<const float4*>(src);
+  if (CH > 0 && (reinterpret_cast<uintptr_t>(src) & (4 * sizeof(T) - 1)) == 0) {
     float4* d4 = reinterpret_cast<float4*>(img);
 #pragma unroll 4
     for (int i = lane; i < npx / 4; i += 32) {
-      const float4 v = ldg_stream(s4 + i);
+      const float4 v = ldg_stream_quad(src, i);
       d4[i] = v;
       vmin = fminf(vmin, fminf(fminf(v.x, v.y), fminf(v.z, v.w)));
     }
   } else {
     for (int i = lane; i < npx; i += 32) {
-      const float v = __ldg(src + i);
+      const float v = ldg_f32(src + i);
       img[i] = v;
       vmin = fminf(vmin, v);
     }
@@ -199,27 +199,28 @@ __device__ __forceinline__ void peak_map_generic(const float* __restrict__ H, lo
   if (lane == 0) peak_scores(peaks, npk, mpe_map + mi, margin_map + mi);
 }
 
-template <int CH, int CW>
+template <int CH, int CW, typename T>
 __global__ void __launch_bounds__(kPeakWarps * 32)
-peak_unc_kernel(const float* __restrict__ H, long long maps, int h_, int w_, float* __restrict__ mpe_map,
+peak_unc_kernel(const T* __restrict__ H, long long maps, int h_, int w_, float* __restrict__ mpe_map,
                 float* __restrict__ margin_map) {
   extern __shared__ __align__(16) float s_peak[];
   const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
   const long long mi = (long long)blockIdx.x * kPeakWarps + wp;
   if (mi >= maps) return;
   const int npx = (CH > 0 ? CH : h_) * (CW > 0 ? CW : w_);
-  peak_map_generic<CH, CW>(H, mi, h_, w_, mpe_map, margin_map, s_peak + (size_t)wp * 2 * npx, lane);
+  peak_map_generic<CH, CW, T>(H, mi, h_, w_, mpe_map, margin_map, s_peak + (size_t)wp * 2 * npx, lane);
 }
 
 // the generic 64 x 48 routine on a list of maps (the fast path's overflow cases); grid-stride over the list
+template <typename T>
 __global__ void __launch_bounds__(kPeakWarps * 32)
-peak_unc_redo_kernel(const float* __restrict__ H, const unsigned int* __restrict__ redo_count, const int* __restrict__ redo_list,
+peak_unc_redo_kernel(const T* __restrict__ H, const unsigned int* __restrict__ redo_count, const int* __restrict__ redo_list,
                      float* __restrict__ mpe_map, float* __restrict__ margin_map) {
   extern __shared__ __align__(16) float s_peak[];
   const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
   const unsigned total = *redo_count;
   for (unsigned slot = blockIdx.x * kPeakWarps + wp; slot < total; slot += gridDim.x * kPeakWarps) {
-    peak_map_generic<64, 48>(H, redo_list[slot], 64, 48, mpe_map, margin_map, s_peak + (size_t)wp * 2 * 64 * 48, lane);
+    peak_map_generic<64, 48, T>(H, redo_list[slot], 64, 48, mpe_map, margin_map, s_peak + (size_t)wp * 2 * 64 * 48, lane);
     __syncwarp();
   }
 }
@@ -399,9 +400,11 @@ peak_unc_fast_kernel(const float* __restrict__ H, long long maps, float* __restr
 // lanes are clamped to 0 .. 31: a clamped lane only repeats rows that are inside the window already, which is exactly
 // what edge replication does to a maximum.  The originals are read a second time (L1 / L2) for the mask test.
 // Shared memory: the candidate list only -> occupancy is set by registers (12 warps per SM instead of 7).
+// T: fp32, or a 16-bit type read as 8-byte quads (same rows per lane) and converted exactly in registers.
 constexpr int kPrWarps = 4;
+template <typename T>
 __global__ void __launch_bounds__(kPrWarps * 32, 3)
-peak_unc_reg_kernel(const float* __restrict__ H, long long maps, float* __restrict__ mpe_map, float* __restrict__ margin_map,
+peak_unc_reg_kernel(const T* __restrict__ H, long long maps, float* __restrict__ mpe_map, float* __restrict__ margin_map,
                     unsigned int* __restrict__ redo_count, int* __restrict__ redo_list) {
   __shared__ float s_cval[kPrWarps][kPfCand];
   __shared__ int s_cidx[kPrWarps][kPfCand];
@@ -413,7 +416,7 @@ peak_unc_reg_kernel(const float* __restrict__ H, long long maps, float* __restri
   int* cidx = s_cidx[wp];
   int* ccount = &s_cnt[wp];
   if (lane == 0) *ccount = 0;
-  const float4* src = reinterpret_cast<const float4*>(H + (size_t)mi * (kPfH * kPfW) + (size_t)lane * (2 * kPfW));
+  const T* src = H + (size_t)mi * (kPfH * kPfW) + (size_t)lane * (2 * kPfW);
   float a[kPfW], b[kPfW];           // row maxima of rows 2l / 2l+1, then their window maxima
   float vmin = INFINITY;
 #pragma unroll
@@ -421,7 +424,7 @@ peak_unc_reg_kernel(const float* __restrict__ H, long long maps, float* __restri
     float p[kPfW + 2 * kPfPad];
 #pragma unroll
     for (int q = 0; q < kPfW / 4; ++q) {
-      const float4 v = __ldg(src + rr * (kPfW / 4) + q);
+      const float4 v = ldg_quad(src, rr * (kPfW / 4) + q);
       p[kPfPad + 4 * q] = v.x; p[kPfPad + 4 * q + 1] = v.y; p[kPfPad + 4 * q + 2] = v.z; p[kPfPad + 4 * q + 3] = v.w;
       vmin = fminf(vmin, fminf(fminf(v.x, v.y), fminf(v.z, v.w)));
     }
@@ -459,7 +462,7 @@ peak_unc_reg_kernel(const float* __restrict__ H, long long maps, float* __restri
     const bool yin = y >= kPfPad && y < kPfH - kPfPad;
 #pragma unroll
     for (int q = 0; q < kPfW / 4; ++q) {
-      const float4 v4 = __ldg(src + rr * (kPfW / 4) + q);
+      const float4 v4 = ldg_quad(src, rr * (kPfW / 4) + q);
       const float vv[4] = {v4.x, v4.y, v4.z, v4.w};
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
@@ -616,53 +619,74 @@ extern "C" size_t vatlq_peak_workspace_bytes(int64_t n, int J, int h, int w) {
   return maps * 8 + ((h == kPfH && w == kPfW) ? 16 + maps * 4 : 0);
 }
 
-extern "C" int vatlq_peak_unc(const float* H, int64_t n, int J, int h, int w, float* mpe, float* margin, void* ws,
-                              size_t ws_bytes, vatlq_stream_t stream_) {
+template <typename T>
+static int launch_peak_unc(const T* H, int64_t n, int J, int h, int w, float* mpe, float* margin, void* ws, size_t smem,
+                           cudaStream_t stream) {
+  const long long maps = (long long)n * J;
+  static size_t configured = 0;
+  if (smem > configured) {
+    VQ_CUDA(cudaFuncSetAttribute((peak_unc_kernel<0, 0, T>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    VQ_CUDA(cudaFuncSetAttribute((peak_unc_kernel<64, 48, T>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    VQ_CUDA(cudaFuncSetAttribute(peak_unc_redo_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)((size_t)kPeakWarps * 2 * kPfH * kPfW * sizeof(float))));
+    if (std::is_same<T, float>::value)
+      VQ_CUDA(cudaFuncSetAttribute(peak_unc_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kPfWarps * kPfSmemWarp)));
+    configured = smem;
+  }
+  float* mm = (float*)ws;
+  const bool no_fast = getenv("VATLQ_PEAK_GENERIC") != nullptr;     // measurement / test switch (read per call)
+  if (h == kPfH && w == kPfW && !no_fast && (reinterpret_cast<uintptr_t>(H) & (4 * sizeof(T) - 1)) == 0) {
+    unsigned int* redo_count = (unsigned int*)((char*)ws + (size_t)maps * 8);
+    int* redo_list = (int*)((char*)ws + (size_t)maps * 8 + 16);
+    VQ_CUDA(cudaMemsetAsync(redo_count, 0, 16, stream));
+    // the shared-memory-staged variant (measurement switch) is fp32 only: 16-bit maps take the register kernel
+    // whatever VATLQ_PEAK_SMEM says
+    if (std::is_same<T, float>::value && getenv("VATLQ_PEAK_SMEM") != nullptr)
+      peak_unc_fast_kernel<<<(unsigned)((maps + kPfWarps - 1) / kPfWarps), kPfWarps * 32, kPfWarps * kPfSmemWarp, stream>>>(
+          (const float*)H, maps, mm, mm + maps, redo_count, redo_list);
+    else
+      peak_unc_reg_kernel<T><<<(unsigned)((maps + kPrWarps - 1) / kPrWarps), kPrWarps * 32, 0, stream>>>(H, maps, mm, mm + maps,
+                                                                                                  redo_count, redo_list);
+    VQ_LAUNCHED();
+    const unsigned rgrid = (unsigned)std::min<long long>((maps + kPeakWarps - 1) / kPeakWarps, (long long)sm_count() * 4);
+    peak_unc_redo_kernel<T><<<rgrid, kPeakWarps * 32, (size_t)kPeakWarps * 2 * kPfH * kPfW * sizeof(float), stream>>>(
+        H, redo_count, redo_list, mm, mm + maps);
+    VQ_LAUNCHED();
+  } else {
+    const unsigned pgrid = (unsigned)((maps + kPeakWarps - 1) / kPeakWarps);
+    if (h == 64 && w == 48) peak_unc_kernel<64, 48, T><<<pgrid, kPeakWarps * 32, smem, stream>>>(H, maps, h, w, mm, mm + maps);
+    else peak_unc_kernel<0, 0, T><<<pgrid, kPeakWarps * 32, smem, stream>>>(H, maps, h, w, mm, mm + maps);
+    VQ_LAUNCHED();
+  }
+  peak_frames_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(mm, mm + maps, (long long)n, J, mpe, margin);
+  VQ_LAUNCHED();
+  return 0;
+}
+
+extern "C" int vatlq_peak_unc_dt(const void* H, int dtype, int64_t n, int J, int h, int w, float* mpe, float* margin, void* ws,
+                                 size_t ws_bytes, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   VQ_REQUIRE(n >= 0 && J > 0 && h > 2 * kPeakMinDist && w > 2 * kPeakMinDist, "bad shape");
+  VQ_REQUIRE(dtype_size(dtype) != 0, "unknown dtype (VATLQ_F32, VATLQ_F16 or VATLQ_BF16)");
   if (n == 0) return 0;
   VQ_REQUIRE(H && ws && (mpe || margin), "null pointer");
   VQ_REQUIRE(h * w <= 128 * 32 * 4, "map too large (<= 16384 pixels)");
   const long long maps = (long long)n * J;
   VQ_REQUIRE(maps < (1LL << 31), "too many maps per call (n*J < 2^31)");
   VQ_REQUIRE(ws_bytes >= vatlq_peak_workspace_bytes(n, J, h, w), "workspace too small (vatlq_peak_workspace_bytes)");
+  // (fp32 keeps its generic fallback for a misaligned H; the 16-bit forms are new and ask for the alignment instead)
+  VQ_REQUIRE(dtype == VATLQ_F32 || h != kPfH || w != kPfW || quad_aligned(H, dtype), "16-bit H must be 8-byte aligned");
   const size_t smem = (size_t)kPeakWarps * 2 * h * w * sizeof(float);
   VQ_REQUIRE(smem <= 200 * 1024, "map too large for the shared-memory staging");
-  static size_t configured = 0;
-  if (smem > configured) {
-    VQ_CUDA(cudaFuncSetAttribute((peak_unc_kernel<0, 0>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    VQ_CUDA(cudaFuncSetAttribute((peak_unc_kernel<64, 48>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    VQ_CUDA(cudaFuncSetAttribute(peak_unc_redo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)((size_t)kPeakWarps * 2 * kPfH * kPfW * sizeof(float))));
-    VQ_CUDA(cudaFuncSetAttribute(peak_unc_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kPfWarps * kPfSmemWarp)));
-    configured = smem;
-  }
-  float* mm = (float*)ws;
-  const bool no_fast = getenv("VATLQ_PEAK_GENERIC") != nullptr;     // measurement / test switch (read per call)
-  if (h == kPfH && w == kPfW && !no_fast && (reinterpret_cast<uintptr_t>(H) & 15) == 0) {
-    unsigned int* redo_count = (unsigned int*)((char*)ws + (size_t)maps * 8);
-    int* redo_list = (int*)((char*)ws + (size_t)maps * 8 + 16);
-    VQ_CUDA(cudaMemsetAsync(redo_count, 0, 16, stream));
-    if (getenv("VATLQ_PEAK_SMEM") != nullptr)      // the shared-memory-staged variant (measurement switch)
-      peak_unc_fast_kernel<<<(unsigned)((maps + kPfWarps - 1) / kPfWarps), kPfWarps * 32, kPfWarps * kPfSmemWarp, stream>>>(
-          H, maps, mm, mm + maps, redo_count, redo_list);
-    else
-      peak_unc_reg_kernel<<<(unsigned)((maps + kPrWarps - 1) / kPrWarps), kPrWarps * 32, 0, stream>>>(H, maps, mm, mm + maps, redo_count,
-                                                                                               redo_list);
-    VQ_LAUNCHED();
-    const unsigned rgrid = (unsigned)std::min<long long>((maps + kPeakWarps - 1) / kPeakWarps, (long long)sm_count() * 4);
-    peak_unc_redo_kernel<<<rgrid, kPeakWarps * 32, (size_t)kPeakWarps * 2 * kPfH * kPfW * sizeof(float), stream>>>(
-        H, redo_count, redo_list, mm, mm + maps);
-    VQ_LAUNCHED();
-  } else {
-    const unsigned pgrid = (unsigned)((maps + kPeakWarps - 1) / kPeakWarps);
-    if (h == 64 && w == 48) peak_unc_kernel<64, 48><<<pgrid, kPeakWarps * 32, smem, stream>>>(H, maps, h, w, mm, mm + maps);
-    else peak_unc_kernel<0, 0><<<pgrid, kPeakWarps * 32, smem, stream>>>(H, maps, h, w, mm, mm + maps);
-    VQ_LAUNCHED();
-  }
-  peak_frames_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(mm, mm + maps, (long long)n, J, mpe, margin);
-  VQ_LAUNCHED();
-  return 0;
+  return with_dtype(dtype, [&](auto tag) {
+    using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+    return launch_peak_unc<T>((const T*)H, n, J, h, w, mpe, margin, ws, smem, stream);
+  });
+}
+
+extern "C" int vatlq_peak_unc(const float* H, int64_t n, int J, int h, int w, float* mpe, float* margin, void* ws,
+                              size_t ws_bytes, vatlq_stream_t stream) {
+  return vatlq_peak_unc_dt(H, VATLQ_F32, n, J, h, w, mpe, margin, ws, ws_bytes, stream);
 }
 
 extern "C" int vatlq_oks(const float* kpts, const float* gt_kpts, const float* bbox_ann_xyxy, int64_t n, double* oks,

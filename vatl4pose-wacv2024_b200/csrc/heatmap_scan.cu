@@ -1,5 +1,6 @@
 // Heat-map scan: THC + local-peak statistics + argmax / quarter-pixel coordinates in ONE
-// streaming pass over the (n,J,h,w) fp32 pool.  See include/vatlq.h for the reference
+// streaming pass over the (n,J,h,w) pool, fp32, fp16 or bf16 (16-bit maps are converted exactly at the load:
+// every output equals the fp32 scan of the upcast, bit for bit).  See include/vatlq.h for the reference
 // functions this replaces and DESIGN.md §scan for the data flow.
 //
 // Work decomposition (fast path): one warp walks a run of consecutive frames of one joint.
@@ -38,8 +39,8 @@ __device__ __forceinline__ bool pair_wanted(int64_t t, int64_t n, const uint8_t*
 }
 
 // 3x3 zero-padded maximum test of pixel (y,x) against the map in shared memory
-template <int HM_H, int HM_W>
-__device__ __forceinline__ bool is_local_max(const float* __restrict__ s_map, int y, int x, float val,
+template <int HM_H, int HM_W, typename T>
+__device__ __forceinline__ bool is_local_max(const T* __restrict__ s_map, int y, int x, float val,
                                              int h_rt, int w_rt) {
   const int hh = HM_H > 0 ? HM_H : h_rt, ww = HM_W > 0 ? HM_W : w_rt;
   bool ok = true;
@@ -49,7 +50,7 @@ __device__ __forceinline__ bool is_local_max(const float* __restrict__ s_map, in
     for (int dx = -1; dx <= 1; ++dx) {
       if (dy == 0 && dx == 0) continue;
       const int yy = y + dy, xx = x + dx;
-      const float nb = (yy >= 0 && yy < hh && xx >= 0 && xx < ww) ? s_map[yy * ww + xx] : 0.0f;
+      const float nb = (yy >= 0 && yy < hh && xx >= 0 && xx < ww) ? to_f32(s_map[yy * ww + xx]) : 0.0f;
       ok = ok && (val >= nb);
     }
   }
@@ -57,7 +58,8 @@ __device__ __forceinline__ bool is_local_max(const float* __restrict__ s_map, in
 }
 
 // quarter-pixel shift of transforms.py:560-566 (strictly interior pixels only; sign(0) = 0)
-__device__ __forceinline__ void quarter_shift(const float* __restrict__ s_map, int y, int x, int hh, int ww,
+template <typename T>
+__device__ __forceinline__ void quarter_shift(const T* __restrict__ s_map, int y, int x, int hh, int ww,
                                               float gmax, float& fx, float& fy) {
   if (!(gmax > 0.0f)) {  // get_max_pred zeroes the coordinates (transforms.py:723-726)
     fx = 0.0f;
@@ -67,8 +69,8 @@ __device__ __forceinline__ void quarter_shift(const float* __restrict__ s_map, i
   fx = (float)x;
   fy = (float)y;
   if (x > 1 && x < ww - 1 && y > 1 && y < hh - 1) {
-    const float dx = s_map[y * ww + x + 1] - s_map[y * ww + x - 1];
-    const float dy = s_map[(y + 1) * ww + x] - s_map[(y - 1) * ww + x];
+    const float dx = to_f32(s_map[y * ww + x + 1]) - to_f32(s_map[y * ww + x - 1]);
+    const float dy = to_f32(s_map[(y + 1) * ww + x]) - to_f32(s_map[(y - 1) * ww + x]);
     fx += (dx > 0.0f) ? 0.25f : ((dx < 0.0f) ? -0.25f : 0.0f);
     fy += (dy > 0.0f) ? 0.25f : ((dy < 0.0f) ? -0.25f : 0.0f);
   }
@@ -78,9 +80,9 @@ constexpr int FH = 64, FW = 48, FPIX = FH * FW, FQ = FPIX / 4;  // 3072 px, 768 
 
 // ------------------------------------------------------------------------------------
 // fast path, 64x48 maps (every config of the reference): one WARP owns a run of consecutive frames of one joint.
-// Lane 0 keeps kStages-1 maps in flight with cp.async.bulk (1-D TMA bulk copy, 12 288 B each,
+// Lane 0 keeps kStages-1 maps in flight with cp.async.bulk (1-D TMA bulk copy, 12 288 B each in fp32, 6 144 B in 16 bits,
 // completion counted on an mbarrier per stage); the warp pulls the landed map into registers
-// (24 float4 per lane), where it stays to serve as frame t-1 of the next step, so every byte
+// (24 float4 per lane, converted from 24 8-byte quads in 16 bits), where it stays to serve as frame t-1 of the next step, so every byte
 // of H crosses HBM once and shared memory is only a landing zone + the 3x3 neighbourhood
 // lookups of the few pixels above half of the map maximum.  No __syncthreads anywhere: all
 // reductions are warp shuffles, warps of a CTA only share the launch.
@@ -91,17 +93,29 @@ constexpr int FH = 64, FW = 48, FPIX = FH * FW, FQ = FPIX / 4;  // 3072 px, 768 
 #ifndef VQ_SCAN_STAGES
 #define VQ_SCAN_STAGES 2
 #endif
+// 16-bit maps (6 144 B per stage): 2, 3 and 4 stages measured within 0.5 % of each other on B200 (170 000 frames,
+// tools/time_heatmap_dtypes.py --stage-libs): the 16-bit scan is not bound by bytes in flight (DESIGN.md §4.1), so it
+// keeps the fp32 kernel's two stages and half its shared memory
+#ifndef VQ_SCAN_STAGES16
+#define VQ_SCAN_STAGES16 2
+#endif
 constexpr int kTmaWarps = VQ_SCAN_WARPS;
-constexpr int kStages = VQ_SCAN_STAGES;
-constexpr int kMapBytes = FPIX * 4;              // 12 288
-constexpr int kLaneQ = FQ / 32;                  // 24 float4 per lane
-constexpr size_t kTmaSmem = (size_t)kTmaWarps * kStages * kMapBytes + (size_t)kTmaWarps * kStages * 8;
+constexpr int kLaneQ = FQ / 32;                  // 24 quads per lane
+template <typename T> struct ScanStages { static constexpr int value = VQ_SCAN_STAGES16; };
+template <> struct ScanStages<float> { static constexpr int value = VQ_SCAN_STAGES; };
+template <typename T>
+constexpr size_t tma_smem() {
+  return (size_t)kTmaWarps * ScanStages<T>::value * (FPIX * sizeof(T)) + (size_t)kTmaWarps * ScanStages<T>::value * 8;
+}
 
+template <typename T>
 __global__ void __launch_bounds__(kTmaWarps * 32, 1)
-scan_tma_64x48(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
+scan_tma_64x48(const T* __restrict__ H, const uint8_t* __restrict__ is_prev,
                const uint8_t* __restrict__ is_next, int64_t n, int J,
-               const float* __restrict__ halo_prev, const float* __restrict__ halo_next,
+               const T* __restrict__ halo_prev, const T* __restrict__ halo_next,
                int run_len, int64_t n_runs, ScanOut out) {
+  constexpr int kStages = ScanStages<T>::value;
+  constexpr int kMapBytes = FPIX * sizeof(T);    // 12 288 (fp32) / 6 144 (16-bit)
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t task = (int64_t)blockIdx.x * kTmaWarps + warp;   // task = run * J + joint
@@ -109,7 +123,7 @@ scan_tma_64x48(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
   const int j = (int)(task % J);
   const int64_t a = (task / J) * run_len;
   const int64_t b = min(n, a + (int64_t)run_len);
-  float* stage0 = reinterpret_cast<float*>(smem_raw) + (size_t)warp * kStages * FPIX;
+  T* stage0 = reinterpret_cast<T*>(smem_raw) + (size_t)warp * kStages * FPIX;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + (size_t)kTmaWarps * kStages * kMapBytes) + warp * kStages;
   const bool has_hp = halo_prev != nullptr, has_hn = halo_next != nullptr;
 
@@ -119,7 +133,7 @@ scan_tma_64x48(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
   const bool tail_pair = (b == n) && pair_wanted(n, n, is_prev, is_next, has_hp, has_hn);
   const int64_t last = tail_pair ? n : b - 1;
   const int64_t count = last - first + 1;
-  auto src_of = [&](int64_t f) -> const float* {
+  auto src_of = [&](int64_t f) -> const T* {
     if (f < 0) return halo_prev + (size_t)j * FPIX;
     if (f >= n) return halo_next + (size_t)j * FPIX;
     return H + ((size_t)f * J + j) * FPIX;
@@ -141,9 +155,8 @@ scan_tma_64x48(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
   for (int64_t i = 0; i < count; ++i) {
     const int64_t f = first + i;
     const int s = (int)(i % kStages);
-    const float* cur = stage0 + (size_t)s * FPIX;
+    const T* cur = stage0 + (size_t)s * FPIX;
     mbar_wait(&bars[s], (uint32_t)((i / kStages) & 1));
-    const float4* cur4 = reinterpret_cast<const float4*>(cur);
     const bool want = (f >= a) && pair_wanted(f, n, is_prev, is_next, has_hp, has_hn);
 
     // ---- pass 1: pull the map into registers; map maximum and |H_f - H_{f-1}|
@@ -151,7 +164,7 @@ scan_tma_64x48(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
     float4 mx = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY), sm = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int r = 0; r < kLaneQ; ++r) {
-      const float4 c = cur4[r * 32 + lane];
+      const float4 c = load_quad(cur, r * 32 + lane);   // LDS.128 (fp32) / LDS.64 + exact conversion
       if (want) {
         sm.x += fabsf(c.x - pv[r].x);
         sm.y += fabsf(c.y - pv[r].y);
@@ -187,7 +200,7 @@ scan_tma_64x48(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
         hot &= hot - 1;
         const int q = r * 32 + lane;
         const int y = q / (FW / 4), x0 = (q % (FW / 4)) * 4;
-        const float4 c4 = cur4[q];
+        const float4 c4 = load_quad(cur, q);
         const float e[4] = {c4.x, c4.y, c4.z, c4.w};
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
@@ -229,11 +242,13 @@ scan_tma_64x48(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
 // ------------------------------------------------------------------------------------
 // generic path: any (h,w) with h*w*4 bytes of shared memory; one CTA per (frame, joint).
 // Reads the previous frame from global memory again (2x traffic) — used for odd shapes only.
+// 16-bit maps are converted while they are staged into the fp32 s_map.
 // ------------------------------------------------------------------------------------
+template <typename T>
 __global__ void __launch_bounds__(kScanThreads)
-scan_generic(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
+scan_generic(const T* __restrict__ H, const uint8_t* __restrict__ is_prev,
              const uint8_t* __restrict__ is_next, int64_t n, int J, int h, int w,
-             const float* __restrict__ halo_prev, const float* __restrict__ halo_next, ScanOut out) {
+             const T* __restrict__ halo_prev, const T* __restrict__ halo_next, ScanOut out) {
   extern __shared__ float s_dyn[];
   float* s_map = s_dyn;
   __shared__ float s_wmax[kWarps];
@@ -247,16 +262,16 @@ scan_generic(const float* __restrict__ H, const uint8_t* __restrict__ is_prev,
   const int npx = h * w;
   const bool has_hp = halo_prev != nullptr, has_hn = halo_next != nullptr;
   const bool want = pair_wanted(t, n, is_prev, is_next, has_hp, has_hn);
-  const float* cur = (t < n) ? H + ((size_t)t * J + j) * npx : (has_hn ? halo_next + (size_t)j * npx : nullptr);
-  const float* prv = (t > 0) ? H + ((size_t)(t - 1) * J + j) * npx : (has_hp ? halo_prev + (size_t)j * npx : nullptr);
+  const T* cur = (t < n) ? H + ((size_t)t * J + j) * npx : (has_hn ? halo_next + (size_t)j * npx : nullptr);
+  const T* prv = (t > 0) ? H + ((size_t)(t - 1) * J + j) * npx : (has_hp ? halo_prev + (size_t)j * npx : nullptr);
   if (tid == 0) s_arg = 0x7fffffff;
   float lmax = -INFINITY, s = 0.0f;
   if (cur) {
     for (int p = tid; p < npx; p += kScanThreads) {
-      const float val = cur[p];
+      const float val = to_f32(cur[p]);
       s_map[p] = val;
       lmax = fmaxf(lmax, val);
-      if (want) s += fabsf(val - prv[p]);
+      if (want) s += fabsf(val - to_f32(prv[p]));
     }
   }
   lmax = warp_max(lmax);
@@ -384,33 +399,31 @@ scan_finalize(int64_t n, int J, int h, int w, const uint8_t* __restrict__ is_pre
 }
 
 // strict three-tensor THC: one CTA per frame, every tensor read once
+template <typename T>
 __global__ void __launch_bounds__(256)
-thc3_kernel(const float* __restrict__ cur, const float* __restrict__ prev, const float* __restrict__ next,
+thc3_kernel(const T* __restrict__ cur, const T* __restrict__ prev, const T* __restrict__ next,
             const uint8_t* __restrict__ is_prev, const uint8_t* __restrict__ is_next, int64_t n, int J,
             int npx, float* __restrict__ thc) {
   __shared__ double s_p[8], s_n[8];
   const int64_t t = blockIdx.x;
   const bool hp = is_prev && is_prev[t] && prev, hn = is_next && is_next[t] && next;
   const size_t fl = (size_t)J * npx;
-  const float* c = cur + t * fl;
+  const T* c = cur + t * fl;
   float sp = 0.f, sn = 0.f;
   double dp = 0.0, dn = 0.0;
   if (hp || hn) {
-    const float* p = prev ? prev + t * fl : nullptr;
-    const float* q = next ? next + t * fl : nullptr;
+    const T* p = prev ? prev + t * fl : nullptr;
+    const T* q = next ? next + t * fl : nullptr;
     if ((fl & 3) == 0) {
-      const float4* c4 = reinterpret_cast<const float4*>(c);
-      const float4* p4 = reinterpret_cast<const float4*>(p);
-      const float4* q4 = reinterpret_cast<const float4*>(q);
       int cnt = 0;
       for (size_t i = threadIdx.x; i < fl / 4; i += blockDim.x) {
-        const float4 x = ldg_stream(c4 + i);
+        const float4 x = ldg_stream_quad(c, i);
         if (hp) {
-          const float4 y = ldg_stream(p4 + i);
+          const float4 y = ldg_stream_quad(p, i);
           sp += fabsf(x.x - y.x) + fabsf(x.y - y.y) + fabsf(x.z - y.z) + fabsf(x.w - y.w);
         }
         if (hn) {
-          const float4 y = ldg_stream(q4 + i);
+          const float4 y = ldg_stream_quad(q, i);
           sn += fabsf(x.x - y.x) + fabsf(x.y - y.y) + fabsf(x.z - y.z) + fabsf(x.w - y.w);
         }
         if (++cnt == 16) {  // bound the fp32 run length
@@ -419,8 +432,8 @@ thc3_kernel(const float* __restrict__ cur, const float* __restrict__ prev, const
       }
     } else {
       for (size_t i = threadIdx.x; i < fl; i += blockDim.x) {
-        if (hp) dp += fabsf(c[i] - p[i]);
-        if (hn) dn += fabsf(c[i] - q[i]);
+        if (hp) dp += fabsf(to_f32(c[i]) - to_f32(p[i]));
+        if (hn) dn += fabsf(to_f32(c[i]) - to_f32(q[i]));
       }
     }
     dp += sp;
@@ -458,17 +471,59 @@ extern "C" size_t vatlq_heatmap_scan_workspace_bytes(int64_t n, int J) {
          align_up(nj * 8, 256);
 }
 
-extern "C" int vatlq_heatmap_scan(const float* H, const uint8_t* is_prev, const uint8_t* is_next,
-                                  int64_t n, int J, int h, int w, const float* halo_prev,
-                                  const float* halo_next, const float* bbox_xyxy, float* thc,
-                                  float* peak_sum, int32_t* peak_cnt, float* peak_mean,
-                                  float* coords_hm, float* kpts, void* ws, size_t ws_bytes,
-                                  vatlq_stream_t stream_) {
+template <typename T>
+static int launch_scan(const T* H, const uint8_t* is_prev, const uint8_t* is_next, int64_t n, int J, int h, int w,
+                       const T* halo_prev, const T* halo_next, const ScanOut& so, cudaStream_t stream) {
+  const bool fast = (h == FH && w == FW) && (halo_prev == nullptr || ((uintptr_t)halo_prev & 15) == 0) &&
+                    (halo_next == nullptr || ((uintptr_t)halo_next & 15) == 0);
+  if (fast) {
+    // one warp per (run, joint) task, ~4 tasks per warp slot so that CTAs finishing early are
+    // replaced; runs no shorter than 8 frames keep the halo re-read <= 1/8 of the traffic.
+    // fp32: 8 warps x 2 stages per SM measured best (6.8 TB/s; 6x3 5.3, 4x4 3.7: tools/tune_scan.py);
+    // 16-bit: 8 warps x VQ_SCAN_STAGES16 stages
+    const int64_t slots = (int64_t)sm_count() * kTmaWarps;
+    int64_t runs = (slots * 4 + J - 1) / J;
+    int64_t run_len = (n + runs - 1) / runs;
+    if (run_len < 8) run_len = 8;
+    if (run_len > n) run_len = n;
+    runs = (n + run_len - 1) / run_len;
+    const int64_t tasks = runs * J;
+    static bool cfg = false;
+    if (!cfg) {
+      VQ_CUDA(cudaFuncSetAttribute(scan_tma_64x48<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tma_smem<T>()));
+      cfg = true;
+    }
+    VQ_REQUIRE((tasks + kTmaWarps - 1) / kTmaWarps <= 2147483647LL, "grid too large");
+    scan_tma_64x48<T><<<(unsigned)((tasks + kTmaWarps - 1) / kTmaWarps), kTmaWarps * 32, tma_smem<T>(), stream>>>(
+        H, is_prev, is_next, n, J, halo_prev, halo_next, (int)run_len, runs, so);
+    VQ_LAUNCHED();
+  } else {
+    const size_t smem = (size_t)h * w * sizeof(float);
+    VQ_REQUIRE(smem <= 200 * 1024, "map too large for the generic path");
+    VQ_REQUIRE(n + 1 <= 2147483647LL && J <= 65535, "grid too large");
+    if (smem > 48 * 1024)
+      VQ_CUDA(cudaFuncSetAttribute(scan_generic<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    dim3 grid((unsigned)(n + 1), (unsigned)J);
+    scan_generic<T><<<grid, kScanThreads, smem, stream>>>(H, is_prev, is_next, n, J, h, w, halo_prev, halo_next, so);
+    VQ_LAUNCHED();
+  }
+  return 0;
+}
+
+extern "C" int vatlq_heatmap_scan_dt(const void* H, int dtype, const uint8_t* is_prev, const uint8_t* is_next,
+                                     int64_t n, int J, int h, int w, const void* halo_prev,
+                                     const void* halo_next, const float* bbox_xyxy, float* thc,
+                                     float* peak_sum, int32_t* peak_cnt, float* peak_mean,
+                                     float* coords_hm, float* kpts, void* ws, size_t ws_bytes,
+                                     vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   VQ_REQUIRE(n >= 0 && J > 0 && h > 0 && w > 0, "bad shape");
+  VQ_REQUIRE(dtype_size(dtype) != 0, "unknown dtype (VATLQ_F32, VATLQ_F16 or VATLQ_BF16)");
   if (n == 0) return 0;
   VQ_REQUIRE(H != nullptr, "H is null");
   VQ_REQUIRE(((uintptr_t)H & 15) == 0, "H must be 16-byte aligned");
+  VQ_REQUIRE(dtype == VATLQ_F32 || ((((uintptr_t)halo_prev | (uintptr_t)halo_next) & 7) == 0),
+             "16-bit halos must be 8-byte aligned");
   VQ_REQUIRE(kpts == nullptr || bbox_xyxy != nullptr, "kpts needs bbox_xyxy");
   VQ_REQUIRE(ws != nullptr && ws_bytes >= vatlq_heatmap_scan_workspace_bytes(n, J), "workspace too small");
   const size_t nj = (size_t)n * J;
@@ -480,38 +535,11 @@ extern "C" int vatlq_heatmap_scan(const float* H, const uint8_t* is_prev, const 
   so.maxv = (float*)p;      p += align_up(nj * 4, 256);
   so.hmxy = (float*)p;
 
-  const bool fast = (h == FH && w == FW) && (halo_prev == nullptr || ((uintptr_t)halo_prev & 15) == 0) &&
-                    (halo_next == nullptr || ((uintptr_t)halo_next & 15) == 0);
-  if (fast) {
-    // one warp per (run, joint) task, ~4 tasks per warp slot so that CTAs finishing early are
-    // replaced; runs no shorter than 8 frames keep the halo re-read <= 1/8 of the traffic.
-    // 8 warps x 2 stages per SM measured best (6.8 TB/s; 6x3 5.3, 4x4 3.7: tools/tune_scan.py)
-    const int64_t slots = (int64_t)sm_count() * kTmaWarps;
-    int64_t runs = (slots * 4 + J - 1) / J;
-    int64_t run_len = (n + runs - 1) / runs;
-    if (run_len < 8) run_len = 8;
-    if (run_len > n) run_len = n;
-    runs = (n + run_len - 1) / run_len;
-    const int64_t tasks = runs * J;
-    static bool cfg = false;
-    if (!cfg) {
-      VQ_CUDA(cudaFuncSetAttribute(scan_tma_64x48, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTmaSmem));
-      cfg = true;
-    }
-    VQ_REQUIRE((tasks + kTmaWarps - 1) / kTmaWarps <= 2147483647LL, "grid too large");
-    scan_tma_64x48<<<(unsigned)((tasks + kTmaWarps - 1) / kTmaWarps), kTmaWarps * 32, kTmaSmem, stream>>>(
-        H, is_prev, is_next, n, J, halo_prev, halo_next, (int)run_len, runs, so);
-    VQ_LAUNCHED();
-  } else {
-    const size_t smem = (size_t)h * w * sizeof(float);
-    VQ_REQUIRE(smem <= 200 * 1024, "map too large for the generic path");
-    VQ_REQUIRE(n + 1 <= 2147483647LL && J <= 65535, "grid too large");
-    if (smem > 48 * 1024)
-      VQ_CUDA(cudaFuncSetAttribute(scan_generic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dim3 grid((unsigned)(n + 1), (unsigned)J);
-    scan_generic<<<grid, kScanThreads, smem, stream>>>(H, is_prev, is_next, n, J, h, w, halo_prev, halo_next, so);
-    VQ_LAUNCHED();
-  }
+  const int rc = with_dtype(dtype, [&](auto tag) {
+    using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+    return launch_scan<T>((const T*)H, is_prev, is_next, n, J, h, w, (const T*)halo_prev, (const T*)halo_next, so, stream);
+  });
+  if (rc != 0) return rc;
   const int fb = 128;
   scan_finalize<<<(unsigned)((n + fb - 1) / fb), fb, 0, stream>>>(
       n, J, h, w, is_prev, is_next, halo_prev != nullptr, halo_next != nullptr, bbox_xyxy, so, thc,
@@ -520,18 +548,40 @@ extern "C" int vatlq_heatmap_scan(const float* H, const uint8_t* is_prev, const 
   return 0;
 }
 
-extern "C" int vatlq_thc3(const float* cur, const float* prev, const float* next, const uint8_t* is_prev,
-                          const uint8_t* is_next, int64_t n, int J, int h, int w, float* thc,
-                          vatlq_stream_t stream_) {
+extern "C" int vatlq_heatmap_scan(const float* H, const uint8_t* is_prev, const uint8_t* is_next,
+                                  int64_t n, int J, int h, int w, const float* halo_prev,
+                                  const float* halo_next, const float* bbox_xyxy, float* thc,
+                                  float* peak_sum, int32_t* peak_cnt, float* peak_mean,
+                                  float* coords_hm, float* kpts, void* ws, size_t ws_bytes,
+                                  vatlq_stream_t stream) {
+  return vatlq_heatmap_scan_dt(H, VATLQ_F32, is_prev, is_next, n, J, h, w, halo_prev, halo_next, bbox_xyxy, thc, peak_sum,
+                               peak_cnt, peak_mean, coords_hm, kpts, ws, ws_bytes, stream);
+}
+
+extern "C" int vatlq_thc3_dt(const void* cur, const void* prev, const void* next, int dtype, const uint8_t* is_prev,
+                             const uint8_t* is_next, int64_t n, int J, int h, int w, float* thc,
+                             vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   VQ_REQUIRE(n >= 0 && J > 0 && h > 0 && w > 0, "bad shape");
+  VQ_REQUIRE(dtype_size(dtype) != 0, "unknown dtype (VATLQ_F32, VATLQ_F16 or VATLQ_BF16)");
   if (n == 0) return 0;
   VQ_REQUIRE(cur && thc, "null pointer");
   VQ_REQUIRE(n <= 2147483647LL, "n too large");
   const size_t fl = (size_t)J * h * w;
   if ((fl & 3) == 0)
-    VQ_REQUIRE((((uintptr_t)cur | (uintptr_t)prev | (uintptr_t)next) & 15) == 0, "tensors must be 16-byte aligned");
-  thc3_kernel<<<(unsigned)n, 256, 0, stream>>>(cur, prev, next, is_prev, is_next, n, J, h * w, thc);
-  VQ_LAUNCHED();
-  return 0;
+    VQ_REQUIRE(quad_aligned((const void*)((uintptr_t)cur | (uintptr_t)prev | (uintptr_t)next), dtype),
+               dtype == VATLQ_F32 ? "tensors must be 16-byte aligned" : "16-bit tensors must be 8-byte aligned");
+  return with_dtype(dtype, [&](auto tag) {
+    using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+    thc3_kernel<T><<<(unsigned)n, 256, 0, stream>>>((const T*)cur, (const T*)prev, (const T*)next, is_prev, is_next, n, J,
+                                                    h * w, thc);
+    VQ_LAUNCHED();
+    return 0;
+  });
+}
+
+extern "C" int vatlq_thc3(const float* cur, const float* prev, const float* next, const uint8_t* is_prev,
+                          const uint8_t* is_next, int64_t n, int J, int h, int w, float* thc,
+                          vatlq_stream_t stream) {
+  return vatlq_thc3_dt(cur, prev, next, VATLQ_F32, is_prev, is_next, n, J, h, w, thc, stream);
 }

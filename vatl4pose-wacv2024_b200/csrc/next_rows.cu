@@ -114,20 +114,21 @@ __device__ __forceinline__ float entr_f32(float p) {
   return e;
 }
 
-template <int NV>  // NV float4 per lane when the map is NV*128 pixels, 0: generic (second read from L2)
+// NV quads per lane when the map is NV*128 pixels, 0: generic (second read from L2).  T: fp32, or a 16-bit type read
+// as 8-byte quads and converted exactly in registers (same pixels per lane and chain: the bits of the fp32 upcast).
+template <int NV, typename T>
 __global__ void __launch_bounds__(256, 2)
-entropy_kernel(const float* __restrict__ H, int64_t maps, int npx, float* __restrict__ per_map) {
+entropy_kernel(const T* __restrict__ H, int64_t maps, int npx, float* __restrict__ per_map) {
   const int lane = threadIdx.x & 31;
   const int64_t mi = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (mi >= maps) return;
-  const float* mp = H + (size_t)mi * npx;
+  const T* mp = H + (size_t)mi * npx;
   double acc = 0.0;
   float e;
   if (NV > 0) {
     float4 v[NV > 0 ? NV : 1];
-    const float4* m4 = reinterpret_cast<const float4*>(mp);
 #pragma unroll
-    for (int q = 0; q < NV; ++q) v[q] = ldg_stream(m4 + q * 32 + lane);
+    for (int q = 0; q < NV; ++q) v[q] = ldg_stream_quad(mp, q * 32 + lane);
     float s = 0.f;
 #pragma unroll
     for (int q = 0; q < NV; ++q) {
@@ -176,10 +177,10 @@ entropy_kernel(const float* __restrict__ H, int64_t maps, int npx, float* __rest
       e = (float)warp_sum(ea);
     }
   } else {
-    for (int i = lane; i < npx; i += 32) acc += (double)mp[i];
+    for (int i = lane; i < npx; i += 32) acc += (double)to_f32(mp[i]);
     const float S = (float)warp_sum(acc);
     double ea = 0.0;
-    for (int i = lane; i < npx; i += 32) ea += (double)entr_f32(__fdiv_rn(mp[i], S));
+    for (int i = lane; i < npx; i += 32) ea += (double)entr_f32(__fdiv_rn(to_f32(mp[i]), S));
     e = (float)warp_sum(ea);
   }
   if (lane == 0) per_map[mi] = e;
@@ -225,7 +226,7 @@ entropy_tma_kernel(const float* __restrict__ H, int64_t maps, int run_len, float
     double acc = 0.0;
     float sm = 0.f;
 #pragma unroll
-    for (int q = 0; q < kEntNV; ++q) {       // (identical order to entropy_kernel<24>: same bits)
+    for (int q = 0; q < kEntNV; ++q) {       // (identical order to entropy_kernel<24, float>: same bits)
       sm += (v[q].x + v[q].y) + (v[q].z + v[q].w);
       if ((q & 3) == 3) {
         acc += (double)sm;
@@ -477,17 +478,34 @@ extern "C" int vatlq_pose_unc(const float* coords_hm, const float* kpts, const f
   return 0;
 }
 
-extern "C" int vatlq_heatmap_entropy(const float* H, int64_t n, int J, int h, int w, float* entropy,
-                                     void* ws, size_t ws_bytes, vatlq_stream_t stream_) {
+extern "C" int vatlq_heatmap_entropy_dt(const void* H_, int dtype, int64_t n, int J, int h, int w, float* entropy,
+                                        void* ws, size_t ws_bytes, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   VQ_REQUIRE(n >= 0 && J > 0 && h > 0 && w > 0, "bad shape");
+  VQ_REQUIRE(dtype_size(dtype) != 0, "unknown dtype (VATLQ_F32, VATLQ_F16 or VATLQ_BF16)");
   if (n == 0) return 0;
-  VQ_REQUIRE(H && entropy, "null pointer");
+  VQ_REQUIRE(H_ && entropy, "null pointer");
   const int64_t maps = n * J;
   VQ_REQUIRE(ws != nullptr && ws_bytes >= (size_t)maps * sizeof(float), "workspace must hold n*J floats");
   VQ_REQUIRE((maps + 7) / 8 <= 2147483647LL, "grid too large");
   const int npx = h * w;
   const unsigned grid = (unsigned)((maps + 7) / 8);
+  if (dtype != VATLQ_F32) {
+    // the TMA variant below is fp32 only: 16-bit maps take the register-staged kernel whatever VATLQ_ENTROPY_TMA says
+    VQ_REQUIRE(npx != 24 * 128 || quad_aligned(H_, dtype), "16-bit H must be 8-byte aligned");
+    const int rc = with_dtype(dtype, [&](auto tag) {
+      using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+      if (npx == 24 * 128) entropy_kernel<24, T><<<grid, 256, 0, stream>>>((const T*)H_, maps, npx, (float*)ws);
+      else entropy_kernel<0, T><<<grid, 256, 0, stream>>>((const T*)H_, maps, npx, (float*)ws);
+      VQ_LAUNCHED();
+      return 0;
+    });
+    if (rc != 0) return rc;
+    entropy_frames_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>((const float*)ws, n, J, entropy);
+    VQ_LAUNCHED();
+    return 0;
+  }
+  const float* H = (const float*)H_;
   // Measured on B200 (tools/time_next_rows.py, 40 000 frames): the TMA-staged variant runs at 2.5 TB/s, the
   // register-staged one at 3.9 TB/s — the kernel is bound by the ~1.4 k instructions per lane and map (MUFU.LG2 chain),
   // and 8 warps per SM (196 KB of stages) hide less of that than 16 resident warps do.  Kept for experiments only.
@@ -507,13 +525,18 @@ extern "C" int vatlq_heatmap_entropy(const float* H, int64_t n, int J, int h, in
     const int64_t tasks = (maps + run_len - 1) / run_len;
     entropy_tma_kernel<<<(unsigned)((tasks + kEntWarps - 1) / kEntWarps), kEntWarps * 32, kEntSmem, stream>>>(H, maps, run_len, (float*)ws);
   } else if (npx == 24 * 128 && ((uintptr_t)H & 15) == 0)
-    entropy_kernel<24><<<grid, 256, 0, stream>>>(H, maps, npx, (float*)ws);
+    entropy_kernel<24, float><<<grid, 256, 0, stream>>>(H, maps, npx, (float*)ws);
   else
-    entropy_kernel<0><<<grid, 256, 0, stream>>>(H, maps, npx, (float*)ws);
+    entropy_kernel<0, float><<<grid, 256, 0, stream>>>(H, maps, npx, (float*)ws);
   VQ_LAUNCHED();
   entropy_frames_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>((const float*)ws, n, J, entropy);
   VQ_LAUNCHED();
   return 0;
+}
+
+extern "C" int vatlq_heatmap_entropy(const float* H, int64_t n, int J, int h, int w, float* entropy,
+                                     void* ws, size_t ws_bytes, vatlq_stream_t stream) {
+  return vatlq_heatmap_entropy_dt(H, VATLQ_F32, n, J, h, w, entropy, ws, ws_bytes, stream);
 }
 
 static int cos_grid(int64_t m) {

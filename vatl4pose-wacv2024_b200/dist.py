@@ -29,17 +29,34 @@ def shard_sizes(n: int, world: int) -> list[int]:
     return [shard_range(n, r, world)[1] - shard_range(n, r, world)[0] for r in range(world)]
 
 
+# dtypes exchange_halo moves (heat maps: the first three); a dtype code is its index here
+_HALO_DTYPES = (torch.float32, torch.float16, torch.bfloat16, torch.float64, torch.int64, torch.int32, torch.int16,
+                torch.int8, torch.uint8, torch.bool)
+
+
 def exchange_halo(first: torch.Tensor | None, last: torch.Tensor | None, rank: int, world: int, group=None):
     """Send this rank's first frame to rank-1 and last frame to rank+1; return
     (halo_prev, halo_next): the frame before / after the local range (None at the pool ends).
-    Frames are one (J,h,w) tensor = 208 896 B at the reference shape.  Every rank must own at
-    least one frame (shard_range guarantees it for n >= world); an empty shard raises."""
+    Frames are one (J,h,w) tensor = 208 896 B at the reference shape (104 448 B in fp16 / bf16).  Every rank
+    must own at least one frame (shard_range guarantees it for n >= world); an empty shard raises.  The ranks
+    first agree on the frames' dtype (one MIN all-reduce on the frames' device): a mismatch raises VatlqError on
+    every rank instead of posting sends and receives of different sizes."""
     if world == 1:
         return None, None
     like = first if first is not None else last
     if like is None:
         raise _lib.VatlqError("exchange_halo: an empty shard is not supported (shard_range never produces one "
                               "for n >= world); give every rank at least one frame")
+    # every rank must hold one heat-map dtype, or the sends and receives below would not match: agree first, and
+    # raise on every rank on a mismatch ({min code, min -code} in one MIN all-reduce: min == max iff all agree)
+    code = _HALO_DTYPES.index(like.dtype) if like.dtype in _HALO_DTYPES else len(_HALO_DTYPES)
+    mm = torch.tensor([code, -code], dtype=torch.int64, device=like.device)
+    td.all_reduce(mm, op=td.ReduceOp.MIN, group=group)
+    lo_code, hi_code = int(mm[0].item()), -int(mm[1].item())
+    if lo_code != hi_code or code == len(_HALO_DTYPES):
+        names = [str(d) for d in _HALO_DTYPES] + ["an unsupported dtype"]
+        raise _lib.VatlqError(f"exchange_halo: the ranks hold frames of different dtypes ({names[lo_code]} .. "
+                              f"{names[hi_code]}); every rank must hold the same dtype")
     halo_prev = torch.empty_like(like) if rank > 0 else None
     halo_next = torch.empty_like(like) if rank < world - 1 else None
     ops_ = []
@@ -131,7 +148,8 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
                       group=None, first_pick: int = -1, representativeness: str = "None", filter: str = "Coreset",
                       w_unc: float = 1.0):
     """One query over a pool sharded across the ranks of `group` (one process per GPU).
-    Every rank passes its slice of the pool and gets the same global pick list back.
+    Every rank passes its slice of the pool and gets the same global pick list back.  Heat-map shards may be
+    fp32, fp16 or bf16 (the same dtype on every rank; the picks equal those of the fp32 upcast).
     uncertainty: any accelerated name (THC*, WPU*, THC+WPU, HP, TPC, Entropy, MPE, Margin, None);
     representativeness: "None" or "Influence" (ActiveLearning.py:467-477); filter: "Coreset" (:609-614),
     "None" (top-k, :533-534), "Diversity" (:581-590), "K-Means" (:593-608) or "weighted" (:553-580; w_unc = cfg.VAL.W_UNC;

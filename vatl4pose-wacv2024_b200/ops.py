@@ -34,6 +34,20 @@ def _cuda(t: torch.Tensor, dtype, name: str) -> torch.Tensor:
     return t.contiguous()
 
 
+# heat-map element types and their VATLQ_* codes: 16-bit maps are read as they are, and every result equals the
+# fp32 path's on their exact upcast, bit for bit (include/vatlq.h)
+HEATMAP_DTYPES = {torch.float32: _lib.F32, torch.float16: _lib.F16, torch.bfloat16: _lib.BF16}
+
+
+def _heatmaps(t: torch.Tensor, name: str) -> torch.Tensor:
+    """A CUDA heat-map tensor in one of HEATMAP_DTYPES, contiguous."""
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise _lib.VatlqError(f"{name} must be a CUDA tensor (the query pass has no CPU path)")
+    if t.dtype not in HEATMAP_DTYPES:
+        raise _lib.VatlqError(f"{name} must be torch.float32, torch.float16 or torch.bfloat16, got {t.dtype}")
+    return t.contiguous()
+
+
 def _flags(t, n: int, dev, name: str):
     if t is None:
         return None
@@ -58,8 +72,9 @@ class ScanResult:
 def heatmap_scan(H: torch.Tensor, is_prev=None, is_next=None, boxes_xyxy: torch.Tensor | None = None,
                  halo_prev: torch.Tensor | None = None, halo_next: torch.Tensor | None = None) -> ScanResult:
     """THC + local-peak statistics + argmax/quarter-pixel coordinates of a whole pool in one pass
-    (vatlq_heatmap_scan).  H (n,J,h,w) fp32 CUDA; flags length n; boxes (n,4) fp32 xyxy."""
-    H = _cuda(H, torch.float32, "H")
+    (vatlq_heatmap_scan_dt).  H (n,J,h,w) fp32 / fp16 / bf16 CUDA (halos of the same dtype); flags length n;
+    boxes (n,4) fp32 xyxy.  Outputs are fp32 whatever H's dtype."""
+    H = _heatmaps(H, "H")
     if H.dim() != 4:
         raise _lib.VatlqError("H must be (n,J,h,w)")
     n, nj, h, w = H.shape
@@ -69,8 +84,8 @@ def heatmap_scan(H: torch.Tensor, is_prev=None, is_next=None, boxes_xyxy: torch.
     bb = None if boxes_xyxy is None else _cuda(boxes_xyxy.to(dev), torch.float32, "boxes_xyxy")
     if bb is not None and tuple(bb.shape) != (n, 4):
         raise _lib.VatlqError("boxes_xyxy must be (n,4)")
-    hp = None if halo_prev is None else _cuda(halo_prev, torch.float32, "halo_prev")
-    hn = None if halo_next is None else _cuda(halo_next, torch.float32, "halo_next")
+    hp = None if halo_prev is None else _cuda(halo_prev, H.dtype, "halo_prev")
+    hn = None if halo_next is None else _cuda(halo_next, H.dtype, "halo_next")
     for t, nm in ((hp, "halo_prev"), (hn, "halo_next")):
         if t is not None and t.numel() != nj * h * w:
             raise _lib.VatlqError(f"{nm} must be one (J,h,w) frame")
@@ -85,26 +100,27 @@ def heatmap_scan(H: torch.Tensor, is_prev=None, is_next=None, boxes_xyxy: torch.
         coords_hm=torch.empty((n, nj, 2), dtype=torch.float32, device=dev),
         kpts=None if bb is None else torch.empty((n, nj, 3), dtype=torch.float32, device=dev))
     with torch.cuda.device(dev):
-        _lib.check(L.vatlq_heatmap_scan(_ptr(H), _ptr(ip), _ptr(inx), n, nj, h, w, _ptr(hp), _ptr(hn), _ptr(bb),
-                                        _ptr(out.thc), _ptr(out.peak_sum), _ptr(out.peak_cnt), _ptr(out.peak_mean),
-                                        _ptr(out.coords_hm), _ptr(out.kpts), _ptr(ws), ws_bytes, _stream()),
-                   "vatlq_heatmap_scan")
+        _lib.check(L.vatlq_heatmap_scan_dt(_ptr(H), HEATMAP_DTYPES[H.dtype], _ptr(ip), _ptr(inx), n, nj, h, w, _ptr(hp),
+                                           _ptr(hn), _ptr(bb), _ptr(out.thc), _ptr(out.peak_sum), _ptr(out.peak_cnt),
+                                           _ptr(out.peak_mean), _ptr(out.coords_hm), _ptr(out.kpts), _ptr(ws), ws_bytes,
+                                           _stream()), "vatlq_heatmap_scan_dt")
     return out
 
 
 def thc3(cur: torch.Tensor, prev: torch.Tensor | None, nxt: torch.Tensor | None, is_prev, is_next) -> torch.Tensor:
-    """Strict three-tensor THC (separately forwarded prev/next crops, ActiveLearning.py:293-297)."""
-    cur = _cuda(cur, torch.float32, "cur")
+    """Strict three-tensor THC (separately forwarded prev/next crops, ActiveLearning.py:293-297).
+    cur / prev / next: one dtype of HEATMAP_DTYPES."""
+    cur = _heatmaps(cur, "cur")
     n, nj, h, w = cur.shape
     dev = cur.device
-    prev = None if prev is None else _cuda(prev, torch.float32, "prev")
-    nxt = None if nxt is None else _cuda(nxt, torch.float32, "next")
+    prev = None if prev is None else _cuda(prev, cur.dtype, "prev")
+    nxt = None if nxt is None else _cuda(nxt, cur.dtype, "next")
     ip = _flags(is_prev, n, dev, "is_prev")
     inx = _flags(is_next, n, dev, "is_next")
     out = torch.empty(n, dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
-        _lib.check(_lib.lib().vatlq_thc3(_ptr(cur), _ptr(prev), _ptr(nxt), _ptr(ip), _ptr(inx), n, nj, h, w,
-                                         _ptr(out), _stream()), "vatlq_thc3")
+        _lib.check(_lib.lib().vatlq_thc3_dt(_ptr(cur), _ptr(prev), _ptr(nxt), HEATMAP_DTYPES[cur.dtype], _ptr(ip),
+                                            _ptr(inx), n, nj, h, w, _ptr(out), _stream()), "vatlq_thc3_dt")
     return out
 
 
@@ -352,16 +368,17 @@ def pose_uncertainty(coords_hm: torch.Tensor, kpts: torch.Tensor, boxes_xyxy: to
 
 
 def heatmap_entropy(H: torch.Tensor) -> torch.Tensor:
-    """Entropy uncertainty (ActiveLearning.py:790-796) of every frame (vatlq_heatmap_entropy)."""
-    H = _cuda(H, torch.float32, "H")
+    """Entropy uncertainty (ActiveLearning.py:790-796) of every frame (vatlq_heatmap_entropy_dt); H in any of
+    HEATMAP_DTYPES, fp32 (n,) out."""
+    H = _heatmaps(H, "H")
     if H.dim() != 4:
         raise _lib.VatlqError("H must be (n,J,h,w)")
     n, nj, h, w = H.shape
     out = torch.empty(n, dtype=torch.float32, device=H.device)
     ws = torch.empty(max(n * nj, 1), dtype=torch.float32, device=H.device)
     with torch.cuda.device(H.device):
-        _lib.check(_lib.lib().vatlq_heatmap_entropy(_ptr(H), n, nj, h, w, _ptr(out), _ptr(ws), ws.numel() * 4, _stream()),
-                   "vatlq_heatmap_entropy")
+        _lib.check(_lib.lib().vatlq_heatmap_entropy_dt(_ptr(H), HEATMAP_DTYPES[H.dtype], n, nj, h, w, _ptr(out), _ptr(ws),
+                                                       ws.numel() * 4, _stream()), "vatlq_heatmap_entropy_dt")
     return out
 
 
@@ -445,8 +462,9 @@ def oks(kpts: torch.Tensor, gt_kpts: torch.Tensor, bbox_ann_xyxy: torch.Tensor) 
 
 
 def peak_uncertainty(H: torch.Tensor, want_mpe: bool = True, want_margin: bool = True):
-    """MPE / Margin uncertainties (ActiveLearning.py:762-788) of every frame (vatlq_peak_unc): fp32 (n,) each."""
-    H = _cuda(H, torch.float32, "H")
+    """MPE / Margin uncertainties (ActiveLearning.py:762-788) of every frame (vatlq_peak_unc_dt): H in any of
+    HEATMAP_DTYPES, fp32 (n,) each."""
+    H = _heatmaps(H, "H")
     if H.dim() != 4:
         raise _lib.VatlqError("H must be (n,J,h,w)")
     n, nj, h, w = H.shape
@@ -454,8 +472,8 @@ def peak_uncertainty(H: torch.Tensor, want_mpe: bool = True, want_margin: bool =
     mar = torch.empty(n, dtype=torch.float32, device=H.device) if want_margin else None
     ws = torch.empty(max(int(_lib.lib().vatlq_peak_workspace_bytes(n, nj, h, w)), 16), dtype=torch.uint8, device=H.device)
     with torch.cuda.device(H.device):
-        _lib.check(_lib.lib().vatlq_peak_unc(_ptr(H), n, nj, h, w, _ptr(mpe), _ptr(mar), _ptr(ws), ws.numel(), _stream()),
-                   "vatlq_peak_unc")
+        _lib.check(_lib.lib().vatlq_peak_unc_dt(_ptr(H), HEATMAP_DTYPES[H.dtype], n, nj, h, w, _ptr(mpe), _ptr(mar), _ptr(ws),
+                                                ws.numel(), _stream()), "vatlq_peak_unc_dt")
     return mpe, mar
 
 

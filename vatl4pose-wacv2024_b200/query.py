@@ -95,12 +95,17 @@ class QueryPass:
         `halo_next` are only for the first / last chunk of a rank's range (frames owned by the
         neighbouring ranks); between chunks the halo is carried automatically: the scan of a
         chunk is given the first frame of the NEXT chunk as halo_next lazily — to keep the
-        stream simple the last frame of every chunk is re-scored with the next chunk instead."""
+        stream simple the last frame of every chunk is re-scored with the next chunk instead.
+        H may be fp32, fp16 or bf16 (ops.HEATMAP_DTYPES); the carried halo frame keeps the chunk's dtype, so every
+        chunk of one pool must share it (converting the carried frame to 16 bits would round it)."""
         m = H.shape[0]
         if m == 0:
             return
         if self._carry is not None and pos != self._carry_pos:
             raise _lib.VatlqError("chunks must be fed in pool order")
+        if self._carry is not None and H.dtype != self._carry.dtype:
+            raise _lib.VatlqError(f"every chunk of a pool must have one heat-map dtype: got {H.dtype} after "
+                                  f"{self._carry.dtype}")
         first = self._carry is None
         hp = halo_prev if first else self._carry
         last_chunk = pos + m >= self.n
@@ -222,7 +227,8 @@ def run_query(H, boxes_xyxy, is_prev, is_next, X, ae_weights, labeled, k: int, m
               batch: int = 16, device="cuda:0", chunk: int | None = None, first_pick: int = -1) -> QueryResult:
     """One full single-GPU query (THC + WPU + fusion + core-set) — the public functional API.
     Inputs may be host numpy arrays / CPU tensors (copied to `device` here, chunk by chunk for
-    the heat maps) or CUDA tensors (used in place)."""
+    the heat maps) or CUDA tensors (used in place).  Heat maps may be fp32, fp16 or bf16 (numpy float16,
+    torch bfloat16): they are copied and scored in their own dtype, never converted."""
     dev = torch.device(device)
 
     def to_dev(a, dtype):
