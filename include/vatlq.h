@@ -208,6 +208,17 @@ int vatlq_coreset_prune_stats(int64_t* host_out4, int reset);
  * 2 verify; min_rows < 0: environment */
 int vatlq_coreset_set_prune(int mode, int64_t min_rows);
 
+/* The TF32 screen of the 16-pick rounds (d == 2048): before a round's fp64 pass each streamed row is
+ * compared with the round's centres on the tensor cores, and only the rows that an error bound cannot
+ * prove unchanged (min_d[i] <= d(i,c) for every centre) go through the exact fp64 arithmetic.  The pick
+ * list and min_d are unchanged bit for bit.  Environment: VATLQ_PASS_SCREEN=0 disables,
+ * VATLQ_PASS_SCREEN=verify computes every streamed row exactly and counts the rows the screen did not
+ * list whose min_d moved.  host_out3 = {rows screened, rows listed, verify violations (must be 0)},
+ * accumulated over the vatlq_coreset_select calls since the last reset. */
+int vatlq_coreset_screen_stats(int64_t* host_out3, int reset);
+/* process-wide override of VATLQ_PASS_SCREEN: -1 environment, 0 off, 1 screen, 2 verify */
+int vatlq_coreset_set_screen(int mode);
+
 /* One pairwise-distance column block, exposed for parity tests of the distance arithmetic:
  * out[i*m + j] = d(X[i], X[centers[j]]) in fp64 (sklearn _euclidean_distances order). */
 int vatlq_pairwise_dist(const float* X, int64_t n, int d, const int64_t* centers, int64_t m,

@@ -35,6 +35,8 @@ SIGNATURES = {
                                     _i64, _i64, _int, _vp, _vp, _vp, _sz, _vp, _vp]),
     "vatlq_coreset_prune_stats": (_int, [_vp, _int]),
     "vatlq_coreset_set_prune": (_int, [_int, _i64]),
+    "vatlq_coreset_screen_stats": (_int, [_vp, _int]),
+    "vatlq_coreset_set_screen": (_int, [_int]),
     "vatlq_pairwise_dist": (_int, [_vp, _i64, _int, _vp, _i64, _vp, _vp, _sz, _vp]),
     "vatlq_pose_unc": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _vp, _vp, _vp, _vp, _vp]),
     "vatlq_heatmap_entropy": (_int, [_vp, _i64, _int, _int, _int, _vp, _vp, _sz, _vp]),

@@ -363,6 +363,10 @@ struct PassArgs {
   unsigned char* seg_skip_out;       // [2][skip_stride] flags written by the filter mode
   int prune_mode;                    // 0 off, 1 skip, 2 verify (stream everything, count rows that changed anyway)
   unsigned long long* prune_stats;   // [0] tiles seen, [1] tiles streamed, [2] verify violations
+  // paired pass only, see "the screen" at pass_kernel_tma: 0 off, 1 DMMA only the rows the TF32 screen cannot
+  // decide, 2 verify (DMMA every streamed row, count unlisted rows whose min_d moved anyway)
+  int screen_mode;
+  unsigned long long* screen_stats;  // [0] rows screened, [1] rows listed, [2] verify violations
 };
 
 // centres of THIS pass: count (<= 0: nothing to do) and whether it is the round's last pass
@@ -655,7 +659,8 @@ __device__ __forceinline__ ApplyConst apply_const(const PassArgs& a, bool final_
   return c;
 }
 // tile_mode: 0 streamed, 1 pruned (no dot products were computed: min_d stays), 2 verify (streamed
-// although the filter flagged it: count the rows whose min_d moved anyway — must stay 0)
+// although the filter flagged it: count the rows whose min_d moved anyway — must stay 0), 3 screen verify
+// (computed although the screen decided the row: the same count, into screen_stats[2])
 // Returns the histogram bin of the row's new score (-1: outside the window / no histogram): the caller adds it
 // warp-aggregated (rows of one track score alike, so per-row shared-memory atomics on one bin — and on the in-window
 // counter — serialised the whole CTA: 145 us of a 1 M-row pass).
@@ -678,6 +683,7 @@ __device__ __forceinline__ int apply_row(const PassArgs& a, const ApplyConst& c,
   const double m_old = a.m[i];
   const double dmin = fmin(m_old, sqrt(fmax(tm, 0.0)));
   if (tile_mode == 2 && (dmin != m_old || picked)) atomicAdd(&a.prune_stats[2], 1ULL);
+  if (tile_mode == 3 && (dmin != m_old || picked)) atomicAdd(&a.screen_stats[2], 1ULL);
   if (tile_mode != 1) a.m[i] = dmin;
   if (a.unc) {
     double u = a.unc[i];
@@ -720,7 +726,8 @@ constexpr int kStageBytesX = 8 * kRowBytesX;               // 66 048
 constexpr int kWsThreads = (kSeg + 4) * 32;                // 8 compute warps + producer + 3 epilogue warps
 constexpr int kMaxTilesCta = 2048;                         // tiles per CTA the pruned-tile list can hold
 constexpr size_t kWsSmem = (size_t)kStagesX * kStageBytesX + sizeof(double) * kPartBufs * kSeg * 64 + 2 * kStagesX * 8 +
-                           2 * kB * 16 + (kNB + 1) * 4 + 128 + kMaxTilesCta * 2 + kMaxTilesCta / 8 + 16;
+                           2 * kB * 16 + (kNB + 1) * 4 + 128 + kMaxTilesCta * 2 + kMaxTilesCta / 8 + 16 +
+                           kMaxTilesCta + 2 * kB * 8 + 16;   // the screen: listed-row mask per tile, centre norms
 
 __device__ __forceinline__ unsigned smem_addr(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void named_sync(int id, int count) {
@@ -748,6 +755,60 @@ __device__ __forceinline__ unsigned cluster_ctarank() {
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
+// 32-bit word at the same shared-memory offset in CTA `rank` of the cluster
+__device__ __forceinline__ unsigned ld_dsmem_u32(const void* p, unsigned rank) {
+  unsigned remote, v;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_addr(p)), "r"(rank));
+  asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(remote) : "memory");
+  return v;
+}
+
+// ---- the screen (paired pass, screen_mode != 0) ------------------------------------------------
+// A round only needs to know which rows get closer to one of its <= 16 centres: min_d[i] changes iff
+// d(i,c) < m_old = min_d[i] for some c.  Before the DMMA tile loop each CTA of a pair streams the tiles of ITS
+// parity (the rows it finishes) through the same TMA ring and the compute warps evaluate S~ = x.c for all 16
+// centres with mma.sync m16n8k8 TF32 (A = 16 centres from registers, B = the tile's 8 rows, fp32
+// accumulation; warp w = K segment w as in the DMMA loop).  A row is DECIDED when for every centre
+//     S~ finite  and  fl(t~ - 2E) > m_old^2 rounded up,   t~ = (|x|^2 + |c|^2) - 2 S~,
+//     E = 2u |x||c| + 2^-20 (|x|^2 + |c|^2),  u = 2^-8,
+// with m_old finite and the row not one of the picks.  Proof that a decided row keeps min_d bit for bit: the
+// TF32 operands carry >= 10 mantissa bits and the fp32 accumulation over K = 2048 adds at most 2048 * 2^-23
+// relative to sum |x_k c_k| <= |x||c| (Cauchy-Schwarz), so |S~ - S| <= (2^-9 + 2^-12) |x||c| <= u |x||c| (S: the
+// exact dot of the fp32 features).  The canonical fp64 value t = fl(fl(-2 dot + xx_i) + xx_c) is within
+// 2^-48 (|x|^2 + |c|^2) of |x|^2 + |c|^2 - 2S, so t >= t~ - 2u|x||c| - 2^-48(..) = (t~ - 2E) + 2u|x||c|
+// + 2^-19 (|x|^2 + |c|^2) - 2^-48 (..), which exceeds the computed fl(t~ - 2E) by more than that subtraction's
+// own rounding (and that of |x|, |c|, which enter E only scaled by u): t > m_old^2.  sqrt is correctly rounded and
+// monotone and m_old is a double, so d = sqrt(max(t, 0)) >= m_old and fmin(m_old, d) == m_old: the row's
+// min_d, score and candidate record are exactly what the full pass writes.  Any NaN / Inf makes the test false
+// (the row is listed).  The undecided rows are then gathered 8 per tile (the same per-row TMA copies the
+// producer always issues) and only those go through the canonical DMMA tile machine.
+constexpr double kScreenU = 0.00390625;               // 2^-8
+constexpr double kScreenAbs = 9.5367431640625e-07;    // 2^-20
+__device__ __forceinline__ void mma_tf32(float (&d)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
+  asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+// entry e of the list of undecided rows -> the walker's tile k and row r (s_pre: inclusive prefix of the listed
+// rows per tile, nt entries; s_mask: the listed rows of every tile)
+__device__ __forceinline__ int listed_row(const unsigned short* s_pre, const unsigned char* s_mask, int nt, int e) {
+  int lo = 0, hi = nt - 1;   // smallest k with s_pre[k] > e
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if ((int)s_pre[mid] > e) hi = mid;
+    else lo = mid + 1;
+  }
+  int skip = e - (lo ? (int)s_pre[lo - 1] : 0);
+  const unsigned m = s_mask[lo];
+  int r = 0;
+#pragma unroll
+  for (int b = 0; b < 8; ++b)
+    if ((m >> b) & 1u) {
+      if (skip == 0) r = b;
+      --skip;
+    }
+  return lo * 8 + r;
+}
 
 template <int STEPS, bool PAIR, bool FILTER = false>
 __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
@@ -765,7 +826,11 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
   // flagged ones, and the number of streamed tiles
   unsigned short* s_tiles = reinterpret_cast<unsigned short*>(s_hist + (kNB + 1) + 3);
   unsigned int* s_flagged = reinterpret_cast<unsigned int*>(s_tiles + kMaxTilesCta);
-  int* s_na = reinterpret_cast<int*>(s_flagged + kMaxTilesCta / 32);
+  int* s_na = reinterpret_cast<int*>(s_flagged + kMaxTilesCta / 32);   // [0] streamed tiles, [1] of them of this CTA's
+                                                                        // parity, [2] rows the screen listed
+  // the screen: listed (undecided) rows of every tile of the walker as a bit mask, |c| of the 16 centres
+  unsigned char* s_mask = reinterpret_cast<unsigned char*>(s_na + 4);
+  double* s_nc = reinterpret_cast<double*>(s_mask + kMaxTilesCta);
 
   pdl_enter();
   const int total = a.n_centers ? *a.n_centers : a.n_centers_imm;
@@ -801,6 +866,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     const int last = PAIR ? total - 1 : nb - 1;
     const long long p = (a.centers + a.center_off)[min((int)threadIdx.x, last)];
     s_xxc[threadIdx.x] = a.xx[p];
+    s_nc[threadIdx.x] = sqrt(a.xx[p]);
     s_pick[threadIdx.x] = p;
   }
   for (int b = threadIdx.x; b < kNB + 1; b += blockDim.x) s_hist[b] = 0u;
@@ -816,6 +882,10 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
   const int nt = ((long long)cid < ntiles) ? (int)((ntiles - cid + ncl - 1) / ncl) : 0;
   // tile j of the streamed sequence is tile k = tile_of(j) of the walker (rows (cid + k*ncl)*8 ...)
   const bool use_list = !FILTER && a.seg_skip != nullptr && a.prune_mode != 0 && nt <= kMaxTilesCta;
+  const int screen = (PAIR && !FILTER && nt <= kMaxTilesCta) ? a.screen_mode : 0;   // the same on both CTAs of a pair
+  const unsigned own_par = crank ? 0xaaaaaaaau : 0x55555555u;   // tiles base + lane of this CTA's parity (base % 32 == 0)
+  if (screen)
+    for (int k = threadIdx.x; k < nt; k += blockDim.x) s_mask[k] = 0;
   // The list of streamed tiles is built by ALL warps (chunks of 32 tiles dealt round-robin: the two dependent loads per
   // tile — segment ids, then their flags — are one memory round trip per chunk instead of one per 32 tiles of the
   // whole CTA); the chunk counts are scanned by one warp and every warp then writes its chunks at their offsets.
@@ -844,12 +914,16 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
       if (lane == 0) {
         s_flagged[base >> 5] = fm;
         s_cnt[base >> 5] = __popc(sm);
+        s_cnt[kMaxTilesCta / 32 + (base >> 5)] = __popc(sm & own_par);
       }
     }
     __syncthreads();
     if (warp == 0) {                     // exclusive scan of the chunk counts (<= 64 chunks: two per lane)
       const int nch = (nt + 31) >> 5;
       const unsigned c0 = (2 * lane < nch) ? s_cnt[2 * lane] : 0u, c1 = (2 * lane + 1 < nch) ? s_cnt[2 * lane + 1] : 0u;
+      const int n1 = warp_sum((int)((2 * lane < nch ? s_cnt[kMaxTilesCta / 32 + 2 * lane] : 0u) +
+                                    (2 * lane + 1 < nch ? s_cnt[kMaxTilesCta / 32 + 2 * lane + 1] : 0u)));
+      if (lane == 0) s_na[1] = n1;
       unsigned incl = c0 + c1;
 #pragma unroll
       for (int o = 1; o < 32; o <<= 1) {
@@ -875,6 +949,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     }
   } else if (threadIdx.x == 0) {
     *s_na = nt;
+    s_na[1] = (nt + 1 - crank) / 2;
     if (a.prune_stats && nt > 0 && crank == 0) {
       atomicAdd(&a.prune_stats[0], (unsigned long long)nt);
       atomicAdd(&a.prune_stats[1], (unsigned long long)nt);
@@ -884,11 +959,101 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
   if (clocked) tq1 = gtime_ns();
   const int na = *s_na;
   auto tile_of = [&](int j) -> int { return use_list ? (int)s_tiles[j] : j; };
+  // the screen's tiles are the streamed tiles of this CTA's parity (the rows it finishes): n1 of them
+  const int n1 = s_na[1];
+  // between the screen and the DMMA tiles (every thread of both CTAs): merge the partner's listed rows, so that
+  // both CTAs of the pair walk the same list of undecided rows, and (list mode) count them per tile
+  auto screen_join = [&]() {
+    named_sync(7, kWsThreads);
+    cluster_sync_all();
+    for (int w = threadIdx.x; w < (nt + 3) / 4; w += blockDim.x)
+      reinterpret_cast<unsigned*>(s_mask)[w] |= ld_dsmem_u32(s_mask + 4 * w, (unsigned)crank ^ 1u);
+    named_sync(7, kWsThreads);
+    if (screen == 1) {
+      if (warp == kSeg) {   // inclusive prefix of the listed rows per tile (s_tiles is no longer read)
+        const int k0 = lane * (kMaxTilesCta / 32), k1 = min(nt, k0 + kMaxTilesCta / 32);
+        int sum = 0;
+        for (int k = k0; k < k1; ++k) sum += __popc(s_mask[k]);
+        int incl = sum;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const int t = __shfl_up_sync(0xffffffffu, incl, o);
+          if (lane >= o) incl += t;
+        }
+        int run = incl - sum;
+        for (int k = k0; k < k1; ++k) {
+          run += __popc(s_mask[k]);
+          s_tiles[k] = (unsigned short)run;
+        }
+        if (lane == 31) s_na[2] = incl;
+      }
+      named_sync(7, kWsThreads);
+    }
+  };
+  // row (relative to a.lo) of entry e of the listed rows
+  auto list_row = [&](int e) -> long long {
+    const int q = listed_row(s_tiles, s_mask, nt, e);
+    return ((long long)cid + (long long)(q >> 3) * ncl) * 8 + (q & 7);
+  };
 
   if (warp < kSeg) {
     // ------------------------------------------------------------------ compute warps
     asm volatile("setmaxnreg.inc.sync.aligned.u32 216;");
     const int seg = warp, g = lane >> 2, kk = lane & 3;
+    const unsigned a_off = smem_addr(stage0) + g * kRowBytesX + seg * (STEPS * 64) + kk * 16;
+    int st = 0, pb = 0;
+    unsigned phase = 0;
+    if (screen) {
+      // A operand of mma.m16n8k8: centres g and g + 8 of the round at the features this lane reads of a row (the
+      // k slots of the two MMAs of a super-step are features 16s + 4kk + {0, 1} and {2, 3}: the same permutation
+      // of K for A and B)
+      unsigned af[STEPS][8];
+      {
+        const long long* allc = a.centers + a.center_off;
+        const long long p0 = allc[min(g, total - 1)], p1 = allc[min(g + kB, total - 1)];
+        const float4* c0 = reinterpret_cast<const float4*>(a.X) + (size_t)p0 * a.d4 + seg * (STEPS * 4) + kk;
+        const float4* c1 = reinterpret_cast<const float4*>(a.X) + (size_t)p1 * a.d4 + seg * (STEPS * 4) + kk;
+#pragma unroll
+        for (int s = 0; s < STEPS; ++s) {
+          const float4 v0 = __ldg(c0 + 4 * s), v1 = __ldg(c1 + 4 * s);
+          af[s][0] = __float_as_uint(v0.x); af[s][1] = __float_as_uint(v0.y);
+          af[s][2] = __float_as_uint(v0.z); af[s][3] = __float_as_uint(v0.w);
+          af[s][4] = __float_as_uint(v1.x); af[s][5] = __float_as_uint(v1.y);
+          af[s][6] = __float_as_uint(v1.z); af[s][7] = __float_as_uint(v1.w);
+        }
+      }
+      const unsigned my_partf = smem_addr(&s_part[0][seg][0]) + lane * 16;
+      for (int k = 0; k < n1; ++k) {
+        mbar_wait(&full[st], phase);
+        const unsigned ap = a_off + st * kStageBytesX;
+        float d0[4] = {0.f, 0.f, 0.f, 0.f}, d1[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+        for (int s = 0; s < STEPS; ++s) {
+          const float4 x = lds128(ap + s * 64);
+          const unsigned A0[4] = {af[s][0], af[s][4], af[s][1], af[s][5]};
+          const unsigned A1[4] = {af[s][2], af[s][6], af[s][3], af[s][7]};
+          mma_tf32(d0, A0, __float_as_uint(x.x), __float_as_uint(x.y));
+          mma_tf32(d1, A1, __float_as_uint(x.z), __float_as_uint(x.w));
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty[st]);
+        if (++st == kStagesX) {
+          st = 0;
+          phase ^= 1u;
+        }
+        if (k >= kPartBufs) named_sync(1 + kPartBufs + pb, kSeg * 32 + 32);
+        // lane (g,kk): centre g at rows 2kk, 2kk+1, centre g+8 at rows 2kk, 2kk+1
+        asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(my_partf + pb * (unsigned)(sizeof(double) * kSeg * 64)),
+                     "f"(d0[0] + d1[0]), "f"(d0[1] + d1[1]), "f"(d0[2] + d1[2]), "f"(d0[3] + d1[3])
+                     : "memory");
+        asm volatile("fence.acq_rel.cta;" ::: "memory");
+        named_arrive(1 + pb, kSeg * 32 + 32);
+        if (++pb == kPartBufs) pb = 0;
+      }
+      screen_join();
+      pb = 0;
+    }
+    const int nd = screen == 1 ? (s_na[2] + 7) / 8 : na;   // DMMA tiles
     double breg[STEPS][4];
     {
       const long long pg = centers[min(g, nb - 1)];
@@ -902,11 +1067,8 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
         breg[s][3] = (double)v.w;
       }
     }
-    const unsigned a_off = smem_addr(stage0) + g * kRowBytesX + seg * (STEPS * 64) + kk * 16;
     const unsigned my_part = smem_addr(&s_part[0][seg][lane * 2]);
-    int st = 0, pb = 0;
-    unsigned phase = 0;
-    for (int k = 0; k < na; ++k) {
+    for (int k = 0; k < nd; ++k) {
       mbar_wait(&full[st], phase);
       const unsigned ap = a_off + st * kStageBytesX;
       double c[4][2];
@@ -940,34 +1102,110 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     if (warp == kSeg) {
       // ---------------------------------------------------------------- producer warp
       // lane r < 8 copies row r of every tile; rows past the end re-read the last row
-      int st = 0;
+      int st = 0, fills = 0;
       unsigned phase = 0;
-      for (int j = 0; j < na; ++j) {
-        const int k = tile_of(j);
-        if (j >= kStagesX) mbar_wait(&empty[st], phase ^ 1u);   // the stage's previous tile was released
+      auto fill = [&](auto row_of_lane) {
+        if (fills++ >= kStagesX) mbar_wait(&empty[st], phase ^ 1u);   // the stage's previous tile was released
         if (lane == 0) mbar_expect_tx(&full[st], 8u * 2048u * 4u);
         __syncwarp();
         if (lane < 8) {
-          long long row;
-          if (FILTER) row = a.lo + a.seg_start[min((int)(((long long)cid + (long long)k * ncl) * 8 + lane), nseg - 1)];   // anchor rows
-          else row = min(a.lo + ((long long)cid + (long long)k * ncl) * 8 + lane, a.hi - 1);
+          const long long row = row_of_lane();
           tma_load_1d(stage0 + (size_t)st * kStageBytesX + lane * kRowBytesX, a.X + (size_t)row * 2048, 2048u * 4u, &full[st]);
         }
         if (++st == kStagesX) {
           st = 0;
           phase ^= 1u;
         }
+      };
+      if (screen) {
+        for (int j = 0; j < na; ++j) {
+          const int k = tile_of(j);
+          if ((k & 1) != crank) continue;
+          fill([&]() { return min(a.lo + ((long long)cid + (long long)k * ncl) * 8 + lane, a.hi - 1); });
+        }
+        screen_join();
+      }
+      if (screen == 1) {
+        const int nl = s_na[2];
+        for (int j = 0; j < (nl + 7) / 8; ++j) fill([&]() { return a.lo + list_row(min(j * 8 + lane, nl - 1)); });
+      } else {
+        for (int j = 0; j < na; ++j) {
+          const int k = tile_of(j);
+          fill([&]() {
+            if (FILTER) return a.lo + a.seg_start[min((int)(((long long)cid + (long long)k * ncl) * 8 + lane), nseg - 1)];   // anchor rows
+            return min(a.lo + ((long long)cid + (long long)k * ncl) * 8 + lane, a.hi - 1);
+          });
+        }
       }
     } else {
       // ---------------------------------------------------------------- epilogue warps
       const int ew = warp - kSeg - 1;             // partial buffer of this warp: tiles k = ew, ew+3, ...
       const int r = lane >> 2;                    // lane (r,kk): row r, centres 2kk, 2kk+1 (the DMMA C layout)
-      for (int j = ew; j < na; j += kPartBufs) {
-        const int k = tile_of(j);
+      if (screen) {
+        // lane (r, q): row r of the tile against centres q, q+4, q+8, q+12
+        const int q = lane & 3;
+        const float* sf = reinterpret_cast<const float*>(&s_part[ew][0][0]);
+        unsigned long long n_rows = 0, n_listed = 0;
+        for (int j = 0, jj = 0; j < na; ++j) {
+          const int k = tile_of(j);
+          if ((k & 1) != crank) continue;
+          if (jj++ % kPartBufs != ew) continue;
+          const long long i = a.lo + ((long long)cid + (long long)k * ncl) * 8 + r;
+          const bool valid = i < a.hi;
+          const long long ic = valid ? i : a.hi - 1;
+          const double xxi = a.xx[ic], m_old = a.m[ic];
+          named_sync(1 + ew, kSeg * 32 + 32);
+          double S[4];
+#pragma unroll
+          for (int c4 = 0; c4 < 4; ++c4) {
+            const int c = q + 4 * c4;
+            const int at = ((c & 7) * 4 + (r >> 1)) * 4 + ((c >> 3) << 1) + (r & 1);
+            double s = 0.0;
+#pragma unroll
+            for (int w = 0; w < kSeg; ++w) s += (double)sf[w * 128 + at];
+            S[c4] = s;
+          }
+          if (jj - 1 + kPartBufs < n1) named_arrive(1 + kPartBufs + ew, kSeg * 32 + 32);
+          const double nx = sqrt(xxi), m2 = __dmul_ru(m_old, m_old);
+          bool und = !isfinite(m_old);
+#pragma unroll
+          for (int c4 = 0; c4 < 4; ++c4) {
+            const int c = q + 4 * c4;
+            const double xs = xxi + s_xxc[c];
+            const double t = xs - 2.0 * S[c4];
+            const double E = 2.0 * kScreenU * nx * s_nc[c] + kScreenAbs * xs;
+            und = und || !(isfinite(S[c4]) && t - 2.0 * E > m2) || s_pick[c] == i;
+          }
+          const unsigned ub = __ballot_sync(0xffffffffu, und && valid);
+          unsigned byte = 0;
+#pragma unroll
+          for (int rr = 0; rr < 8; ++rr)
+            if ((ub >> (4 * rr)) & 0xfu) byte |= 1u << rr;
+          if (lane == 0) {
+            s_mask[k] = (unsigned char)byte;
+            n_rows += (unsigned long long)min(8LL, a.hi - (a.lo + ((long long)cid + (long long)k * ncl) * 8));
+            n_listed += __popc(byte);
+          }
+        }
+        if (lane == 0 && a.screen_stats && n_rows) {
+          atomicAdd(&a.screen_stats[0], n_rows);
+          atomicAdd(&a.screen_stats[1], n_listed);
+        }
+        screen_join();
+      }
+      const int nl = screen == 1 ? s_na[2] : 0;
+      const int nd = screen == 1 ? (nl + 7) / 8 : na;
+      for (int j = ew; j < nd; j += kPartBufs) {
         named_sync(1 + ew, kSeg * 32 + 32);
         const double dot0 = combine8(&s_part[ew][0][lane * 2], 64);
         const double dot1 = combine8(&s_part[ew][0][lane * 2 + 1], 64);
-        if (j + kPartBufs < na) named_arrive(1 + kPartBufs + ew, kSeg * 32 + 32);   // partials consumed
+        if (j + kPartBufs < nd) named_arrive(1 + kPartBufs + ew, kSeg * 32 + 32);   // partials consumed
+        if (screen == 1) {
+          if (j * 8 + r < nl)
+            *reinterpret_cast<double2*>(a.dots + list_row(j * 8 + r) * NC + crank * kB + (lane & 3) * 2) = make_double2(dot0, dot1);
+          continue;
+        }
+        const int k = tile_of(j);
         const long long row = ((long long)cid + (long long)k * ncl) * 8 + r;   // relative to a.lo (FILTER: segment id)
         if (FILTER) {
           // segment `row`: nearest of this group's centres to its anchor, largest min_d of its rows, the test of
@@ -1018,7 +1256,9 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
       if (q < nrows) {
         const int k = PAIR ? 2 * (q >> 3) + crank : (q >> 3);
         const long long i = a.lo + ((long long)cid + (long long)k * ncl) * 8 + (q & 7);
-        const int tile_mode = (use_list && ((s_flagged[k >> 5] >> (k & 31)) & 1u)) ? a.prune_mode : 0;
+        int tile_mode = (use_list && ((s_flagged[k >> 5] >> (k & 31)) & 1u)) ? a.prune_mode : 0;
+        // a row the screen decided: no dot products (list mode) or a verify count
+        if (screen && !((s_mask[k] >> (q & 7)) & 1u)) tile_mode = (screen == 1) ? 1 : (tile_mode ? tile_mode : 3);
         if (i < a.hi) bin = apply_row<NC>(a, ac, i, s_xxc, s_pick, best, tile_mode);
       }
       if (ac.do_hist) {                                            // one shared atomic per distinct bin per warp
@@ -1064,6 +1304,7 @@ struct PruneCtl {
   unsigned long long cnt;
   int nseg, pad;
   unsigned long long stats[3];     // tiles seen, tiles streamed, verify violations (PassArgs::prune_stats)
+  unsigned long long screen[3];    // rows screened, rows listed, verify violations (PassArgs::screen_stats)
 };
 
 // squared distance of two rows as sum((x-y)^2) in fp64 (every lane returns the warp total)
@@ -1999,6 +2240,8 @@ static PassProfiler g_prof;
 static long long g_prune[4] = {0, 0, 0, 0};   // tiles seen, tiles streamed, verify violations, segments (last call)
 static int g_prune_mode_set = -1;              // vatlq_coreset_set_prune: -1 = take VATLQ_PRUNE
 static long long g_prune_min_set = -1;         //                          -1 = take VATLQ_PRUNE_MIN_ROWS
+static long long g_screen[3] = {0, 0, 0};      // rows screened, rows listed, verify violations (paired passes)
+static int g_screen_mode_set = -1;             // vatlq_coreset_set_screen: -1 = take VATLQ_PASS_SCREEN
 
 }  // namespace vatlq
 
@@ -2205,6 +2448,7 @@ static void prune_collect(const PruneState& P) {
     g_prune[1] += (long long)hp.stats[1];
     g_prune[2] += (long long)hp.stats[2];
     g_prune[3] = hp.nseg;
+    for (int q = 0; q < 3; ++q) g_screen[q] += (long long)hp.screen[q];
   }
 }
 
@@ -2340,6 +2584,14 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
     return e ? atoll(e) : 0LL;
   }();
   const bool tma_filter = (row_hi - row_lo) >= tma_filter_min;
+  // the TF32 screen of the paired pass (see "the screen" at pass_kernel_tma): 0 off, 1 on, 2 verify
+  static const int screen_env = []() {
+    const char* e = getenv("VATLQ_PASS_SCREEN");
+    if (!e) return 1;
+    if (!strcmp(e, "0") || !strcmp(e, "off")) return 0;
+    return !strcmp(e, "verify") ? 2 : 1;
+  }();
+  const int screen_mode = g_screen_mode_set >= 0 ? g_screen_mode_set : screen_env;
   static const size_t plan_smem = getenv("VATLQ_PLAN_SMEM") ? (size_t)atoi(getenv("VATLQ_PLAN_SMEM")) * 1024 : (size_t)kPlanSmem;   // 0: L2 path
   static bool pairs_cfg = false;
   if (!pairs_cfg) {
@@ -2468,6 +2720,8 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
         fill_pass(a);
         a.skip_stride = P.skip_stride;
         a.push = push_of(seq0 + round_no + 1);   // the block this round's (only) pass publishes
+        a.screen_mode = screen_mode;
+        a.screen_stats = P.pc->screen;
         rc = timed_launch(a, true);
         if (rc == 0) {
           PassArgs b{};
@@ -2569,6 +2823,19 @@ extern "C" int vatlq_coreset_set_prune(int mode, int64_t min_rows) {
   VQ_REQUIRE(mode >= -1 && mode <= 2, "mode must be -1 (environment), 0 (off), 1 (prune) or 2 (verify)");
   g_prune_mode_set = mode;
   g_prune_min_set = min_rows < 0 ? -1 : (long long)min_rows;
+  return 0;
+}
+
+extern "C" int vatlq_coreset_set_screen(int mode) {
+  VQ_REQUIRE(mode >= -1 && mode <= 2, "mode must be -1 (environment), 0 (off), 1 (screen) or 2 (verify)");
+  g_screen_mode_set = mode;
+  return 0;
+}
+
+extern "C" int vatlq_coreset_screen_stats(int64_t* host_out3, int reset) {
+  if (host_out3)
+    for (int i = 0; i < 3; ++i) host_out3[i] = g_screen[i];
+  if (reset) g_screen[0] = g_screen[1] = g_screen[2] = 0;
   return 0;
 }
 

@@ -321,6 +321,21 @@ def prune_stats(reset: bool = False) -> dict:
     return {"tiles": int(out[0]), "streamed": int(out[1]), "violations": int(out[2]), "segments": int(out[3])}
 
 
+SCREEN_MODES = {"env": -1, "off": 0, "on": 1, "verify": 2}
+
+
+def set_screen(mode: str = "env"):
+    """TF32 screen of the 16-pick rounds (include/vatlq.h): "env" (VATLQ_PASS_SCREEN), "off", "on" or "verify"."""
+    _lib.check(_lib.lib().vatlq_coreset_set_screen(SCREEN_MODES[mode]), "vatlq_coreset_set_screen")
+
+
+def screen_stats(reset: bool = False) -> dict:
+    """Rows screened / listed for the exact fp64 pass and verify violations, since the last reset."""
+    out = (C.c_int64 * 3)()
+    _lib.check(_lib.lib().vatlq_coreset_screen_stats(C.cast(out, C.c_void_p), int(reset)), "vatlq_coreset_screen_stats")
+    return {"screened": int(out[0]), "listed": int(out[1]), "violations": int(out[2])}
+
+
 def pairwise_dist(X: torch.Tensor, centers) -> torch.Tensor:
     """(n,m) fp64 Euclidean distances of every row to X[centers] with the library's canonical
     fp64 arithmetic (sklearn order: sqrt(max(0, -2 x.c + |x|^2 + |c|^2)))."""
