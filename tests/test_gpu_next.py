@@ -234,7 +234,7 @@ def test_peak_uncertainties_match_oracle(built_lib, kind):
 
 
 def test_peak_fast_path_equals_generic(built_lib, monkeypatch):
-    """The 64 x 48 paths (register / shuffle: the default; shared-memory staged) against the generic routine (bit-equal), on smooth maps, noise maps, tied
+    """The 64 x 48 register / shuffle kernel against the generic routine (bit-equal), on smooth maps, noise maps, tied
     peaks and plateau maps whose candidate list overflows (redone by the generic routine on a list)."""
     v = built_lib
     rng = np.random.default_rng(21)
@@ -265,10 +265,6 @@ def test_peak_fast_path_equals_generic(built_lib, monkeypatch):
     gen = v.ops.peak_uncertainty(Hd)
     monkeypatch.delenv("VATLQ_PEAK_GENERIC")
     assert torch.equal(fast[0], gen[0]) and torch.equal(fast[1], gen[1])
-    monkeypatch.setenv("VATLQ_PEAK_SMEM", "1")         # the shared-memory-staged 64 x 48 variant
-    staged = v.ops.peak_uncertainty(Hd)
-    monkeypatch.delenv("VATLQ_PEAK_SMEM")
-    assert torch.equal(staged[0], gen[0]) and torch.equal(staged[1], gen[1])
     from oracle import vatl_oracle as O
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")

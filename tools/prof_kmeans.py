@@ -1,7 +1,7 @@
 """Short driver for ncu captures of the K-Means filter kernels and the MPE / Margin fast path:
-    ncu --set full --clock-control none --import-source on -k regex:'km_gemm_kernel|peak_unc_fast_kernel' -c 8 \
+    ncu --set full --clock-control none --import-source on -k regex:'km_gemm_kernel|peak_unc_reg_kernel' -c 8 \
         -o gpurun_out/prof_kmeans python tools/prof_kmeans.py
-Launch order: 3 x peak_unc_fast_kernel, 12 seeding distance GEMMs (km_gemm_kernel<128,16,..,1>), 3 assignment GEMMs
+Launch order: 3 x peak_unc_reg_kernel, 12 seeding distance GEMMs (km_gemm_kernel<128,16,..,1>), 3 assignment GEMMs
 (km_gemm_kernel<64,64,2,2,0>)."""
 import ctypes as C
 import os

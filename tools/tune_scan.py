@@ -21,5 +21,5 @@ for frames in [int(x) for x in os.environ.get("SCAN_FRAMES", "60000,1080").split
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / reps
-    print(f"scan[{os.environ.get('VATLQ_SCAN', 'tma')}] frames={frames} {ms:.3f} ms  {frames * 208896 / ms / 1e6:.0f} GB/s")
+    print(f"scan frames={frames} {ms:.3f} ms  {frames * 208896 / ms / 1e6:.0f} GB/s")
     del H

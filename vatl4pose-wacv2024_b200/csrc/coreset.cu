@@ -201,10 +201,6 @@ constexpr int kSeg = 8;
 #define VQ_DEPTH 8
 #endif
 constexpr int kDepth = VQ_DEPTH;     // super-steps of x in flight per lane (register ring)
-#ifndef VQ_PREFETCH
-#define VQ_PREFETCH 0
-#endif
-constexpr int kPrefetch = VQ_PREFETCH;  // super-steps the L2 prefetch cursor runs ahead of the ring
 
 __device__ __forceinline__ void dmma(double (&c)[2], double a, double b) {
   asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
@@ -570,22 +566,6 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
     long long lt = t0;                 // load cursor
     int ls = 0;
     const float4* lp = (nt > 0) ? row_ptr(lt) : X4;
-    // a third cursor runs kPrefetch steps ahead of the loads and only touches L2
-    // (prefetch.global.L2): DRAM latency is hidden without holding registers
-    long long qt = t0;
-    int qs = 0;
-    const float4* qp = lp;
-    auto l2_prefetch = [&]() {
-      if (kPrefetch > 0 && qt < ntiles) {
-        if (kk == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(qp + 4 * qs));
-        if (++qs == mylen) {
-          qs = 0;
-          qt += tstride;
-          if (qt < ntiles) qp = row_ptr(qt);
-        }
-      }
-    };
-    for (int p = 0; p < kPrefetch; ++p) l2_prefetch();
     float4 ring[kDepth];
 #pragma unroll
     for (int p = 0; p < kDepth; ++p) {
@@ -607,7 +587,6 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
           const double2 b01 = *reinterpret_cast<const double2*>(bptr + 16 * cs);
           const double2 b23 = *reinterpret_cast<const double2*>(bptr + 16 * cs + 2);
           const double x0 = (double)ring[p].x, x1 = (double)ring[p].y, x2 = (double)ring[p].z, x3 = (double)ring[p].w;
-          l2_prefetch();
           if (f + kDepth < F) {          // refill the slot that was just consumed
             ring[p] = load_x<GUARD>(lp, 4 * ls, a.d4 - 4 * seg_beg - kk);
             if (++ls == mylen) {
@@ -2304,8 +2283,6 @@ static int pair_grid() {
   static int grid = -1;
   if (grid < 0) {
     grid = 0;
-    if (const char* e = getenv("VATLQ_PAIR"))
-      if (!strcmp(e, "0") || !strcmp(e, "off")) return grid;
     if (configure_pass() != 0) return grid;   // (the occupancy query needs the opt-in shared-memory size)
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3((unsigned)(sm_count() & ~1));
@@ -2327,15 +2304,6 @@ static int pair_grid() {
 
 // the paired pass of a 16-pick round (d = 2048 only): applies picks [0, nb) when nb > 8, reading X once
 // (filter = true: the same tile machine over the segment anchors, writing both centre groups' skip flags)
-// VATLQ_PDL=0: plain stream-ordered launches (measurement switch)
-static bool pdl_on() {
-  static const bool on = []() {
-    const char* e = getenv("VATLQ_PDL");
-    return !(e && (!strcmp(e, "0") || !strcmp(e, "off")));
-  }();
-  return on;
-}
-
 static int launch_pass_pair(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr,
                             bool filter = false, bool pdl = false) {
   if (int e = configure_pass()) return e;
@@ -2351,7 +2319,7 @@ static int launch_pass_pair(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = 
   at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = (pdl && pdl_on()) ? 2 : 1;
+  cfg.numAttrs = pdl ? 2 : 1;
   if (ev0) cudaEventRecord(ev0, stream);
   if (filter) VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, true, true>, a));
   else VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, true, false>, a));
@@ -2364,19 +2332,7 @@ static int launch_pass(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = nullp
   if (int e = configure_pass()) return e;
   if (ev0) cudaEventRecord(ev0, stream);
   const bool fast = a.d4 == kSeg * 4 * 16 && a.dots != nullptr;   // d = 2048
-  if (fast && pdl && pdl_on()) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)sm_count());
-    cfg.blockDim = dim3(kWsThreads);
-    cfg.dynamicSmemBytes = kWsSmem;
-    cfg.stream = stream;
-    cudaLaunchAttribute at{};
-    at.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at.val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = &at;
-    cfg.numAttrs = 1;
-    VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, false, false>, a));
-  } else if (fast) pass_kernel_tma<16, false><<<sm_count(), kWsThreads, kWsSmem, stream>>>(a);
+  if (fast) VQ_CUDA(launch_pdl(pass_kernel_tma<16, false>, dim3(sm_count()), dim3(kWsThreads), kWsSmem, stream, pdl, a));
   else if ((a.d4 & 3) != 0) pass_kernel_generic<true><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
   else pass_kernel_generic<false><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
   if (ev1) cudaEventRecord(ev1, stream);
@@ -2579,11 +2535,6 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
   const size_t pairs_smem = G.smem;
   const bool fast_d = (G.d4 == kSeg * 4 * 16);   // d = 2048: register-resident centres
   const bool use_pair = fast_d && nbk > kB && pair_grid() >= 2;   // 16 picks per round in one read of X
-  static const long long tma_filter_min = []() {
-    const char* e = getenv("VATLQ_TMA_FILTER_MIN_ROWS");
-    return e ? atoll(e) : 0LL;
-  }();
-  const bool tma_filter = (row_hi - row_lo) >= tma_filter_min;
   // the TF32 screen of the paired pass (see "the screen" at pass_kernel_tma): 0 off, 1 on, 2 verify
   static const int screen_env = []() {
     const char* e = getenv("VATLQ_PASS_SCREEN");
@@ -2592,7 +2543,6 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
     return !strcmp(e, "verify") ? 2 : 1;
   }();
   const int screen_mode = g_screen_mode_set >= 0 ? g_screen_mode_set : screen_env;
-  static const size_t plan_smem = getenv("VATLQ_PLAN_SMEM") ? (size_t)atoi(getenv("VATLQ_PLAN_SMEM")) * 1024 : (size_t)kPlanSmem;   // 0: L2 path
   static bool pairs_cfg = false;
   if (!pairs_cfg) {
     // the same shared-memory carve-out as the pass kernels on either side of it: no SM reconfiguration between them
@@ -2666,18 +2616,9 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
       if (nbk > 1) {
         dim3 pg(kCap / kB, 4);
         if (fast_d) {
-          cudaLaunchConfig_t cfg{};
-          cfg.gridDim = dim3((unsigned)sm_count(), 1);
-          cfg.blockDim = dim3(kSeg * 32);
-          cfg.dynamicSmemBytes = plan_smem;
-          cfg.stream = stream;
-          cudaLaunchAttribute at{};
-          at.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-          at.val.programmaticStreamSerializationAllowed = 1;
-          cfg.attrs = &at;
-          cfg.numAttrs = pdl_on() ? 1 : 0;
-          const cudaError_t le = cudaLaunchKernelEx(&cfg, pairs_plan_kernel<16>, X, G.d4, (const double*)xx, blocks, send, hist,
-                                                    (long long*)out_idx, ctl, Dcc, mail, (unsigned long long)(seq0 + round_no), (int)(plan_smem / 8));
+          const cudaError_t le = launch_pdl(pairs_plan_kernel<16>, dim3(sm_count()), dim3(kSeg * 32), kPlanSmem, stream, true, X, G.d4,
+                                            (const double*)xx, blocks, send, hist, (long long*)out_idx, ctl, Dcc, mail,
+                                            (unsigned long long)(seq0 + round_no), kPlanSmem / 8);
           if (le != cudaSuccess) {
             snprintf(g_err, sizeof(g_err), "pairs_plan launch failed: %s", cudaGetErrorString(le));
             rc = (int)le;
@@ -2698,7 +2639,7 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
       if (prune_mode) {   // flags of every centre group of the round in one launch
         PassArgs a{};
         fill_pass(a);
-        if (use_pair && tma_filter) {   // the pass's own TMA / DMMA tile machine over the anchor rows (bandwidth-bound)
+        if (use_pair) {   // the pass's own TMA / DMMA tile machine over the anchor rows (bandwidth-bound)
           a.seg_start = P.seg_start; a.seg_r = P.seg_r; a.nseg = &P.pc->nseg; a.seg_skip_out = P.seg_skip;
           a.skip_stride = P.skip_stride;
           rc = launch_pass_pair(a, stream, nullptr, nullptr, true, true);

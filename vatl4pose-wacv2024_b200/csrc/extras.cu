@@ -228,20 +228,14 @@ peak_unc_redo_kernel(const T* __restrict__ H, const unsigned int* __restrict__ r
 
 // ---- 64 x 48 fast path.  The generic kernel above spends ~10 k instructions per lane and map on the two 11-tap
 // window passes (22 shared loads + clamps per pixel) and on five full-map scans for the peaks.  Here:
-//   * the map sits in shared memory with 5 replicated columns on each side (row stride 59: conflict-free when the
-//     lanes walk different rows), the row maxima with 5 replicated rows above and below (row stride 49);
-//   * a lane takes whole rows (then whole columns) into REGISTERS and gets the 11-wide maxima by doubling
-//     (w2 = max(p[i], p[i+1]), w4, w8, out[x] = max(w8[x], w8[x+3])): 4 max ops per element, no clamps;
+//   * a lane takes whole rows into REGISTERS and gets their 11-wide maxima by doubling
+//     (w2 = max(p[i], p[i+1]), w4, w8, out[x] = max(w8[x], w8[x+3])): 4 max ops per element, no clamps; the
+//     11-tall column maxima come from the neighbouring lanes' row maxima by shuffles;
 //   * mask pixels (a few dozen per map) are appended to a candidate list; the five rounds of "best remaining
 //     peak + Chebyshev-< 5 suppression" run on the list.  A list overflow (large plateaus) is flagged and the map
 //     is redone by the generic kernel.
 constexpr int kPfW = 48, kPfH = 64, kPfPad = kPeakMinDist;
-constexpr int kPfPS = kPfW + 2 * kPfPad + 1;            // 59: padded image row stride
-constexpr int kPfRS = kPfW + 1;                         // 49: row-maxima row stride
-constexpr int kPfRows = kPfH + 2 * kPfPad;              // 74 rows of row maxima
 constexpr int kPfCand = 256;
-constexpr int kPfWarps = 7;
-constexpr size_t kPfSmemWarp = (size_t)(kPfH * kPfPS + kPfRows * kPfRS) * 4 + kPfCand * 8 + 16;
 
 template <int N>
 __device__ __forceinline__ void window11(float (&p)[N]) {   // p[i] <- max(p[i .. i+10]) for i < N - 10, in place
@@ -299,107 +293,13 @@ __device__ __forceinline__ void peak_select(const float* cval, const int* cidx, 
   if (lane == 0) peak_scores(peaks, npk, mpe_out, margin_out);
 }
 
-__global__ void __launch_bounds__(kPfWarps * 32, 1)
-peak_unc_fast_kernel(const float* __restrict__ H, long long maps, float* __restrict__ mpe_map, float* __restrict__ margin_map,
-                     unsigned int* __restrict__ redo_count, int* __restrict__ redo_list) {
-  extern __shared__ __align__(16) unsigned char pf_smem[];
-  const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
-  const long long mi = (long long)blockIdx.x * kPfWarps + wp;
-  if (mi >= maps) return;
-  float* P = reinterpret_cast<float*>(pf_smem + (size_t)wp * kPfSmemWarp);     // [64][59]
-  float* R = P + kPfH * kPfPS;                                                  // [74][49]
-  float* cval = R + kPfRows * kPfRS;                                            // [256]
-  int* cidx = reinterpret_cast<int*>(cval + kPfCand);                           // [256]
-  int* ccount = cidx + kPfCand;
-  const float4* src = reinterpret_cast<const float4*>(H + (size_t)mi * (kPfH * kPfW));
-  float vmin = INFINITY;
-  if (lane == 0) *ccount = 0;
-#pragma unroll 4
-  for (int i = lane; i < kPfH * kPfW / 4; i += 32) {       // 12 float4 per row
-    const float4 v = ldg_stream(src + i);
-    const int y = i / 12, x = (i - y * 12) * 4;
-    float* d = P + y * kPfPS + kPfPad + x;
-    d[0] = v.x; d[1] = v.y; d[2] = v.z; d[3] = v.w;
-    vmin = fminf(vmin, fminf(fminf(v.x, v.y), fminf(v.z, v.w)));
-  }
-#pragma unroll
-  for (int o = 16; o; o >>= 1) vmin = fminf(vmin, __shfl_xor_sync(0xffffffffu, vmin, o));
-  __syncwarp();
-  // row pass: lane takes rows lane and lane + 32 into registers (edge columns replicated)
-#pragma unroll 1
-  for (int rr = 0; rr < 2; ++rr) {
-    const int y = lane + 32 * rr;
-    float p[kPfW + 2 * kPfPad];
-    const float* row = P + y * kPfPS;
-#pragma unroll
-    for (int i = 0; i < kPfW; ++i) p[kPfPad + i] = row[kPfPad + i];
-#pragma unroll
-    for (int i = 0; i < kPfPad; ++i) {
-      p[i] = p[kPfPad];
-      p[kPfPad + kPfW + i] = p[kPfPad + kPfW - 1];
-    }
-    window11(p);
-    float* out = R + (y + kPfPad) * kPfRS;
-#pragma unroll
-    for (int x = 0; x < kPfW; ++x) out[x] = p[x];
-    if (y == 0) {
-#pragma unroll 1
-      for (int e = 0; e < kPfPad; ++e)
-#pragma unroll
-        for (int x = 0; x < kPfW; ++x) R[e * kPfRS + x] = p[x];
-    }
-    if (y == kPfH - 1) {
-#pragma unroll 1
-      for (int e = 0; e < kPfPad; ++e)
-#pragma unroll
-        for (int x = 0; x < kPfW; ++x) R[(kPfH + kPfPad + e) * kPfRS + x] = p[x];
-    }
-  }
-  __syncwarp();
-  // column pass: lane takes columns lane and lane + 32 (< 48); mask and candidates
-  int n_eq = 0;
-#pragma unroll 1
-  for (int cc = 0; cc < 2; ++cc) {
-    const int x = lane + 32 * cc;
-    if (x < kPfW) {
-      float c[kPfRows];
-#pragma unroll
-      for (int i = 0; i < kPfRows; ++i) c[i] = R[i * kPfRS + x];
-      window11(c);
-      const bool xin = x >= kPfPad && x < kPfW - kPfPad;
-#pragma unroll
-      for (int y = 0; y < kPfH; ++y) {
-        const float v = P[y * kPfPS + kPfPad + x];
-        const bool eq = v == c[y];
-        n_eq += eq ? 1 : 0;
-        if (eq && xin && y >= kPfPad && y < kPfH - kPfPad && v > vmin) {
-          const int pos = atomicAdd(ccount, 1);
-          if (pos < kPfCand) {
-            cval[pos] = v;
-            cidx[pos] = y * kPfW + x;
-          }
-        }
-      }
-    }
-  }
-  n_eq = warp_sum(n_eq);
-  __syncwarp();
-  int ncand = *ccount;
-  if (n_eq == kPfH * kPfW) ncand = 0;                       // trivial image: no peak at all
-  if (ncand > kPfCand) {                                     // large plateaus: the generic kernel redoes this map
-    if (lane == 0) redo_list[atomicAdd(redo_count, 1u)] = (int)mi;
-    return;
-  }
-  peak_select(cval, cidx, ncand, lane, mpe_map + mi, margin_map + mi);
-}
-
-// ---- 64 x 48 register path (the default).  No staging of the map at all: lane l reads rows 2l and 2l+1 straight from
+// The 64 x 48 kernel.  No staging of the map at all: lane l reads rows 2l and 2l+1 straight from
 // global memory (96 contiguous floats), gets their 11-wide row maxima by doubling in registers, and the 11-tall column
 // maxima from its neighbours' row maxima with six shuffles per column: rows 2l-4 .. 2l+5 are the row pairs of lanes
 // l-2 .. l+2 (pair maximum m), row 2l-5 is the second row of lane l-3, row 2l+6 the first row of lane l+3.  Source
 // lanes are clamped to 0 .. 31: a clamped lane only repeats rows that are inside the window already, which is exactly
 // what edge replication does to a maximum.  The originals are read a second time (L1 / L2) for the mask test.
-// Shared memory: the candidate list only -> occupancy is set by registers (12 warps per SM instead of 7).
+// Shared memory: the candidate list only -> occupancy is set by registers (12 warps per SM).
 // T: fp32, or a 16-bit type read as 8-byte quads (same rows per lane) and converted exactly in registers.
 constexpr int kPrWarps = 4;
 template <typename T>
@@ -629,8 +529,6 @@ static int launch_peak_unc(const T* H, int64_t n, int J, int h, int w, float* mp
     VQ_CUDA(cudaFuncSetAttribute((peak_unc_kernel<64, 48, T>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     VQ_CUDA(cudaFuncSetAttribute(peak_unc_redo_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)((size_t)kPeakWarps * 2 * kPfH * kPfW * sizeof(float))));
-    if (std::is_same<T, float>::value)
-      VQ_CUDA(cudaFuncSetAttribute(peak_unc_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kPfWarps * kPfSmemWarp)));
     configured = smem;
   }
   float* mm = (float*)ws;
@@ -639,14 +537,8 @@ static int launch_peak_unc(const T* H, int64_t n, int J, int h, int w, float* mp
     unsigned int* redo_count = (unsigned int*)((char*)ws + (size_t)maps * 8);
     int* redo_list = (int*)((char*)ws + (size_t)maps * 8 + 16);
     VQ_CUDA(cudaMemsetAsync(redo_count, 0, 16, stream));
-    // the shared-memory-staged variant (measurement switch) is fp32 only: 16-bit maps take the register kernel
-    // whatever VATLQ_PEAK_SMEM says
-    if (std::is_same<T, float>::value && getenv("VATLQ_PEAK_SMEM") != nullptr)
-      peak_unc_fast_kernel<<<(unsigned)((maps + kPfWarps - 1) / kPfWarps), kPfWarps * 32, kPfWarps * kPfSmemWarp, stream>>>(
-          (const float*)H, maps, mm, mm + maps, redo_count, redo_list);
-    else
-      peak_unc_reg_kernel<T><<<(unsigned)((maps + kPrWarps - 1) / kPrWarps), kPrWarps * 32, 0, stream>>>(H, maps, mm, mm + maps,
-                                                                                                  redo_count, redo_list);
+    peak_unc_reg_kernel<T><<<(unsigned)((maps + kPrWarps - 1) / kPrWarps), kPrWarps * 32, 0, stream>>>(H, maps, mm, mm + maps,
+                                                                                                redo_count, redo_list);
     VQ_LAUNCHED();
     const unsigned rgrid = (unsigned)std::min<long long>((maps + kPeakWarps - 1) / kPeakWarps, (long long)sm_count() * 4);
     peak_unc_redo_kernel<T><<<rgrid, kPeakWarps * 32, (size_t)kPeakWarps * 2 * kPfH * kPfW * sizeof(float), stream>>>(

@@ -25,8 +25,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
-#include <cstring>
 
 #include "common.cuh"
 
@@ -823,35 +821,31 @@ extern "C" int vatlq_kmeans_pp(const float* X, int64_t n, int d, const double* w
   g.X = X; g.n = n; g.d = d; g.C = Cbuf; g.m = bn; g.cn = cc; g.xx = xx; g.out = D;
   km_pp_seed_kernel<<<1, 1, 0, stream>>>(st, (int)first_center);
   VQ_LAUNCHED();
-  static const bool pdl = []() {
-    const char* e = getenv("VATLQ_PDL");
-    return !(e && (!strcmp(e, "0") || !strcmp(e, "off")));
-  }();
   for (int64_t c = 0; c < k; ++c) {
     const int tr = c == 0 ? 1 : trials;       // step 0: the first centre alone (closest = its distances)
     // (with rand_vals == NULL the state's seed row is used and no block writes the state).  Every kernel of the chain
     // is a programmatic dependent of the one before it (pdl_enter() at kernel entry keeps the data flow in stream order)
-    VQ_CUDA(launch_pdl(km_candidates_kernel, dim3(bn), dim3(256), 0, stream, pdl && c > 0, X, d, (long long)n, (const double*)cum,
+    VQ_CUDA(launch_pdl(km_candidates_kernel, dim3(bn), dim3(256), 0, stream, c > 0, X, d, (long long)n, (const double*)cum,
                        c == 0 ? (const double*)nullptr : rand_vals + (size_t)(c - 1) * trials, st, tr, (const double*)xx, Cbuf, cc));
-    rc = narrow ? launch_gemm<128, 8, 4, 1, 1>(g, stream, pdl) : launch_gemm<128, 16, 4, 1, 1>(g, stream, pdl);
+    rc = narrow ? launch_gemm<128, 8, 4, 1, 1>(g, stream, true) : launch_gemm<128, 16, 4, 1, 1>(g, stream, true);
     if (rc) return rc;
     if (narrow)
-      VQ_CUDA(launch_pdl(km_pot_partial_kernel<8>, dim3(pot_blocks), dim3(256), 0, stream, pdl, (const double*)D, (const double*)closest, w,
+      VQ_CUDA(launch_pdl(km_pot_partial_kernel<8>, dim3(pot_blocks), dim3(256), 0, stream, true, (const double*)D, (const double*)closest, w,
                          (long long)n, part));
     else
-      VQ_CUDA(launch_pdl(km_pot_partial_kernel<16>, dim3(pot_blocks), dim3(256), 0, stream, pdl, (const double*)D, (const double*)closest, w,
+      VQ_CUDA(launch_pdl(km_pot_partial_kernel<16>, dim3(pot_blocks), dim3(256), 0, stream, true, (const double*)D, (const double*)closest, w,
                          (long long)n, part));
-    VQ_CUDA(launch_pdl(km_pot_final_kernel, dim3(1), dim3(512), 0, stream, pdl, (const double*)part, pot_blocks, tr, st, center_ids, (int)c));
+    VQ_CUDA(launch_pdl(km_pot_final_kernel, dim3(1), dim3(512), 0, stream, true, (const double*)part, pot_blocks, tr, st, center_ids, (int)c));
     if (narrow)
-      VQ_CUDA(launch_pdl(km_commit_tiles_kernel<8>, dim3(tiles), dim3(256), 0, stream, pdl, (const double*)D, (const PpState*)st, w, (long long)n,
+      VQ_CUDA(launch_pdl(km_commit_tiles_kernel<8>, dim3(tiles), dim3(256), 0, stream, true, (const double*)D, (const PpState*)st, w, (long long)n,
                          closest, wc, tile_off));
     else
-      VQ_CUDA(launch_pdl(km_commit_tiles_kernel<16>, dim3(tiles), dim3(256), 0, stream, pdl, (const double*)D, (const PpState*)st, w, (long long)n,
+      VQ_CUDA(launch_pdl(km_commit_tiles_kernel<16>, dim3(tiles), dim3(256), 0, stream, true, (const double*)D, (const PpState*)st, w, (long long)n,
                          closest, wc, tile_off));
     g_launches.fetch_add(4);
     if (c + 1 < k) {
-      VQ_CUDA(launch_pdl(km_scan_offsets_kernel, dim3(1), dim3(256), 0, stream, pdl, tile_off, tiles));
-      VQ_CUDA(launch_pdl(km_scan_apply_kernel, dim3(tiles), dim3(256), 0, stream, pdl, (const double*)wc, (long long)n, (const double*)tile_off, cum));
+      VQ_CUDA(launch_pdl(km_scan_offsets_kernel, dim3(1), dim3(256), 0, stream, true, tile_off, tiles));
+      VQ_CUDA(launch_pdl(km_scan_apply_kernel, dim3(tiles), dim3(256), 0, stream, true, (const double*)wc, (long long)n, (const double*)tile_off, cum));
       g_launches.fetch_add(2);
     }
   }

@@ -4,7 +4,6 @@
 //   * Influence / Diversity: row sums of the cosine-distance matrix (ActiveLearning.py:467-483,581-590)
 //   * the uncertainty / representativeness blend                   (ActiveLearning.py:517-521)
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -184,71 +183,6 @@ entropy_kernel(const T* __restrict__ H, int64_t maps, int npx, float* __restrict
     e = (float)warp_sum(ea);
   }
   if (lane == 0) per_map[mi] = e;
-}
-
-// The same arithmetic with the scan's staging (heatmap_scan.cu): one warp walks a run of consecutive 64x48 maps, each
-// map fetched by ONE 12 288-byte cp.async.bulk (TMA, UBLKCP) into the warp's own two-stage shared-memory ring, so the
-// next map is in flight while this one is summed and turned into entr() — no occupancy-bound register staging.
-constexpr int kEntWarps = 8, kEntStages = 2, kEntNV = 24, kEntPix = kEntNV * 128;
-constexpr size_t kEntSmem = (size_t)kEntWarps * kEntStages * kEntPix * 4 + (size_t)kEntWarps * kEntStages * 8;
-__global__ void __launch_bounds__(kEntWarps * 32, 1)
-entropy_tma_kernel(const float* __restrict__ H, int64_t maps, int run_len, float* __restrict__ per_map) {
-  extern __shared__ __align__(128) unsigned char ent_smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int64_t a = ((int64_t)blockIdx.x * kEntWarps + warp) * run_len;
-  if (a >= maps) return;
-  const int64_t count = min((int64_t)run_len, maps - a);
-  float* stage0 = reinterpret_cast<float*>(ent_smem) + (size_t)warp * kEntStages * kEntPix;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(ent_smem + (size_t)kEntWarps * kEntStages * kEntPix * 4) + warp * kEntStages;
-  if (lane == 0) {
-    for (int st = 0; st < kEntStages; ++st) mbar_init(&bars[st], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    for (int st = 0; st < kEntStages && st < count; ++st) {
-      mbar_expect_tx(&bars[st], kEntPix * 4);
-      tma_load_1d(stage0 + (size_t)st * kEntPix, H + (size_t)(a + st) * kEntPix, kEntPix * 4, &bars[st]);
-    }
-  }
-  __syncwarp();
-  for (int64_t i = 0; i < count; ++i) {
-    const int st = (int)(i % kEntStages);
-    mbar_wait(&bars[st], (uint32_t)((i / kEntStages) & 1));
-    const float4* m4 = reinterpret_cast<const float4*>(stage0 + (size_t)st * kEntPix);
-    float4 v[kEntNV];
-#pragma unroll
-    for (int q = 0; q < kEntNV; ++q) v[q] = m4[q * 32 + lane];
-    // the stage is free as soon as the map sits in registers: refill it now (maximum lead time)
-    __syncwarp();
-    if (lane == 0 && i + kEntStages < count) {
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      mbar_expect_tx(&bars[st], kEntPix * 4);
-      tma_load_1d(stage0 + (size_t)st * kEntPix, H + (size_t)(a + i + kEntStages) * kEntPix, kEntPix * 4, &bars[st]);
-    }
-    double acc = 0.0;
-    float sm = 0.f;
-#pragma unroll
-    for (int q = 0; q < kEntNV; ++q) {       // (identical order to entropy_kernel<24, float>: same bits)
-      sm += (v[q].x + v[q].y) + (v[q].z + v[q].w);
-      if ((q & 3) == 3) {
-        acc += (double)sm;
-        sm = 0.f;
-      }
-    }
-    acc += (double)sm;
-    const float S = (float)warp_sum(acc);
-    const float rS = __frcp_rn(S);
-    const bool mul = fabsf(rS) > 1e-30f && fabsf(rS) < 1e30f;
-    double ea = 0.0;
-#pragma unroll
-    for (int q = 0; q < kEntNV; ++q) {
-      float4 p;
-      if (mul) p = make_float4(v[q].x * rS, v[q].y * rS, v[q].z * rS, v[q].w * rS);
-      else p = make_float4(__fdiv_rn(v[q].x, S), __fdiv_rn(v[q].y, S), __fdiv_rn(v[q].z, S), __fdiv_rn(v[q].w, S));
-      const float e4 = (entr_f32(p.x) + entr_f32(p.y)) + (entr_f32(p.z) + entr_f32(p.w));
-      ea += (double)e4;
-    }
-    const float e = (float)warp_sum(ea);
-    if (lane == 0) per_map[a + i] = e;
-  }
 }
 
 // entropy_value += entropy(heatmap) over the joints, in joint order (:793-795)
@@ -490,45 +424,16 @@ extern "C" int vatlq_heatmap_entropy_dt(const void* H_, int dtype, int64_t n, in
   VQ_REQUIRE((maps + 7) / 8 <= 2147483647LL, "grid too large");
   const int npx = h * w;
   const unsigned grid = (unsigned)((maps + 7) / 8);
-  if (dtype != VATLQ_F32) {
-    // the TMA variant below is fp32 only: 16-bit maps take the register-staged kernel whatever VATLQ_ENTROPY_TMA says
-    VQ_REQUIRE(npx != 24 * 128 || quad_aligned(H_, dtype), "16-bit H must be 8-byte aligned");
-    const int rc = with_dtype(dtype, [&](auto tag) {
-      using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
-      if (npx == 24 * 128) entropy_kernel<24, T><<<grid, 256, 0, stream>>>((const T*)H_, maps, npx, (float*)ws);
-      else entropy_kernel<0, T><<<grid, 256, 0, stream>>>((const T*)H_, maps, npx, (float*)ws);
-      VQ_LAUNCHED();
-      return 0;
-    });
-    if (rc != 0) return rc;
-    entropy_frames_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>((const float*)ws, n, J, entropy);
+  // fp32 falls back to the generic kernel for a map not 16-byte aligned; 16-bit maps must be 8-byte aligned
+  VQ_REQUIRE(dtype == VATLQ_F32 || npx != 24 * 128 || quad_aligned(H_, dtype), "16-bit H must be 8-byte aligned");
+  const int rc = with_dtype(dtype, [&](auto tag) {
+    using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+    if (npx == 24 * 128 && quad_aligned(H_, dtype)) entropy_kernel<24, T><<<grid, 256, 0, stream>>>((const T*)H_, maps, npx, (float*)ws);
+    else entropy_kernel<0, T><<<grid, 256, 0, stream>>>((const T*)H_, maps, npx, (float*)ws);
     VQ_LAUNCHED();
     return 0;
-  }
-  const float* H = (const float*)H_;
-  // Measured on B200 (tools/time_next_rows.py, 40 000 frames): the TMA-staged variant runs at 2.5 TB/s, the
-  // register-staged one at 3.9 TB/s — the kernel is bound by the ~1.4 k instructions per lane and map (MUFU.LG2 chain),
-  // and 8 warps per SM (196 KB of stages) hide less of that than 16 resident warps do.  Kept for experiments only.
-  static const bool use_tma = []() {
-    const char* e = getenv("VATLQ_ENTROPY_TMA");
-    return e && e[0] == '1';
-  }();
-  if (npx == kEntPix && ((uintptr_t)H & 15) == 0 && use_tma && maps >= 4096) {
-    static bool cfg = false;
-    if (!cfg) {
-      VQ_CUDA(cudaFuncSetAttribute(entropy_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEntSmem));
-      cfg = true;
-    }
-    // runs long enough to amortise the ring fill, short enough for ~4 waves of warps over the SMs
-    const int64_t warps = (int64_t)sm_count() * kEntWarps * 4;
-    const int run_len = (int)std::max<int64_t>(4, std::min<int64_t>(64, (maps + warps - 1) / warps));
-    const int64_t tasks = (maps + run_len - 1) / run_len;
-    entropy_tma_kernel<<<(unsigned)((tasks + kEntWarps - 1) / kEntWarps), kEntWarps * 32, kEntSmem, stream>>>(H, maps, run_len, (float*)ws);
-  } else if (npx == 24 * 128 && ((uintptr_t)H & 15) == 0)
-    entropy_kernel<24, float><<<grid, 256, 0, stream>>>(H, maps, npx, (float*)ws);
-  else
-    entropy_kernel<0, float><<<grid, 256, 0, stream>>>(H, maps, npx, (float*)ws);
-  VQ_LAUNCHED();
+  });
+  if (rc != 0) return rc;
   entropy_frames_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>((const float*)ws, n, J, entropy);
   VQ_LAUNCHED();
   return 0;

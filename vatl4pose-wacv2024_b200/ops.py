@@ -7,7 +7,6 @@ falls back: a missing library or a non-CUDA tensor raises.
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass
 
 import numpy as np
@@ -286,7 +285,7 @@ def coreset_select(X: torch.Tensor, unc: torch.Tensor, labeled, k: int, moks: fl
     out = torch.empty(max(k, 1), dtype=torch.int64, device=dev)
     stats = (C.c_int64 * 16)()
     if tc_init is None:    # the labelled-set contraction on the tcgen05 tensor cores when it is large enough to pay
-        tc_init = d == 2048 and lab.numel() >= TC_INIT_MIN_LABELED and hi > lo and os.environ.get("VATLQ_TC_INIT", "1") != "0"
+        tc_init = d == 2048 and lab.numel() >= TC_INIT_MIN_LABELED and hi > lo
     done = False
     if tc_init and lab.numel() > 0:
         done, _, _ = coreset_init_tc(X, lab, min_d, lo, hi)
