@@ -168,6 +168,9 @@ int vatlq_fuse_final(const uint8_t* unlabeled, int64_t n, const double* stats2,
  * tiles / in the planner (summed over the rounds), [11..14] this call's pruning statistics: tiles seen,
  * tiles streamed, verify violations, segments; [15] reserved.
  * ------------------------------------------------------------------------------------ */
+/* The workspace of vatlq_coreset_init / vatlq_coreset_select.  With d == 2048 and batch >= 16 (rounds of 16 picks,
+ * screened in fp16) it includes an fp16 copy of the owned rows, n * 4096 bytes; vatlq_coreset_init does not need
+ * that part. */
 size_t vatlq_coreset_workspace_bytes(int64_t n, int d, int batch);
 int vatlq_coreset_init(const float* X, int64_t n, int d, int64_t row_lo, int64_t row_hi,
                        const int64_t* labeled, int64_t n_labeled,
@@ -208,8 +211,9 @@ int vatlq_coreset_prune_stats(int64_t* host_out4, int reset);
  * 2 verify; min_rows < 0: environment */
 int vatlq_coreset_set_prune(int mode, int64_t min_rows);
 
-/* The TF32 screen of the 16-pick rounds (d == 2048): before a round's fp64 pass each streamed row is
- * compared with the round's centres on the tensor cores, and only the rows that an error bound cannot
+/* The fp16 screen of the 16-pick rounds (d == 2048): before a round's fp64 pass each streamed row is
+ * compared with the round's centres on the tensor cores (an fp16 copy of the owned rows that
+ * vatlq_coreset_select fills in its workspace), and only the rows that an error bound cannot
  * prove unchanged (min_d[i] <= d(i,c) for every centre) go through the exact fp64 arithmetic.  The pick
  * list and min_d are unchanged bit for bit.  Environment: VATLQ_PASS_SCREEN=0 disables,
  * VATLQ_PASS_SCREEN=verify computes every streamed row exactly and counts the rows the screen did not

@@ -359,10 +359,11 @@ struct PassArgs {
   unsigned char* seg_skip_out;       // [2][skip_stride] flags written by the filter mode
   int prune_mode;                    // 0 off, 1 skip, 2 verify (stream everything, count rows that changed anyway)
   unsigned long long* prune_stats;   // [0] tiles seen, [1] tiles streamed, [2] verify violations
-  // paired pass only, see "the screen" at pass_kernel_tma: 0 off, 1 DMMA only the rows the TF32 screen cannot
+  // paired pass only, see "the screen" at pass_kernel_tma: 0 off, 1 DMMA only the rows the fp16 screen cannot
   // decide, 2 verify (DMMA every streamed row, count unlisted rows whose min_d moved anyway)
   int screen_mode;
   unsigned long long* screen_stats;  // [0] rows screened, [1] rows listed, [2] verify violations
+  const __half* Xh;                  // screen_mode != 0: X[lo, hi) as fp16, row r - lo at Xh + (r - lo) * 2048
 };
 
 // centres of THIS pass: count (<= 0: nothing to do) and whether it is the round's last pass
@@ -702,6 +703,10 @@ constexpr int kStagesX = 3;
 constexpr int kPartBufs = 3;
 constexpr int kRowBytesX = 2048 * 4 + 64;                  // stage row stride
 constexpr int kStageBytesX = 8 * kRowBytesX;               // 66 048
+// the screen's stages hold TWO tiles of fp16 rows (16 x 4 KB, the bytes of one fp32 tile).  Row stride = 32 mod 128
+// bytes: the 8-byte loads of rows g = 0..3 (lanes 4g .. 4g+3, 32 contiguous bytes each) hit all 32 banks
+constexpr int kRowBytesH = 2048 * 2 + 32;
+static_assert(16 * kRowBytesH == kStageBytesX, "an fp16 stage of two tiles fills an fp32 stage exactly");
 constexpr int kWsThreads = (kSeg + 4) * 32;                // 8 compute warps + producer + 3 epilogue warps
 constexpr int kMaxTilesCta = 2048;                         // tiles per CTA the pruned-tile list can hold
 constexpr size_t kWsSmem = (size_t)kStagesX * kStageBytesX + sizeof(double) * kPartBufs * kSeg * 64 + 2 * kStagesX * 8 +
@@ -718,6 +723,11 @@ __device__ __forceinline__ void named_arrive(int id, int count) {
 __device__ __forceinline__ float4 lds128(unsigned addr) {
   float4 r;
   asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "r"(addr));
+  return r;
+}
+__device__ __forceinline__ uint2 lds64(unsigned addr) {
+  uint2 r;
+  asm volatile("ld.shared.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "r"(addr));
   return r;
 }
 
@@ -745,28 +755,53 @@ __device__ __forceinline__ unsigned ld_dsmem_u32(const void* p, unsigned rank) {
 // ---- the screen (paired pass, screen_mode != 0) ------------------------------------------------
 // A round only needs to know which rows get closer to one of its <= 16 centres: min_d[i] changes iff
 // d(i,c) < m_old = min_d[i] for some c.  Before the DMMA tile loop each CTA of a pair streams the tiles of ITS
-// parity (the rows it finishes) through the same TMA ring and the compute warps evaluate S~ = x.c for all 16
-// centres with mma.sync m16n8k8 TF32 (A = 16 centres from registers, B = the tile's 8 rows, fp32
-// accumulation; warp w = K segment w as in the DMMA loop).  A row is DECIDED when for every centre
+// parity (the rows it finishes) through the same TMA ring, read from an fp16 copy of the owned rows (PassArgs::Xh,
+// filled once per selection call by half_copy_kernel: half the bytes of the fp32 rows), and the compute warps
+// evaluate S~ = x~.c~ for all 16 centres with mma.sync m16n8k16 f16 (A = 16 centres from registers, read from the
+// fp32 X and rounded the same way, B = a tile's 8 rows, fp32 accumulation; warp w = K segment w as in the DMMA
+// loop).  A row is DECIDED when for every centre
 //     S~ finite  and  fl(t~ - 2E) > m_old^2 rounded up,   t~ = (|x|^2 + |c|^2) - 2 S~,
-//     E = 2u |x||c| + 2^-20 (|x|^2 + |c|^2),  u = 2^-8,
-// with m_old finite and the row not one of the picks.  Proof that a decided row keeps min_d bit for bit: the
-// TF32 operands carry >= 10 mantissa bits and the fp32 accumulation over K = 2048 adds at most 2048 * 2^-23
-// relative to sum |x_k c_k| <= |x||c| (Cauchy-Schwarz), so |S~ - S| <= (2^-9 + 2^-12) |x||c| <= u |x||c| (S: the
-// exact dot of the fp32 features).  The canonical fp64 value t = fl(fl(-2 dot + xx_i) + xx_c) is within
-// 2^-48 (|x|^2 + |c|^2) of |x|^2 + |c|^2 - 2S, so t >= t~ - 2u|x||c| - 2^-48(..) = (t~ - 2E) + 2u|x||c|
-// + 2^-19 (|x|^2 + |c|^2) - 2^-48 (..), which exceeds the computed fl(t~ - 2E) by more than that subtraction's
-// own rounding (and that of |x|, |c|, which enter E only scaled by u): t > m_old^2.  sqrt is correctly rounded and
-// monotone and m_old is a double, so d = sqrt(max(t, 0)) >= m_old and fmin(m_old, d) == m_old: the row's
+//     E = 2u |x||c| + 2^-20 (|x|^2 + |c|^2) + 2^-17 (|x| + |c|),  u = 2^-8,
+// with m_old finite and the row not one of the picks.  Proof that a decided row keeps min_d bit for bit (S: the
+// exact dot of the fp32 features, K = 2048).  cvt.rn to fp16 moves an element v by |dv| <= 2^-11 |v| in the normal
+// range and by |dv| <= 2^-25 in the subnormal range (|v| < 2^-14), so |dv| <= 2^-11 |v| + 2^-25 and, 0 being
+// representable, |dv| <= |v|.  Then x~c~ - xc = dx c + x dc + dx dc with |dx dc| <= (2^-11|x_k| + 2^-25)|dc| <=
+// 2^-22 |x_k c_k| + 2^-36 |x_k| + 2^-25 |c_k|, so the exact dot of the fp16 operands is within
+//     (2^-10 + 2^-22) sum|x_k c_k| + 2^-24 (|x|_1 + |c|_1)
+// of S; with sum|x_k c_k| <= |x||c| (Cauchy-Schwarz) and |v|_1 <= sqrt(2048) |v|_2 this is
+// <= (2^-10 + 2^-22) |x||c| + 2^-18.5 (|x| + |c|).  The products of two fp16 values are exact in fp32, and the fp32
+// accumulation is ASSUMED to add at most 2048 * 2^-23 = 2^-12 relative to sum |x~_k c~_k| (not proven for the
+// tensor core's internal order; the verify mode of tests/test_gpu_pass_screen*.py checks it): in all
+//     |S~ - S| <= (2^-10 + 2^-12 + 2^-20) |x||c| + 2^-18.4 (|x| + |c|) <= u |x||c| + 2^-18 (|x| + |c|).
+// The canonical fp64 value t = fl(fl(-2 dot + xx_i) + xx_c) is within 2^-48 (|x|^2 + |c|^2) of |x|^2 + |c|^2 - 2S,
+// so t >= t~ - 2u|x||c| - 2^-17 (|x| + |c|) - 2^-48(..) = (t~ - 2E) + 2u|x||c| + 2^-19 (|x|^2 + |c|^2)
+// + 2^-17 (|x| + |c|) - 2^-48 (..), which exceeds the computed fl(t~ - 2E) by more than that subtraction's own
+// rounding (and that of |x|, |c|, which enter E only scaled by u or 2^-17): t > m_old^2.  sqrt is correctly rounded
+// and monotone and m_old is a double, so d = sqrt(max(t, 0)) >= m_old and fmin(m_old, d) == m_old: the row's
 // min_d, score and candidate record are exactly what the full pass writes.  Any NaN / Inf makes the test false
-// (the row is listed).  The undecided rows are then gathered 8 per tile (the same per-row TMA copies the
-// producer always issues) and only those go through the canonical DMMA tile machine.
+// (the row is listed); in particular an element with |v| >= 65520 becomes +-Inf in fp16, and S~ is then +-Inf or
+// NaN (Inf x 0), never finite.  The undecided rows are then gathered 8 per tile (the per-row TMA copies of the fp32
+// rows the producer always issues) and only those go through the canonical DMMA tile machine.
 constexpr double kScreenU = 0.00390625;               // 2^-8
 constexpr double kScreenAbs = 9.5367431640625e-07;    // 2^-20
-__device__ __forceinline__ void mma_tf32(float (&d)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
-  asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+constexpr double kScreenAbs1 = 7.62939453125e-06;     // 2^-17
+__device__ __forceinline__ void mma_f16(float (&d)[4], const unsigned (&a)[4], uint2 b) {
+  asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
                : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b.x), "r"(b.y));
+}
+__device__ __forceinline__ unsigned half2_bits(float lo, float hi) {   // cvt.rn.f16x2.f32: lo in the low half
+  const __half2 h = __floats2half2_rn(lo, hi);
+  return *reinterpret_cast<const unsigned*>(&h);
+}
+// the screen's fp16 copy of rows [lo, lo + n4 / 512) of X (d = 2048): one float4 -> four halves per thread and step
+__global__ void __launch_bounds__(256) half_copy_kernel(const float4* __restrict__ X, long long lo, long long n4,
+                                                        uint2* __restrict__ Xh) {
+  const float4* src = X + lo * 512;
+  for (long long q = (long long)blockIdx.x * 256 + threadIdx.x; q < n4; q += (long long)gridDim.x * 256) {
+    const float4 v = ldg_stream(src + q);
+    Xh[q] = make_uint2(half2_bits(v.x, v.y), half2_bits(v.z, v.w));
+  }
 }
 // entry e of the list of undecided rows -> the walker's tile k and row r (s_pre: inclusive prefix of the listed
 // rows per tile, nt entries; s_mask: the listed rows of every tile)
@@ -983,10 +1018,10 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     int st = 0, pb = 0;
     unsigned phase = 0;
     if (screen) {
-      // A operand of mma.m16n8k8: centres g and g + 8 of the round at the features this lane reads of a row (the
-      // k slots of the two MMAs of a super-step are features 16s + 4kk + {0, 1} and {2, 3}: the same permutation
-      // of K for A and B)
-      unsigned af[STEPS][8];
+      // A operand of mma.m16n8k16: centres g and g + 8 of the round at the features this lane reads of a row, as
+      // fp16 (the k slots {2kk, 2kk+1} and {2kk+8, 2kk+9} of super-step s are features 16s + 4kk + {0, 1} and
+      // {2, 3}: the same permutation of K for A and B)
+      unsigned af[STEPS][4];
       {
         const long long* allc = a.centers + a.center_off;
         const long long p0 = allc[min(g, total - 1)], p1 = allc[min(g + kB, total - 1)];
@@ -995,24 +1030,23 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
 #pragma unroll
         for (int s = 0; s < STEPS; ++s) {
           const float4 v0 = __ldg(c0 + 4 * s), v1 = __ldg(c1 + 4 * s);
-          af[s][0] = __float_as_uint(v0.x); af[s][1] = __float_as_uint(v0.y);
-          af[s][2] = __float_as_uint(v0.z); af[s][3] = __float_as_uint(v0.w);
-          af[s][4] = __float_as_uint(v1.x); af[s][5] = __float_as_uint(v1.y);
-          af[s][6] = __float_as_uint(v1.z); af[s][7] = __float_as_uint(v1.w);
+          af[s][0] = half2_bits(v0.x, v0.y);
+          af[s][1] = half2_bits(v1.x, v1.y);
+          af[s][2] = half2_bits(v0.z, v0.w);
+          af[s][3] = half2_bits(v1.z, v1.w);
         }
       }
+      const unsigned h_off = smem_addr(stage0) + g * kRowBytesH + seg * (STEPS * 32) + kk * 8;
       const unsigned my_partf = smem_addr(&s_part[0][seg][0]) + lane * 16;
-      for (int k = 0; k < n1; ++k) {
+      // a stage holds tiles k and k + 1 (rows 0-7, 8-15); with n1 odd the last stage's second half repeats tile k
+      for (int k = 0; k < n1; k += 2) {
         mbar_wait(&full[st], phase);
-        const unsigned ap = a_off + st * kStageBytesX;
-        float d0[4] = {0.f, 0.f, 0.f, 0.f}, d1[4] = {0.f, 0.f, 0.f, 0.f};
+        const unsigned ap = h_off + st * kStageBytesX;
+        float d[2][4] = {{0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
 #pragma unroll
         for (int s = 0; s < STEPS; ++s) {
-          const float4 x = lds128(ap + s * 64);
-          const unsigned A0[4] = {af[s][0], af[s][4], af[s][1], af[s][5]};
-          const unsigned A1[4] = {af[s][2], af[s][6], af[s][3], af[s][7]};
-          mma_tf32(d0, A0, __float_as_uint(x.x), __float_as_uint(x.y));
-          mma_tf32(d1, A1, __float_as_uint(x.z), __float_as_uint(x.w));
+          mma_f16(d[0], af[s], lds64(ap + s * 32));
+          mma_f16(d[1], af[s], lds64(ap + 8 * kRowBytesH + s * 32));
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty[st]);
@@ -1020,14 +1054,17 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
           st = 0;
           phase ^= 1u;
         }
-        if (k >= kPartBufs) named_sync(1 + kPartBufs + pb, kSeg * 32 + 32);
-        // lane (g,kk): centre g at rows 2kk, 2kk+1, centre g+8 at rows 2kk, 2kk+1
-        asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(my_partf + pb * (unsigned)(sizeof(double) * kSeg * 64)),
-                     "f"(d0[0] + d1[0]), "f"(d0[1] + d1[1]), "f"(d0[2] + d1[2]), "f"(d0[3] + d1[3])
-                     : "memory");
-        asm volatile("fence.acq_rel.cta;" ::: "memory");
-        named_arrive(1 + pb, kSeg * 32 + 32);
-        if (++pb == kPartBufs) pb = 0;
+        // one partial buffer per tile, as the epilogue warps expect them
+        for (int h = 0; h < 2 && k + h < n1; ++h) {
+          if (k + h >= kPartBufs) named_sync(1 + kPartBufs + pb, kSeg * 32 + 32);
+          // lane (g,kk): centre g at rows 2kk, 2kk+1, centre g+8 at rows 2kk, 2kk+1
+          asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(my_partf + pb * (unsigned)(sizeof(double) * kSeg * 64)),
+                       "f"(d[h][0]), "f"(d[h][1]), "f"(d[h][2]), "f"(d[h][3])
+                       : "memory");
+          asm volatile("fence.acq_rel.cta;" ::: "memory");
+          named_arrive(1 + pb, kSeg * 32 + 32);
+          if (++pb == kPartBufs) pb = 0;
+        }
       }
       screen_join();
       pb = 0;
@@ -1097,11 +1134,34 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
         }
       };
       if (screen) {
+        // two tiles of this CTA's parity per stage, fp16 rows of 4 KB from the copy: lane r < 16 copies row r & 7 of
+        // the first (r < 8) or second tile; a lone last tile fills both halves
+        auto fill_half = [&](int k0, int k1) {
+          if (fills++ >= kStagesX) mbar_wait(&empty[st], phase ^ 1u);
+          if (lane == 0) mbar_expect_tx(&full[st], 16u * 2048u * 2u);
+          __syncwarp();
+          if (lane < 16) {
+            const int k = lane < 8 ? k0 : k1;
+            const long long row = min(((long long)cid + (long long)k * ncl) * 8 + (lane & 7), a.hi - a.lo - 1);   // relative to a.lo
+            tma_load_1d(stage0 + (size_t)st * kStageBytesX + lane * kRowBytesH, a.Xh + (size_t)row * 2048, 2048u * 2u, &full[st]);
+          }
+          if (++st == kStagesX) {
+            st = 0;
+            phase ^= 1u;
+          }
+        };
+        int held = -1;
         for (int j = 0; j < na; ++j) {
           const int k = tile_of(j);
           if ((k & 1) != crank) continue;
-          fill([&]() { return min(a.lo + ((long long)cid + (long long)k * ncl) * 8 + lane, a.hi - 1); });
+          if (held < 0) {
+            held = k;
+          } else {
+            fill_half(held, k);
+            held = -1;
+          }
         }
+        if (held >= 0) fill_half(held, held);
         screen_join();
       }
       if (screen == 1) {
@@ -1152,7 +1212,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
             const int c = q + 4 * c4;
             const double xs = xxi + s_xxc[c];
             const double t = xs - 2.0 * S[c4];
-            const double E = 2.0 * kScreenU * nx * s_nc[c] + kScreenAbs * xs;
+            const double E = 2.0 * kScreenU * nx * s_nc[c] + kScreenAbs * xs + kScreenAbs1 * (nx + s_nc[c]);
             und = und || !(isfinite(S[c4]) && t - 2.0 * E > m2) || s_pick[c] == i;
           }
           const unsigned ub = __ballot_sync(0xffffffffu, und && valid);
@@ -2177,7 +2237,13 @@ struct Comm {
 struct WsLayout {
   size_t xx, score, hist, partial, send, recv, dcc, ctl, dots, flags, total;
   size_t prune, seg_of_row, seg_start, seg_r, seg_skip, skip_stride;   // pruning state (cd aliases dots during set-up)
+  size_t xh;   // the screen's fp16 copy of the owned rows, n * 4096 bytes from here (beyond `total`: only a
+               // selection whose rounds take the paired pass needs it; sized by n, so a rank of an 8-way shard
+               // uses an eighth of it)
 };
+// rounds of 16 picks, applied by the paired pass (and screened): d == 2048 and batch >= 16 (vatlq_coreset_select
+// rounds batch down to a power of two)
+static bool paired_rounds(int d, int batch) { return d == kSeg * 16 * 16 && batch >= 2 * kB; }
 static WsLayout ws_layout(long long n, int world) {
   WsLayout L;
   size_t o = 0;
@@ -2203,6 +2269,7 @@ static WsLayout ws_layout(long long n, int world) {
   L.seg_skip = take((size_t)n * (kMaxPicks / kB));   // one flag array per centre group of a round
   L.skip_stride = align_up((size_t)n, 256);
   L.total = o;
+  L.xh = o;
   return L;
 }
 
@@ -2227,10 +2294,9 @@ static int g_screen_mode_set = -1;             // vatlq_coreset_set_screen: -1 =
 using namespace vatlq;
 
 extern "C" size_t vatlq_coreset_workspace_bytes(int64_t n, int d, int batch) {
-  (void)d;
-  (void)batch;
   if (n < 0) return 0;
-  return ws_layout(n, kMaxRanks).total;
+  const WsLayout L = ws_layout(n, kMaxRanks);
+  return paired_rounds(d, batch) ? L.xh + (size_t)n * 4096 : L.total;
 }
 
 struct Geom {
@@ -2466,7 +2532,8 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
   VQ_REQUIRE(world >= 1 && world <= kMaxRanks, "world size not supported");
   VQ_REQUIRE(world > 1 || (row_lo == 0 && row_hi == n), "single GPU must own every row");
   const WsLayout L = ws_layout(n, kMaxRanks);
-  VQ_REQUIRE(ws != nullptr && ws_bytes >= L.total, "workspace too small");
+  VQ_REQUIRE(ws != nullptr && ws_bytes >= vatlq_coreset_workspace_bytes(n, d, batch),
+             "workspace too small (vatlq_coreset_workspace_bytes(n, d, batch))");
   if (k == 0) return 0;
   char* w = (char*)ws;
   Ctl* ctl = (Ctl*)(w + L.ctl);
@@ -2534,8 +2601,8 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
   VQ_REQUIRE(fgrid <= 4096 && sm_count() <= 4096, "grid too large for the arg-max scratch");
   const size_t pairs_smem = G.smem;
   const bool fast_d = (G.d4 == kSeg * 4 * 16);   // d = 2048: register-resident centres
-  const bool use_pair = fast_d && nbk > kB && pair_grid() >= 2;   // 16 picks per round in one read of X
-  // the TF32 screen of the paired pass (see "the screen" at pass_kernel_tma): 0 off, 1 on, 2 verify
+  const bool use_pair = paired_rounds(d, batch) && pair_grid() >= 2;   // 16 picks per round in one read of X
+  // the fp16 screen of the paired pass (see "the screen" at pass_kernel_tma): 0 off, 1 on, 2 verify
   static const int screen_env = []() {
     const char* e = getenv("VATLQ_PASS_SCREEN");
     if (!e) return 1;
@@ -2543,6 +2610,12 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
     return !strcmp(e, "verify") ? 2 : 1;
   }();
   const int screen_mode = g_screen_mode_set >= 0 ? g_screen_mode_set : screen_env;
+  // the screen reads the owned rows from their fp16 copy at the end of the workspace, filled once per call
+  const __half* Xh = (use_pair && screen_mode) ? (const __half*)(w + L.xh) : nullptr;
+  if (Xh && row_hi > row_lo) {
+    half_copy_kernel<<<sm_count() * 8, 256, 0, stream>>>((const float4*)X, row_lo, (row_hi - row_lo) * 512, (uint2*)(w + L.xh));
+    VQ_LAUNCHED();
+  }
   static bool pairs_cfg = false;
   if (!pairs_cfg) {
     // the same shared-memory carve-out as the pass kernels on either side of it: no SM reconfiguration between them
@@ -2663,6 +2736,7 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
         a.push = push_of(seq0 + round_no + 1);   // the block this round's (only) pass publishes
         a.screen_mode = screen_mode;
         a.screen_stats = P.pc->screen;
+        a.Xh = Xh;
         rc = timed_launch(a, true);
         if (rc == 0) {
           PassArgs b{};

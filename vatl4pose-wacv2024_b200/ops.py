@@ -324,7 +324,7 @@ SCREEN_MODES = {"env": -1, "off": 0, "on": 1, "verify": 2}
 
 
 def set_screen(mode: str = "env"):
-    """TF32 screen of the 16-pick rounds (include/vatlq.h): "env" (VATLQ_PASS_SCREEN), "off", "on" or "verify"."""
+    """fp16 screen of the 16-pick rounds (include/vatlq.h): "env" (VATLQ_PASS_SCREEN), "off", "on" or "verify"."""
     _lib.check(_lib.lib().vatlq_coreset_set_screen(SCREEN_MODES[mode]), "vatlq_coreset_set_screen")
 
 
