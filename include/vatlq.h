@@ -172,6 +172,23 @@ int vatlq_fuse_final(const uint8_t* unlabeled, int64_t n, const double* stats2,
  * screened in fp16) it includes an fp16 copy of the owned rows, n * 4096 bytes; vatlq_coreset_init does not need
  * that part. */
 size_t vatlq_coreset_workspace_bytes(int64_t n, int d, int batch);
+/* The core-set calls on X in any VATLQ_* dtype (the fp32 entries are these calls with VATLQ_F32).  Every 16-bit
+ * value converts exactly to fp64 and every kernel reads the same values in the same order, so min_d, unc, the pick
+ * list and the counting statistics equal, bit for bit, those of the same call on X's fp32 upcast, in every screen and
+ * prune mode.  A 16-bit X must be 8-byte aligned (16-byte when d == 2048: the passes copy whole rows with TMA); an
+ * unknown dtype or a misaligned X returns VATLQ_EINVAL before any device work.  The 16-pick rounds screen a 16-bit X
+ * itself, so its workspace has no fp16 copy: vatlq_coreset_workspace_bytes_dt(n, d, batch, F16 or BF16) is smaller
+ * by n * 4096 bytes when d == 2048 and batch >= 16 (an unknown dtype: 0). */
+size_t vatlq_coreset_workspace_bytes_dt(int64_t n, int d, int batch, int dtype);
+int vatlq_coreset_init_dt(const void* X, int dtype, int64_t n, int d, int64_t row_lo, int64_t row_hi,
+                          const int64_t* labeled, int64_t n_labeled,
+                          double* min_d, void* ws, size_t ws_bytes, vatlq_stream_t stream);
+int vatlq_coreset_select_dt(const void* X, int dtype, int64_t n, int d, int64_t row_lo, int64_t row_hi,
+                            double* min_d, double* unc,
+                            int rule, double moks, double lambda, int64_t n_labeled,
+                            int64_t first_pick, int64_t k, int batch,
+                            int64_t* out_idx, void* comm,
+                            void* ws, size_t ws_bytes, int64_t* host_stats, vatlq_stream_t stream);
 int vatlq_coreset_init(const float* X, int64_t n, int d, int64_t row_lo, int64_t row_hi,
                        const int64_t* labeled, int64_t n_labeled,
                        double* min_d, void* ws, size_t ws_bytes, vatlq_stream_t stream);
@@ -212,8 +229,8 @@ int vatlq_coreset_prune_stats(int64_t* host_out4, int reset);
 int vatlq_coreset_set_prune(int mode, int64_t min_rows);
 
 /* The fp16 screen of the 16-pick rounds (d == 2048): before a round's fp64 pass each streamed row is
- * compared with the round's centres on the tensor cores (an fp16 copy of the owned rows that
- * vatlq_coreset_select fills in its workspace), and only the rows that an error bound cannot
+ * compared with the round's centres on the tensor cores (an fp32 X through an fp16 copy of the owned rows that
+ * vatlq_coreset_select fills in its workspace; a 16-bit X as it is, in its own type), and only the rows that an error bound cannot
  * prove unchanged (min_d[i] <= d(i,c) for every centre) go through the exact fp64 arithmetic.  The pick
  * list and min_d are unchanged bit for bit.  Environment: VATLQ_PASS_SCREEN=0 disables,
  * VATLQ_PASS_SCREEN=verify computes every streamed row exactly and counts the rows the screen did not
@@ -227,6 +244,9 @@ int vatlq_coreset_set_screen(int mode);
  * out[i*m + j] = d(X[i], X[centers[j]]) in fp64 (sklearn _euclidean_distances order). */
 int vatlq_pairwise_dist(const float* X, int64_t n, int d, const int64_t* centers, int64_t m,
                         double* out, void* ws /* >= n*8 bytes */, size_t ws_bytes, vatlq_stream_t stream);
+/* The same on X in any VATLQ_* dtype (8-byte aligned in 16 bits): equal, bit for bit, to the fp32 call on the upcast. */
+int vatlq_pairwise_dist_dt(const void* X, int dtype, int64_t n, int d, const int64_t* centers, int64_t m,
+                           double* out, void* ws, size_t ws_bytes, vatlq_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
  * SURVEY.md 8f "next" rows: the other per-item uncertainties and the representativeness step.

@@ -33,11 +33,16 @@ SIGNATURES = {
     "vatlq_coreset_init_tc": (_int, [_vp, _i64, _int, _i64, _i64, _vp, _i64, _vp, _vp, _sz, _int, _vp, _vp, _vp]),
     "vatlq_coreset_select": (_int, [_vp, _i64, _int, _i64, _i64, _vp, _vp, _int, _dbl, _dbl, _i64,
                                     _i64, _i64, _int, _vp, _vp, _vp, _sz, _vp, _vp]),
+    "vatlq_coreset_workspace_bytes_dt": (_sz, [_i64, _int, _int, _int]),
+    "vatlq_coreset_init_dt": (_int, [_vp, _int, _i64, _int, _i64, _i64, _vp, _i64, _vp, _vp, _sz, _vp]),
+    "vatlq_coreset_select_dt": (_int, [_vp, _int, _i64, _int, _i64, _i64, _vp, _vp, _int, _dbl, _dbl, _i64,
+                                       _i64, _i64, _int, _vp, _vp, _vp, _sz, _vp, _vp]),
     "vatlq_coreset_prune_stats": (_int, [_vp, _int]),
     "vatlq_coreset_set_prune": (_int, [_int, _i64]),
     "vatlq_coreset_screen_stats": (_int, [_vp, _int]),
     "vatlq_coreset_set_screen": (_int, [_int]),
     "vatlq_pairwise_dist": (_int, [_vp, _i64, _int, _vp, _i64, _vp, _vp, _sz, _vp]),
+    "vatlq_pairwise_dist_dt": (_int, [_vp, _int, _i64, _int, _vp, _i64, _vp, _vp, _sz, _vp]),
     "vatlq_pose_unc": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _vp, _vp, _vp, _vp, _vp]),
     "vatlq_heatmap_entropy": (_int, [_vp, _i64, _int, _int, _int, _vp, _vp, _sz, _vp]),
     "vatlq_heatmap_entropy_dt": (_int, [_vp, _int, _i64, _int, _int, _int, _vp, _vp, _sz, _vp]),
@@ -74,7 +79,7 @@ SIGNATURES = {
 
 _lib = None
 EINVAL, ECOMM, ESTATE = -1, -3, -4     # VATLQ_E* of include/vatlq.h
-F32, F16, BF16 = 0, 1, 2               # VATLQ_F32 / VATLQ_F16 / VATLQ_BF16: heat-map element types of the *_dt entries
+F32, F16, BF16 = 0, 1, 2               # VATLQ_F32 / VATLQ_F16 / VATLQ_BF16: element types of the *_dt entries
 
 
 class VatlqError(RuntimeError):

@@ -45,6 +45,15 @@ def _as_cuda(a, dtype=torch.float32):
     return t.to(device=_dev(), dtype=dtype).contiguous()
 
 
+def embedding_store_dtype(filter_: str, representativeness: str, dtype: torch.dtype) -> torch.dtype:
+    """The dtype eval_and_query stores the embeddings in: fp16 / bf16 as they are when only the core-set reads them
+    (filter Coreset, representativeness None or Random) — its picks equal those of the exact fp32 upcast, at half
+    the memory — fp32 (`.float()`, like the reference) for every other consumer."""
+    if dtype in (torch.float16, torch.bfloat16) and filter_ == "Coreset" and representativeness in ("None", "Random"):
+        return dtype
+    return torch.float32
+
+
 def _heatmaps(out: torch.Tensor) -> torch.Tensor:
     """The estimator's heat maps as the kernels read them: fp16 / bf16 (autocast or a .half() model) as they are —
     the scores equal those of their exact fp32 upcast — every other dtype as `.float()` like the reference."""
@@ -202,7 +211,9 @@ def coreset_selection(self, embeddings, uncertainty):
     labeled_id, moks_queried, unc_lambda, uncertainty (the strategy name), cfg.VAL.UNC_LAMBDA,
     opt.fixed_lambda, query_size.  `uncertainty` (the array) is modified in place like the
     reference (:848).  Returns the list of picked indices in pick order."""
-    X = _as_cuda(embeddings, torch.float32)
+    # (fp16 / bf16 tensors as they are: the selection equals that on their exact fp32 upcast)
+    keep = isinstance(embeddings, torch.Tensor) and embeddings.dtype in (torch.float16, torch.bfloat16)
+    X = _as_cuda(embeddings, embeddings.dtype if keep else torch.float32)
     if isinstance(embeddings, np.ndarray) and embeddings.dtype == np.float64:
         if not np.array_equal(X.cpu().numpy().astype(np.float64), embeddings):
             raise _lib.VatlqError("embeddings must hold fp32-representable values (ActiveLearning.py:270,286)")
@@ -351,8 +362,9 @@ class ActiveLearning:
         # embeddings are collected when the filter OR the representativeness needs them (:283)
         want_feat = self.filter not in ("None", "Random") or self.representativeness not in ("None", "Random")
         qp = QueryPass(n, dev, ae_weights=self.AE if use_wpu else None, uncertainty=self.uncertainty)
-        # (the reference keeps an all-zero fvecs_matrix otherwise, :270)
-        X = torch.zeros((n, 2048), dtype=torch.float32, device=dev) if want_feat else None
+        # (the reference keeps an all-zero fvecs_matrix otherwise, :270); allocated at the first batch, in
+        # embedding_store_dtype of the estimator's embeddings
+        X = None
         oks_dev = torch.zeros(n, dtype=torch.float64, device=dev)
         have_gt = True
         m = self.model
@@ -372,7 +384,12 @@ class ActiveLearning:
             out, emb = forward_with_embedding(m, cur, want_feat, fuse=bool(getattr(self.opt, "fuse_embedding", True)))
             H = _heatmaps(out[:, self.eval_joints])                       # (:277-281)
             if want_feat:
-                X[pos:pos + b] = emb.float()                              # (:283-286)
+                if X is None:
+                    X = torch.zeros((n, 2048), device=dev,
+                                    dtype=embedding_store_dtype(self.filter, self.representativeness, emb.dtype))
+                if X.dtype != torch.float32 and emb.dtype != X.dtype:
+                    raise _lib.VatlqError(f"the estimator's embeddings changed dtype mid-pool ({X.dtype} -> {emb.dtype})")
+                X[pos:pos + b] = emb if emb.dtype == X.dtype else emb.float()   # (:283-286)
             boxes = torch.as_tensor(np.asarray(bboxes_crop), dtype=torch.float32).reshape(b, 4).to(dev)
             ip = torch.as_tensor(np.asarray(isPrev)).to(torch.uint8)
             inx = torch.as_tensor(np.asarray(isNext)).to(torch.uint8)

@@ -216,14 +216,24 @@ __device__ __forceinline__ void dmma_v(double (&c)[2], double a, double b) {
                : "d"(a), "d"(b));
 }
 
+// ELEMENT TYPES of X (VATLQ_F32 / F16 / BF16): every kernel that reads X is a template on the element type T and
+// reads it a quad (four consecutive features: a float4 in fp32, a uint2 in 16 bits, common.cuh) at a time, widened
+// exactly to fp32 at the load; from there on the fp64 arithmetic is the same instruction sequence in every type, so
+// a 16-bit X gives every output of its fp32 upcast bit for bit.
+template <typename T>
+using quad_t = typename QuadOf<T>::type;
+template <typename T>
+__device__ __forceinline__ float4 ldg_q(const quad_t<T>* p) { return quad_f32(__ldg(p), (const T*)nullptr); }
+
 // centers in shared memory: fp64, row stride S = dpad + 2 doubles (== 16 bytes mod 128, which
 // makes the two 16-byte B loads of a quarter-warp conflict free), features >= d zero
-__device__ __forceinline__ void stage_center(const float* __restrict__ X, int d4, int dpad, int S, long long row, int j,
+template <typename T>
+__device__ __forceinline__ void stage_center(const T* __restrict__ X, int d4, int dpad, int S, long long row, int j,
                                              double* s_c) {
-  const float4* src = reinterpret_cast<const float4*>(X) + (size_t)row * d4;
+  const quad_t<T>* src = reinterpret_cast<const quad_t<T>*>(X) + (size_t)row * d4;
   for (int q = threadIdx.x; q < dpad / 4; q += blockDim.x) {
     float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (q < d4) v = __ldg(src + q);
+    if (q < d4) v = ldg_q<T>(src + q);
     double2* dst = reinterpret_cast<double2*>(s_c + (size_t)j * S + 4 * q);
     dst[0] = make_double2((double)v.x, (double)v.y);
     dst[1] = make_double2((double)v.z, (double)v.w);
@@ -231,10 +241,10 @@ __device__ __forceinline__ void stage_center(const float* __restrict__ X, int d4
 }
 
 // x[row][4q..4q+3]; GUARD only when d is not a multiple of 16 (the last super-step is ragged)
-template <bool GUARD>
-__device__ __forceinline__ float4 load_x(const float4* p, int q, int d4) {
+template <bool GUARD, typename T>
+__device__ __forceinline__ float4 load_x(const quad_t<T>* p, int q, int d4) {
   if (GUARD && q >= d4) return make_float4(0.f, 0.f, 0.f, 0.f);
-  return ldg_stream(p + q);
+  return quad_f32(ldg_stream(p + q), (const T*)nullptr);
 }
 
 __device__ __forceinline__ void dmma_step(double (&c)[4][2], const float4& x, const double* bp) {
@@ -265,8 +275,8 @@ __device__ __forceinline__ double combine8(const double* p, int stride) {
 // canonical dots of one 8-row block (this lane's row pointer `rowp`, never null) against the 8
 // staged centers, all four segments by one warp (four independent chains): used by the small
 // kernels.  self != 0: B = A (row norms, no shared memory).
-template <bool GUARD, bool SELF>
-__device__ __forceinline__ void dmma_block(const float4* rowp, int d4, int nss, const double* __restrict__ s_c, int S,
+template <bool GUARD, bool SELF, typename T>
+__device__ __forceinline__ void dmma_block(const quad_t<T>* rowp, int d4, int nss, const double* __restrict__ s_c, int S,
                                            int lane, double (&out)[2]) {
   const int g = lane >> 2, kk = lane & 3;
   const int seglen = (nss + kSeg - 1) / kSeg;
@@ -285,7 +295,7 @@ __device__ __forceinline__ void dmma_block(const float4* rowp, int d4, int nss, 
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
         const int ss = (grp * 4 + q) * seglen + s;
-        x[q] = (ss < nss) ? load_x<GUARD>(rowp, 4 * ss + kk, d4) : make_float4(0.f, 0.f, 0.f, 0.f);
+        x[q] = (ss < nss) ? load_x<GUARD, T>(rowp, 4 * ss + kk, d4) : make_float4(0.f, 0.f, 0.f, 0.f);
       }
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
@@ -308,8 +318,8 @@ __device__ __forceinline__ void dmma_block(const float4* rowp, int d4, int nss, 
 // ---------------------------------------------------------------- squared row norms
 // xx_i = dot(x_i, x_i): in the diagonal 8x8 block the B operand of lane (g,kk) is its own A
 // operand; the diagonal element (g,g) lives in lane (g, g>>1), slot g&1.
-template <bool GUARD>
-__global__ void __launch_bounds__(256) row_norms_kernel(const float* __restrict__ X, long long n, int d4, int nss,
+template <bool GUARD, typename T>
+__global__ void __launch_bounds__(256) row_norms_kernel(const T* __restrict__ X, long long n, int d4, int nss,
                                                         double* __restrict__ xx) {
   const int lane = threadIdx.x & 31, g = lane >> 2, kk = lane & 3;
   const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -317,14 +327,14 @@ __global__ void __launch_bounds__(256) row_norms_kernel(const float* __restrict_
   for (long long r0 = w * 8; r0 < n; r0 += nw * 8) {
     const long long row = min(r0 + g, n - 1);
     double c[2];
-    dmma_block<GUARD, true>(reinterpret_cast<const float4*>(X) + (size_t)row * d4, d4, nss, nullptr, 0, lane, c);
+    dmma_block<GUARD, true, T>(reinterpret_cast<const quad_t<T>*>(X) + (size_t)row * d4, d4, nss, nullptr, 0, lane, c);
     if (kk == (g >> 1) && r0 + g < n) xx[r0 + g] = (g & 1) ? c[1] : c[0];
   }
 }
 
 // ---------------------------------------------------------------- the pass over X
 struct PassArgs {
-  const float* X;
+  const void* X;             // [n][d] of the kernel's element type T
   long long n;
   int d4, nss, S;
   long long lo, hi;          // owned rows
@@ -363,7 +373,8 @@ struct PassArgs {
   // decide, 2 verify (DMMA every streamed row, count unlisted rows whose min_d moved anyway)
   int screen_mode;
   unsigned long long* screen_stats;  // [0] rows screened, [1] rows listed, [2] verify violations
-  const __half* Xh;                  // screen_mode != 0: X[lo, hi) as fp16, row r - lo at Xh + (r - lo) * 2048
+  const __half* Xh;                  // screen_mode != 0: X[lo, hi) in 16 bits, row r - lo at Xh + (r - lo) * 2048: the
+                                     // fp16 copy for an fp32 X, X itself for a 16-bit X (bf16 bits: only addressed)
 };
 
 // centres of THIS pass: count (<= 0: nothing to do) and whether it is the round's last pass
@@ -447,8 +458,9 @@ __device__ void publish_pass(const PassArgs& a, Best best, bool do_hist, const u
 
 constexpr int kTeams = kPassThreads / 32 / kSeg;   // 2 teams of 8 warps
 
-template <bool GUARD>
+template <bool GUARD, typename T>
 __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs a) {
+  using Q = quad_t<T>;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   bool final_pass;
   const int nb = pass_centers(a, final_pass);
@@ -468,7 +480,7 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
   }
   for (int j = 0; j < kB; ++j) {
     const long long p = centers[min(j, nb - 1)];  // pad with the last center: min() is idempotent
-    stage_center(a.X, a.d4, dpad, a.S, p, j, s_c);
+    stage_center(static_cast<const T*>(a.X), a.d4, dpad, a.S, p, j, s_c);
     if (threadIdx.x == 0) {
       s_xxc[j] = a.xx[p];
       s_pick[j] = p;
@@ -491,7 +503,7 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
   }
   __syncthreads();
 
-  const float4* X4 = reinterpret_cast<const float4*>(a.X);
+  const Q* X4 = reinterpret_cast<const Q*>(a.X);
   const long long ntiles = (a.hi - a.lo + 7) / 8;
   const long long t0 = (long long)blockIdx.x * kTeams + team, tstride = (long long)gridDim.x * kTeams;
   const long long nt = (t0 < ntiles) ? (ntiles - t0 + tstride - 1) / tstride : 0;
@@ -566,13 +578,13 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
     int cs = 0;                        // step inside its segment
     long long lt = t0;                 // load cursor
     int ls = 0;
-    const float4* lp = (nt > 0) ? row_ptr(lt) : X4;
+    const Q* lp = (nt > 0) ? row_ptr(lt) : X4;
     float4 ring[kDepth];
 #pragma unroll
     for (int p = 0; p < kDepth; ++p) {
       ring[p] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (p < F) {
-        ring[p] = load_x<GUARD>(lp, 4 * ls, a.d4 - 4 * seg_beg - kk);
+        ring[p] = load_x<GUARD, T>(lp, 4 * ls, a.d4 - 4 * seg_beg - kk);
         if (++ls == mylen) {
           ls = 0;
           lt += tstride;
@@ -589,7 +601,7 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
           const double2 b23 = *reinterpret_cast<const double2*>(bptr + 16 * cs + 2);
           const double x0 = (double)ring[p].x, x1 = (double)ring[p].y, x2 = (double)ring[p].z, x3 = (double)ring[p].w;
           if (f + kDepth < F) {          // refill the slot that was just consumed
-            ring[p] = load_x<GUARD>(lp, 4 * ls, a.d4 - 4 * seg_beg - kk);
+            ring[p] = load_x<GUARD, T>(lp, 4 * ls, a.d4 - 4 * seg_beg - kk);
             if (++ls == mylen) {
               ls = 0;
               lt += tstride;
@@ -707,6 +719,7 @@ constexpr int kStageBytesX = 8 * kRowBytesX;               // 66 048
 // bytes: the 8-byte loads of rows g = 0..3 (lanes 4g .. 4g+3, 32 contiguous bytes each) hit all 32 banks
 constexpr int kRowBytesH = 2048 * 2 + 32;
 static_assert(16 * kRowBytesH == kStageBytesX, "an fp16 stage of two tiles fills an fp32 stage exactly");
+
 constexpr int kWsThreads = (kSeg + 4) * 32;                // 8 compute warps + producer + 3 epilogue warps
 constexpr int kMaxTilesCta = 2048;                         // tiles per CTA the pruned-tile list can hold
 constexpr size_t kWsSmem = (size_t)kStagesX * kStageBytesX + sizeof(double) * kPartBufs * kSeg * 64 + 2 * kStagesX * 8 +
@@ -729,6 +742,12 @@ __device__ __forceinline__ uint2 lds64(unsigned addr) {
   uint2 r;
   asm volatile("ld.shared.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "r"(addr));
   return r;
+}
+// quad of a staged row, widened to fp32 (16 bytes in fp32, 8 in 16 bits)
+template <typename T>
+__device__ __forceinline__ float4 lds_quad(unsigned addr) {
+  if constexpr (sizeof(T) == 4) return lds128(addr);
+  else return quad_f32(lds64(addr), (const T*)nullptr);
 }
 
 // PAIR = true ("paired pass"): the grid is launched as clusters of two CTAs (one TPC).  Both CTAs of a pair walk the
@@ -782,13 +801,35 @@ __device__ __forceinline__ unsigned ld_dsmem_u32(const void* p, unsigned rank) {
 // (the row is listed); in particular an element with |v| >= 65520 becomes +-Inf in fp16, and S~ is then +-Inf or
 // NaN (Inf x 0), never finite.  The undecided rows are then gathered 8 per tile (the per-row TMA copies of the fp32
 // rows the producer always issues) and only those go through the canonical DMMA tile machine.
+//
+// 16-BIT X (fp16 or bf16): the screen streams X itself through the same stages (its rows are the copy's 4 KB), reads
+// the 16 centres from X as they are, and issues mma.sync m16n8k16 in X's own type (f16 or bf16).  No operand is
+// rounded: x~ = x and c~ = c, so the input terms above vanish.  A product of two fp16 (11 x 11 significant bits) or two
+// bf16 values (8 x 8 bits) is exact in fp32, so S~ differs from S only by the fp32 accumulation, which is ASSUMED, as
+// above, to add at most 2048 * 2^-23 = 2^-12 relative to sum |x_k c_k| <= |x||c| (checked by verify mode, not proven).
+// bf16 has fp32's exponent range, so an input below 2^-126 may be flushed by the tensor core (moving the dot by
+// < 2^-126 |c|_1 <= 2^-120.5 |c|, likewise for x), a product or a partial sum may fall below 2^-126 (at worst flushed:
+// < 2^-114 over the 2048 products and additions), and a product or a sum may overflow to Inf / NaN.  Hence
+//     |S~ - S| <= 2^-12 |x||c| + 2^-120 (|x| + |c|) + 2^-114,
+//     E16 = 2 u16 |x||c| + 2^-20 (|x|^2 + |c|^2) + 2^-100 (1 + |x| + |c|),   u16 = 2^-12,
+// and the proof above goes through with E16 for E: t >= t~ - 2|S~ - S| - 2^-48 (..) exceeds fl(t~ - 2 E16) by more than
+// its rounding.  A row whose S~ overflowed is not finite and is listed, never decided.  (An fp16 dot product cannot
+// overflow fp32: 2048 x 65504^2 < 2^44; its products are >= 2^-48 and never underflow.)
 constexpr double kScreenU = 0.00390625;               // 2^-8
 constexpr double kScreenAbs = 9.5367431640625e-07;    // 2^-20
 constexpr double kScreenAbs1 = 7.62939453125e-06;     // 2^-17
+constexpr double kScreenU16 = 0.000244140625;         // 2^-12
+constexpr double kScreenAbs16 = 7.888609052210118e-31;  // 2^-100
+template <typename T = __half>
 __device__ __forceinline__ void mma_f16(float (&d)[4], const unsigned (&a)[4], uint2 b) {
-  asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b.x), "r"(b.y));
+  if constexpr (std::is_same<T, __nv_bfloat16>::value)
+    asm("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b.x), "r"(b.y));
+  else
+    asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b.x), "r"(b.y));
 }
 __device__ __forceinline__ unsigned half2_bits(float lo, float hi) {   // cvt.rn.f16x2.f32: lo in the low half
   const __half2 h = __floats2half2_rn(lo, hi);
@@ -824,9 +865,15 @@ __device__ __forceinline__ int listed_row(const unsigned short* s_pre, const uns
   return lo * 8 + r;
 }
 
-template <int STEPS, bool PAIR, bool FILTER = false>
+template <int STEPS, bool PAIR, bool FILTER = false, typename T = float>
 __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
   static_assert(STEPS * 16 * kSeg * 4 + 64 == kRowBytesX, "stage geometry is for d = 2048");
+  using Q = quad_t<T>;
+  constexpr bool X16 = sizeof(T) == 2;            // 16-bit X: the screen reads X itself (see "the screen")
+  // stage row stride of the DMMA tiles: a 16-bit X keeps its rows at the screen's stride (8-byte loads, conflict
+  // free), one tile in the first half of a stage
+  constexpr int kRowB = X16 ? kRowBytesH : kRowBytesX;
+  constexpr unsigned kXRowBytes = 2048u * sizeof(T);
   constexpr int NC = PAIR ? 2 * kB : kB;          // dot products per row the finishing reads
   extern __shared__ __align__(128) unsigned char smem_raw[];
   unsigned char* stage0 = smem_raw;
@@ -1014,26 +1061,33 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     // ------------------------------------------------------------------ compute warps
     asm volatile("setmaxnreg.inc.sync.aligned.u32 216;");
     const int seg = warp, g = lane >> 2, kk = lane & 3;
-    const unsigned a_off = smem_addr(stage0) + g * kRowBytesX + seg * (STEPS * 64) + kk * 16;
+    const unsigned a_off = smem_addr(stage0) + g * kRowB + seg * (STEPS * 4 * (int)sizeof(Q)) + kk * (int)sizeof(Q);
     int st = 0, pb = 0;
     unsigned phase = 0;
     if (screen) {
       // A operand of mma.m16n8k16: centres g and g + 8 of the round at the features this lane reads of a row, as
-      // fp16 (the k slots {2kk, 2kk+1} and {2kk+8, 2kk+9} of super-step s are features 16s + 4kk + {0, 1} and
-      // {2, 3}: the same permutation of K for A and B)
+      // fp16 or X's 16-bit type (the k slots {2kk, 2kk+1} and {2kk+8, 2kk+9} of super-step s are features
+      // 16s + 4kk + {0, 1} and {2, 3}: the same permutation of K for A and B)
       unsigned af[STEPS][4];
       {
         const long long* allc = a.centers + a.center_off;
         const long long p0 = allc[min(g, total - 1)], p1 = allc[min(g + kB, total - 1)];
-        const float4* c0 = reinterpret_cast<const float4*>(a.X) + (size_t)p0 * a.d4 + seg * (STEPS * 4) + kk;
-        const float4* c1 = reinterpret_cast<const float4*>(a.X) + (size_t)p1 * a.d4 + seg * (STEPS * 4) + kk;
+        const Q* c0 = reinterpret_cast<const Q*>(a.X) + (size_t)p0 * a.d4 + seg * (STEPS * 4) + kk;
+        const Q* c1 = reinterpret_cast<const Q*>(a.X) + (size_t)p1 * a.d4 + seg * (STEPS * 4) + kk;
 #pragma unroll
         for (int s = 0; s < STEPS; ++s) {
-          const float4 v0 = __ldg(c0 + 4 * s), v1 = __ldg(c1 + 4 * s);
-          af[s][0] = half2_bits(v0.x, v0.y);
-          af[s][1] = half2_bits(v1.x, v1.y);
-          af[s][2] = half2_bits(v0.z, v0.w);
-          af[s][3] = half2_bits(v1.z, v1.w);
+          const Q v0 = __ldg(c0 + 4 * s), v1 = __ldg(c1 + 4 * s);
+          if constexpr (X16) {   // the centres as they are (element 2j in the low half of word j)
+            af[s][0] = v0.x;
+            af[s][1] = v1.x;
+            af[s][2] = v0.y;
+            af[s][3] = v1.y;
+          } else {
+            af[s][0] = half2_bits(v0.x, v0.y);
+            af[s][1] = half2_bits(v1.x, v1.y);
+            af[s][2] = half2_bits(v0.z, v0.w);
+            af[s][3] = half2_bits(v1.z, v1.w);
+          }
         }
       }
       const unsigned h_off = smem_addr(stage0) + g * kRowBytesH + seg * (STEPS * 32) + kk * 8;
@@ -1045,8 +1099,8 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
         float d[2][4] = {{0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
 #pragma unroll
         for (int s = 0; s < STEPS; ++s) {
-          mma_f16(d[0], af[s], lds64(ap + s * 32));
-          mma_f16(d[1], af[s], lds64(ap + 8 * kRowBytesH + s * 32));
+          mma_f16<T>(d[0], af[s], lds64(ap + s * 32));
+          mma_f16<T>(d[1], af[s], lds64(ap + 8 * kRowBytesH + s * 32));
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty[st]);
@@ -1073,10 +1127,10 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     double breg[STEPS][4];
     {
       const long long pg = centers[min(g, nb - 1)];
-      const float4* cp = reinterpret_cast<const float4*>(a.X) + (size_t)pg * a.d4 + seg * (STEPS * 4) + kk;
+      const Q* cp = reinterpret_cast<const Q*>(a.X) + (size_t)pg * a.d4 + seg * (STEPS * 4) + kk;
 #pragma unroll
       for (int s = 0; s < STEPS; ++s) {
-        const float4 v = __ldg(cp + 4 * s);
+        const float4 v = ldg_q<T>(cp + 4 * s);
         breg[s][0] = (double)v.x;
         breg[s][1] = (double)v.y;
         breg[s][2] = (double)v.z;
@@ -1092,7 +1146,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
       for (int e = 0; e < 4; ++e) c[e][0] = c[e][1] = 0.0;
 #pragma unroll
       for (int s = 0; s < STEPS; ++s) {
-        const float4 x = lds128(ap + s * 64);
+        const float4 x = lds_quad<T>(ap + s * 4 * (unsigned)sizeof(Q));
         dmma(c[0], (double)x.x, breg[s][0]);
         dmma(c[1], (double)x.y, breg[s][1]);
         dmma(c[2], (double)x.z, breg[s][2]);
@@ -1122,11 +1176,12 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
       unsigned phase = 0;
       auto fill = [&](auto row_of_lane) {
         if (fills++ >= kStagesX) mbar_wait(&empty[st], phase ^ 1u);   // the stage's previous tile was released
-        if (lane == 0) mbar_expect_tx(&full[st], 8u * 2048u * 4u);
+        if (lane == 0) mbar_expect_tx(&full[st], 8u * kXRowBytes);
         __syncwarp();
         if (lane < 8) {
           const long long row = row_of_lane();
-          tma_load_1d(stage0 + (size_t)st * kStageBytesX + lane * kRowBytesX, a.X + (size_t)row * 2048, 2048u * 4u, &full[st]);
+          tma_load_1d(stage0 + (size_t)st * kStageBytesX + lane * kRowB, static_cast<const T*>(a.X) + (size_t)row * 2048,
+                      kXRowBytes, &full[st]);
         }
         if (++st == kStagesX) {
           st = 0;
@@ -1134,8 +1189,8 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
         }
       };
       if (screen) {
-        // two tiles of this CTA's parity per stage, fp16 rows of 4 KB from the copy: lane r < 16 copies row r & 7 of
-        // the first (r < 8) or second tile; a lone last tile fills both halves
+        // two tiles of this CTA's parity per stage, 16-bit rows of 4 KB (the fp16 copy, or a 16-bit X itself): lane
+        // r < 16 copies row r & 7 of the first (r < 8) or second tile; a lone last tile fills both halves
         auto fill_half = [&](int k0, int k1) {
           if (fills++ >= kStagesX) mbar_wait(&empty[st], phase ^ 1u);
           if (lane == 0) mbar_expect_tx(&full[st], 16u * 2048u * 2u);
@@ -1212,7 +1267,8 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
             const int c = q + 4 * c4;
             const double xs = xxi + s_xxc[c];
             const double t = xs - 2.0 * S[c4];
-            const double E = 2.0 * kScreenU * nx * s_nc[c] + kScreenAbs * xs + kScreenAbs1 * (nx + s_nc[c]);
+            const double E = X16 ? 2.0 * kScreenU16 * nx * s_nc[c] + kScreenAbs * xs + kScreenAbs16 * (1.0 + nx + s_nc[c])
+                                 : 2.0 * kScreenU * nx * s_nc[c] + kScreenAbs * xs + kScreenAbs1 * (nx + s_nc[c]);
             und = und || !(isfinite(S[c4]) && t - 2.0 * E > m2) || s_pick[c] == i;
           }
           const unsigned ub = __ballot_sync(0xffffffffu, und && valid);
@@ -1347,10 +1403,11 @@ struct PruneCtl {
 };
 
 // squared distance of two rows as sum((x-y)^2) in fp64 (every lane returns the warp total)
-__device__ __forceinline__ double warp_sqdist(const float4* __restrict__ x, const float4* __restrict__ y, int d4, int lane) {
+template <typename T>
+__device__ __forceinline__ double warp_sqdist(const quad_t<T>* __restrict__ x, const quad_t<T>* __restrict__ y, int d4, int lane) {
   double acc = 0.0;
   for (int c = lane; c < d4; c += 32) {
-    const float4 u = __ldg(x + c), v = __ldg(y + c);
+    const float4 u = ldg_q<T>(x + c), v = ldg_q<T>(y + c);
     const double a0 = (double)u.x - (double)v.x, a1 = (double)u.y - (double)v.y;
     const double a2 = (double)u.z - (double)v.z, a3 = (double)u.w - (double)v.w;
     acc = fma(a0, a0, acc);
@@ -1362,17 +1419,18 @@ __device__ __forceinline__ double warp_sqdist(const float4* __restrict__ x, cons
 }
 
 // cd[r] = d(row lo+r-1, row lo+r) for r >= 1 (cd[0] = +inf), and their sum / count
-__global__ void __launch_bounds__(256) consec_kernel(const float* __restrict__ X, int d4, long long lo, long long hi,
+template <typename T>
+__global__ void __launch_bounds__(256) consec_kernel(const T* __restrict__ X, int d4, long long lo, long long hi,
                                                      double* __restrict__ cd, PruneCtl* pc) {
   const int lane = threadIdx.x & 31;
   const long long w0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
-  const float4* X4 = reinterpret_cast<const float4*>(X);
+  const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
   double local = 0.0;
   unsigned long long cnt = 0;
   for (long long r = w0; r < hi - lo; r += nwarps) {
     double dist = INFINITY;
     if (r > 0) {
-      dist = sqrt(warp_sqdist(X4 + (size_t)(lo + r) * d4, X4 + (size_t)(lo + r - 1) * d4, d4, lane));
+      dist = sqrt(warp_sqdist<T>(X4 + (size_t)(lo + r) * d4, X4 + (size_t)(lo + r - 1) * d4, d4, lane));
       if (isfinite(dist)) {
         local += dist;
         cnt += 1;
@@ -1440,18 +1498,19 @@ __global__ void __launch_bounds__(1024) segment_kernel(const double* __restrict_
 }
 
 // R_s = max_i d(anchor_s, i): one warp per segment
-__global__ void __launch_bounds__(256) seg_radius_kernel(const float* __restrict__ X, int d4, long long lo,
+template <typename T>
+__global__ void __launch_bounds__(256) seg_radius_kernel(const T* __restrict__ X, int d4, long long lo,
                                                          const int* __restrict__ seg_start, const PruneCtl* pc,
                                                          double* __restrict__ segR) {
   const int lane = threadIdx.x & 31;
   const int w0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
-  const float4* X4 = reinterpret_cast<const float4*>(X);
+  const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
   const int nseg = pc->nseg;
   for (int sg = w0; sg < nseg; sg += nwarps) {
     const int a = seg_start[sg], e = seg_start[sg + 1];
     double R = 0.0;
     for (int r = a + 1; r < e; ++r)
-      R = fmax(R, sqrt(warp_sqdist(X4 + (size_t)(lo + r) * d4, X4 + (size_t)(lo + a) * d4, d4, lane)));
+      R = fmax(R, sqrt(warp_sqdist<T>(X4 + (size_t)(lo + r) * d4, X4 + (size_t)(lo + a) * d4, d4, lane)));
     if (lane == 0) segR[sg] = R;
   }
 }
@@ -1463,8 +1522,8 @@ __global__ void __launch_bounds__(256) seg_radius_kernel(const float* __restrict
 // this one is multiplied, so the kernel is not a chain of memory round trips); after the split-K
 // exchange warp w finishes segment w of the tile: canonical distances of its anchor to the 8
 // centres, the maximum of min_d over its rows, and the test.
-template <int STEPS>
-__global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const float* __restrict__ X, int d4, long long lo,
+template <int STEPS, typename T>
+__global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const T* __restrict__ X, int d4, long long lo,
                                                                     const int* __restrict__ seg_start,
                                                                     const double* __restrict__ segR,
                                                                     const double* __restrict__ m, const double* __restrict__ xx,
@@ -1486,24 +1545,24 @@ __global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const float*
   const int ntiles = (nseg + 7) / 8;
   if ((int)blockIdx.x >= ntiles) return;
   const int lane = threadIdx.x & 31, seg = threadIdx.x >> 5, g = lane >> 2, kk = lane & 3;
-  const float4* X4 = reinterpret_cast<const float4*>(X);
+  const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
   const int lane_off = seg * (STEPS * 4) + kk;
   auto anchor = [&](int sg) -> long long { return lo + seg_start[min(sg, nseg - 1)]; };
   int t = blockIdx.x;
   // the first tile's anchor rows and the centres are requested back to back (one memory round trip)
   float4 ring[STEPS];
   {
-    const float4* p0 = X4 + (size_t)anchor(t * 8 + g) * d4 + lane_off;
+    const quad_t<T>* p0 = X4 + (size_t)anchor(t * 8 + g) * d4 + lane_off;
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) ring[s] = __ldg(p0 + 4 * s);
+    for (int s = 0; s < STEPS; ++s) ring[s] = ldg_q<T>(p0 + 4 * s);
   }
   double breg[STEPS][4];
   {
     const long long p = centers[min(g, nb - 1)];   // padded with the last centre
-    const float4* cp = X4 + (size_t)p * d4 + lane_off;
+    const quad_t<T>* cp = X4 + (size_t)p * d4 + lane_off;
 #pragma unroll
     for (int s = 0; s < STEPS; ++s) {
-      const float4 c4 = __ldg(cp + 4 * s);
+      const float4 c4 = ldg_q<T>(cp + 4 * s);
       breg[s][0] = (double)c4.x;
       breg[s][1] = (double)c4.y;
       breg[s][2] = (double)c4.z;
@@ -1515,7 +1574,7 @@ __global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const float*
   for (; t < ntiles; t += gridDim.x) {
     const int tn = t + gridDim.x;
     const bool has_next = tn < ntiles;
-    const float4* np = X4 + (size_t)anchor((has_next ? tn : t) * 8 + g) * d4 + lane_off;
+    const quad_t<T>* np = X4 + (size_t)anchor((has_next ? tn : t) * 8 + g) * d4 + lane_off;
     const int myseg = t * 8 + seg;                       // the segment this warp finishes
     // everything the test needs is requested BEFORE the multiply loop and consumed after it:
     // min_d of the segment's rows (segments hold <= kSegMax = 64 rows: two per lane), |a|^2, R
@@ -1533,7 +1592,7 @@ __global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const float*
 #pragma unroll
     for (int s = 0; s < STEPS; ++s) {
       const float4 x = ring[s];
-      if (has_next) ring[s] = __ldg(np + 4 * s);
+      if (has_next) ring[s] = ldg_q<T>(np + 4 * s);
       dmma(c[0], (double)x.x, breg[s][0]);
       dmma(c[1], (double)x.y, breg[s][1]);
       dmma(c[2], (double)x.z, breg[s][2]);
@@ -1670,7 +1729,8 @@ __device__ __forceinline__ void locate(const CandView& v, int world, int pos, in
 }
 
 // ---------------------------------------------------------------- candidate x candidate distances
-__global__ void __launch_bounds__(256) pairs_kernel(const float* __restrict__ X, int d4, int nss, int S, int guard,
+template <typename T>
+__global__ void __launch_bounds__(256) pairs_kernel(const T* __restrict__ X, int d4, int nss, int S, int guard,
                                                     const double* __restrict__ xx, const RankBlock* blocks,
                                                     const Ctl* ctl, double* __restrict__ Dcc) {
   if (ctl->n_picked >= ctl->k) return;
@@ -1691,15 +1751,15 @@ __global__ void __launch_bounds__(256) pairs_kernel(const float* __restrict__ X,
   }
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5, g = lane >> 2, kk = lane & 3;
-  const float4* X4 = reinterpret_cast<const float4*>(X);
+  const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
   for (int r0 = (blockIdx.y * nwarp + warp) * 8; r0 < v.total; r0 += gridDim.y * nwarp * 8) {
     const int pos = min(r0 + g, v.total - 1);
     int rr, ss;
     locate(v, world, pos, rr, ss);
     const long long ridx = blocks[rr].idx[ss];
     double c[2];
-    if (guard) dmma_block<true, false>(X4 + (size_t)ridx * d4, d4, nss, s_c, S, lane, c);
-    else dmma_block<false, false>(X4 + (size_t)ridx * d4, d4, nss, s_c, S, lane, c);
+    if (guard) dmma_block<true, false, T>(X4 + (size_t)ridx * d4, d4, nss, s_c, S, lane, c);
+    else dmma_block<false, false, T>(X4 + (size_t)ridx * d4, d4, nss, s_c, S, lane, c);
     if (r0 + g < v.total) {
       const double xxi = xx[ridx];
 #pragma unroll
@@ -1718,12 +1778,12 @@ __device__ void plan_body(const RankBlock* blocks, RankBlock* send, const double
 // every 8 x 8 block is written twice (d is symmetric; both halves hold the SAME bits, so the planner may read rows).
 // The pairs are dealt round-robin to the CTAs of the grid: with ~250 candidates that is 528 pairs over 148 CTAs
 // (3-4 each, all loads of a pair in flight together) instead of 8 sequential tiles per CTA on a quarter of the SMs.
-template <int STEPS>
-__device__ __forceinline__ void pairs_tiles(const float* __restrict__ X, int d4, const double* __restrict__ xx,
+template <int STEPS, typename T>
+__device__ __forceinline__ void pairs_tiles(const T* __restrict__ X, int d4, const double* __restrict__ xx,
                                             const RankBlock* blocks, const CandView& v, int world,
                                             double* __restrict__ Dcc, double (*s_part)[kSeg][64], double* s_xxc) {
   const int lane = threadIdx.x & 31, seg = threadIdx.x >> 5, g = lane >> 2, kk = lane & 3;
-  const float4* X4 = reinterpret_cast<const float4*>(X);
+  const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
   const int lane_off = seg * (STEPS * 4) + kk;
   auto cand_row = [&](int pos) {
     int r, q;
@@ -1743,13 +1803,13 @@ __device__ __forceinline__ void pairs_tiles(const float* __restrict__ X, int d4,
     const int t = cb + q, col0 = cb * kB;
     // both operand tiles are requested back to back: one memory round trip per pair
     const long long crow = cand_row(col0 + g), arow = cand_row(t * 8 + g);
-    const float4* cp = X4 + (size_t)crow * d4 + lane_off;
-    const float4* ap = X4 + (size_t)arow * d4 + lane_off;
+    const quad_t<T>* cp = X4 + (size_t)crow * d4 + lane_off;
+    const quad_t<T>* ap = X4 + (size_t)arow * d4 + lane_off;
     float4 cb4[STEPS], ring[STEPS];
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) cb4[s] = __ldg(cp + 4 * s);
+    for (int s = 0; s < STEPS; ++s) cb4[s] = ldg_q<T>(cp + 4 * s);
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) ring[s] = __ldg(ap + 4 * s);
+    for (int s = 0; s < STEPS; ++s) ring[s] = ldg_q<T>(ap + 4 * s);
     if (threadIdx.x < kB) s_xxc[buf * kB + threadIdx.x] = xx[cand_row(col0 + threadIdx.x)];
     const int myrow = t * 8 + seg;                       // the row this warp finishes
     const double xxi = (myrow < v.total) ? xx[cand_row(myrow)] : 0.0;
@@ -1787,8 +1847,8 @@ __device__ __forceinline__ void pairs_tiles(const float* __restrict__ X, int d4,
 // The last CTA of the grid to finish runs the planner (plan_body) on the completed matrix, so a
 // round needs no separate plan launch.
 constexpr int kPlanSmem = 208 * 1024;    // dynamic shared memory of pairs_plan_kernel: the planner's staged distance rows
-template <int STEPS>
-__global__ void __launch_bounds__(kSeg * 32, 1) pairs_plan_kernel(const float* __restrict__ X, int d4,
+template <int STEPS, typename T>
+__global__ void __launch_bounds__(kSeg * 32, 1) pairs_plan_kernel(const T* __restrict__ X, int d4,
                                                                   const double* __restrict__ xx, const RankBlock* blocks,
                                                                   RankBlock* send, unsigned int* hist, long long* out_idx,
                                                                   Ctl* ctl, double* __restrict__ Dcc, Mailbox* mail,
@@ -1816,7 +1876,7 @@ __global__ void __launch_bounds__(kSeg * 32, 1) pairs_plan_kernel(const float* _
   {
     const int world = ctl->world;
     const CandView v = view_of(blocks, world);
-    if (!v.fallback) pairs_tiles<STEPS>(X, d4, xx, blocks, v, world, Dcc, s_part, s_xxc);
+    if (!v.fallback) pairs_tiles<STEPS, T>(X, d4, xx, blocks, v, world, Dcc, s_part, s_xxc);
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -2159,7 +2219,8 @@ __global__ void wait_blocks_kernel(Mailbox* mail, const Ctl* ctl, unsigned long 
 }
 
 // distances of every row to a list of centers, for the parity tests
-__global__ void __launch_bounds__(256) pairwise_kernel(const float* __restrict__ X, long long n, int d4, int nss, int S,
+template <typename T>
+__global__ void __launch_bounds__(256) pairwise_kernel(const T* __restrict__ X, long long n, int d4, int nss, int S,
                                                        int guard, const double* __restrict__ xx, const long long* __restrict__ centers,
                                                        long long mcols, double* __restrict__ out) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -2167,7 +2228,7 @@ __global__ void __launch_bounds__(256) pairwise_kernel(const float* __restrict__
   double* s_c = reinterpret_cast<double*>(smem_raw);
   const long long col0 = (long long)blockIdx.x * kB;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5, g = lane >> 2, kk = lane & 3;
-  const float4* X4 = reinterpret_cast<const float4*>(X);
+  const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
   for (int j = 0; j < kB; ++j) {
     const long long p = centers[min(col0 + j, mcols - 1)];
     stage_center(X, d4, nss * 16, S, p, j, s_c);
@@ -2177,8 +2238,8 @@ __global__ void __launch_bounds__(256) pairwise_kernel(const float* __restrict__
   for (long long r0 = ((long long)blockIdx.y * nwarp + warp) * 8; r0 < n; r0 += (long long)gridDim.y * nwarp * 8) {
     const long long i = min(r0 + g, n - 1);
     double c[2];
-    if (guard) dmma_block<true, false>(X4 + (size_t)i * d4, d4, nss, s_c, S, lane, c);
-    else dmma_block<false, false>(X4 + (size_t)i * d4, d4, nss, s_c, S, lane, c);
+    if (guard) dmma_block<true, false, T>(X4 + (size_t)i * d4, d4, nss, s_c, S, lane, c);
+    else dmma_block<false, false, T>(X4 + (size_t)i * d4, d4, nss, s_c, S, lane, c);
     if (r0 + g < n) {
       const double xxi = xx[i];
 #pragma unroll
@@ -2293,10 +2354,14 @@ static int g_screen_mode_set = -1;             // vatlq_coreset_set_screen: -1 =
 
 using namespace vatlq;
 
-extern "C" size_t vatlq_coreset_workspace_bytes(int64_t n, int d, int batch) {
-  if (n < 0) return 0;
+extern "C" size_t vatlq_coreset_workspace_bytes_dt(int64_t n, int d, int batch, int dtype) {
+  if (n < 0 || dtype_size(dtype) == 0) return 0;
   const WsLayout L = ws_layout(n, kMaxRanks);
-  return paired_rounds(d, batch) ? L.xh + (size_t)n * 4096 : L.total;
+  // the fp16 copy only for an fp32 X: the screen reads a 16-bit X itself
+  return (dtype == VATLQ_F32 && paired_rounds(d, batch)) ? L.xh + (size_t)n * 4096 : L.total;
+}
+extern "C" size_t vatlq_coreset_workspace_bytes(int64_t n, int d, int batch) {
+  return vatlq_coreset_workspace_bytes_dt(n, d, batch, VATLQ_F32);
 }
 
 struct Geom {
@@ -2313,8 +2378,9 @@ static Geom geom_of(int d) {
   return g;
 }
 
-static int check_x(const float* X, int64_t n, int d, int64_t lo, int64_t hi) {
-  VQ_REQUIRE(X != nullptr && ((uintptr_t)X & 15) == 0, "X must be a 16-byte aligned device pointer");
+static int check_x(const void* X, int dtype, int64_t n, int d, int64_t lo, int64_t hi) {
+  VQ_REQUIRE(dtype_size(dtype) != 0, "dtype must be VATLQ_F32, VATLQ_F16 or VATLQ_BF16");
+  VQ_REQUIRE(X != nullptr && quad_aligned(X, dtype), "X must be a device pointer aligned to 16 bytes (fp32) or 8 bytes (16 bits)");
   VQ_REQUIRE(n > 0 && d > 0 && (d & 3) == 0, "d must be a positive multiple of 4");
   VQ_REQUIRE(n < 0xffffffffLL, "n must be below 2^32 - 1 (the planner reduces 32-bit row ids)");
   VQ_REQUIRE(0 <= lo && lo <= hi && hi <= n, "bad row range");
@@ -2322,23 +2388,36 @@ static int check_x(const float* X, int64_t n, int d, int64_t lo, int64_t hi) {
   return 0;
 }
 
-static int launch_norms(const float* X, int64_t n, int d, double* xx, cudaStream_t stream) {
+template <typename T>
+static int launch_norms(const T* X, int64_t n, int d, double* xx, cudaStream_t stream) {
   const Geom g = geom_of(d);
   const int grid = sm_count() * 8;
-  if (g.guard) row_norms_kernel<true><<<grid, 256, 0, stream>>>(X, n, g.d4, g.nss, xx);
-  else row_norms_kernel<false><<<grid, 256, 0, stream>>>(X, n, g.d4, g.nss, xx);
+  if (g.guard) row_norms_kernel<true, T><<<grid, 256, 0, stream>>>(X, n, g.d4, g.nss, xx);
+  else row_norms_kernel<false, T><<<grid, 256, 0, stream>>>(X, n, g.d4, g.nss, xx);
   VQ_LAUNCHED();
   return 0;
 }
 
+template <typename T>
+static int configure_pass_of() {
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_generic<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_generic<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<16, false, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<16, true, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<16, true, true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<16, T>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<16, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPlanSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pairs_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pairwise_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+  return 0;
+}
+// the opt-in shared-memory sizes (and the planner's carve-out) of every kernel of every element type, once
 static int configure_pass() {
   static bool configured = false;
   if (!configured) {
-    VQ_CUDA(cudaFuncSetAttribute(pass_kernel_generic<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-    VQ_CUDA(cudaFuncSetAttribute(pass_kernel_generic<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-    VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
-    VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
-    VQ_CUDA(cudaFuncSetAttribute((pass_kernel_tma<16, true, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
+    if (int e = configure_pass_of<float>()) return e;
+    if (int e = configure_pass_of<__half>()) return e;
+    if (int e = configure_pass_of<__nv_bfloat16>()) return e;
     configured = true;
   }
   return 0;
@@ -2370,6 +2449,7 @@ static int pair_grid() {
 
 // the paired pass of a 16-pick round (d = 2048 only): applies picks [0, nb) when nb > 8, reading X once
 // (filter = true: the same tile machine over the segment anchors, writing both centre groups' skip flags)
+template <typename T>
 static int launch_pass_pair(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr,
                             bool filter = false, bool pdl = false) {
   if (int e = configure_pass()) return e;
@@ -2387,20 +2467,21 @@ static int launch_pass_pair(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = 
   cfg.attrs = at;
   cfg.numAttrs = pdl ? 2 : 1;
   if (ev0) cudaEventRecord(ev0, stream);
-  if (filter) VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, true, true>, a));
-  else VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, true, false>, a));
+  if (filter) VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, true, true, T>, a));
+  else VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, true, false, T>, a));
   if (ev1) cudaEventRecord(ev1, stream);
   VQ_LAUNCHED();
   return 0;
 }
 
+template <typename T>
 static int launch_pass(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr, bool pdl = false) {
   if (int e = configure_pass()) return e;
   if (ev0) cudaEventRecord(ev0, stream);
   const bool fast = a.d4 == kSeg * 4 * 16 && a.dots != nullptr;   // d = 2048
-  if (fast) VQ_CUDA(launch_pdl(pass_kernel_tma<16, false>, dim3(sm_count()), dim3(kWsThreads), kWsSmem, stream, pdl, a));
-  else if ((a.d4 & 3) != 0) pass_kernel_generic<true><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
-  else pass_kernel_generic<false><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
+  if (fast) VQ_CUDA(launch_pdl(pass_kernel_tma<16, false, false, T>, dim3(sm_count()), dim3(kWsThreads), kWsSmem, stream, pdl, a));
+  else if ((a.d4 & 3) != 0) pass_kernel_generic<true, T><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
+  else pass_kernel_generic<false, T><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
   if (ev1) cudaEventRecord(ev1, stream);
   VQ_LAUNCHED();
   return 0;
@@ -2417,7 +2498,8 @@ struct PruneState {
   size_t skip_stride = 0;
   int filter_grid = 1;
 };
-static int prune_setup(PruneState& P, const float* X, const Geom& G, int64_t row_lo, int64_t row_hi, char* w,
+template <typename T>
+static int prune_setup(PruneState& P, const T* X, const Geom& G, int64_t row_lo, int64_t row_hi, char* w,
                        const WsLayout& L, cudaStream_t stream) {
   static const int prune_env = []() {
     const char* e = getenv("VATLQ_PRUNE");
@@ -2443,20 +2525,21 @@ static int prune_setup(PruneState& P, const float* X, const Geom& G, int64_t row
   VQ_CUDA(cudaMemsetAsync(P.pc, 0, sizeof(PruneCtl), stream));
   if (P.mode) {
     double* cd = (double*)(w + L.dots);   // the dot-product scratch is idle until the first pass
-    consec_kernel<<<sm_count() * 8, 256, 0, stream>>>(X, G.d4, row_lo, row_hi, cd, P.pc);
+    consec_kernel<T><<<sm_count() * 8, 256, 0, stream>>>(X, G.d4, row_lo, row_hi, cd, P.pc);
     VQ_LAUNCHED();
     segment_kernel<<<1, 1024, 0, stream>>>(cd, (int)own, P.pc, P.seg_of_row, P.seg_start);
     VQ_LAUNCHED();
-    seg_radius_kernel<<<sm_count() * 8, 256, 0, stream>>>(X, G.d4, row_lo, P.seg_start, P.pc, P.seg_r);
+    seg_radius_kernel<T><<<sm_count() * 8, 256, 0, stream>>>(X, G.d4, row_lo, P.seg_start, P.pc, P.seg_r);
     VQ_LAUNCHED();
   }
   return 0;
 }
 // flags for the `groups` passes that apply centers[center_off + 8g ..), g = 0 .. groups-1 (flag array g):
 // ONE launch before the first of those passes
+template <typename T>
 static int launch_filter(const PruneState& P, const PassArgs& a, cudaStream_t stream, int groups = 1) {
   dim3 grid((unsigned)P.filter_grid, (unsigned)groups);
-  prune_filter_kernel<16><<<grid, kSeg * 32, 0, stream>>>(a.X, a.d4, a.lo, P.seg_start, P.seg_r, a.m, a.xx, a.centers,
+  prune_filter_kernel<16, T><<<grid, kSeg * 32, 0, stream>>>(static_cast<const T*>(a.X), a.d4, a.lo, P.seg_start, P.seg_r, a.m, a.xx, a.centers,
                                                           a.n_centers, a.n_centers_imm, a.center_off, P.pc, P.seg_skip,
                                                           P.skip_stride);
   VQ_LAUNCHED();
@@ -2478,12 +2561,17 @@ namespace vatlq {
 int vq_launch_norms(const float* X, int64_t n, int d, double* xx, cudaStream_t stream) { return launch_norms(X, n, d, xx, stream); }
 }  // namespace vatlq
 
-extern "C" int vatlq_coreset_init(const float* X, int64_t n, int d, int64_t row_lo, int64_t row_hi,
-                                  const int64_t* labeled, int64_t n_labeled, double* min_d, void* ws,
-                                  size_t ws_bytes, vatlq_stream_t stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  if (int e = check_x(X, n, d, row_lo, row_hi)) return e;
-  VQ_REQUIRE(min_d != nullptr && n_labeled >= 0, "null min_d");
+// X of the core-set calls: check_x, plus 16-byte alignment when d = 2048 (the TMA passes copy whole rows with
+// cp.async.bulk, which needs a 16-byte aligned source in every dtype)
+static int check_coreset_x(const void* X, int dtype, int64_t n, int d, int64_t lo, int64_t hi) {
+  if (int e = check_x(X, dtype, n, d, lo, hi)) return e;
+  VQ_REQUIRE(d != kSeg * 16 * 16 || ((uintptr_t)X & 15) == 0, "X must be 16-byte aligned when d = 2048");
+  return 0;
+}
+
+template <typename T>
+static int coreset_init(const T* X, int64_t n, int d, int64_t row_lo, int64_t row_hi, const int64_t* labeled,
+                        int64_t n_labeled, double* min_d, void* ws, size_t ws_bytes, cudaStream_t stream) {
   const WsLayout L = ws_layout(n, kMaxRanks);
   VQ_REQUIRE(ws != nullptr && ws_bytes >= L.total, "workspace too small");
   char* w = (char*)ws;
@@ -2505,9 +2593,9 @@ extern "C" int vatlq_coreset_init(const float* X, int64_t n, int d, int64_t row_
     a.n_centers_imm = (int)std::min<int64_t>(kB, n_labeled - c0); a.ctl = nullptr; a.hist = nullptr;
     if (P.mode) {
       a.seg_of_row = P.seg_of_row; a.seg_skip = P.seg_skip; a.prune_mode = P.mode; a.prune_stats = P.pc->stats;
-      if (int e = launch_filter(P, a, stream)) return e;
+      if (int e = launch_filter<T>(P, a, stream)) return e;
     }
-    if (int e = launch_pass(a, stream)) return e;
+    if (int e = launch_pass<T>(a, stream)) return e;
   }
   if (P.mode == 2) {   // verify mode only: wait and collect the violation count of the initialisation passes
     VQ_CUDA(cudaStreamSynchronize(stream));
@@ -2516,13 +2604,28 @@ extern "C" int vatlq_coreset_init(const float* X, int64_t n, int d, int64_t row_
   return 0;
 }
 
-extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t row_lo, int64_t row_hi,
-                                    double* min_d, double* unc, int rule, double moks, double lambda,
-                                    int64_t n_labeled, int64_t first_pick, int64_t k, int batch,
-                                    int64_t* out_idx, void* comm_, void* ws, size_t ws_bytes,
-                                    int64_t* host_stats, vatlq_stream_t stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  if (int e = check_x(X, n, d, row_lo, row_hi)) return e;
+extern "C" int vatlq_coreset_init_dt(const void* X, int dtype, int64_t n, int d, int64_t row_lo, int64_t row_hi,
+                                     const int64_t* labeled, int64_t n_labeled, double* min_d, void* ws,
+                                     size_t ws_bytes, vatlq_stream_t stream) {
+  if (int e = check_coreset_x(X, dtype, n, d, row_lo, row_hi)) return e;
+  VQ_REQUIRE(min_d != nullptr && n_labeled >= 0, "null min_d");
+  return with_dtype(dtype, [&](auto t) {
+    using T = std::remove_cv_t<std::remove_pointer_t<decltype(t)>>;
+    return coreset_init<T>(static_cast<const T*>(X), n, d, row_lo, row_hi, labeled, n_labeled, min_d, ws, ws_bytes,
+                           (cudaStream_t)stream);
+  });
+}
+extern "C" int vatlq_coreset_init(const float* X, int64_t n, int d, int64_t row_lo, int64_t row_hi,
+                                  const int64_t* labeled, int64_t n_labeled, double* min_d, void* ws,
+                                  size_t ws_bytes, vatlq_stream_t stream) {
+  return vatlq_coreset_init_dt(X, VATLQ_F32, n, d, row_lo, row_hi, labeled, n_labeled, min_d, ws, ws_bytes, stream);
+}
+
+template <typename T>
+static int coreset_select(const T* X, int dtype, int64_t n, int d, int64_t row_lo, int64_t row_hi, double* min_d,
+                          double* unc, int rule, double moks, double lambda, int64_t n_labeled, int64_t first_pick,
+                          int64_t k, int batch, int64_t* out_idx, void* comm_, void* ws, size_t ws_bytes,
+                          int64_t* host_stats, cudaStream_t stream) {
   VQ_REQUIRE(min_d && unc && out_idx, "null pointer");
   VQ_REQUIRE(rule >= 0 && rule <= 2, "rule must be 0, 1 or 2");
   VQ_REQUIRE(k >= 0 && k <= n, "k must be in [0, n]");
@@ -2532,8 +2635,8 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
   VQ_REQUIRE(world >= 1 && world <= kMaxRanks, "world size not supported");
   VQ_REQUIRE(world > 1 || (row_lo == 0 && row_hi == n), "single GPU must own every row");
   const WsLayout L = ws_layout(n, kMaxRanks);
-  VQ_REQUIRE(ws != nullptr && ws_bytes >= vatlq_coreset_workspace_bytes(n, d, batch),
-             "workspace too small (vatlq_coreset_workspace_bytes(n, d, batch))");
+  VQ_REQUIRE(ws != nullptr && ws_bytes >= vatlq_coreset_workspace_bytes_dt(n, d, batch, dtype),
+             "workspace too small (vatlq_coreset_workspace_bytes_dt(n, d, batch, dtype))");
   if (k == 0) return 0;
   char* w = (char*)ws;
   Ctl* ctl = (Ctl*)(w + L.ctl);
@@ -2610,20 +2713,23 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
     return !strcmp(e, "verify") ? 2 : 1;
   }();
   const int screen_mode = g_screen_mode_set >= 0 ? g_screen_mode_set : screen_env;
-  // the screen reads the owned rows from their fp16 copy at the end of the workspace, filled once per call
-  const __half* Xh = (use_pair && screen_mode) ? (const __half*)(w + L.xh) : nullptr;
-  if (Xh && row_hi > row_lo) {
-    half_copy_kernel<<<sm_count() * 8, 256, 0, stream>>>((const float4*)X, row_lo, (row_hi - row_lo) * 512, (uint2*)(w + L.xh));
-    VQ_LAUNCHED();
+  // the screen reads the owned rows in 16 bits: an fp32 X from its fp16 copy at the end of the workspace, filled once
+  // per call; a 16-bit X as it is
+  const __half* Xh = nullptr;
+  if (use_pair && screen_mode) {
+    if constexpr (sizeof(T) == 2) {
+      Xh = reinterpret_cast<const __half*>(X) + (size_t)row_lo * 2048;
+    } else {
+      Xh = (const __half*)(w + L.xh);
+      if (row_hi > row_lo) {
+        half_copy_kernel<<<sm_count() * 8, 256, 0, stream>>>((const float4*)X, row_lo, (row_hi - row_lo) * 512, (uint2*)(w + L.xh));
+        VQ_LAUNCHED();
+      }
+    }
   }
-  static bool pairs_cfg = false;
-  if (!pairs_cfg) {
-    // the same shared-memory carve-out as the pass kernels on either side of it: no SM reconfiguration between them
-    VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<16>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPlanSmem));
-    VQ_CUDA(cudaFuncSetAttribute(pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-    pairs_cfg = true;
-  }
+  // (the same shared-memory carve-out for the planner as for the pass kernels on either side of it: no SM
+  // reconfiguration between them)
+  if (int e = configure_pass()) return e;
   auto fill_pass = [&](PassArgs& a) {
     a.X = X; a.n = n; a.d4 = G.d4; a.nss = G.nss; a.S = G.S; a.lo = row_lo; a.hi = row_hi; a.xx = xx; a.m = min_d;
     a.unc = unc; a.score = score; a.centers = ctl->picks; a.n_centers = &ctl->nb; a.n_centers_imm = 0; a.ctl = ctl;
@@ -2644,7 +2750,7 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
     fill_pass(a);
     a.send = nullptr;   // the bootstrap below computes the arg-max of the scores this pass writes
     a.seg_skip = nullptr; a.prune_mode = 0;
-    if (int e = launch_pass(a, stream)) return e;
+    if (int e = launch_pass<T>(a, stream)) return e;
   } else {
     const long long cnt = row_hi - row_lo;
     if (cnt > 0) {
@@ -2689,7 +2795,7 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
       if (nbk > 1) {
         dim3 pg(kCap / kB, 4);
         if (fast_d) {
-          const cudaError_t le = launch_pdl(pairs_plan_kernel<16>, dim3(sm_count()), dim3(kSeg * 32), kPlanSmem, stream, true, X, G.d4,
+          const cudaError_t le = launch_pdl(pairs_plan_kernel<16, T>, dim3(sm_count()), dim3(kSeg * 32), kPlanSmem, stream, true, X, G.d4,
                                             (const double*)xx, blocks, send, hist, (long long*)out_idx, ctl, Dcc, mail,
                                             (unsigned long long)(seq0 + round_no), kPlanSmem / 8);
           if (le != cudaSuccess) {
@@ -2699,7 +2805,7 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
           }
         } else {
           if (p2p) wait_blocks_kernel<<<1, 1, 0, stream>>>(mail, ctl, seq0 + round_no);
-          pairs_kernel<<<pg, 256, pairs_smem, stream>>>(X, G.d4, G.nss, G.S, G.guard, xx, blocks, ctl, Dcc);
+          pairs_kernel<T><<<pg, 256, pairs_smem, stream>>>(X, G.d4, G.nss, G.S, G.guard, xx, blocks, ctl, Dcc);
         }
         g_launches.fetch_add(1);
       } else if (p2p) {
@@ -2715,16 +2821,16 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
         if (use_pair) {   // the pass's own TMA / DMMA tile machine over the anchor rows (bandwidth-bound)
           a.seg_start = P.seg_start; a.seg_r = P.seg_r; a.nseg = &P.pc->nseg; a.seg_skip_out = P.seg_skip;
           a.skip_stride = P.skip_stride;
-          rc = launch_pass_pair(a, stream, nullptr, nullptr, true, true);
+          rc = launch_pass_pair<T>(a, stream, nullptr, nullptr, true, true);
         } else {
-          rc = launch_filter(P, a, stream, (nbk + kB - 1) / kB);
+          rc = launch_filter<T>(P, a, stream, (nbk + kB - 1) / kB);
         }
       }
       auto timed_launch = [&](PassArgs& a, bool pair) {
         const bool timed = g_prof.on && g_prof.used + 2 <= g_prof.ev.size() && g_prof.used / 2 < 1024;
         if (timed) a.did_work = flags + g_prof.used / 2;
         cudaEvent_t e0 = timed ? g_prof.ev[g_prof.used] : nullptr, e1 = timed ? g_prof.ev[g_prof.used + 1] : nullptr;
-        const int r = pair ? launch_pass_pair(a, stream, e0, e1, false, true) : launch_pass(a, stream, e0, e1, true);
+        const int r = pair ? launch_pass_pair<T>(a, stream, e0, e1, false, true) : launch_pass<T>(a, stream, e0, e1, true);
         if (timed) g_prof.used += 2;
         return r;
       };
@@ -2834,6 +2940,27 @@ extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t ro
   return rc;
 }
 
+extern "C" int vatlq_coreset_select_dt(const void* X, int dtype, int64_t n, int d, int64_t row_lo, int64_t row_hi,
+                                       double* min_d, double* unc, int rule, double moks, double lambda,
+                                       int64_t n_labeled, int64_t first_pick, int64_t k, int batch, int64_t* out_idx,
+                                       void* comm, void* ws, size_t ws_bytes, int64_t* host_stats,
+                                       vatlq_stream_t stream) {
+  if (int e = check_coreset_x(X, dtype, n, d, row_lo, row_hi)) return e;
+  return with_dtype(dtype, [&](auto t) {
+    using T = std::remove_cv_t<std::remove_pointer_t<decltype(t)>>;
+    return coreset_select<T>(static_cast<const T*>(X), dtype, n, d, row_lo, row_hi, min_d, unc, rule, moks, lambda,
+                             n_labeled, first_pick, k, batch, out_idx, comm, ws, ws_bytes, host_stats, (cudaStream_t)stream);
+  });
+}
+extern "C" int vatlq_coreset_select(const float* X, int64_t n, int d, int64_t row_lo, int64_t row_hi,
+                                    double* min_d, double* unc, int rule, double moks, double lambda,
+                                    int64_t n_labeled, int64_t first_pick, int64_t k, int batch,
+                                    int64_t* out_idx, void* comm, void* ws, size_t ws_bytes,
+                                    int64_t* host_stats, vatlq_stream_t stream) {
+  return vatlq_coreset_select_dt(X, VATLQ_F32, n, d, row_lo, row_hi, min_d, unc, rule, moks, lambda, n_labeled,
+                                 first_pick, k, batch, out_idx, comm, ws, ws_bytes, host_stats, stream);
+}
+
 extern "C" int vatlq_coreset_set_prune(int mode, int64_t min_rows) {
   VQ_REQUIRE(mode >= -1 && mode <= 2, "mode must be -1 (environment), 0 (off), 1 (prune) or 2 (verify)");
   g_prune_mode_set = mode;
@@ -2861,27 +2988,31 @@ extern "C" int vatlq_coreset_prune_stats(int64_t* host_out4, int reset) {
   return 0;
 }
 
-extern "C" int vatlq_pairwise_dist(const float* X, int64_t n, int d, const int64_t* centers, int64_t m,
-                                   double* out, void* ws, size_t ws_bytes, vatlq_stream_t stream_) {
+extern "C" int vatlq_pairwise_dist_dt(const void* X, int dtype, int64_t n, int d, const int64_t* centers, int64_t m,
+                                      double* out, void* ws, size_t ws_bytes, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  if (int e = check_x(X, n, d, 0, n)) return e;
+  if (int e = check_x(X, dtype, n, d, 0, n)) return e;
   VQ_REQUIRE(centers && out && m > 0, "null pointer");
   VQ_REQUIRE(ws != nullptr && ws_bytes >= (size_t)n * sizeof(double), "workspace must hold n doubles");
-  const Geom G = geom_of(d);
-  double* xx = (double*)ws;
-  if (int e = launch_norms(X, n, d, xx, stream)) return e;
-  static bool cfg = false;
-  if (!cfg) {
-    VQ_CUDA(cudaFuncSetAttribute(pairwise_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-    cfg = true;
-  }
   const long long colblocks = (m + kB - 1) / kB;
   VQ_REQUIRE(colblocks <= 2147483647LL, "too many centers");
+  if (int e = configure_pass()) return e;
+  const Geom G = geom_of(d);
+  double* xx = (double*)ws;
   const int gy = (int)std::max<long long>(1, std::min<long long>(64, (n + 127) / 128));
   dim3 grid((unsigned)colblocks, (unsigned)gy);
-  pairwise_kernel<<<grid, 256, G.smem, stream>>>(X, n, G.d4, G.nss, G.S, G.guard, xx, (const long long*)centers, m, out);
-  VQ_LAUNCHED();
-  return 0;
+  return with_dtype(dtype, [&](auto t) {
+    using T = std::remove_cv_t<std::remove_pointer_t<decltype(t)>>;
+    const T* XT = static_cast<const T*>(X);
+    if (int e = launch_norms(XT, n, d, xx, stream)) return e;
+    pairwise_kernel<T><<<grid, 256, G.smem, stream>>>(XT, n, G.d4, G.nss, G.S, G.guard, xx, (const long long*)centers, m, out);
+    VQ_LAUNCHED();
+    return 0;
+  });
+}
+extern "C" int vatlq_pairwise_dist(const float* X, int64_t n, int d, const int64_t* centers, int64_t m,
+                                   double* out, void* ws, size_t ws_bytes, vatlq_stream_t stream) {
+  return vatlq_pairwise_dist_dt(X, VATLQ_F32, n, d, centers, m, out, ws, ws_bytes, stream);
 }
 
 // ---------------------------------------------------------------- communicator

@@ -34,6 +34,19 @@ _HALO_DTYPES = (torch.float32, torch.float16, torch.bfloat16, torch.float64, tor
                 torch.int8, torch.uint8, torch.bool)
 
 
+def _agree_dtype(t: torch.Tensor, what: str, group=None):
+    """Raise VatlqError on every rank unless every rank's t has the same dtype (one MIN all-reduce on t's device:
+    {min code, min -code}, and min == max iff all agree)."""
+    code = _HALO_DTYPES.index(t.dtype) if t.dtype in _HALO_DTYPES else len(_HALO_DTYPES)
+    mm = torch.tensor([code, -code], dtype=torch.int64, device=t.device)
+    td.all_reduce(mm, op=td.ReduceOp.MIN, group=group)
+    lo_code, hi_code = int(mm[0].item()), -int(mm[1].item())
+    if lo_code != hi_code or code == len(_HALO_DTYPES):
+        names = [str(d) for d in _HALO_DTYPES] + ["an unsupported dtype"]
+        raise _lib.VatlqError(f"{what}: the ranks hold {'frames' if what == 'exchange_halo' else 'rows'} of different "
+                              f"dtypes ({names[lo_code]} .. {names[hi_code]}); every rank must hold the same dtype")
+
+
 def exchange_halo(first: torch.Tensor | None, last: torch.Tensor | None, rank: int, world: int, group=None):
     """Send this rank's first frame to rank-1 and last frame to rank+1; return
     (halo_prev, halo_next): the frame before / after the local range (None at the pool ends).
@@ -47,16 +60,8 @@ def exchange_halo(first: torch.Tensor | None, last: torch.Tensor | None, rank: i
     if like is None:
         raise _lib.VatlqError("exchange_halo: an empty shard is not supported (shard_range never produces one "
                               "for n >= world); give every rank at least one frame")
-    # every rank must hold one heat-map dtype, or the sends and receives below would not match: agree first, and
-    # raise on every rank on a mismatch ({min code, min -code} in one MIN all-reduce: min == max iff all agree)
-    code = _HALO_DTYPES.index(like.dtype) if like.dtype in _HALO_DTYPES else len(_HALO_DTYPES)
-    mm = torch.tensor([code, -code], dtype=torch.int64, device=like.device)
-    td.all_reduce(mm, op=td.ReduceOp.MIN, group=group)
-    lo_code, hi_code = int(mm[0].item()), -int(mm[1].item())
-    if lo_code != hi_code or code == len(_HALO_DTYPES):
-        names = [str(d) for d in _HALO_DTYPES] + ["an unsupported dtype"]
-        raise _lib.VatlqError(f"exchange_halo: the ranks hold frames of different dtypes ({names[lo_code]} .. "
-                              f"{names[hi_code]}); every rank must hold the same dtype")
+    # every rank must hold one heat-map dtype, or the sends and receives below would not match
+    _agree_dtype(like, "exchange_halo", group)
     halo_prev = torch.empty_like(like) if rank > 0 else None
     halo_next = torch.empty_like(like) if rank < world - 1 else None
     ops_ = []
@@ -149,7 +154,8 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
                       w_unc: float = 1.0):
     """One query over a pool sharded across the ranks of `group` (one process per GPU).
     Every rank passes its slice of the pool and gets the same global pick list back.  Heat-map shards may be
-    fp32, fp16 or bf16 (the same dtype on every rank; the picks equal those of the fp32 upcast).
+    fp32, fp16 or bf16 (the same dtype on every rank; the picks equal those of the fp32 upcast), and so may the
+    embedding shards X_local for the Coreset filter: they are gathered and selected on as they are.
     uncertainty: any accelerated name (THC*, WPU*, THC+WPU, HP, TPC, Entropy, MPE, Margin, None);
     representativeness: "None" or "Influence" (ActiveLearning.py:467-477); filter: "Coreset" (:609-614),
     "None" (top-k, :533-534), "Diversity" (:581-590), "K-Means" (:593-608) or "weighted" (:553-580; w_unc = cfg.VAL.W_UNC;
@@ -189,6 +195,8 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
         raise ValueError("Representativeness type is not supported by distributed_query")
     score = allgather_rows(score_local, n, world, group)
     if filter == "Coreset":
+        if world > 1:   # the all-gather below needs one row size on every rank
+            _agree_dtype(X_local, "distributed_query", group)
         X = allgather_rows(X_local, n, world, group)
         picks, st = ops.coreset_select(X, score, lab, k, moks, lam, rule=rule, batch=batch, first_pick=first_pick,
                                        comm=comm.handle if comm is not None else None,

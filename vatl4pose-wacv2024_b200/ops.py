@@ -36,6 +36,17 @@ def _cuda(t: torch.Tensor, dtype, name: str) -> torch.Tensor:
 # heat-map element types and their VATLQ_* codes: 16-bit maps are read as they are, and every result equals the
 # fp32 path's on their exact upcast, bit for bit (include/vatlq.h)
 HEATMAP_DTYPES = {torch.float32: _lib.F32, torch.float16: _lib.F16, torch.bfloat16: _lib.BF16}
+# embedding element types of the core-set and pairwise-distance entries: the same contract, for X
+EMBEDDING_DTYPES = HEATMAP_DTYPES
+
+
+def _embeddings(t: torch.Tensor, name: str) -> torch.Tensor:
+    """A CUDA (n,d) embedding tensor in one of EMBEDDING_DTYPES, contiguous."""
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise _lib.VatlqError(f"{name} must be a CUDA tensor (the query pass has no CPU path)")
+    if t.dtype not in EMBEDDING_DTYPES:
+        raise _lib.VatlqError(f"{name} must be torch.float32, torch.float16 or torch.bfloat16, got {t.dtype}")
+    return t.contiguous()
 
 
 def _heatmaps(t: torch.Tensor, name: str) -> torch.Tensor:
@@ -264,11 +275,18 @@ def coreset_init_tc(X: torch.Tensor, lab: torch.Tensor, min_d: torch.Tensor, lo:
 def coreset_select(X: torch.Tensor, unc: torch.Tensor, labeled, k: int, moks: float, lam: float,
                    rule: str = "w_unc", first_pick: int = -1, batch: int = 16, comm=None,
                    row_range: tuple[int, int] | None = None, return_state: bool = False, tc_init: bool | None = None):
-    """k-center greedy selection (vatlq_coreset_init + vatlq_coreset_select).
-    X (n,d) fp32 CUDA (replicated on every rank when comm is given), unc (n,) fp64 CUDA — a
+    """k-center greedy selection (vatlq_coreset_init_dt + vatlq_coreset_select_dt).
+    X (n,d) CUDA in one of EMBEDDING_DTYPES (replicated on every rank when comm is given): a 16-bit X is read as it
+    is and gives, bit for bit, the picks, min_d, unc and counting stats of its fp32 upcast.  unc (n,) fp64 CUDA — a
     private copy is made, like the caller's deepcopy at ActiveLearning.py:612-613.
+    tc_init: labelled-set initialisation on the TF32 tcgen05 GEMM (coreset_init_tc, fp32 X only); None picks it for
+    fp32 X at d = 2048 with >= TC_INIT_MIN_LABELED labelled rows.  A 16-bit X takes the exact fp64 init (at
+    L = 17 000 about 204 ms against 39 ms, DESIGN.md §4.5); tc_init=True with a 16-bit X raises.
     Returns the picks as an int64 CUDA tensor in pick order (and stats / min_d / unc)."""
-    X = _cuda(X, torch.float32, "X")
+    X = _embeddings(X, "X")
+    dt = EMBEDDING_DTYPES[X.dtype]
+    if tc_init and dt != _lib.F32:
+        raise _lib.VatlqError("tc_init=True needs an fp32 X (the tcgen05 init is TF32); use tc_init=None for 16-bit X")
     n, d = X.shape
     dev = X.device
     unc = _cuda(unc, torch.float64, "unc").clone()
@@ -279,24 +297,25 @@ def coreset_select(X: torch.Tensor, unc: torch.Tensor, labeled, k: int, moks: fl
                                      dtype=np.int64)).to(dev)
     lo, hi = (0, n) if row_range is None else row_range
     L = _lib.lib()
-    ws_bytes = L.vatlq_coreset_workspace_bytes(n, d, batch)
+    ws_bytes = L.vatlq_coreset_workspace_bytes_dt(n, d, batch, dt)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     min_d = torch.empty(n, dtype=torch.float64, device=dev)
     out = torch.empty(max(k, 1), dtype=torch.int64, device=dev)
     stats = (C.c_int64 * 16)()
     if tc_init is None:    # the labelled-set contraction on the tcgen05 tensor cores when it is large enough to pay
-        tc_init = d == 2048 and lab.numel() >= TC_INIT_MIN_LABELED and hi > lo
+        tc_init = dt == _lib.F32 and d == 2048 and lab.numel() >= TC_INIT_MIN_LABELED and hi > lo
     done = False
     if tc_init and lab.numel() > 0:
         done, _, _ = coreset_init_tc(X, lab, min_d, lo, hi)
     with torch.cuda.device(dev):
         if not done:
-            _lib.check(L.vatlq_coreset_init(_ptr(X), n, d, lo, hi, _ptr(lab) if lab.numel() else None, lab.numel(),
-                                            _ptr(min_d), _ptr(ws), ws_bytes, _stream()), "vatlq_coreset_init")
-        _lib.check(L.vatlq_coreset_select(_ptr(X), n, d, lo, hi, _ptr(min_d), _ptr(unc), RULES[rule], float(moks),
-                                          float(lam), lab.numel(), int(first_pick), int(k), int(batch), _ptr(out),
-                                          C.c_void_p(comm) if comm else None, _ptr(ws), ws_bytes,
-                                          C.cast(stats, C.c_void_p), _stream()), "vatlq_coreset_select")
+            _lib.check(L.vatlq_coreset_init_dt(_ptr(X), dt, n, d, lo, hi, _ptr(lab) if lab.numel() else None,
+                                               lab.numel(), _ptr(min_d), _ptr(ws), ws_bytes, _stream()),
+                       "vatlq_coreset_init_dt")
+        _lib.check(L.vatlq_coreset_select_dt(_ptr(X), dt, n, d, lo, hi, _ptr(min_d), _ptr(unc), RULES[rule], float(moks),
+                                             float(lam), lab.numel(), int(first_pick), int(k), int(batch), _ptr(out),
+                                             C.c_void_p(comm) if comm else None, _ptr(ws), ws_bytes,
+                                             C.cast(stats, C.c_void_p), _stream()), "vatlq_coreset_select_dt")
     picks = out[:k]
     st = CoresetStats(*[int(v) for v in stats][:15])
     if return_state:
@@ -337,15 +356,15 @@ def screen_stats(reset: bool = False) -> dict:
 
 def pairwise_dist(X: torch.Tensor, centers) -> torch.Tensor:
     """(n,m) fp64 Euclidean distances of every row to X[centers] with the library's canonical
-    fp64 arithmetic (sklearn order: sqrt(max(0, -2 x.c + |x|^2 + |c|^2)))."""
-    X = _cuda(X, torch.float32, "X")
+    fp64 arithmetic (sklearn order: sqrt(max(0, -2 x.c + |x|^2 + |c|^2))).  X in any of EMBEDDING_DTYPES."""
+    X = _embeddings(X, "X")
     n, d = X.shape
     c = torch.as_tensor(np.asarray(centers, dtype=np.int64)).to(X.device)
     out = torch.empty((n, c.numel()), dtype=torch.float64, device=X.device)
     ws = torch.empty(n, dtype=torch.float64, device=X.device)
     with torch.cuda.device(X.device):
-        _lib.check(_lib.lib().vatlq_pairwise_dist(_ptr(X), n, d, _ptr(c), c.numel(), _ptr(out), _ptr(ws), n * 8, _stream()),
-                   "vatlq_pairwise_dist")
+        _lib.check(_lib.lib().vatlq_pairwise_dist_dt(_ptr(X), EMBEDDING_DTYPES[X.dtype], n, d, _ptr(c), c.numel(), _ptr(out),
+                                                     _ptr(ws), n * 8, _stream()), "vatlq_pairwise_dist_dt")
     return out
 
 
