@@ -1,8 +1,8 @@
 // k-center greedy core-set selection (ActiveLearning.coreset_selection,
 // active_learning/ActiveLearning.py:798-850) with fp64 distance arithmetic on fp32 features.
 //
-// One canonical distance d(i,c) is used everywhere (the same instruction sequence in every
-// kernel, see "the fp64 tensor-core tile" below):
+// One canonical distance d(i,c) is used everywhere (every kernel builds it from the shared tile of
+// canonical.cuh, see "the fp64 tensor-core tile" there):
 //   dot(i,c): fp64 tensor-core MMAs (mma.sync.m8n8k4.f64) over the features in a fixed order,
 //             fp32 inputs widened exactly, fp64 accumulation;
 //   d(i,c) = sqrt(max(0, (-2*dot + xx_i) + xx_c))   (sklearn _euclidean_distances order).
@@ -27,7 +27,7 @@
 #include <cstdlib>
 #include <cstring>
 
-#include "common.cuh"
+#include "canonical.cuh"
 
 namespace vatlq {
 
@@ -170,60 +170,10 @@ __device__ __forceinline__ double score_of(int rule, double wd, double wu, doubl
   return m;                                                              // :832
 }
 
-__device__ __forceinline__ double sq_from_dot(double dot, double xxi, double xxc) {
-  double t = __dmul_rn(-2.0, dot);
-  t = __dadd_rn(t, xxi);
-  return __dadd_rn(t, xxc);
-}
-__device__ __forceinline__ double dist_from_dot(double dot, double xxi, double xxc) {
-  return sqrt(fmax(sq_from_dot(dot, xxi, xxc), 0.0));
-}
-
-// ---- the fp64 tensor-core tile --------------------------------------------------------------
-// mma.sync.m8n8k4.f64 (DMMA; measured 18.5 T FMA/s on B200, tools/micro/fp64_rate.cu): a warp
-// computes 8 rows x 8 centers per instruction with ONE A and ONE B operand per lane, so the
-// register tile is tiny (2 doubles per 8x8 block) and shared-memory traffic is 1/8 of a scalar
-// DFMA register tile.  Lane (g = lane>>2, kk = lane&3) owns row g of an 8-row block and feeds,
-// for super-step s (16 features), the float4 x[row][16s+4kk .. +3]; element e of that float4
-// is k-slot kk of MMA e, i.e. feature 16s+4kk+e.  The B operand of lane (g, kk) is center g
-// at the same feature.  Output: lane holds (row g, centers 2kk and 2kk+1).
-//
-// CANONICAL DOT: the feature axis is cut into kSeg = 8 segments of ceil(nss/8) super-steps.
-// Inside a segment, element e (0..3) of every float4 feeds its own sequential DMMA chain
-// (four independent chains hide the dependent-issue latency of DMMA), and
-//   P_seg = (c_0 + c_1) + (c_2 + c_3),   dot = ((P0 + P1) + (P2 + P3)) + ((P4 + P5) + (P6 + P7)).
-// Every kernel (norms, pass, candidate pairs, pairwise) evaluates exactly this, so d(i,c) has
-// the same bits wherever it is computed and dot(x,x) == xx (d(c,c) == 0).  In the pass the eight
-// segments of a block are computed by eight warps in parallel (split-K): a warp then only ever
-// needs 1/8 of every centre, which fits its REGISTERS (see pass_kernel_tma).
-constexpr int kSeg = 8;
 #ifndef VQ_DEPTH
 #define VQ_DEPTH 8
 #endif
 constexpr int kDepth = VQ_DEPTH;     // super-steps of x in flight per lane (register ring)
-
-__device__ __forceinline__ void dmma(double (&c)[2], double a, double b) {
-  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-      : "+d"(c[0]), "+d"(c[1])
-      : "d"(a), "d"(b));
-}
-// volatile twin for the streaming kernels: keeps program order against the (volatile) ring loads,
-// so that the load of super-step s of the NEXT tile is issued right before the MMAs of step s of
-// this tile (a full tile of lead time) instead of wherever the scheduler lets it sink to
-__device__ __forceinline__ void dmma_v(double (&c)[2], double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(c[0]), "+d"(c[1])
-               : "d"(a), "d"(b));
-}
-
-// ELEMENT TYPES of X (VATLQ_F32 / F16 / BF16): every kernel that reads X is a template on the element type T and
-// reads it a quad (four consecutive features: a float4 in fp32, a uint2 in 16 bits, common.cuh) at a time, widened
-// exactly to fp32 at the load; from there on the fp64 arithmetic is the same instruction sequence in every type, so
-// a 16-bit X gives every output of its fp32 upcast bit for bit.
-template <typename T>
-using quad_t = typename QuadOf<T>::type;
-template <typename T>
-__device__ __forceinline__ float4 ldg_q(const quad_t<T>* p) { return quad_f32(__ldg(p), (const T*)nullptr); }
 
 // centers in shared memory: fp64, row stride S = dpad + 2 doubles (== 16 bytes mod 128, which
 // makes the two 16-byte B loads of a quarter-warp conflict free), features >= d zero
@@ -262,14 +212,6 @@ __device__ __forceinline__ void dmma_step_self(double (&c)[4][2], const float4& 
   dmma(c[1], x1, x1);
   dmma(c[2], x2, x2);
   dmma(c[3], x3, x3);
-}
-
-__device__ __forceinline__ double combine4(double p0, double p1, double p2, double p3) {
-  return __dadd_rn(__dadd_rn(p0, p1), __dadd_rn(p2, p3));
-}
-__device__ __forceinline__ double combine8(const double* p, int stride) {
-  return __dadd_rn(combine4(p[0], p[stride], p[2 * stride], p[3 * stride]),
-                   combine4(p[4 * stride], p[5 * stride], p[6 * stride], p[7 * stride]));
 }
 
 // canonical dots of one 8-row block (this lane's row pointer `rowp`, never null) against the 8
@@ -695,13 +637,13 @@ __device__ __forceinline__ int apply_row(const PassArgs& a, const ApplyConst& c,
 }
 
 // ---------------------------------------------------------------- the pass over X, fast path
-// d == 8 * 16 * STEPS (2048 for STEPS = 16).  Warp-specialised, one CTA per SM, 8-row tiles:
+// d == kFastD (2048).  Warp-specialised, one CTA per SM, 8-row tiles:
 //   * PRODUCER (one warp): streams tiles into a ring of kStagesX shared-memory stages with 1-D TMA
 //     bulk copies (one 8 KB cp.async.bulk per row, completion counted on the stage's mbarrier) and
 //     refills a stage as soon as the 8 compute warps have released it, so two to three tiles
 //     (128-192 KB per SM) are always in flight no matter how the math is scheduled.
 //   * 8 COMPUTE warps = the 8 K-segments of a tile.  Warp w keeps ITS 1/8 of the 8 centres in
-//     registers as fp64 B operands (STEPS x 4 doubles per lane); per super-step it reads one
+//     registers as fp64 B operands (kSteps x 4 doubles per lane); per super-step it reads one
 //     float4 of A from the stage (row stride 8 KB + 64 B: conflict free), converts and issues four
 //     DMMAs.  A tile ends with one 16-byte shared store of the segment's partial dots and a
 //     non-blocking bar.arrive.
@@ -713,11 +655,11 @@ __device__ __forceinline__ int apply_row(const PassArgs& a, const ApplyConst& c,
 // setmaxnreg: compute warpgroups 216 registers, the producer/epilogue warpgroup 72.
 constexpr int kStagesX = 3;
 constexpr int kPartBufs = 3;
-constexpr int kRowBytesX = 2048 * 4 + 64;                  // stage row stride
+constexpr int kRowBytesX = kFastD * 4 + 64;                // stage row stride
 constexpr int kStageBytesX = 8 * kRowBytesX;               // 66 048
 // the screen's stages hold TWO tiles of fp16 rows (16 x 4 KB, the bytes of one fp32 tile).  Row stride = 32 mod 128
 // bytes: the 8-byte loads of rows g = 0..3 (lanes 4g .. 4g+3, 32 contiguous bytes each) hit all 32 banks
-constexpr int kRowBytesH = 2048 * 2 + 32;
+constexpr int kRowBytesH = kFastD * 2 + 32;
 static_assert(16 * kRowBytesH == kStageBytesX, "an fp16 stage of two tiles fills an fp32 stage exactly");
 
 constexpr int kWsThreads = (kSeg + 4) * 32;                // 8 compute warps + producer + 3 epilogue warps
@@ -865,15 +807,14 @@ __device__ __forceinline__ int listed_row(const unsigned short* s_pre, const uns
   return lo * 8 + r;
 }
 
-template <int STEPS, bool PAIR, bool FILTER = false, typename T = float>
+template <bool PAIR, bool FILTER = false, typename T = float>
 __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
-  static_assert(STEPS * 16 * kSeg * 4 + 64 == kRowBytesX, "stage geometry is for d = 2048");
   using Q = quad_t<T>;
   constexpr bool X16 = sizeof(T) == 2;            // 16-bit X: the screen reads X itself (see "the screen")
   // stage row stride of the DMMA tiles: a 16-bit X keeps its rows at the screen's stride (8-byte loads, conflict
   // free), one tile in the first half of a stage
   constexpr int kRowB = X16 ? kRowBytesH : kRowBytesX;
-  constexpr unsigned kXRowBytes = 2048u * sizeof(T);
+  constexpr unsigned kXRowBytes = kFastD * sizeof(T);
   constexpr int NC = PAIR ? 2 * kB : kB;          // dot products per row the finishing reads
   extern __shared__ __align__(128) unsigned char smem_raw[];
   unsigned char* stage0 = smem_raw;
@@ -1061,21 +1002,21 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     // ------------------------------------------------------------------ compute warps
     asm volatile("setmaxnreg.inc.sync.aligned.u32 216;");
     const int seg = warp, g = lane >> 2, kk = lane & 3;
-    const unsigned a_off = smem_addr(stage0) + g * kRowB + seg * (STEPS * 4 * (int)sizeof(Q)) + kk * (int)sizeof(Q);
+    const unsigned a_off = smem_addr(stage0) + g * kRowB + seg * (kSteps * 4 * (int)sizeof(Q)) + kk * (int)sizeof(Q);
     int st = 0, pb = 0;
     unsigned phase = 0;
     if (screen) {
       // A operand of mma.m16n8k16: centres g and g + 8 of the round at the features this lane reads of a row, as
       // fp16 or X's 16-bit type (the k slots {2kk, 2kk+1} and {2kk+8, 2kk+9} of super-step s are features
       // 16s + 4kk + {0, 1} and {2, 3}: the same permutation of K for A and B)
-      unsigned af[STEPS][4];
+      unsigned af[kSteps][4];
       {
         const long long* allc = a.centers + a.center_off;
         const long long p0 = allc[min(g, total - 1)], p1 = allc[min(g + kB, total - 1)];
-        const Q* c0 = reinterpret_cast<const Q*>(a.X) + (size_t)p0 * a.d4 + seg * (STEPS * 4) + kk;
-        const Q* c1 = reinterpret_cast<const Q*>(a.X) + (size_t)p1 * a.d4 + seg * (STEPS * 4) + kk;
+        const Q* c0 = reinterpret_cast<const Q*>(a.X) + (size_t)p0 * a.d4 + seg * (kSteps * 4) + kk;
+        const Q* c1 = reinterpret_cast<const Q*>(a.X) + (size_t)p1 * a.d4 + seg * (kSteps * 4) + kk;
 #pragma unroll
-        for (int s = 0; s < STEPS; ++s) {
+        for (int s = 0; s < kSteps; ++s) {
           const Q v0 = __ldg(c0 + 4 * s), v1 = __ldg(c1 + 4 * s);
           if constexpr (X16) {   // the centres as they are (element 2j in the low half of word j)
             af[s][0] = v0.x;
@@ -1090,7 +1031,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
           }
         }
       }
-      const unsigned h_off = smem_addr(stage0) + g * kRowBytesH + seg * (STEPS * 32) + kk * 8;
+      const unsigned h_off = smem_addr(stage0) + g * kRowBytesH + seg * (kSteps * 32) + kk * 8;
       const unsigned my_partf = smem_addr(&s_part[0][seg][0]) + lane * 16;
       // a stage holds tiles k and k + 1 (rows 0-7, 8-15); with n1 odd the last stage's second half repeats tile k
       for (int k = 0; k < n1; k += 2) {
@@ -1098,7 +1039,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
         const unsigned ap = h_off + st * kStageBytesX;
         float d[2][4] = {{0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
 #pragma unroll
-        for (int s = 0; s < STEPS; ++s) {
+        for (int s = 0; s < kSteps; ++s) {
           mma_f16<T>(d[0], af[s], lds64(ap + s * 32));
           mma_f16<T>(d[1], af[s], lds64(ap + 8 * kRowBytesH + s * 32));
         }
@@ -1124,19 +1065,8 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
       pb = 0;
     }
     const int nd = screen == 1 ? (s_na[2] + 7) / 8 : na;   // DMMA tiles
-    double breg[STEPS][4];
-    {
-      const long long pg = centers[min(g, nb - 1)];
-      const Q* cp = reinterpret_cast<const Q*>(a.X) + (size_t)pg * a.d4 + seg * (STEPS * 4) + kk;
-#pragma unroll
-      for (int s = 0; s < STEPS; ++s) {
-        const float4 v = ldg_q<T>(cp + 4 * s);
-        breg[s][0] = (double)v.x;
-        breg[s][1] = (double)v.y;
-        breg[s][2] = (double)v.z;
-        breg[s][3] = (double)v.w;
-      }
-    }
+    double breg[kSteps][4];
+    centre_slice(static_cast<const T*>(a.X), a.d4, centers[min(g, nb - 1)], seg, kk, breg);
     const unsigned my_part = smem_addr(&s_part[0][seg][lane * 2]);
     for (int k = 0; k < nd; ++k) {
       mbar_wait(&full[st], phase);
@@ -1145,13 +1075,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
 #pragma unroll
       for (int e = 0; e < 4; ++e) c[e][0] = c[e][1] = 0.0;
 #pragma unroll
-      for (int s = 0; s < STEPS; ++s) {
-        const float4 x = lds_quad<T>(ap + s * 4 * (unsigned)sizeof(Q));
-        dmma(c[0], (double)x.x, breg[s][0]);
-        dmma(c[1], (double)x.y, breg[s][1]);
-        dmma(c[2], (double)x.z, breg[s][2]);
-        dmma(c[3], (double)x.w, breg[s][3]);
-      }
+      for (int s = 0; s < kSteps; ++s) seg_step(c, lds_quad<T>(ap + s * 4 * (unsigned)sizeof(Q)), breg[s]);
       __syncwarp();
       if (lane == 0) mbar_arrive(&empty[st]);          // this warp has read its slice of the stage
       if (++st == kStagesX) {
@@ -1160,9 +1084,9 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
       }
       if (k >= kPartBufs) named_sync(1 + kPartBufs + pb, kSeg * 32 + 32);   // buffer released by its epilogue warp
       // lane (g,kk) holds (row g, centres 2kk, 2kk+1)
+      const double2 part = seg_partial(c);
       asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"(my_part + pb * (unsigned)(sizeof(double) * kSeg * 64)),
-                   "d"(combine4(c[0][0], c[1][0], c[2][0], c[3][0])), "d"(combine4(c[0][1], c[1][1], c[2][1], c[3][1]))
-                   : "memory");
+                   "d"(part.x), "d"(part.y) : "memory");
       asm volatile("fence.acq_rel.cta;" ::: "memory");   // partials visible before the arrive is counted
       named_arrive(1 + pb, kSeg * 32 + 32);
       if (++pb == kPartBufs) pb = 0;
@@ -1180,7 +1104,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
         __syncwarp();
         if (lane < 8) {
           const long long row = row_of_lane();
-          tma_load_1d(stage0 + (size_t)st * kStageBytesX + lane * kRowB, static_cast<const T*>(a.X) + (size_t)row * 2048,
+          tma_load_1d(stage0 + (size_t)st * kStageBytesX + lane * kRowB, static_cast<const T*>(a.X) + (size_t)row * kFastD,
                       kXRowBytes, &full[st]);
         }
         if (++st == kStagesX) {
@@ -1319,9 +1243,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
             double cn = 0.0;
 #pragma unroll
             for (int jc = 0; jc < kB; ++jc) cn = fmax(cn, s_xxc[crank * kB + jc]);
-            const double margin = 1e-6 * (1.0 + sqrt(xxa) + sqrt(cn));
-            a.seg_skip_out[(size_t)crank * a.skip_stride + row] =
-                (isfinite(M) && sqrt(fmax(sq, 0.0)) - a.seg_r[row] - M >= margin) ? 1 : 0;
+            a.seg_skip_out[(size_t)crank * a.skip_stride + row] = segment_skip(sq, a.seg_r[row], M, xxa, cn) ? 1 : 0;
           }
         } else if (a.lo + row < a.hi) {
           *reinterpret_cast<double2*>(a.dots + row * NC + crank * kB + (lane & 3) * 2) = make_double2(dot0, dot1);
@@ -1516,13 +1438,13 @@ __global__ void __launch_bounds__(256) seg_radius_kernel(const T* __restrict__ X
 }
 
 // per pass: seg_skip[s] = 1 when no row of segment s can get closer to this pass's centres.
-// Same tile machine as the candidate-pairs kernel (d == 8 * 16 * STEPS): the 8 warps of a CTA are
+// Same tile machine as the candidate-pairs kernel (d == kFastD): the 8 warps of a CTA are
 // the 8 K-segments, each holding its 1/8 of the pass's 8 centres in registers as fp64 B operands;
 // tiles of 8 anchor rows stream through a register ring (the next tile's loads are in flight while
 // this one is multiplied, so the kernel is not a chain of memory round trips); after the split-K
 // exchange warp w finishes segment w of the tile: canonical distances of its anchor to the 8
 // centres, the maximum of min_d over its rows, and the test.
-template <int STEPS, typename T>
+template <typename T>
 __global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const T* __restrict__ X, int d4, long long lo,
                                                                     const int* __restrict__ seg_start,
                                                                     const double* __restrict__ segR,
@@ -1546,29 +1468,18 @@ __global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const T* __r
   if ((int)blockIdx.x >= ntiles) return;
   const int lane = threadIdx.x & 31, seg = threadIdx.x >> 5, g = lane >> 2, kk = lane & 3;
   const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
-  const int lane_off = seg * (STEPS * 4) + kk;
+  const int lane_off = seg * (kSteps * 4) + kk;
   auto anchor = [&](int sg) -> long long { return lo + seg_start[min(sg, nseg - 1)]; };
   int t = blockIdx.x;
   // the first tile's anchor rows and the centres are requested back to back (one memory round trip)
-  float4 ring[STEPS];
+  float4 ring[kSteps];
   {
     const quad_t<T>* p0 = X4 + (size_t)anchor(t * 8 + g) * d4 + lane_off;
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) ring[s] = ldg_q<T>(p0 + 4 * s);
+    for (int s = 0; s < kSteps; ++s) ring[s] = ldg_q<T>(p0 + 4 * s);
   }
-  double breg[STEPS][4];
-  {
-    const long long p = centers[min(g, nb - 1)];   // padded with the last centre
-    const quad_t<T>* cp = X4 + (size_t)p * d4 + lane_off;
-#pragma unroll
-    for (int s = 0; s < STEPS; ++s) {
-      const float4 c4 = ldg_q<T>(cp + 4 * s);
-      breg[s][0] = (double)c4.x;
-      breg[s][1] = (double)c4.y;
-      breg[s][2] = (double)c4.z;
-      breg[s][3] = (double)c4.w;
-    }
-  }
+  double breg[kSteps][4];
+  centre_slice(X, d4, centers[min(g, nb - 1)], seg, kk, breg);   // padded with the last centre
   if (threadIdx.x < kB) s_xxc[threadIdx.x] = xx[centers[min((int)threadIdx.x, nb - 1)]];
   int buf = 0;
   for (; t < ntiles; t += gridDim.x) {
@@ -1590,16 +1501,12 @@ __global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const T* __r
 #pragma unroll
     for (int e = 0; e < 4; ++e) c[e][0] = c[e][1] = 0.0;
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) {
+    for (int s = 0; s < kSteps; ++s) {
       const float4 x = ring[s];
       if (has_next) ring[s] = ldg_q<T>(np + 4 * s);
-      dmma(c[0], (double)x.x, breg[s][0]);
-      dmma(c[1], (double)x.y, breg[s][1]);
-      dmma(c[2], (double)x.z, breg[s][2]);
-      dmma(c[3], (double)x.w, breg[s][3]);
+      seg_step(c, x, breg[s]);
     }
-    *reinterpret_cast<double2*>(&s_part[buf][seg][lane * 2]) =
-        make_double2(combine4(c[0][0], c[1][0], c[2][0], c[3][0]), combine4(c[0][1], c[1][1], c[2][1], c[3][1]));
+    *reinterpret_cast<double2*>(&s_part[buf][seg][lane * 2]) = seg_partial(c);
     __syncthreads();
     if (myseg < nseg) {
       double M = fmax(m0, m1);
@@ -1614,8 +1521,7 @@ __global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const T* __r
         double cn = 0.0;
 #pragma unroll
         for (int j = 0; j < kB; ++j) cn = fmax(cn, s_xxc[j]);
-        const double margin = 1e-6 * (1.0 + sqrt(xxa) + sqrt(cn));
-        seg_skip[myseg] = (isfinite(M) && sqrt(fmax(d2, 0.0)) - R - M >= margin) ? 1 : 0;
+        seg_skip[myseg] = segment_skip(d2, R, M, xxa, cn) ? 1 : 0;
       }
     }
     buf ^= 1;
@@ -1778,13 +1684,13 @@ __device__ void plan_body(const RankBlock* blocks, RankBlock* send, const double
 // every 8 x 8 block is written twice (d is symmetric; both halves hold the SAME bits, so the planner may read rows).
 // The pairs are dealt round-robin to the CTAs of the grid: with ~250 candidates that is 528 pairs over 148 CTAs
 // (3-4 each, all loads of a pair in flight together) instead of 8 sequential tiles per CTA on a quarter of the SMs.
-template <int STEPS, typename T>
+template <typename T>
 __device__ __forceinline__ void pairs_tiles(const T* __restrict__ X, int d4, const double* __restrict__ xx,
                                             const RankBlock* blocks, const CandView& v, int world,
                                             double* __restrict__ Dcc, double (*s_part)[kSeg][64], double* s_xxc) {
   const int lane = threadIdx.x & 31, seg = threadIdx.x >> 5, g = lane >> 2, kk = lane & 3;
   const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
-  const int lane_off = seg * (STEPS * 4) + kk;
+  const int lane_off = seg * (kSteps * 4) + kk;
   auto cand_row = [&](int pos) {
     int r, q;
     locate(v, world, min(pos, v.total - 1), r, q);
@@ -1805,11 +1711,11 @@ __device__ __forceinline__ void pairs_tiles(const T* __restrict__ X, int d4, con
     const long long crow = cand_row(col0 + g), arow = cand_row(t * 8 + g);
     const quad_t<T>* cp = X4 + (size_t)crow * d4 + lane_off;
     const quad_t<T>* ap = X4 + (size_t)arow * d4 + lane_off;
-    float4 cb4[STEPS], ring[STEPS];
+    float4 cb4[kSteps], ring[kSteps];
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) cb4[s] = ldg_q<T>(cp + 4 * s);
+    for (int s = 0; s < kSteps; ++s) cb4[s] = ldg_q<T>(cp + 4 * s);
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) ring[s] = ldg_q<T>(ap + 4 * s);
+    for (int s = 0; s < kSteps; ++s) ring[s] = ldg_q<T>(ap + 4 * s);
     if (threadIdx.x < kB) s_xxc[buf * kB + threadIdx.x] = xx[cand_row(col0 + threadIdx.x)];
     const int myrow = t * 8 + seg;                       // the row this warp finishes
     const double xxi = (myrow < v.total) ? xx[cand_row(myrow)] : 0.0;
@@ -1817,14 +1723,8 @@ __device__ __forceinline__ void pairs_tiles(const T* __restrict__ X, int d4, con
 #pragma unroll
     for (int e = 0; e < 4; ++e) c[e][0] = c[e][1] = 0.0;
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) {
-      dmma(c[0], (double)ring[s].x, (double)cb4[s].x);
-      dmma(c[1], (double)ring[s].y, (double)cb4[s].y);
-      dmma(c[2], (double)ring[s].z, (double)cb4[s].z);
-      dmma(c[3], (double)ring[s].w, (double)cb4[s].w);
-    }
-    *reinterpret_cast<double2*>(&s_part[buf][seg][lane * 2]) =
-        make_double2(combine4(c[0][0], c[1][0], c[2][0], c[3][0]), combine4(c[0][1], c[1][1], c[2][1], c[3][1]));
+    for (int s = 0; s < kSteps; ++s) seg_step(c, ring[s], cb4[s]);
+    *reinterpret_cast<double2*>(&s_part[buf][seg][lane * 2]) = seg_partial(c);
     __syncthreads();
     if (myrow < v.total && lane < kB && col0 + lane < v.total) {
       // Dcc[w * kCap + c] = d(row c, centre w) with the pass's operand roles (sklearn: (-2 x.c + |x|^2) + |c|^2, the
@@ -1839,7 +1739,7 @@ __device__ __forceinline__ void pairs_tiles(const T* __restrict__ X, int d4, con
   }
 }
 
-// fast path (d == 8 * 16 * STEPS): the pass kernel's tile machine on the gathered candidates.
+// fast path (d == kFastD): the pass kernel's tile machine on the gathered candidates.
 // CTA (cb, y): the 8 candidates of column block cb are the centres (their 1/8 K-slices live in the
 // registers of the 8 warps), row tiles y, y + gridDim.y, ... of the candidate list stream through
 // a register ring (from L2 mostly: the rows were just touched by the pass).  After the split-K
@@ -1847,7 +1747,7 @@ __device__ __forceinline__ void pairs_tiles(const T* __restrict__ X, int d4, con
 // The last CTA of the grid to finish runs the planner (plan_body) on the completed matrix, so a
 // round needs no separate plan launch.
 constexpr int kPlanSmem = 208 * 1024;    // dynamic shared memory of pairs_plan_kernel: the planner's staged distance rows
-template <int STEPS, typename T>
+template <typename T>
 __global__ void __launch_bounds__(kSeg * 32, 1) pairs_plan_kernel(const T* __restrict__ X, int d4,
                                                                   const double* __restrict__ xx, const RankBlock* blocks,
                                                                   RankBlock* send, unsigned int* hist, long long* out_idx,
@@ -1876,7 +1776,7 @@ __global__ void __launch_bounds__(kSeg * 32, 1) pairs_plan_kernel(const T* __res
   {
     const int world = ctl->world;
     const CandView v = view_of(blocks, world);
-    if (!v.fallback) pairs_tiles<STEPS, T>(X, d4, xx, blocks, v, world, Dcc, s_part, s_xxc);
+    if (!v.fallback) pairs_tiles<T>(X, d4, xx, blocks, v, world, Dcc, s_part, s_xxc);
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -2304,7 +2204,7 @@ struct WsLayout {
 };
 // rounds of 16 picks, applied by the paired pass (and screened): d == 2048 and batch >= 16 (vatlq_coreset_select
 // rounds batch down to a power of two)
-static bool paired_rounds(int d, int batch) { return d == kSeg * 16 * 16 && batch >= 2 * kB; }
+static bool paired_rounds(int d, int batch) { return d == kFastD && batch >= 2 * kB; }
 static WsLayout ws_layout(long long n, int world) {
   WsLayout L;
   size_t o = 0;
@@ -2402,11 +2302,11 @@ template <typename T>
 static int configure_pass_of() {
   VQ_CUDA(cudaFuncSetAttribute(pass_kernel_generic<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
   VQ_CUDA(cudaFuncSetAttribute(pass_kernel_generic<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<16, false, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
-  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<16, true, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
-  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<16, true, true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
-  VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<16, T>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-  VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<16, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPlanSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<false, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<true, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<true, true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<T>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPlanSmem));
   VQ_CUDA(cudaFuncSetAttribute(pairs_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
   VQ_CUDA(cudaFuncSetAttribute(pairwise_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
   return 0;
@@ -2440,7 +2340,7 @@ static int pair_grid() {
     cfg.attrs = &at;
     cfg.numAttrs = 1;
     int ncl = 0;
-    if (cudaOccupancyMaxActiveClusters(&ncl, pass_kernel_tma<16, true>, &cfg) == cudaSuccess && ncl > 0)
+    if (cudaOccupancyMaxActiveClusters(&ncl, pass_kernel_tma<true>, &cfg) == cudaSuccess && ncl > 0)
       grid = 2 * std::min(ncl, sm_count() / 2);
     cudaGetLastError();
   }
@@ -2467,8 +2367,8 @@ static int launch_pass_pair(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = 
   cfg.attrs = at;
   cfg.numAttrs = pdl ? 2 : 1;
   if (ev0) cudaEventRecord(ev0, stream);
-  if (filter) VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, true, true, T>, a));
-  else VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<16, true, false, T>, a));
+  if (filter) VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<true, true, T>, a));
+  else VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<true, false, T>, a));
   if (ev1) cudaEventRecord(ev1, stream);
   VQ_LAUNCHED();
   return 0;
@@ -2478,8 +2378,8 @@ template <typename T>
 static int launch_pass(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr, bool pdl = false) {
   if (int e = configure_pass()) return e;
   if (ev0) cudaEventRecord(ev0, stream);
-  const bool fast = a.d4 == kSeg * 4 * 16 && a.dots != nullptr;   // d = 2048
-  if (fast) VQ_CUDA(launch_pdl(pass_kernel_tma<16, false, false, T>, dim3(sm_count()), dim3(kWsThreads), kWsSmem, stream, pdl, a));
+  const bool fast = a.d4 == kFastD / 4 && a.dots != nullptr;
+  if (fast) VQ_CUDA(launch_pdl(pass_kernel_tma<false, false, T>, dim3(sm_count()), dim3(kWsThreads), kWsSmem, stream, pdl, a));
   else if ((a.d4 & 3) != 0) pass_kernel_generic<true, T><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
   else pass_kernel_generic<false, T><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
   if (ev1) cudaEventRecord(ev1, stream);
@@ -2519,7 +2419,7 @@ static int prune_setup(PruneState& P, const T* X, const Geom& G, int64_t row_lo,
   P.seg_skip = (unsigned char*)(w + L.seg_skip);
   P.skip_stride = L.skip_stride;
   const long long prune_min = g_prune_min_set >= 0 ? g_prune_min_set : prune_min_rows;
-  P.mode = (G.d4 == kSeg * 4 * 16 && own >= prune_min && own >= 8 && own < (1LL << 30))
+  P.mode = (G.d4 == kFastD / 4 && own >= prune_min && own >= 8 && own < (1LL << 30))
                ? (g_prune_mode_set >= 0 ? g_prune_mode_set : prune_env) : 0;
   P.filter_grid = (int)std::max<long long>(1, std::min<long long>(sm_count(), own / 8 + 1));   // tiles of 8 segments, grid-stride
   VQ_CUDA(cudaMemsetAsync(P.pc, 0, sizeof(PruneCtl), stream));
@@ -2539,7 +2439,7 @@ static int prune_setup(PruneState& P, const T* X, const Geom& G, int64_t row_lo,
 template <typename T>
 static int launch_filter(const PruneState& P, const PassArgs& a, cudaStream_t stream, int groups = 1) {
   dim3 grid((unsigned)P.filter_grid, (unsigned)groups);
-  prune_filter_kernel<16, T><<<grid, kSeg * 32, 0, stream>>>(static_cast<const T*>(a.X), a.d4, a.lo, P.seg_start, P.seg_r, a.m, a.xx, a.centers,
+  prune_filter_kernel<T><<<grid, kSeg * 32, 0, stream>>>(static_cast<const T*>(a.X), a.d4, a.lo, P.seg_start, P.seg_r, a.m, a.xx, a.centers,
                                                           a.n_centers, a.n_centers_imm, a.center_off, P.pc, P.seg_skip,
                                                           P.skip_stride);
   VQ_LAUNCHED();
@@ -2565,7 +2465,7 @@ int vq_launch_norms(const float* X, int64_t n, int d, double* xx, cudaStream_t s
 // cp.async.bulk, which needs a 16-byte aligned source in every dtype)
 static int check_coreset_x(const void* X, int dtype, int64_t n, int d, int64_t lo, int64_t hi) {
   if (int e = check_x(X, dtype, n, d, lo, hi)) return e;
-  VQ_REQUIRE(d != kSeg * 16 * 16 || ((uintptr_t)X & 15) == 0, "X must be 16-byte aligned when d = 2048");
+  VQ_REQUIRE(d != kFastD || ((uintptr_t)X & 15) == 0, "X must be 16-byte aligned when d = 2048");
   return 0;
 }
 
@@ -2703,7 +2603,7 @@ static int coreset_select(const T* X, int dtype, int64_t n, int d, int64_t row_l
   int fgrid = std::max(1, std::min(sm_count() * 4, (own + 255) / 256));
   VQ_REQUIRE(fgrid <= 4096 && sm_count() <= 4096, "grid too large for the arg-max scratch");
   const size_t pairs_smem = G.smem;
-  const bool fast_d = (G.d4 == kSeg * 4 * 16);   // d = 2048: register-resident centres
+  const bool fast_d = (G.d4 == kFastD / 4);   // register-resident centres
   const bool use_pair = paired_rounds(d, batch) && pair_grid() >= 2;   // 16 picks per round in one read of X
   // the fp16 screen of the paired pass (see "the screen" at pass_kernel_tma): 0 off, 1 on, 2 verify
   static const int screen_env = []() {
@@ -2795,7 +2695,7 @@ static int coreset_select(const T* X, int dtype, int64_t n, int d, int64_t row_l
       if (nbk > 1) {
         dim3 pg(kCap / kB, 4);
         if (fast_d) {
-          const cudaError_t le = launch_pdl(pairs_plan_kernel<16, T>, dim3(sm_count()), dim3(kSeg * 32), kPlanSmem, stream, true, X, G.d4,
+          const cudaError_t le = launch_pdl(pairs_plan_kernel<T>, dim3(sm_count()), dim3(kSeg * 32), kPlanSmem, stream, true, X, G.d4,
                                             (const double*)xx, blocks, send, hist, (long long*)out_idx, ctl, Dcc, mail,
                                             (unsigned long long)(seq0 + round_no), kPlanSmem / 8);
           if (le != cudaSuccess) {

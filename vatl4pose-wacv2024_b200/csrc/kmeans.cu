@@ -26,17 +26,12 @@
 #include <algorithm>
 #include <cmath>
 
-#include "common.cuh"
+#include "canonical.cuh"
 
 namespace vatlq {
 
 namespace km {
 
-__device__ __forceinline__ void dmma(double (&c)[2], double a, double b) {
-  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-      : "+d"(c[0]), "+d"(c[1])
-      : "d"(a), "d"(b));
-}
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem, bool valid) {
   const unsigned sz = valid ? 16u : 0u;      // src-size 0: the 16 bytes are zero-filled
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(smem)), "l"(gmem), "r"(sz) : "memory");

@@ -9,9 +9,10 @@
 //            per row = TMEM lane, so the minimum lives in a register).
 //   sweep 2  the same GEMM again for the same 128 rows: every (row, group of 8 centres) with
 //            t~(i,c) <= t~min(i) + 2 E(i) is appended to a list.
-//   rescore  the list, sorted by centre group, goes through the canonical fp64 DMMA tile machine of
-//            coreset.cu (8 centres as register-resident B operands, 8 listed rows per tile) and
-//            min_d is lowered with atomicMin on the bit pattern of the (non-negative) distance.
+//   rescore  the list, sorted by centre group, goes through the canonical fp64 DMMA tile the exact
+//            passes of coreset.cu use (canonical.cuh: 8 centres as register-resident B operands, 8
+//            listed rows per tile) and min_d is lowered with atomicMin on the bit pattern of the
+//            (non-negative) distance.
 //
 // Error bound.  kind::tf32 uses the upper 19 bits of each fp32 operand (relative error <= 2^-10 per
 // operand, whether truncated or rounded), products are accumulated in fp32 over K = 2048.  With
@@ -28,7 +29,7 @@
 #include <cstdlib>
 #include <cstring>
 
-#include "common.cuh"
+#include "canonical.cuh"
 
 namespace vatlq {
 
@@ -37,6 +38,7 @@ constexpr int TC_BN = 256;          // centres per tile (UMMA N)
 constexpr int TC_BK = 32;           // fp32 per k-block: 128 bytes = one 128B-swizzle atom row
 constexpr int TC_STAGES = 4;
 constexpr int TC_D = 2048;
+static_assert(TC_D == kFastD, "the re-score keeps 1/8 of a centre in registers (canonical.cuh)");
 constexpr int TC_KB = TC_D / TC_BK; // 64 k-blocks
 constexpr int TC_A_BYTES = TC_BM * TC_BK * 4;    // 16 KB
 constexpr int TC_B_BYTES = TC_BN * TC_BK * 4;    // 32 KB
@@ -303,27 +305,15 @@ __global__ void __launch_bounds__(256) tc_gather_kernel(const float* __restrict_
   }
 }
 
-// ---- exact re-scoring of the listed (centre group, row) pairs: the canonical fp64 tile of coreset.cu --------
-// (same instruction sequence: 8 K-segments by 8 warps, four DMMA chains per segment, fixed combine tree)
-constexpr int kSegT = 8;
-__device__ __forceinline__ void tdmma(double (&c)[2], double a, double b) {
-  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(c[0]), "+d"(c[1]) : "d"(a), "d"(b));
-}
-__device__ __forceinline__ double tcomb4(double p0, double p1, double p2, double p3) {
-  return __dadd_rn(__dadd_rn(p0, p1), __dadd_rn(p2, p3));
-}
-__device__ __forceinline__ double tcomb8(const double* p, int stride) {
-  return __dadd_rn(tcomb4(p[0], p[stride], p[2 * stride], p[3 * stride]),
-                   tcomb4(p[4 * stride], p[5 * stride], p[6 * stride], p[7 * stride]));
-}
-
+// ---- exact re-scoring of the listed (centre group, row) pairs on the canonical fp64 tile (canonical.cuh) --------
+// (the helpers the exact passes of coreset.cu use: 8 K-segments by 8 warps, four DMMA chains per segment, fixed
+// combine tree, so the re-scored distances are theirs bit for bit)
 // one CTA per centre group (8 labelled centres): its slice of the sorted pair list is found by binary search
-__global__ void __launch_bounds__(kSegT * 32, 1)
+__global__ void __launch_bounds__(kSeg * 32, 1)
 tc_rescore_kernel(const float* __restrict__ X, long long lo, const long long* __restrict__ centers, int L,
                   const double* __restrict__ xx, const int* __restrict__ sorted_group, const int* __restrict__ sorted_row,
                   const unsigned int* __restrict__ pair_count, unsigned int cap, double* __restrict__ min_d) {
-  constexpr int STEPS = 16;
-  __shared__ __align__(16) double s_part[kSegT][64];
+  __shared__ __align__(16) double s_part[kSeg][64];
   __shared__ double s_xxc[8];
   __shared__ int s_rng[2];
   const unsigned int npairs = min(pair_count[0], cap);
@@ -347,53 +337,32 @@ tc_rescore_kernel(const float* __restrict__ X, long long lo, const long long* __
   if (beg >= end) return;
   const int lane = threadIdx.x & 31, seg = threadIdx.x >> 5, g = lane >> 2, kk = lane & 3;
   const float4* X4 = reinterpret_cast<const float4*>(X);
-  const int lane_off = seg * (STEPS * 4) + kk;
+  const int lane_off = seg * (kSteps * 4) + kk;
   const int nc = min(8, L - grp * 8);
-  double breg[STEPS][4];
-  {
-    const long long p = centers[grp * 8 + min(g, nc - 1)];
-    const float4* cp = X4 + (size_t)p * (TC_D / 4) + lane_off;
-#pragma unroll
-    for (int s = 0; s < STEPS; ++s) {
-      const float4 c4 = __ldg(cp + 4 * s);
-      breg[s][0] = (double)c4.x;
-      breg[s][1] = (double)c4.y;
-      breg[s][2] = (double)c4.z;
-      breg[s][3] = (double)c4.w;
-    }
-  }
+  double breg[kSteps][4];
+  centre_slice(X, TC_D / 4, centers[grp * 8 + min(g, nc - 1)], seg, kk, breg);
   if (threadIdx.x < 8) s_xxc[threadIdx.x] = xx[centers[grp * 8 + min((int)threadIdx.x, nc - 1)]];
   for (int t0 = beg; t0 < end; t0 += 8) {
     const long long row = lo + sorted_row[min(t0 + g, end - 1)];
     const float4* rp = X4 + (size_t)row * (TC_D / 4) + lane_off;
-    float4 xr[STEPS];
+    float4 xr[kSteps];
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) xr[s] = __ldg(rp + 4 * s);
+    for (int s = 0; s < kSteps; ++s) xr[s] = __ldg(rp + 4 * s);
     double c[4][2];
 #pragma unroll
     for (int e = 0; e < 4; ++e) c[e][0] = c[e][1] = 0.0;
 #pragma unroll
-    for (int s = 0; s < STEPS; ++s) {
-      tdmma(c[0], (double)xr[s].x, breg[s][0]);
-      tdmma(c[1], (double)xr[s].y, breg[s][1]);
-      tdmma(c[2], (double)xr[s].z, breg[s][2]);
-      tdmma(c[3], (double)xr[s].w, breg[s][3]);
-    }
+    for (int s = 0; s < kSteps; ++s) seg_step(c, xr[s], breg[s]);
     __syncthreads();                               // (the previous tile's partials have been consumed)
-    *reinterpret_cast<double2*>(&s_part[seg][lane * 2]) =
-        make_double2(tcomb4(c[0][0], c[1][0], c[2][0], c[3][0]), tcomb4(c[0][1], c[1][1], c[2][1], c[3][1]));
+    *reinterpret_cast<double2*>(&s_part[seg][lane * 2]) = seg_partial(c);
     __syncthreads();
     // warp w finishes row w of the tile: lane j < 8 holds centre j
     const int myrow = t0 + seg;
     if (myrow < end) {
       const long long ri = lo + sorted_row[myrow];
       double sq = INFINITY;
-      if (lane < 8) {
-        const double dot = tcomb8(&s_part[0][seg * 8 + lane], 64);
-        double t = __dmul_rn(-2.0, dot);
-        t = __dadd_rn(t, xx[ri]);
-        sq = __dadd_rn(t, s_xxc[lane]);            // (padded centres repeat the last one: min is idempotent)
-      }
+      // (padded centres repeat the last one: min is idempotent)
+      if (lane < 8) sq = sq_from_dot(combine8(&s_part[0][seg * 8 + lane], 64), xx[ri], s_xxc[lane]);
 #pragma unroll
       for (int o = 4; o; o >>= 1) sq = fmin(sq, __shfl_xor_sync(0xffffffffu, sq, o));
       if (lane == 0) {
@@ -541,7 +510,7 @@ extern "C" int vatlq_coreset_init_tc(const float* X, int64_t n, int d, int64_t r
                                           (int*)(w + T.sr), (int)h_count[0], 0, 32, stream));
   g_launches.fetch_add(1);
   if (int e = fill_f64(min_d + row_lo, own, INFINITY, stream)) return e;
-  tc_rescore_kernel<<<(L + 7) / 8, kSegT * 32, 0, stream>>>(X, row_lo, (const long long*)labeled, L, xx, (const int*)(w + T.sg),
+  tc_rescore_kernel<<<(L + 7) / 8, kSeg * 32, 0, stream>>>(X, row_lo, (const long long*)labeled, L, xx, (const int*)(w + T.sg),
                                                             (const int*)(w + T.sr), count, T.cap, min_d);
   VQ_LAUNCHED();
   return 0;
