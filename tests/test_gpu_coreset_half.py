@@ -75,7 +75,7 @@ def test_batches(built_lib, batch, dtype):
     unc = v.synth.pool_unc(n, device="cuda:0")
     s = _check(v, X, unc, [], 48 if batch == 1 else 160, 0.0, f"batch {batch} {dtype}", batch=batch)
     if batch < 16:
-        assert s["screened"] == 0                # the solo pass does not screen
+        assert s["screened"] == 0                # an unpaired selection (the solo pass) does not screen
 
 
 @pytest.mark.parametrize("dtype", DTYPES)

@@ -97,3 +97,21 @@ def test_labelled_set_initialisation_is_pruned_exactly(built_lib):
     assert torch.equal(p_off, p_on) and torch.equal(md_off, md_on) and torch.equal(md_off, md_ver)
     assert s_ver["violations"] == 0
     assert s_ver["tiles"] > 700 * (n // 8)                 # the 750 initialisation passes were counted (verify collects them)
+
+
+@pytest.mark.parametrize("batch", [8, 16])
+def test_tile_counts_are_the_passes_rows(built_lib, batch):
+    """Every pass that applies centres sees each owned 8-row tile once, and nothing else counts as a tile: in
+    particular not the segment filter's tiles of anchor rows (batch 8: the solo filter, batch 16: the paired one)."""
+    v = built_lib
+    n = 20005
+    X = torch.from_numpy(_ragged_clusters(n, 2048, 21)).cuda()
+    unc = torch.from_numpy(np.random.default_rng(22).uniform(0, 1, n)).cuda()
+    v.ops.set_prune("on", 0)
+    try:
+        _, st = v.ops.coreset_select(X, unc, [], 300, 0.6, 0.01, batch=batch, tc_init=False)
+        torch.cuda.synchronize()
+    finally:
+        v.ops.set_prune("env", -1)
+    assert st.passes > 0 and st.tiles_streamed < st.tiles       # tiles were pruned, so the filter ran
+    assert st.tiles == st.passes * ((n + 7) // 8), (st.tiles, st.passes)

@@ -1,6 +1,6 @@
 """Short driver for ncu captures at bench scale: one heat-map scan, the 8f kernels, and a core-set
 selection long enough to reach the pruned steady state.
-    ncu --set full --clock-control none --import-source on -k regex:'pass_kernel_tma|prune_filter|pairs_plan' \
+    ncu --set full --clock-control none --import-source on -k regex:'pass_kernel_tma|pairs_plan' \
         --launch-skip 1500 -c 8 -o gpurun_out/prof_coreset python tools/prof_kernels.py
     ncu --set full --clock-control none -k regex:'scan_tma|entropy_kernel|cos_colsum_kernel|cos_rowsum' -c 6 \
         -o gpurun_out/prof_stream python tools/prof_kernels.py

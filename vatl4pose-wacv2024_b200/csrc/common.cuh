@@ -149,7 +149,7 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // ---------------------------------------------------------------- programmatic dependent launch
-// Chains of short kernels (a core-set round: candidate tiles + planner, segment filter, paired pass, solo pass; a
+// Chains of short kernels (a core-set round: candidate tiles + planner, segment filter, pass; a
 // k-means++ step: seven kernels) are launched with cudaLaunchAttributeProgrammaticStreamSerialization.  Each starts with pdl_enter(): wait until
 // the previous kernel has completed and flushed (so the data flow is exactly the stream order), then let the NEXT
 // kernel's CTAs be scheduled as SMs free up — they sit in their own pdl_enter() until this grid is done.  What is

@@ -17,9 +17,11 @@
 // tiles; its last CTA replays the greedy rule on the candidates, emits the picks and chooses the next
 // theta from the score histogram) -> the segment filter (exact pruning flags of both centre groups: the
 // FILTER mode of the pass kernel on the segment anchors) -> the paired pass (a cluster of two CTAs
-// applies 16 picks per read of X; its epilogue lists the next candidates, the exact arg-max for the
-// fallback and the next histogram, and pushes the rank's block to the peers' mailboxes).  Rounds of
-// <= 8 picks take the solo pass.  Other feature widths use the generic kernels (pairs / plan / pass).
+// applies the round's 1..16 picks in one read of X; its epilogue lists the next candidates, the exact
+// arg-max for the fallback and the next histogram, and pushes the rank's block to the peers' mailboxes).
+// Selections that do not pair (batch < 16, or no clusters of two) and the labelled-set initialisation take
+// the solo forms of the same kernel (filter, then pass, per 8 centres).  Other feature widths use the
+// generic kernels (pairs / plan / pass).
 #include <dlfcn.h>
 
 #include <algorithm>
@@ -297,9 +299,7 @@ struct PassArgs {
   unsigned char* did_work;   // optional: set to 1 when this launch applied centres (pass timing bookkeeping)
   double* dots;              // fast path: [owned row][8 or 16] canonical dot products: epilogue warps -> row finishing
   // exact pruning (fast path only, see "pruning" below): tiles whose segments were all flagged by
-  // prune_filter_kernel are not streamed; their rows keep min_d and only take part in the epilogue
-  int only_if_le8;           // solo pass of a 16-pick round: run only when the round planned <= 8 picks (else the
-                             // paired pass applies all of them in ONE read of X)
+  // the filter mode are not streamed; their rows keep min_d and only take part in the epilogue
   const int* seg_of_row;             // [owned row] -> segment id, or null
   size_t skip_stride;                // paired pass: the flags of centre group 1 start at seg_skip + skip_stride
   const unsigned char* seg_skip;     // [segment] 1: no row of the segment can get closer to this pass's centres
@@ -308,7 +308,7 @@ struct PassArgs {
   const int* seg_start;              // [nseg + 1] first owned row of every segment
   const double* seg_r;               // [nseg] segment radius
   const int* nseg;                   // device count of segments
-  unsigned char* seg_skip_out;       // [2][skip_stride] flags written by the filter mode
+  unsigned char* seg_skip_out;       // flags written by the filter mode (paired: group 1's at + skip_stride)
   int prune_mode;                    // 0 off, 1 skip, 2 verify (stream everything, count rows that changed anyway)
   unsigned long long* prune_stats;   // [0] tiles seen, [1] tiles streamed, [2] verify violations
   // paired pass only, see "the screen" at pass_kernel_tma: 0 off, 1 DMMA only the rows the fp16 screen cannot
@@ -345,26 +345,23 @@ __device__ __forceinline__ void emit_row(RankBlock* send, double theta_emit, lon
   }
 }
 
-// flush the CTA's histogram, reduce the arg-max over the CTA, and let the last CTA of the grid
-// finish the rank's block header (every thread of the CTA calls this)
-__device__ void publish_pass(const PassArgs& a, Best best, bool do_hist, const unsigned int* s_hist, bool final_pass) {
+// reduce the arg-max over the CTA and let the last CTA of the grid finish the rank's block header `out`: the exact
+// arg-max, theta, mode, the in-window count (*inwin, read once every CTA is done; null: 0) and, with reset_count,
+// count = 0; then push it to the peers (every thread of the CTA calls this; nw: warps of the CTA)
+__device__ void publish_header(int nw, Best best, Best* partial, Ctl* ctl, RankBlock* out, const PushArgs& push,
+                               double theta, long long mode, const unsigned int* inwin, bool reset_count) {
   __shared__ Best s_best[32];
   __shared__ unsigned int s_last;
-  const int tid = threadIdx.x, nw = (blockDim.x + 31) >> 5;
-  if (do_hist) {
-    for (int b = tid; b < kNB + 1; b += blockDim.x)
-      if (s_hist[b]) atomicAdd(&a.hist[b], s_hist[b]);
-  }
-  if (a.send == nullptr || !final_pass) return;
+  const int tid = threadIdx.x;
   best = warp_best(best);
   if ((tid & 31) == 0) s_best[tid >> 5] = best;
   __syncthreads();
   if (tid == 0) {
     for (int k = 1; k < nw; ++k)
       if (better(s_best[k].s, s_best[k].i, best.s, best.i)) best = s_best[k];
-    a.partial[blockIdx.x] = best;
+    partial[blockIdx.x] = best;
     __threadfence();
-    s_last = (atomicAdd(&a.ctl->filter_ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
+    s_last = (atomicAdd(&ctl->filter_ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
   }
   __syncthreads();
   if (s_last) {
@@ -372,8 +369,8 @@ __device__ void publish_pass(const PassArgs& a, Best best, bool do_hist, const u
     Best b{-INFINITY, 0x7fffffffffffffffLL};
     for (int k = tid; k < (int)gridDim.x; k += blockDim.x) {
       Best q;
-      q.s = ((volatile Best*)a.partial)[k].s;
-      q.i = ((volatile Best*)a.partial)[k].i;
+      q.s = ((volatile Best*)partial)[k].s;
+      q.i = ((volatile Best*)partial)[k].i;
       if (better(q.s, q.i, b.s, b.i)) b = q;
     }
     b = warp_best(b);
@@ -383,19 +380,74 @@ __device__ void publish_pass(const PassArgs& a, Best best, bool do_hist, const u
     if (tid == 0) {
       for (int k = 1; k < nw; ++k)
         if (better(s_best[k].s, s_best[k].i, b.s, b.i)) b = s_best[k];
-      a.send->smax = b.s;
-      a.send->smax_idx = b.i;
-      a.send->theta = a.ctl->theta_emit;
-      a.send->mode = a.ctl->emit_mode;
-      a.send->inwin = do_hist ? (long long)((volatile unsigned int*)a.hist)[kNB] : 0;
-      a.ctl->filter_ticket = 0;
+      if (reset_count) out->count = 0;
+      out->smax = b.s;
+      out->smax_idx = b.i;
+      out->theta = theta;
+      out->mode = mode;
+      out->inwin = inwin ? (long long)*(volatile const unsigned int*)inwin : 0;
+      ctl->filter_ticket = 0;
       __threadfence();
     }
-    if (a.push.peers != nullptr) {
+    if (push.peers != nullptr) {
       __syncthreads();
-      push_block(a.push, a.send);
+      push_block(push, out);
     }
   }
+}
+
+// flush the CTA's histogram; the round's last pass publishes the block header (every thread of the CTA calls this)
+__device__ void publish_pass(const PassArgs& a, Best best, bool do_hist, const unsigned int* s_hist, bool final_pass) {
+  if (do_hist) {
+    for (int b = threadIdx.x; b < kNB + 1; b += blockDim.x)
+      if (s_hist[b]) atomicAdd(&a.hist[b], s_hist[b]);
+  }
+  if (a.send == nullptr || !final_pass) return;
+  publish_header((blockDim.x + 31) >> 5, best, a.partial, a.ctl, a.send, a.push, a.ctl->theta_emit, a.ctl->emit_mode,
+                 do_hist ? a.hist + kNB : nullptr, false);
+}
+
+// what a pass reads from the control block to finish its rows
+struct ApplyConst {
+  double h_lo, h_inv, wd, wu, theta_emit;
+  int rule;
+  bool do_hist, emit;
+};
+__device__ __forceinline__ ApplyConst apply_const(const PassArgs& a, bool final_pass) {
+  ApplyConst c{0.0, 0.0, 0.0, 0.0, INFINITY, 0, false, false};
+  c.do_hist = a.hist != nullptr && a.ctl != nullptr && a.ctl->W > 0.0 && final_pass;
+  c.emit = a.send != nullptr && final_pass;
+  if (a.ctl) {
+    c.rule = a.ctl->rule;
+    c.wd = a.ctl->wd;
+    c.wu = a.ctl->wu;
+    c.theta_emit = a.ctl->theta_emit;
+    if (c.do_hist) {
+      c.h_lo = a.ctl->U - a.ctl->W;
+      c.h_inv = (double)kNB / a.ctl->W;
+    }
+  }
+  return c;
+}
+// the end of a row's finishing once its new min_d is known (and written): unc := 0 for a pick, the score, the
+// candidate record and the arg-max.  Returns the histogram bin of the new score (-1: outside the window / no histogram)
+__device__ __forceinline__ int finish_row(const PassArgs& a, const ApplyConst& c, long long i, double dmin, bool picked,
+                                          Best& best) {
+  if (a.unc) {
+    double u = a.unc[i];
+    if (picked) {
+      u = 0.0;  // uncertainty[ind] = 0  (:848)
+      a.unc[i] = 0.0;
+    }
+    const double sc = score_of(c.rule, c.wd, c.wu, dmin, u);
+    a.score[i] = sc;
+    if (c.emit) emit_row(a.send, c.theta_emit, i, dmin, u, sc, best);
+    if (c.do_hist) {
+      const double fb = (sc - c.h_lo) * c.h_inv;
+      if (fb >= 0.0) return (int)fmin(fb, (double)(kNB - 1));
+    }
+  }
+  return -1;
 }
 
 constexpr int kTeams = kPassThreads / 32 / kSeg;   // 2 teams of 8 warps
@@ -428,21 +480,10 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
       s_pick[j] = p;
     }
   }
-  const bool do_hist = a.hist != nullptr && a.ctl != nullptr && a.ctl->W > 0.0 && final_pass;
-  double h_lo = 0.0, h_inv = 0.0, wd = 0.0, wu = 0.0, theta_emit = INFINITY;
-  int rule = 0;
+  const ApplyConst ac = apply_const(a, final_pass);
   Best best{-INFINITY, 0x7fffffffffffffffLL};
-  if (a.ctl) {
-    rule = a.ctl->rule;
-    wd = a.ctl->wd;
-    wu = a.ctl->wu;
-    theta_emit = a.ctl->theta_emit;
-    if (do_hist) {
-      h_lo = a.ctl->U - a.ctl->W;
-      h_inv = (double)kNB / a.ctl->W;
-      for (int b = threadIdx.x; b < kNB + 1; b += blockDim.x) s_hist[b] = 0u;
-    }
-  }
+  if (ac.do_hist)
+    for (int b = threadIdx.x; b < kNB + 1; b += blockDim.x) s_hist[b] = 0u;
   __syncthreads();
 
   const Q* X4 = reinterpret_cast<const Q*>(a.X);
@@ -479,26 +520,13 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
       if (live && kk == 0) {
         const double dmin = fmin(a.m[i], dm);
         a.m[i] = dmin;
-        if (a.unc) {
-          bool picked = false;
+        bool picked = false;
 #pragma unroll
-          for (int j = 0; j < kB; ++j) picked = picked || (s_pick[j] == i);
-          double u = a.unc[i];
-          if (picked) {
-            u = 0.0;  // uncertainty[ind] = 0  (:848)
-            a.unc[i] = 0.0;
-          }
-          const double sc = score_of(rule, wd, wu, dmin, u);
-          a.score[i] = sc;
-          if (a.send && final_pass) emit_row(a.send, theta_emit, i, dmin, u, sc, best);
-          if (do_hist) {
-            const double fb = (sc - h_lo) * h_inv;
-            if (fb >= 0.0) {
-              const int b = (int)fmin(fb, (double)(kNB - 1));
-              atomicAdd(&s_hist[b], 1u);
-              atomicAdd(&s_hist[kNB], 1u);
-            }
-          }
+        for (int j = 0; j < kB; ++j) picked = picked || (s_pick[j] == i);
+        const int b = finish_row(a, ac, i, dmin, picked, best);
+        if (b >= 0) {
+          atomicAdd(&s_hist[b], 1u);
+          atomicAdd(&s_hist[kNB], 1u);
         }
       }
     }
@@ -564,34 +592,13 @@ __global__ void __launch_bounds__(kPassThreads, 1) pass_kernel_generic(PassArgs 
     }
   }
   __syncthreads();
-  publish_pass(a, best, do_hist, s_hist, final_pass);
+  publish_pass(a, best, ac.do_hist, s_hist, final_pass);
 }
 
 // second half of the fast-path pass: one thread per row turns the kB canonical dot products
 // into the distance to the nearest new centre (min_j sqrt(max(t_j, 0)) == sqrt(max(min_j t_j, 0))
 // bit for bit, sqrt being monotone and correctly rounded: one square root per row instead of kB),
 // the running minimum, unc/score, the candidate list, the histogram and the arg-max
-struct ApplyConst {
-  double h_lo, h_inv, wd, wu, theta_emit;
-  int rule;
-  bool do_hist, emit;
-};
-__device__ __forceinline__ ApplyConst apply_const(const PassArgs& a, bool final_pass) {
-  ApplyConst c{0.0, 0.0, 0.0, 0.0, INFINITY, 0, false, false};
-  c.do_hist = a.hist != nullptr && a.ctl != nullptr && a.ctl->W > 0.0 && final_pass;
-  c.emit = a.send != nullptr && final_pass;
-  if (a.ctl) {
-    c.rule = a.ctl->rule;
-    c.wd = a.ctl->wd;
-    c.wu = a.ctl->wu;
-    c.theta_emit = a.ctl->theta_emit;
-    if (c.do_hist) {
-      c.h_lo = a.ctl->U - a.ctl->W;
-      c.h_inv = (double)kNB / a.ctl->W;
-    }
-  }
-  return c;
-}
 // tile_mode: 0 streamed, 1 pruned (no dot products were computed: min_d stays), 2 verify (streamed
 // although the filter flagged it: count the rows whose min_d moved anyway — must stay 0), 3 screen verify
 // (computed although the screen decided the row: the same count, into screen_stats[2])
@@ -619,21 +626,7 @@ __device__ __forceinline__ int apply_row(const PassArgs& a, const ApplyConst& c,
   if (tile_mode == 2 && (dmin != m_old || picked)) atomicAdd(&a.prune_stats[2], 1ULL);
   if (tile_mode == 3 && (dmin != m_old || picked)) atomicAdd(&a.screen_stats[2], 1ULL);
   if (tile_mode != 1) a.m[i] = dmin;
-  if (a.unc) {
-    double u = a.unc[i];
-    if (picked) {
-      u = 0.0;  // uncertainty[ind] = 0  (:848)
-      a.unc[i] = 0.0;
-    }
-    const double sc = score_of(c.rule, c.wd, c.wu, dmin, u);
-    a.score[i] = sc;
-    if (c.emit) emit_row(a.send, c.theta_emit, i, dmin, u, sc, best);
-    if (c.do_hist) {
-      const double fb = (sc - c.h_lo) * c.h_inv;
-      if (fb >= 0.0) return (int)fmin(fb, (double)(kNB - 1));
-    }
-  }
-  return -1;
+  return finish_row(a, c, i, dmin, picked, best);
 }
 
 // ---------------------------------------------------------------- the pass over X, fast path
@@ -835,24 +828,14 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
   double* s_nc = reinterpret_cast<double*>(s_mask + kMaxTilesCta);
 
   pdl_enter();
-  const int total = a.n_centers ? *a.n_centers : a.n_centers_imm;
+  // this launch applies centres [center_off, center_off + NC) of the list, CTA r of a pair group r (the filter: the
+  // flags of group r); a short group is padded with the last centre (min() is idempotent), so a paired pass applies
+  // any round of 1..16 picks and a group without centres of its own only repeats the last one
+  const int total = (a.n_centers ? *a.n_centers : a.n_centers_imm) - a.center_off;
+  if (total <= 0) return;
+  const bool final_pass = NC >= total;
+  auto centre = [&](int j) { return (a.centers + a.center_off)[min(j, total - 1)]; };
   const int crank = PAIR ? (int)cluster_ctarank() : 0;
-  bool final_pass;
-  int nb;
-  if (PAIR && FILTER) {
-    nb = min(kB, total - kB * crank);              // group r's flags; a group without centres has nothing to do
-    final_pass = false;
-    if (nb <= 0) return;
-  } else if (PAIR) {
-    if (total <= kB) return;                       // (both CTAs of the pair: the solo pass handles short rounds)
-    nb = min(kB, total - kB * crank);
-    final_pass = true;
-  } else {
-    if (a.only_if_le8 && total > kB) return;
-    nb = pass_centers(a, final_pass);
-    if (nb <= 0) return;
-  }
-  const long long* centers = a.centers + a.center_off + kB * crank;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const bool clocked = !FILTER && a.ctl != nullptr && blockIdx.x == 0 && threadIdx.x == 0;
   unsigned long long tq0 = 0, tq1 = 0, tq2 = 0, tq3 = 0;
@@ -864,9 +847,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     if (a.did_work) *a.did_work = 1;
   }
   if (threadIdx.x < NC) {
-    // every centre the finishing sees (padded with the last one: min() is idempotent)
-    const int last = PAIR ? total - 1 : nb - 1;
-    const long long p = (a.centers + a.center_off)[min((int)threadIdx.x, last)];
+    const long long p = centre(threadIdx.x);   // every centre the finishing sees
     s_xxc[threadIdx.x] = a.xx[p];
     s_nc[threadIdx.x] = sqrt(a.xx[p]);
     s_pick[threadIdx.x] = p;
@@ -952,7 +933,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
   } else if (threadIdx.x == 0) {
     *s_na = nt;
     s_na[1] = (nt + 1 - crank) / 2;
-    if (a.prune_stats && nt > 0 && crank == 0) {
+    if (!FILTER && a.prune_stats && nt > 0 && crank == 0) {   // (the filter's anchor tiles are not rows streamed)
       atomicAdd(&a.prune_stats[0], (unsigned long long)nt);
       atomicAdd(&a.prune_stats[1], (unsigned long long)nt);
     }
@@ -1011,8 +992,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
       // 16s + 4kk + {0, 1} and {2, 3}: the same permutation of K for A and B)
       unsigned af[kSteps][4];
       {
-        const long long* allc = a.centers + a.center_off;
-        const long long p0 = allc[min(g, total - 1)], p1 = allc[min(g + kB, total - 1)];
+        const long long p0 = centre(g), p1 = centre(g + kB);
         const Q* c0 = reinterpret_cast<const Q*>(a.X) + (size_t)p0 * a.d4 + seg * (kSteps * 4) + kk;
         const Q* c1 = reinterpret_cast<const Q*>(a.X) + (size_t)p1 * a.d4 + seg * (kSteps * 4) + kk;
 #pragma unroll
@@ -1066,7 +1046,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
     }
     const int nd = screen == 1 ? (s_na[2] + 7) / 8 : na;   // DMMA tiles
     double breg[kSteps][4];
-    centre_slice(static_cast<const T*>(a.X), a.d4, centers[min(g, nb - 1)], seg, kk, breg);
+    centre_slice(static_cast<const T*>(a.X), a.d4, centre(kB * crank + g), seg, kk, breg);
     const unsigned my_part = smem_addr(&s_part[0][seg][lane * 2]);
     for (int k = 0; k < nd; ++k) {
       mbar_wait(&full[st], phase);
@@ -1228,7 +1208,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
         const long long row = ((long long)cid + (long long)k * ncl) * 8 + r;   // relative to a.lo (FILTER: segment id)
         if (FILTER) {
           // segment `row`: nearest of this group's centres to its anchor, largest min_d of its rows, the test of
-          // "pruning (exact)" below — same arithmetic as prune_filter_kernel, on the pass's tile machine
+          // "pruning (exact)" below, on the pass's tile machine
           const int kk = lane & 3, sg = (int)min(row, (long long)nseg - 1);
           const int a0 = a.seg_start[sg], e0 = a.seg_start[sg + 1];
           const double xxa = a.xx[a.lo + a0];
@@ -1315,7 +1295,11 @@ __global__ void __launch_bounds__(kWsThreads, 1) pass_kernel_tma(PassArgs a) {
 // the pruned pass writes exactly the bits the full pass would: the pick list cannot change.  A
 // picked row is never pruned (its own segment has d(a_s,c) <= R_s).  VATLQ_PRUNE=verify streams
 // everything and counts rows of flagged tiles whose min_d moved (tests assert 0).
-constexpr int kSegMax = 64;   // <= 64: the filter reads a segment's min_d as two values per lane
+// The flags come from the FILTER mode of pass_kernel_tma: its tiles are 8 anchor rows, and its epilogue takes the
+// canonical distances of each anchor to the group's 8 centres, the largest min_d of the segment's rows and the test.
+// Every group of a round is flagged before the round's first pass: the largest min_d a later group reads can only
+// be larger than what its pass will see, so its flags stay exact.
+constexpr int kSegMax = 64;   // longest segment (rows): bounds the min_d reads of the filter per segment
 struct PruneCtl {
   double sum;                      // sum of the finite consecutive-row distances
   unsigned long long cnt;
@@ -1437,97 +1421,6 @@ __global__ void __launch_bounds__(256) seg_radius_kernel(const T* __restrict__ X
   }
 }
 
-// per pass: seg_skip[s] = 1 when no row of segment s can get closer to this pass's centres.
-// Same tile machine as the candidate-pairs kernel (d == kFastD): the 8 warps of a CTA are
-// the 8 K-segments, each holding its 1/8 of the pass's 8 centres in registers as fp64 B operands;
-// tiles of 8 anchor rows stream through a register ring (the next tile's loads are in flight while
-// this one is multiplied, so the kernel is not a chain of memory round trips); after the split-K
-// exchange warp w finishes segment w of the tile: canonical distances of its anchor to the 8
-// centres, the maximum of min_d over its rows, and the test.
-template <typename T>
-__global__ void __launch_bounds__(kSeg * 32, 1) prune_filter_kernel(const T* __restrict__ X, int d4, long long lo,
-                                                                    const int* __restrict__ seg_start,
-                                                                    const double* __restrict__ segR,
-                                                                    const double* __restrict__ m, const double* __restrict__ xx,
-                                                                    const long long* __restrict__ centers_all,
-                                                                    const int* n_centers, int n_centers_imm, int center_off,
-                                                                    const PruneCtl* pc, unsigned char* __restrict__ seg_skip,
-                                                                    size_t skip_stride) {
-  __shared__ __align__(16) double s_part[2][kSeg][64];
-  __shared__ double s_xxc[kB];
-  // blockIdx.y = centre group of the round: group y's flags are for the pass that applies centres
-  // [center_off + 8y, +8).  All groups are evaluated BEFORE the round's first pass: the max min_d a later
-  // group reads can only be larger than what its pass will see, so its flags are conservative (exact).
-  center_off += (int)blockIdx.y * kB;
-  seg_skip += (size_t)blockIdx.y * skip_stride;
-  const int nb = min(kB, (n_centers ? *n_centers : n_centers_imm) - center_off);   // like pass_centers()
-  if (nb <= 0) return;
-  const long long* centers = centers_all + center_off;
-  const int nseg = pc->nseg;
-  const int ntiles = (nseg + 7) / 8;
-  if ((int)blockIdx.x >= ntiles) return;
-  const int lane = threadIdx.x & 31, seg = threadIdx.x >> 5, g = lane >> 2, kk = lane & 3;
-  const quad_t<T>* X4 = reinterpret_cast<const quad_t<T>*>(X);
-  const int lane_off = seg * (kSteps * 4) + kk;
-  auto anchor = [&](int sg) -> long long { return lo + seg_start[min(sg, nseg - 1)]; };
-  int t = blockIdx.x;
-  // the first tile's anchor rows and the centres are requested back to back (one memory round trip)
-  float4 ring[kSteps];
-  {
-    const quad_t<T>* p0 = X4 + (size_t)anchor(t * 8 + g) * d4 + lane_off;
-#pragma unroll
-    for (int s = 0; s < kSteps; ++s) ring[s] = ldg_q<T>(p0 + 4 * s);
-  }
-  double breg[kSteps][4];
-  centre_slice(X, d4, centers[min(g, nb - 1)], seg, kk, breg);   // padded with the last centre
-  if (threadIdx.x < kB) s_xxc[threadIdx.x] = xx[centers[min((int)threadIdx.x, nb - 1)]];
-  int buf = 0;
-  for (; t < ntiles; t += gridDim.x) {
-    const int tn = t + gridDim.x;
-    const bool has_next = tn < ntiles;
-    const quad_t<T>* np = X4 + (size_t)anchor((has_next ? tn : t) * 8 + g) * d4 + lane_off;
-    const int myseg = t * 8 + seg;                       // the segment this warp finishes
-    // everything the test needs is requested BEFORE the multiply loop and consumed after it:
-    // min_d of the segment's rows (segments hold <= kSegMax = 64 rows: two per lane), |a|^2, R
-    double m0 = 0.0, m1 = 0.0, xxa = 0.0, R = 0.0;
-    if (myseg < nseg) {
-      const int a = seg_start[myseg], e = seg_start[myseg + 1];
-      if (a + lane < e) m0 = m[lo + a + lane];
-      if (a + lane + 32 < e) m1 = m[lo + a + lane + 32];
-      xxa = xx[lo + a];
-      R = segR[myseg];
-    }
-    double c[4][2];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) c[e][0] = c[e][1] = 0.0;
-#pragma unroll
-    for (int s = 0; s < kSteps; ++s) {
-      const float4 x = ring[s];
-      if (has_next) ring[s] = ldg_q<T>(np + 4 * s);
-      seg_step(c, x, breg[s]);
-    }
-    *reinterpret_cast<double2*>(&s_part[buf][seg][lane * 2]) = seg_partial(c);
-    __syncthreads();
-    if (myseg < nseg) {
-      double M = fmax(m0, m1);
-      double d2 = INFINITY;
-      if (lane < kB) d2 = sq_from_dot(combine8(&s_part[buf][0][seg * 8 + lane], 64), xxa, s_xxc[lane]);
-#pragma unroll
-      for (int o = 16; o; o >>= 1) {
-        M = fmax(M, __shfl_xor_sync(0xffffffffu, M, o));
-        d2 = fmin(d2, __shfl_xor_sync(0xffffffffu, d2, o));
-      }
-      if (lane == 0) {
-        double cn = 0.0;
-#pragma unroll
-        for (int j = 0; j < kB; ++j) cn = fmax(cn, s_xxc[j]);
-        seg_skip[myseg] = segment_skip(d2, R, M, xxa, cn) ? 1 : 0;
-      }
-    }
-    buf ^= 1;
-  }
-}
-
 static size_t pass_smem_bytes(int S) {
   return (size_t)kB * S * sizeof(double) + kB * sizeof(double) + (size_t)kTeams * 2 * kSeg * 64 * sizeof(double) +
          kB * sizeof(long long) + (kNB + 1) * sizeof(unsigned int);
@@ -1547,58 +1440,15 @@ __global__ void __launch_bounds__(256) score_init_kernel(long long lo, long long
 // Only before the first round: afterwards every pass leaves the block header behind itself.
 __global__ void __launch_bounds__(256) bootstrap_kernel(long long lo, long long hi, const double* __restrict__ score,
                                                         Best* partial, RankBlock* out, Ctl* ctl, PushArgs push) {
-  __shared__ Best s_best[8];
-  __shared__ unsigned int s_last;
-  const int tid = threadIdx.x;
   Best best{-INFINITY, 0x7fffffffffffffffLL};
-  for (long long i = lo + (long long)blockIdx.x * blockDim.x + tid; i < hi; i += (long long)gridDim.x * blockDim.x) {
+  for (long long i = lo + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < hi; i += (long long)gridDim.x * blockDim.x) {
     const double s = score[i];
     if (better(s, i, best.s, best.i)) {
       best.s = s;
       best.i = i;
     }
   }
-  best = warp_best(best);
-  if ((tid & 31) == 0) s_best[tid >> 5] = best;
-  __syncthreads();
-  if (tid == 0) {
-    for (int k = 1; k < 8; ++k)
-      if (better(s_best[k].s, s_best[k].i, best.s, best.i)) best = s_best[k];
-    partial[blockIdx.x] = best;
-    __threadfence();
-    s_last = (atomicAdd(&ctl->filter_ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
-  }
-  __syncthreads();
-  if (s_last) {
-    __threadfence();
-    Best b{-INFINITY, 0x7fffffffffffffffLL};
-    for (int k = tid; k < (int)gridDim.x; k += blockDim.x) {
-      Best q;
-      q.s = ((volatile Best*)partial)[k].s;
-      q.i = ((volatile Best*)partial)[k].i;
-      if (better(q.s, q.i, b.s, b.i)) b = q;
-    }
-    b = warp_best(b);
-    __syncthreads();
-    if ((tid & 31) == 0) s_best[tid >> 5] = b;
-    __syncthreads();
-    if (tid == 0) {
-      for (int k = 1; k < 8; ++k)
-        if (better(s_best[k].s, s_best[k].i, b.s, b.i)) b = s_best[k];
-      out->count = 0;
-      out->smax = b.s;
-      out->smax_idx = b.i;
-      out->theta = INFINITY;
-      out->mode = 0;
-      out->inwin = 0;
-      ctl->filter_ticket = 0;
-      __threadfence();
-    }
-    if (push.peers != nullptr) {
-      __syncthreads();
-      push_block(push, out);
-    }
-  }
+  publish_header(8, best, partial, ctl, out, push, INFINITY, 0, nullptr, true);   // (256 threads) no list, exact arg-max
 }
 
 // ---------------------------------------------------------------- candidate bookkeeping
@@ -2303,6 +2153,7 @@ static int configure_pass_of() {
   VQ_CUDA(cudaFuncSetAttribute(pass_kernel_generic<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
   VQ_CUDA(cudaFuncSetAttribute(pass_kernel_generic<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
   VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<false, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
+  VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<false, true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
   VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<true, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
   VQ_CUDA(cudaFuncSetAttribute(pass_kernel_tma<true, true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmem));
   VQ_CUDA(cudaFuncSetAttribute(pairs_plan_kernel<T>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
@@ -2347,40 +2198,49 @@ static int pair_grid() {
   return grid;
 }
 
-// the paired pass of a 16-pick round (d = 2048 only): applies picks [0, nb) when nb > 8, reading X once
-// (filter = true: the same tile machine over the segment anchors, writing both centre groups' skip flags)
+// pass_kernel_tma (d = 2048) in its four forms.  pair: clusters of two CTAs on pair_grid() CTAs, applying a round of up
+// to 16 picks in one read of X; else one CTA per SM applying the 8 centres from center_off.  filter: the segment
+// filter over the anchor rows, which writes the skip flags of those centres instead of applying them.
 template <typename T>
-static int launch_pass_pair(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr,
-                            bool filter = false, bool pdl = false) {
+static int launch_tma(const PassArgs& a, bool pair, bool filter, cudaStream_t stream, bool pdl, cudaEvent_t ev0 = nullptr,
+                      cudaEvent_t ev1 = nullptr) {
   if (int e = configure_pass()) return e;
+  void (*kernel)(PassArgs) = pair ? (filter ? pass_kernel_tma<true, true, T> : pass_kernel_tma<true, false, T>)
+                                  : (filter ? pass_kernel_tma<false, true, T> : pass_kernel_tma<false, false, T>);
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)pair_grid());
+  cfg.gridDim = dim3((unsigned)(pair ? pair_grid() : sm_count()));
   cfg.blockDim = dim3(kWsThreads);
   cfg.dynamicSmemBytes = kWsSmem;
   cfg.stream = stream;
   cudaLaunchAttribute at[2] = {};
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2;
-  at[0].val.clusterDim.y = at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
+  unsigned nat = 0;
+  if (pair) {
+    at[nat].id = cudaLaunchAttributeClusterDimension;
+    at[nat].val.clusterDim.x = 2;
+    at[nat].val.clusterDim.y = at[nat].val.clusterDim.z = 1;
+    ++nat;
+  }
+  if (pdl) {
+    at[nat].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[nat].val.programmaticStreamSerializationAllowed = 1;
+    ++nat;
+  }
   cfg.attrs = at;
-  cfg.numAttrs = pdl ? 2 : 1;
+  cfg.numAttrs = nat;
   if (ev0) cudaEventRecord(ev0, stream);
-  if (filter) VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<true, true, T>, a));
-  else VQ_CUDA(cudaLaunchKernelEx(&cfg, pass_kernel_tma<true, false, T>, a));
+  VQ_CUDA(cudaLaunchKernelEx(&cfg, kernel, a));
   if (ev1) cudaEventRecord(ev1, stream);
   VQ_LAUNCHED();
   return 0;
 }
 
+// the solo pass: the TMA kernel at d = 2048, else the generic kernel
 template <typename T>
 static int launch_pass(PassArgs& a, cudaStream_t stream, cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr, bool pdl = false) {
+  if (a.d4 == kFastD / 4 && a.dots != nullptr) return launch_tma<T>(a, false, false, stream, pdl, ev0, ev1);
   if (int e = configure_pass()) return e;
   if (ev0) cudaEventRecord(ev0, stream);
-  const bool fast = a.d4 == kFastD / 4 && a.dots != nullptr;
-  if (fast) VQ_CUDA(launch_pdl(pass_kernel_tma<false, false, T>, dim3(sm_count()), dim3(kWsThreads), kWsSmem, stream, pdl, a));
-  else if ((a.d4 & 3) != 0) pass_kernel_generic<true, T><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
+  if ((a.d4 & 3) != 0) pass_kernel_generic<true, T><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
   else pass_kernel_generic<false, T><<<sm_count(), kPassThreads, pass_smem_bytes(a.S), stream>>>(a);
   if (ev1) cudaEventRecord(ev1, stream);
   VQ_LAUNCHED();
@@ -2396,7 +2256,12 @@ struct PruneState {
   double* seg_r = nullptr;
   unsigned char* seg_skip = nullptr;
   size_t skip_stride = 0;
-  int filter_grid = 1;
+  // the pruning fields of a pass (mode != 0): the pass reads the flags of its centre group at seg_skip (group g's at
+  // + g * skip_stride), its filter launch writes them at seg_skip_out
+  void fill(PassArgs& a) const {
+    a.seg_of_row = seg_of_row; a.seg_skip = seg_skip; a.prune_mode = mode; a.prune_stats = pc->stats;
+    a.seg_start = seg_start; a.seg_r = seg_r; a.nseg = &pc->nseg; a.seg_skip_out = seg_skip; a.skip_stride = skip_stride;
+  }
 };
 template <typename T>
 static int prune_setup(PruneState& P, const T* X, const Geom& G, int64_t row_lo, int64_t row_hi, char* w,
@@ -2421,7 +2286,6 @@ static int prune_setup(PruneState& P, const T* X, const Geom& G, int64_t row_lo,
   const long long prune_min = g_prune_min_set >= 0 ? g_prune_min_set : prune_min_rows;
   P.mode = (G.d4 == kFastD / 4 && own >= prune_min && own >= 8 && own < (1LL << 30))
                ? (g_prune_mode_set >= 0 ? g_prune_mode_set : prune_env) : 0;
-  P.filter_grid = (int)std::max<long long>(1, std::min<long long>(sm_count(), own / 8 + 1));   // tiles of 8 segments, grid-stride
   VQ_CUDA(cudaMemsetAsync(P.pc, 0, sizeof(PruneCtl), stream));
   if (P.mode) {
     double* cd = (double*)(w + L.dots);   // the dot-product scratch is idle until the first pass
@@ -2432,17 +2296,6 @@ static int prune_setup(PruneState& P, const T* X, const Geom& G, int64_t row_lo,
     seg_radius_kernel<T><<<sm_count() * 8, 256, 0, stream>>>(X, G.d4, row_lo, P.seg_start, P.pc, P.seg_r);
     VQ_LAUNCHED();
   }
-  return 0;
-}
-// flags for the `groups` passes that apply centers[center_off + 8g ..), g = 0 .. groups-1 (flag array g):
-// ONE launch before the first of those passes
-template <typename T>
-static int launch_filter(const PruneState& P, const PassArgs& a, cudaStream_t stream, int groups = 1) {
-  dim3 grid((unsigned)P.filter_grid, (unsigned)groups);
-  prune_filter_kernel<T><<<grid, kSeg * 32, 0, stream>>>(static_cast<const T*>(a.X), a.d4, a.lo, P.seg_start, P.seg_r, a.m, a.xx, a.centers,
-                                                          a.n_centers, a.n_centers_imm, a.center_off, P.pc, P.seg_skip,
-                                                          P.skip_stride);
-  VQ_LAUNCHED();
   return 0;
 }
 // accumulate the device-side tile statistics of a finished call (the caller has synchronised)
@@ -2492,8 +2345,8 @@ static int coreset_init(const T* X, int64_t n, int d, int64_t row_lo, int64_t ro
     a.unc = nullptr; a.score = nullptr; a.centers = (const long long*)labeled + c0; a.n_centers = nullptr;
     a.n_centers_imm = (int)std::min<int64_t>(kB, n_labeled - c0); a.ctl = nullptr; a.hist = nullptr;
     if (P.mode) {
-      a.seg_of_row = P.seg_of_row; a.seg_skip = P.seg_skip; a.prune_mode = P.mode; a.prune_stats = P.pc->stats;
-      if (int e = launch_filter<T>(P, a, stream)) return e;
+      P.fill(a);
+      if (int e = launch_tma<T>(a, false, true, stream, false)) return e;   // the flags of this pass
     }
     if (int e = launch_pass<T>(a, stream)) return e;
   }
@@ -2635,9 +2488,7 @@ static int coreset_select(const T* X, int dtype, int64_t n, int d, int64_t row_l
     a.unc = unc; a.score = score; a.centers = ctl->picks; a.n_centers = &ctl->nb; a.n_centers_imm = 0; a.ctl = ctl;
     a.hist = (nbk > 1) ? hist : nullptr; a.send = send; a.partial = partial; a.dots = (double*)(w + L.dots);
     a.prune_stats = P.pc->stats;
-    if (prune_mode) {
-      a.seg_of_row = P.seg_of_row; a.seg_skip = P.seg_skip; a.prune_mode = prune_mode;
-    }
+    if (prune_mode) P.fill(a);
   };
 
   if (n_labeled == 0 && rule == 2) {
@@ -2715,42 +2566,33 @@ static int coreset_select(const T* X, int dtype, int64_t n, int d, int64_t row_l
         plan_kernel<<<1, kPlanThreads, 0, stream>>>(blocks, send, Dcc, hist, (long long*)out_idx, ctl);
         g_launches.fetch_add(1);
       }
-      if (prune_mode) {   // flags of every centre group of the round in one launch
+      if (prune_mode) {   // the flags of every centre group of the round, before its first pass
         PassArgs a{};
         fill_pass(a);
-        if (use_pair) {   // the pass's own TMA / DMMA tile machine over the anchor rows (bandwidth-bound)
-          a.seg_start = P.seg_start; a.seg_r = P.seg_r; a.nseg = &P.pc->nseg; a.seg_skip_out = P.seg_skip;
-          a.skip_stride = P.skip_stride;
-          rc = launch_pass_pair<T>(a, stream, nullptr, nullptr, true, true);
-        } else {
-          rc = launch_filter<T>(P, a, stream, (nbk + kB - 1) / kB);
+        if (use_pair) rc = launch_tma<T>(a, true, true, stream, true);
+        for (int off = 0; !use_pair && off < nbk && rc == 0; off += kB) {
+          a.center_off = off;
+          a.seg_skip_out = P.seg_skip + (size_t)(off / kB) * P.skip_stride;
+          rc = launch_tma<T>(a, false, true, stream, true);
         }
       }
       auto timed_launch = [&](PassArgs& a, bool pair) {
         const bool timed = g_prof.on && g_prof.used + 2 <= g_prof.ev.size() && g_prof.used / 2 < 1024;
         if (timed) a.did_work = flags + g_prof.used / 2;
         cudaEvent_t e0 = timed ? g_prof.ev[g_prof.used] : nullptr, e1 = timed ? g_prof.ev[g_prof.used + 1] : nullptr;
-        const int r = pair ? launch_pass_pair<T>(a, stream, e0, e1, false, true) : launch_pass<T>(a, stream, e0, e1, true);
+        const int r = pair ? launch_tma<T>(a, true, false, stream, true, e0, e1) : launch_pass<T>(a, stream, e0, e1, true);
         if (timed) g_prof.used += 2;
         return r;
       };
       if (use_pair && rc == 0) {
-        // a round of 9..16 picks is applied by ONE paired pass (X read once); a shorter round by the solo pass
+        // every round, of 1 to 16 picks, is applied by ONE paired pass (X read once)
         PassArgs a{};
         fill_pass(a);
-        a.skip_stride = P.skip_stride;
         a.push = push_of(seq0 + round_no + 1);   // the block this round's (only) pass publishes
         a.screen_mode = screen_mode;
         a.screen_stats = P.pc->screen;
         a.Xh = Xh;
         rc = timed_launch(a, true);
-        if (rc == 0) {
-          PassArgs b{};
-          fill_pass(b);
-          b.only_if_le8 = 1;
-          b.push = push_of(seq0 + round_no + 1);
-          rc = timed_launch(b, false);
-        }
       } else {
         for (int off = 0; off < nbk && rc == 0; off += kB) {   // picks [off, off+8) of the round; the last pass emits
           PassArgs a{};
