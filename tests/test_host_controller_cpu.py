@@ -11,6 +11,7 @@ import pytest
 import torch
 
 from oracle import vatl_oracle as O
+from test_kmeans_host_cpu import km_on_cpu  # noqa: F401  (fixture: the K-Means device calls as NumPy stand-ins)
 
 
 def _install_stand_ins(monkeypatch, v):
@@ -164,3 +165,63 @@ def test_controller_default_strategies_host_logic(built_lib, monkeypatch, unc, f
     import test_gpu_query as T
     _install_stand_ins(monkeypatch, built_lib)
     T.test_two_rounds_match_oracle(built_lib, unc, flt)
+
+
+@pytest.fixture
+def one_rank_group():
+    import torch.distributed as td
+    td.init_process_group("gloo", store=td.HashStore(), rank=0, world_size=1)
+    try:
+        yield td.group.WORLD
+    finally:
+        td.destroy_process_group()
+
+
+@pytest.mark.parametrize("rep,flt,n_unl", [("Influence", "None", None), ("None", "Diversity", None),
+                                           ("None", "K-Means", None), ("Influence", "weighted", None),
+                                           ("Influence", "Coreset", None), ("None", "Coreset", None),
+                                           ("None", "Coreset", 0), ("None", "Coreset", 1),
+                                           ("None", "K-Means", 0), ("None", "K-Means", 1)])
+def test_distributed_query_matches_controller_host_logic(km_on_cpu, one_rank_group, monkeypatch, rep, flt, n_unl):
+    """dist.distributed_query on a one-rank gloo group picks what ActiveLearning._query picks from the same pool,
+    labelled set and rule, with the same scores.  With at most one unlabelled item (n_unl) every filter takes the
+    score-ordered top k and nothing is clustered (ActiveLearning.py:533-534, 541-542)."""
+    import vatlq as v
+    from types import SimpleNamespace
+    from vatlq import _lib, dist, kmeans as KM
+    fake = _lib.lib()
+    _install_stand_ins(monkeypatch, v)
+    monkeypatch.setattr(_lib, "lib", lambda: fake)
+    monkeypatch.setattr(KM, "rank_scores", v.ops.rank_scores)
+    if n_unl is not None:
+        def no_clustering(*a, **kw):
+            raise AssertionError("a pool with at most one unlabelled item is not clustered")
+        monkeypatch.setattr(KM, "kmeans_fit_select", no_clustering)
+    n = 60
+    ids, ip, inx = v.synth.track_flags(n, np.random.default_rng(3), 6.0)
+    H = torch.from_numpy(v.synth.heatmaps(n, seed=3, track_ids=ids))
+    boxes = torch.from_numpy(v.synth.boxes_xyxy(n, 3))
+    ip, inx = torch.from_numpy(ip.astype(np.uint8)), torch.from_numpy(inx.astype(np.uint8))
+    X = v.synth.embeddings(n, d=64, seed=3)
+    X[40:45] = X[20:25]                                   # duplicates for the weighted filter's np.unique
+    labeled = list(range(0, n, 5)) if n_unl is None else list(range(n - n_unl))
+    cfg = SimpleNamespace(VAL=SimpleNamespace(QUERY_RATIO=[0.1, 0.2], W_UNC=0.8, UNC_LAMBDA=0.01),
+                          DATA_PRESET=SimpleNamespace(HEATMAP_SIZE=[64, 48]), AE=SimpleNamespace(Z_DIM=4))
+    opt = SimpleNamespace(strategy=f"THC+{rep}_{flt}filter", uncertainty="THC", representativeness=rep, filter=flt,
+                          video_id="0", THCvsWPU="const", fixed_lambda=False, onebyone=False)
+    al = v.ActiveLearning(cfg, opt, eval_len=n)
+    al.labeled_id.update(labeled)
+    al.unlabeled_id.difference_update(labeled)
+    k = al.query_size
+    cand = sorted(set(range(n)) - set(labeled))
+    fake.n = len(cand) if flt != "weighted" else len(np.unique(X[cand].astype(np.float64), axis=0))
+    fake.k = min(k, fake.n)
+    qp = v.QueryPass(n, "cpu", uncertainty="THC")
+    qp.score_pool(H, boxes, ip, inx)
+    al._query(qp, torch.from_numpy(X))
+    res = dist.distributed_query(H, boxes, ip, inx, torch.from_numpy(X), None, labeled, n, k, 0.0, al.unc_lambda,
+                                 uncertainty="THC", rule="w_unc", representativeness=rep, filter=flt, w_unc=al.w_unc,
+                                 group=one_rank_group)
+    assert res.picks.tolist() == al.last_query.query_list
+    assert len(res.picks) == min(k, len(cand))
+    assert torch.equal(res.unc, al.last_query.score)

@@ -28,7 +28,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib, ops
-from .query import QueryPass
+from .query import FILTERS, QueryPass, classify_uncertainty, influence, select, unlabelled_mask
 
 __all__ = ["ActiveLearning", "IndexCollection", "WholeBodyAE", "compute_thc", "compute_entropy", "localpeak_mean",
            "heatmap_to_coord_simple", "compute_hybrid", "coreset_selection"]
@@ -218,23 +218,23 @@ def coreset_selection(self, embeddings, uncertainty):
         if not np.array_equal(X.cpu().numpy().astype(np.float64), embeddings):
             raise _lib.VatlqError("embeddings must hold fp32-representable values (ActiveLearning.py:270,286)")
     unc = _as_cuda(uncertainty, torch.float64)
-    labeled = list(self.labeled_id.index)
-    first_pick = -1
-    if self.uncertainty == "None" or self.cfg.VAL.UNC_LAMBDA == 0:
-        rule = "dist"
-        if len(labeled) == 0:   # _query (:828-833): random first pick, drawn like the reference
-            first_pick = int(np.random.choice(np.arange(X.shape[0])))
-    elif self.opt.fixed_lambda:
-        rule = "fixed_lambda"
-    else:
-        rule = "w_unc"
+    rule, first_pick = _coreset_rule(self, X.shape[0])
     picks, stats, _, unc_after = ops.coreset_select(
-        X, unc, labeled, int(self.query_size), float(self.moks_queried), float(self.unc_lambda), rule=rule,
-        first_pick=first_pick, batch=int(getattr(self, "coreset_batch", 16)), return_state=True)
+        X, unc, list(self.labeled_id.index), int(self.query_size), float(self.moks_queried), float(self.unc_lambda),
+        rule=rule, first_pick=first_pick, batch=int(getattr(self, "coreset_batch", 16)), return_state=True)
     self.coreset_stats = stats
     if isinstance(uncertainty, np.ndarray):
         uncertainty[:] = unc_after.cpu().numpy()
     return [int(i) for i in picks.cpu().tolist()]
+
+
+def _coreset_rule(self, n: int) -> tuple[str, int]:
+    """(rule, first_pick) of the core-set for the strategy of `self` (ActiveLearning.py:815-833): "dist" without an
+    uncertainty to weigh, its first pick drawn from np.random like the reference when nothing is labelled;
+    "fixed_lambda" / "w_unc" otherwise."""
+    if self.uncertainty == "None" or self.cfg.VAL.UNC_LAMBDA == 0:
+        return "dist", int(np.random.choice(np.arange(n))) if len(self.labeled_id.index) == 0 else -1
+    return ("fixed_lambda" if self.opt.fixed_lambda else "w_unc"), -1
 
 
 # ----------------------------------------------------------------------------------------
@@ -242,8 +242,6 @@ def coreset_selection(self, embeddings, uncertainty):
 # ----------------------------------------------------------------------------------------
 
 _REFERENCE_ONLY_UNC = ("VL4Pose",)                      # the reference's own VL4Pose branch is an unfinished stub (:390-391)
-_PEAK_UNC = ("MPE", "Margin")                           # skimage.peak_local_max based (:762-788)
-_SINGLE_UNC = ("HP", "TPC", "Entropy", "MPE", "Margin")
 
 
 class ActiveLearning:
@@ -268,14 +266,11 @@ class ActiveLearning:
         self.model, self.eval_loader, self.AE = model, eval_loader, AE
         self.oks_fn, self.eval_hook, self.retrain_hook, self.metrics_hook = oks_fn, eval_hook, retrain_hook, metrics_hook
         # dispatch keys: accept exactly the reference's names (:329-401,467-481,533-619)
-        u = self.uncertainty
-        known = u in ("None", "THC+WPU") or "THC" in u or "WPU" in u or u in _REFERENCE_ONLY_UNC or u in _SINGLE_UNC \
-            or u in _PEAK_UNC
-        if not known:
+        if not (any(classify_uncertainty(self.uncertainty)) or self.uncertainty in ("None",) + _REFERENCE_ONLY_UNC):
             raise ValueError("Uncertainty type is not supported")
         if self.representativeness not in ("None", "Influence", "Random"):
             raise ValueError("Representativeness type is not supported")
-        if self.filter not in ("None", "weighted", "K-Means", "Coreset", "Diversity", "Random"):
+        if self.filter not in FILTERS + ("Random",):
             raise ValueError("Filter type is not supported")
         if eval_len is None and eval_loader is None:
             self._build_from_reference()          # the two-argument form of the reference (:52-164)
@@ -358,10 +353,10 @@ class ActiveLearning:
         self._require_accelerated()
         dev = _dev()
         n = self.eval_len
-        use_wpu = "WPU" in self.uncertainty and self.uncertainty not in _SINGLE_UNC
         # embeddings are collected when the filter OR the representativeness needs them (:283)
         want_feat = self.filter not in ("None", "Random") or self.representativeness not in ("None", "Random")
-        qp = QueryPass(n, dev, ae_weights=self.AE if use_wpu else None, uncertainty=self.uncertainty)
+        qp = QueryPass(n, dev, ae_weights=self.AE if classify_uncertainty(self.uncertainty)[2] else None,
+                       uncertainty=self.uncertainty)
         # (the reference keeps an all-zero fvecs_matrix otherwise, :270); allocated at the first batch, in
         # embedding_store_dtype of the estimator's embeddings
         X = None
@@ -434,9 +429,7 @@ class ActiveLearning:
         dev = qp.dev
         n = self.eval_len
         unl_idx = self.unlabeled_id.index
-        unl = torch.zeros(n, dtype=torch.uint8, device=dev)
-        if unl_idx:
-            unl[torch.as_tensor(unl_idx, device=dev)] = 1
+        unl = unlabelled_mask(n, self.labeled_id.index, dev)
         thc_h = qp.thc.cpu().numpy() if qp.use_thc else None
         wpu_h = qp.wpu.cpu().numpy() if qp.use_wpu else None
         if self.uncertainty == "THC+WPU":
@@ -457,8 +450,7 @@ class ActiveLearning:
             if len(unl_idx) in (0, 1):
                 infl_u = np.zeros(len(unl_idx))
             elif self.representativeness == "Influence":
-                rs = ops.cosine_rowsum(X, rows=unl_t)                                 # row sums of the cosine graph (:471-473)
-                infl[unl_t] = ops.minmax_f64(rs)                                      # (:475)
+                infl = influence(X, unl)
                 infl_u = infl[unl_t].cpu().numpy()
             else:                                                                     # "Random" (:476-477)
                 infl_u = np.random.rand(len(unl_idx))
@@ -473,35 +465,25 @@ class ActiveLearning:
             self.combine_weight.append(qp.combine_weight)                             # (:486-488)
         if self.uncertainty != "None" and len(unl_idx) not in (0, 1):
             self.uncertainty_dict["Round" + str(self.round_cnt)] = UNC                # (:510,514)
-        order = None
-        if len(unl_idx) in (0, 1) or self.filter in ("None", "Diversity", "Random"):
-            # unlabelled ids by descending score, ties in id order (sorted() is stable) (:527-530): ranked on the
-            # device, only the ids that are used come back
-            want = self.query_size if (len(unl_idx) in (0, 1) or self.filter == "None") else 8 * self.query_size
-            order = ops.rank_scores(score, unl, descending=True, count=want).cpu().tolist() if unl_idx else []
-        if len(unl_idx) in (0, 1) or self.filter == "None":                           # (:533-534,541-542)
-            query_list = sorted(int(i) for i in order[:self.query_size])
-        elif self.filter == "Diversity":                                              # (:537-538,581-590)
-            cand = sorted(int(i) for i in order[:8 * self.query_size])
-            cand_t = torch.as_tensor(cand, dtype=torch.int64, device=dev)
-            div = ops.cosine_rowsum(X, rows=cand_t)
-            by_div = ops.rank_scores(div, None, descending=False, count=self.query_size).cpu().tolist()
-            query_list = [cand[t] for t in by_div]
-        elif self.filter == "Random":                                                 # (:591-592, random_query :727-734)
-            cand = sorted(int(i) for i in order[:8 * self.query_size])
+        if self.filter == "Random" and len(unl_idx) > 1:                              # (:591-592, random_query :727-734)
+            # unlabelled ids by descending score, ties in id order (sorted() is stable) (:527-530)
+            cand = sorted(ops.rank_scores(score, unl, descending=True, count=8 * self.query_size).cpu().tolist())
             query_list = []
             while len(query_list) < self.query_size and len(cand) > 0:
                 q = int(np.random.choice(cand))
                 query_list.append(q)
                 cand.remove(q)
-        elif self.filter in ("K-Means", "weighted"):                                   # (:553-580, 593-608)
+        elif self.filter in ("K-Means", "weighted") and len(unl_idx) > 1:
             query_list = self._kmeans_query(X, score, unl_idx, qp.combine_weight)
-        else:                                                                          # Coreset (:609-614)
-            holder = SimpleNamespace(labeled_id=self.labeled_id, moks_queried=self.moks_queried,
-                                     unc_lambda=self.unc_lambda, uncertainty=self.uncertainty, cfg=self.cfg,
-                                     opt=self.opt, query_size=self.query_size, coreset_batch=self.coreset_batch)
-            query_list = coreset_selection(holder, X, score)
-            self.coreset_stats = holder.coreset_stats
+        else:
+            # (the first pick of "dist" is drawn only when the core-set runs: never with <= 1 unlabelled item)
+            rule, first_pick = _coreset_rule(self, n) if self.filter == "Coreset" and len(unl_idx) > 1 else ("w_unc", -1)
+            picks, _, stats = select(score, unl, X, self.query_size, self.filter, labeled=list(self.labeled_id.index),
+                                     moks=float(self.moks_queried), lam=float(self.unc_lambda), rule=rule,
+                                     first_pick=first_pick, batch=self.coreset_batch)
+            query_list = [int(i) for i in picks.cpu().tolist()]
+            if stats is not None:
+                self.coreset_stats = stats
         self.last_query = SimpleNamespace(thc=qp.thc, wpu=qp.wpu, single=qp.aux, peak_mean=qp.peak_mean, kpts=qp.kpts,
                                           score=score, query_list=list(query_list))
         OKS_dict = self.OKS_dict
@@ -539,33 +521,13 @@ class ActiveLearning:
         return None
 
     def _kmeans_query(self, X, score, unl_idx, combine_weight):
-        """filter == "K-Means" (:593-608) / "weighted" (:553-580): sklearn's KMeans(n_clusters=query_size,
-        random_state=318) on the embeddings of every unlabelled item, restated on the device (kmeans.py), then per
-        cluster the member closest to its centre.  `weighted` first drops duplicate embeddings with
-        np.unique(axis=0) — which also sorts the rows — weighs every row with 1 + w_unc * combine_weight * score, and
-        maps the chosen rows of that sorted matrix straight through candidate_list (:580, kept as the reference has
-        it).  self.query_size is clamped in place like the reference does."""
-        from . import kmeans as KM
-        dev = X.device
-        cand = sorted(int(i) for i in unl_idx)                                        # (:535-536)
-        cand_t = torch.as_tensor(cand, dtype=torch.int64, device=dev)
-        emb = X[cand_t]
-        if self.filter == "weighted":
-            embed_idx = KM.unique_rows_first_index(emb)                                # (:555-556)
-            e_t = torch.as_tensor(embed_idx, dtype=torch.int64, device=dev)
-            emb = emb[e_t]
-            weight = (1 + self.w_unc * combine_weight * score[cand_t])[e_t].contiguous()   # (:560-562)
-            if len(unl_idx) <= self.query_size:
-                self.query_size = len(unl_idx)
-            if self.query_size > emb.shape[0]:
-                self.query_size = int(emb.shape[0])
-            res = KM.kmeans_fit_select(emb, self.query_size, sample_weight=weight)
-        else:
-            if len(unl_idx) < self.query_size:
-                self.query_size = len(unl_idx)
-            res = KM.kmeans_fit_select(emb, self.query_size)
-        self.kmeans_stats = {"n_iter": res.n_iter, "relocations": res.relocations}
-        return [int(cand[i]) for i in res.query_rows]
+        """filter K-Means / weighted over the unlabelled ids `unl_idx` (query.select); self.query_size is clamped in
+        place like the reference does (:558-561, 564-565)."""
+        n = score.numel()
+        unl = unlabelled_mask(n, np.setdiff1d(np.arange(n), np.asarray(unl_idx, dtype=np.int64)), score.device)
+        picks, self.query_size, self.kmeans_stats = select(score, unl, X, self.query_size, self.filter, w_unc=self.w_unc,
+                                                           combine_weight=combine_weight)
+        return [int(i) for i in picks.cpu().tolist()]
 
     # ---- host bookkeeping on the per-item OKS values (tiny; ActiveLearning.py:707-725, 852-884) ----
     def get_retrain_id(self, query_list, OKS_dict):

@@ -159,11 +159,17 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
     uncertainty: any accelerated name (THC*, WPU*, THC+WPU, HP, TPC, Entropy, MPE, Margin, None);
     representativeness: "None" or "Influence" (ActiveLearning.py:467-477); filter: "Coreset" (:609-614),
     "None" (top-k, :533-534), "Diversity" (:581-590), "K-Means" (:593-608) or "weighted" (:553-580; w_unc = cfg.VAL.W_UNC;
-    the assignment step of Lloyd is sharded by rows, seeding and the M step run replicated).  Scoring is sharded (halo frame / halo coordinates for
+    the assignment step of Lloyd is sharded by rows, seeding and the M step run replicated).  With at most one
+    unlabelled item every filter returns the score-ordered top k of the unlabelled items, like the reference
+    (:533-534, 541-542).  Scoring is sharded (halo frame / halo coordinates for
     THC / TPC, MIN all-reduces for the normalisations, a SUM all-reduce of the cosine column sums for
-    Influence); the fused scores are all-gathered (8 B per item) and the final ordering runs replicated."""
+    Influence); the fused scores are all-gathered (8 B per item) and the filter runs replicated (query.select)."""
     from . import ops
-    from .query import QueryPass, QueryResult
+    from .query import FILTERS, QueryPass, QueryResult, influence, select, unlabelled_mask
+    if representativeness not in ("None", "Influence"):
+        raise ValueError("Representativeness type is not supported by distributed_query")
+    if filter not in FILTERS:
+        raise ValueError("Filter type is not supported by distributed_query")
     rank, world = td.get_rank(group), td.get_world_size(group)
     lo, hi = shard_range(n, rank, world)
     dev = X_local.device
@@ -177,60 +183,24 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
     hp, hn = exchange_halo(first, last, rank, world, group)
     qp.score_pool(H_local, boxes_local, is_prev_local, is_next_local, halo_prev=hp, halo_next=hn)
     lab = np.asarray(list(labeled_global), dtype=np.int64)
-    unl = torch.ones(hi - lo, dtype=torch.uint8, device=dev)
-    mine = lab[(lab >= lo) & (lab < hi)] - lo
-    if mine.size:
-        unl[torch.from_numpy(mine).to(dev)] = 0
+    unl = unlabelled_mask(n, lab, dev)
     # (group=None means the default group to torch.distributed but "single GPU" to QueryPass.fuse)
     fuse_group = (group if group is not None else td.group.WORLD) if world > 1 else None
     n_unl = n - lab.size
-    score_local = qp.fuse(unl, thc_vs_wpu, labeled_ratio=lab.size / max(n, 1), group=fuse_group, n_unlabeled_global=n_unl)
+    score_local = qp.fuse(unl[lo:hi], thc_vs_wpu, labeled_ratio=lab.size / max(n, 1), group=fuse_group,
+                          n_unlabeled_global=n_unl)
     if representativeness == "Influence" and n_unl > 1:                      # (:467-477, 517-526)
-        rows = torch.nonzero(unl, as_tuple=False).flatten()
-        infl = torch.zeros(hi - lo, dtype=torch.float64, device=dev)
-        infl[rows] = ops.cosine_rowsum(X_local, rows=rows, group=fuse_group)
-        infl = ops.minmax_f64(infl, unl, group=fuse_group)
-        score_local = ops.blend_scores(score_local, infl, qp.combine_weight, unl) if uncertainty != "None" else infl
-    elif representativeness not in ("None", "Influence"):
-        raise ValueError("Representativeness type is not supported by distributed_query")
+        infl = influence(X_local, unl[lo:hi], group=fuse_group)
+        score_local = ops.blend_scores(score_local, infl, qp.combine_weight, unl[lo:hi]) if uncertainty != "None" else infl
     score = allgather_rows(score_local, n, world, group)
-    if filter == "Coreset":
-        if world > 1:   # the all-gather below needs one row size on every rank
+
+    def gather_X():
+        if world > 1:   # the all-gather needs one row size on every rank
             _agree_dtype(X_local, "distributed_query", group)
-        X = allgather_rows(X_local, n, world, group)
-        picks, st = ops.coreset_select(X, score, lab, k, moks, lam, rule=rule, batch=batch, first_pick=first_pick,
-                                       comm=comm.handle if comm is not None else None,
-                                       row_range=(lo, hi) if world > 1 else None)
-    elif filter in ("None", "Diversity"):
-        unl_g = torch.ones(n, dtype=torch.uint8, device=dev)
-        if lab.size:
-            unl_g[torch.from_numpy(lab).to(dev)] = 0
-        st = None
-        if filter == "None" or n_unl <= 1:                                   # (:533-534, 541-542)
-            picks = torch.sort(ops.rank_scores(score, unl_g, descending=True, count=k)).values
-        else:                                                                # (:537-538, 581-590)
-            X = allgather_rows(X_local, n, world, group)
-            cand = torch.sort(ops.rank_scores(score, unl_g, descending=True, count=8 * k)).values
-            div = ops.cosine_rowsum(X, rows=cand)
-            picks = cand[ops.rank_scores(div, None, descending=False, count=k)]
-    elif filter in ("K-Means", "weighted"):                                  # (:553-580, 593-608)
-        from . import kmeans as KM
-        st = None
-        X = allgather_rows(X_local, n, world, group)
-        cand = np.setdiff1d(np.arange(n, dtype=np.int64), lab)               # sorted unlabelled ids (:535-536)
-        cand_t = torch.from_numpy(cand).to(dev)
-        emb = X[cand_t]
-        kk = min(k, int(cand.size))
-        if filter == "weighted":
-            eidx = torch.as_tensor(KM.unique_rows_first_index(emb), dtype=torch.int64, device=dev)
-            emb = emb[eidx]
-            weight = (1 + w_unc * qp.combine_weight * score[cand_t])[eidx].contiguous()
-            kk = min(kk, int(emb.shape[0]))
-            res = KM.kmeans_fit_select(emb, kk, sample_weight=weight, group=fuse_group)
-        else:
-            res = KM.kmeans_fit_select(emb, kk, group=fuse_group)
-        picks = torch.as_tensor([int(cand[i]) for i in res.query_rows], dtype=torch.int64, device=dev)
-    else:
-        raise ValueError("Filter type is not supported by distributed_query")
+        return allgather_rows(X_local, n, world, group)
+    picks, _, st = select(score, unl, gather_X, k, filter, labeled=lab, moks=moks, lam=lam, rule=rule,
+                          first_pick=first_pick, batch=batch, comm=comm.handle if comm is not None else None,
+                          row_range=(lo, hi) if world > 1 else None, w_unc=w_unc, combine_weight=qp.combine_weight,
+                          group=fuse_group)
     return QueryResult(picks=picks, thc=qp.thc, wpu=qp.wpu, peak_mean=qp.peak_mean, kpts=qp.kpts, unc=score,
                        combine_weight=qp.combine_weight, stats=st)

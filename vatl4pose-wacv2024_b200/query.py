@@ -38,6 +38,80 @@ def _require_cuda(dev: torch.device):
 
 
 SINGLE_UNCERTAINTIES = ("HP", "TPC", "Entropy", "MPE", "Margin")   # one fp32 score per item, min-max normalised (:511-516)
+FILTERS = ("None", "Diversity", "Coreset", "K-Means", "weighted")   # the filters `select` runs (:533-614)
+
+
+def classify_uncertainty(name: str) -> tuple[str | None, bool, bool]:
+    """(single, use_thc, use_wpu) of an uncertainty name, in the dispatch order of ActiveLearning.py:329-401: exact
+    names first, then the substring tests.  In the elif order of the reference a name containing "THC" is THC (even
+    "THC_WPU..."); only the exact string "THC+WPU" enables the two-criterion path (:345,364,403,494).  All three
+    empty: "None", or a name without a device path."""
+    single = name if name in SINGLE_UNCERTAINTIES else None
+    use_thc = single is None and "THC" in name
+    use_wpu = single is None and (name == "THC+WPU" or ("WPU" in name and "THC" not in name))
+    return single, use_thc, use_wpu
+
+
+def unlabelled_mask(n: int, labeled, device) -> torch.Tensor:
+    """uint8 (n,) on `device`: 1 on every row whose id is not in `labeled`."""
+    lab = np.asarray(labeled, dtype=np.int64)
+    unl = torch.ones(n, dtype=torch.uint8, device=device)
+    if lab.size:
+        unl[torch.from_numpy(lab).to(device)] = 0
+    return unl
+
+
+def influence(X: torch.Tensor, unl: torch.Tensor, group=None) -> torch.Tensor:
+    """Influence representativeness (ActiveLearning.py:467-475): row sums of the cosine-distance graph of the
+    unlabelled rows, min-max normalised over them; fp64 (len(unl),), 0 on labelled rows.  X holds the rows `unl`
+    masks.  `group`: the ranks hold disjoint row ranges of one pool (column sums and min / max are all-reduced)."""
+    rows = torch.nonzero(unl, as_tuple=False).flatten()
+    infl = torch.zeros(unl.numel(), dtype=torch.float64, device=unl.device)
+    infl[rows] = ops.minmax_f64(ops.cosine_rowsum(X, rows=rows, group=group), group=group)
+    return infl
+
+
+def select(score: torch.Tensor, unl: torch.Tensor, X, k: int, filter: str, *, labeled=(), moks: float = 0.0,
+           lam: float = 0.01, rule: str = "w_unc", first_pick: int = -1, batch: int = 16, comm=None,
+           row_range: tuple[int, int] | None = None, w_unc: float = 1.0, combine_weight: float | None = None, group=None):
+    """The filter stage after fusion (ActiveLearning.py:527-614) over the whole pool: `score` fp64 (n,), `unl` its
+    uint8 unlabelled mask, X the (n, d) embeddings or a function returning them (called only by the filters that
+    read X).  With at most one unlabelled item every filter returns the score-ordered top k (:533-534, 541-542).
+    None: the top k by score, in id order.  Diversity: of the top 8k by score (in id order), the k of least cosine
+    row sum (:581-590).  Coreset: ops.coreset_select (labeled, moks, lam, rule, first_pick, batch, comm, row_range;
+    :609-614).  K-Means / weighted: kmeans_fit_select on the unlabelled rows in id order (:593-608); weighted first
+    drops duplicate rows (np.unique(axis=0), which also sorts them), weighs each row 1 + w_unc * combine_weight *
+    score and maps the chosen rows of that sorted matrix straight through the candidate ids (:553-580, kept as the
+    reference has it); both clamp k to the rows they cluster, like the reference clamps query_size.
+    `group`: the ranks hold the same X and share the K-Means assignment step.
+    Returns (picks, k, stats): int64 ids on score's device in the reference's order, the k the filter used, and
+    its CoresetStats or K-Means {"n_iter", "relocations"} (None for the other filters)."""
+    n_unl = int(unl.sum().item())
+    if n_unl <= 1 or filter == "None":
+        return torch.sort(ops.rank_scores(score, unl, descending=True, count=k)).values, k, None
+    X = X() if callable(X) else X
+    if filter == "Diversity":
+        cand = torch.sort(ops.rank_scores(score, unl, descending=True, count=8 * k)).values
+        return cand[ops.rank_scores(ops.cosine_rowsum(X, rows=cand), None, descending=False, count=k)], k, None
+    if filter == "Coreset":
+        picks, st = ops.coreset_select(X, score, labeled, k, moks, lam, rule=rule, batch=batch, first_pick=first_pick,
+                                       comm=comm, row_range=row_range)
+        return picks, k, st
+    if filter not in ("K-Means", "weighted"):
+        raise ValueError(f"Filter type is not supported: {filter}")
+    from . import kmeans as KM
+    cand = torch.nonzero(unl, as_tuple=False).flatten()
+    emb = X[cand]
+    k = min(k, n_unl)
+    weight = None
+    if filter == "weighted":
+        eidx = torch.as_tensor(KM.unique_rows_first_index(emb), dtype=torch.int64, device=emb.device)
+        emb = emb[eidx]
+        weight = (1 + w_unc * combine_weight * score[cand])[eidx].contiguous()
+        k = min(k, int(emb.shape[0]))
+    res = KM.kmeans_fit_select(emb, k, sample_weight=weight, group=group)
+    picks = cand[torch.as_tensor(res.query_rows, dtype=torch.int64, device=cand.device)]
+    return picks, k, {"n_iter": res.n_iter, "relocations": res.relocations}
 
 
 class QueryPass:
@@ -50,12 +124,7 @@ class QueryPass:
         _lib.lib()  # fail now, loudly, if the CUDA library is missing
         self.n = int(n_local)
         self.uncertainty = uncertainty
-        # dispatch order of ActiveLearning.py:329-401: exact names first, then the substring tests
-        self.single = uncertainty if uncertainty in SINGLE_UNCERTAINTIES else None
-        # elif order of the reference: a name containing "THC" is THC (even "THC_WPU..."); only the exact string
-        # "THC+WPU" enables the two-criterion path (:345,364,403,494)
-        self.use_thc = self.single is None and "THC" in uncertainty
-        self.use_wpu = self.single is None and (uncertainty == "THC+WPU" or ("WPU" in uncertainty and "THC" not in uncertainty))
+        self.single, self.use_thc, self.use_wpu = classify_uncertainty(uncertainty)
         if not (self.use_thc or self.use_wpu or self.single or uncertainty == "None"):
             raise ValueError("Uncertainty type is not supported by the accelerated path")
         self.nj, self.hm = n_joints, tuple(hm_shape)
@@ -252,9 +321,7 @@ def run_query(H, boxes_xyxy, is_prev, is_next, X, ae_weights, labeled, k: int, m
             qp.score_chunk(a, Ht[a:b].to(dev, non_blocking=True), bb[a:b], ip[a:b], inx[a:b])
     Xd = to_dev(X, torch.float32)
     lab = np.asarray(list(labeled), dtype=np.int64)
-    unl = torch.ones(n, dtype=torch.uint8, device=dev)
-    if lab.size:
-        unl[torch.from_numpy(lab).to(dev)] = 0
+    unl = unlabelled_mask(n, lab, dev)
     unc = qp.fuse(unl, thc_vs_wpu, labeled_ratio=lab.size / max(n, 1))
     picks, st = ops.coreset_select(Xd, unc, lab, k, moks, lam, rule=rule, batch=batch, first_pick=first_pick)
     return QueryResult(picks=picks, thc=qp.thc, wpu=qp.wpu, peak_mean=qp.peak_mean, kpts=qp.kpts, unc=unc,
