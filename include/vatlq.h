@@ -284,6 +284,15 @@ int vatlq_cosine_colsum(const float* X, int64_t n, int d, const int64_t* rows, i
                         double* S, void* ws, size_t ws_bytes, vatlq_stream_t stream);
 int vatlq_cosine_rowsum(const float* X, int64_t n, int d, const int64_t* rows, int64_t m,
                         const double* S, double m_total, double* out, vatlq_stream_t stream);
+/* The two cosine calls on X in any VATLQ_* dtype (the fp32 entries are these calls with VATLQ_F32).  Every 16-bit
+ * value is widened exactly to fp32 at the load and the fp64 arithmetic after it is unchanged, so S and out equal, bit
+ * for bit, those of the fp32 calls on X's upcast (NaN rows included); a 16-bit X is read as it is, half the bytes.
+ * X must be 16-byte aligned in fp32 and 8-byte aligned in 16 bits; an unknown dtype or a misaligned X returns
+ * VATLQ_EINVAL before any device work.  The workspace is vatlq_cosine_workspace_bytes(d) in every dtype. */
+int vatlq_cosine_colsum_dt(const void* X, int dtype, int64_t n, int d, const int64_t* rows, int64_t m,
+                           double* S, void* ws, size_t ws_bytes, vatlq_stream_t stream);
+int vatlq_cosine_rowsum_dt(const void* X, int dtype, int64_t n, int d, const int64_t* rows, int64_t m,
+                           const double* S, double m_total, double* out, vatlq_stream_t stream);
 
 /* stats2[2] = {min v, -max v} over rows with mask != 0 (mask NULL: all rows): the statistics
  * vatlq_fuse_final consumes, for fp64 score vectors (influence normalisation, :477). */

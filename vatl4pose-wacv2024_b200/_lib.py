@@ -49,6 +49,8 @@ SIGNATURES = {
     "vatlq_cosine_workspace_bytes": (_sz, [_int]),
     "vatlq_cosine_colsum": (_int, [_vp, _i64, _int, _vp, _i64, _vp, _vp, _sz, _vp]),
     "vatlq_cosine_rowsum": (_int, [_vp, _i64, _int, _vp, _i64, _vp, _dbl, _vp, _vp]),
+    "vatlq_cosine_colsum_dt": (_int, [_vp, _int, _i64, _int, _vp, _i64, _vp, _vp, _sz, _vp]),
+    "vatlq_cosine_rowsum_dt": (_int, [_vp, _int, _i64, _int, _vp, _i64, _vp, _dbl, _vp, _vp]),
     "vatlq_minmax_stats_f64": (_int, [_vp, _vp, _i64, _vp, _vp]),
     "vatlq_fuse_blend": (_int, [_vp, _vp, _vp, _i64, _dbl, _vp, _vp]),
     "vatlq_peak_workspace_bytes": (_sz, [_i64, _int, _int, _int]),

@@ -208,21 +208,28 @@ entropy_frames_kernel(const float* __restrict__ per_map, int64_t n, int J, float
 //   colsum: every warp walks rows, keeps its share of S in registers (d <= 2048: 16 float4
 //           columns per lane), CTA partials land in the workspace and are added in a fixed order.
 //   rowsum: out_i = m_total - (x_i . S) / |x_i|.
+// T: fp32, or a 16-bit X read as 8-byte quads and widened exactly to fp32 in registers; the lane that
+// owns quad q owns the same four features in every type and the fp64 instruction sequence after the
+// load is the same, so every output equals the fp32 kernel's on the upcast, bit for bit.  The colsum
+// grid (cos_grid) depends on m and the SM count only: the fixed-order sum over the CTA partials is
+// then the same in every type.
 // ------------------------------------------------------------------------------------
 constexpr int kCosNV = 16;        // float4 per lane per row: d <= 2048
 constexpr int kCosThreads = 256;
 constexpr int kCosRows = kCosThreads / 32;   // rows per tile: one per warp
 
-__device__ __forceinline__ const float4* cos_row(const float* X, int d, const int64_t* rows, int64_t i) {
+template <typename T>
+__device__ __forceinline__ const T* cos_row(const T* X, int d, const int64_t* rows, int64_t i) {
   const int64_t r = rows ? rows[i] : i;
-  return reinterpret_cast<const float4*>(X + (size_t)r * d);
+  return X + (size_t)r * d;
 }
 
 // column sums of the normalised rows.  A CTA takes tiles of 8 rows: warp w loads row w (streamed
-// through shared memory, the squared norm reduced on the way), then every thread adds the 8
-// scaled rows into the (up to two) float4 columns it owns.  CTA partials -> workspace.
+// through shared memory as fp32 in every type, the squared norm reduced on the way), then every
+// thread adds the 8 scaled rows into the (up to two) float4 columns it owns.  CTA partials -> workspace.
+template <typename T>
 __global__ void __launch_bounds__(kCosThreads, 2)
-cos_colsum_kernel(const float* __restrict__ X, int d, const int64_t* __restrict__ rows, int64_t m,
+cos_colsum_kernel(const T* __restrict__ X, int d, const int64_t* __restrict__ rows, int64_t m,
                   double* __restrict__ partial /* gridDim.x x d */) {
   extern __shared__ __align__(16) unsigned char cos_smem[];
   float4* s_x = reinterpret_cast<float4*>(cos_smem);   // kCosRows x d4
@@ -235,12 +242,12 @@ cos_colsum_kernel(const float* __restrict__ X, int d, const int64_t* __restrict_
     const int64_t i = tile * kCosRows + warp;
     double nn = 0.0;
     if (i < m) {
-      const float4* rp = cos_row(X, d, rows, i);
+      const T* rp = cos_row(X, d, rows, i);
 #pragma unroll 8
       for (int q = 0; q < kCosNV; ++q) {
         const int c = q * 32 + lane;
         if (c < d4) {
-          const float4 v = ldg_stream(rp + c);
+          const float4 v = ldg_stream_quad(rp, c);
           s_x[warp * d4 + c] = v;
           nn = fma((double)v.x, (double)v.x, nn);
           nn = fma((double)v.y, (double)v.y, nn);
@@ -290,8 +297,9 @@ cos_colsum_reduce_kernel(const double* __restrict__ partial, int parts, int d, d
 }
 
 // out_i = m_total - (x_i . S) / |x_i|: one warp per row, S in shared memory
+template <typename T>
 __global__ void __launch_bounds__(kCosThreads)
-cos_rowsum_kernel(const float* __restrict__ X, int d, const int64_t* __restrict__ rows, int64_t m,
+cos_rowsum_kernel(const T* __restrict__ X, int d, const int64_t* __restrict__ rows, int64_t m,
                   const double* __restrict__ S, double m_total, double* __restrict__ out) {
   extern __shared__ __align__(16) unsigned char cos_smem[];
   double* s_S = reinterpret_cast<double*>(cos_smem);   // d doubles
@@ -300,7 +308,7 @@ cos_rowsum_kernel(const float* __restrict__ X, int d, const int64_t* __restrict_
   for (int c = threadIdx.x; c < d; c += blockDim.x) s_S[c] = S[c];
   __syncthreads();
   for (int64_t i = (int64_t)blockIdx.x * nw + warp; i < m; i += (int64_t)gridDim.x * nw) {
-    const float4* rp = cos_row(X, d, rows, i);
+    const T* rp = cos_row(X, d, rows, i);
     double nn = 0.0, dot = 0.0;
 #pragma unroll
     for (int q0 = 0; q0 < kCosNV; q0 += 8) {
@@ -308,7 +316,7 @@ cos_rowsum_kernel(const float* __restrict__ X, int d, const int64_t* __restrict_
 #pragma unroll
       for (int q = 0; q < 8; ++q) {
         const int c = (q0 + q) * 32 + lane;
-        v[q] = (c < d4) ? ldg_stream(rp + c) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[q] = (c < d4) ? ldg_stream_quad(rp, c) : make_float4(0.f, 0.f, 0.f, 0.f);
       }
 #pragma unroll
       for (int q = 0; q < 8; ++q) {
@@ -456,12 +464,27 @@ extern "C" size_t vatlq_cosine_workspace_bytes(int d) {
   return (size_t)sm_count() * 2 * (size_t)d * sizeof(double);
 }
 
-extern "C" int vatlq_cosine_colsum(const float* X, int64_t n, int d, const int64_t* rows, int64_t m,
-                                   double* S, void* ws, size_t ws_bytes, vatlq_stream_t stream_) {
+// the colsum kernel of element type T: the stage holds fp32 rows in every type, so one smem limit serves
+template <typename T>
+static int launch_cos_colsum(const T* X, int d, const int64_t* rows, int64_t m, int grid, double* partial,
+                             cudaStream_t stream) {
+  static bool cfg = false;
+  if (!cfg) {
+    VQ_CUDA(cudaFuncSetAttribute(cos_colsum_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kCosRows * kCosNV * 128 * 4));
+    cfg = true;
+  }
+  cos_colsum_kernel<T><<<grid, kCosThreads, (size_t)kCosRows * d * sizeof(float), stream>>>(X, d, rows, m, partial);
+  VQ_LAUNCHED();
+  return 0;
+}
+
+extern "C" int vatlq_cosine_colsum_dt(const void* X, int dtype, int64_t n, int d, const int64_t* rows, int64_t m,
+                                      double* S, void* ws, size_t ws_bytes, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  VQ_REQUIRE(dtype_size(dtype) != 0, "dtype must be VATLQ_F32, VATLQ_F16 or VATLQ_BF16");
   VQ_REQUIRE(X && S && n >= 0 && m >= 0, "null pointer");
   VQ_REQUIRE(d > 0 && (d & 3) == 0 && d <= kCosNV * 128, "d must be a multiple of 4 and <= 2048");
-  VQ_REQUIRE(((uintptr_t)X & 15) == 0, "X must be 16-byte aligned");
+  VQ_REQUIRE(quad_aligned(X, dtype), "X must be aligned to 16 bytes (fp32) or 8 bytes (16 bits)");
   VQ_REQUIRE(rows != nullptr || m == n, "m must equal n without a row list");
   VQ_REQUIRE(ws != nullptr && ws_bytes >= vatlq_cosine_workspace_bytes(d), "workspace too small");
   if (m == 0) {
@@ -469,31 +492,42 @@ extern "C" int vatlq_cosine_colsum(const float* X, int64_t n, int d, const int64
     return 0;
   }
   const int grid = cos_grid(m);
-  const size_t smem = (size_t)kCosRows * d * sizeof(float);
-  static bool cfg = false;
-  if (!cfg) {
-    VQ_CUDA(cudaFuncSetAttribute(cos_colsum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCosRows * kCosNV * 128 * 4));
-    cfg = true;
-  }
-  cos_colsum_kernel<<<grid, kCosThreads, smem, stream>>>(X, d, rows, m, (double*)ws);
-  VQ_LAUNCHED();
+  const int rc = with_dtype(dtype, [&](auto tag) {
+    using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+    return launch_cos_colsum((const T*)X, d, rows, m, grid, (double*)ws, stream);
+  });
+  if (rc != 0) return rc;
   cos_colsum_reduce_kernel<<<(d + 255) / 256, 256, 0, stream>>>((const double*)ws, grid, d, S);
   VQ_LAUNCHED();
   return 0;
 }
 
-extern "C" int vatlq_cosine_rowsum(const float* X, int64_t n, int d, const int64_t* rows, int64_t m,
-                                   const double* S, double m_total, double* out, vatlq_stream_t stream_) {
+extern "C" int vatlq_cosine_colsum(const float* X, int64_t n, int d, const int64_t* rows, int64_t m,
+                                   double* S, void* ws, size_t ws_bytes, vatlq_stream_t stream) {
+  return vatlq_cosine_colsum_dt(X, VATLQ_F32, n, d, rows, m, S, ws, ws_bytes, stream);
+}
+
+extern "C" int vatlq_cosine_rowsum_dt(const void* X, int dtype, int64_t n, int d, const int64_t* rows, int64_t m,
+                                      const double* S, double m_total, double* out, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  VQ_REQUIRE(dtype_size(dtype) != 0, "dtype must be VATLQ_F32, VATLQ_F16 or VATLQ_BF16");
   VQ_REQUIRE(X && S && out && n >= 0 && m >= 0, "null pointer");
   VQ_REQUIRE(d > 0 && (d & 3) == 0 && d <= kCosNV * 128, "d must be a multiple of 4 and <= 2048");
-  VQ_REQUIRE(((uintptr_t)X & 15) == 0, "X must be 16-byte aligned");
+  VQ_REQUIRE(quad_aligned(X, dtype), "X must be aligned to 16 bytes (fp32) or 8 bytes (16 bits)");
   VQ_REQUIRE(rows != nullptr || m == n, "m must equal n without a row list");
   if (m == 0) return 0;
   const int grid = (int)std::min<int64_t>((m + kCosRows - 1) / kCosRows, (int64_t)sm_count() * 6);
-  cos_rowsum_kernel<<<grid, kCosThreads, (size_t)d * sizeof(double), stream>>>(X, d, rows, m, S, m_total, out);
-  VQ_LAUNCHED();
-  return 0;
+  return with_dtype(dtype, [&](auto tag) {
+    using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+    cos_rowsum_kernel<T><<<grid, kCosThreads, (size_t)d * sizeof(double), stream>>>((const T*)X, d, rows, m, S, m_total, out);
+    VQ_LAUNCHED();
+    return 0;
+  });
+}
+
+extern "C" int vatlq_cosine_rowsum(const float* X, int64_t n, int d, const int64_t* rows, int64_t m,
+                                   const double* S, double m_total, double* out, vatlq_stream_t stream) {
+  return vatlq_cosine_rowsum_dt(X, VATLQ_F32, n, d, rows, m, S, m_total, out, stream);
 }
 
 extern "C" int vatlq_minmax_stats_f64(const double* v, const uint8_t* mask, int64_t n, double* stats2,

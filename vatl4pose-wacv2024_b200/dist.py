@@ -155,7 +155,11 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
     """One query over a pool sharded across the ranks of `group` (one process per GPU).
     Every rank passes its slice of the pool and gets the same global pick list back.  Heat-map shards may be
     fp32, fp16 or bf16 (the same dtype on every rank; the picks equal those of the fp32 upcast), and so may the
-    embedding shards X_local for the Coreset filter: they are gathered and selected on as they are.
+    embedding shards X_local for representativeness "Influence" and the Coreset and Diversity filters: Influence
+    reads each rank's shard as it is, the filters gather the shards and select on them as they are, and the
+    scores and picks equal those of the fp32 upcast.  Every rank must hold X_local in one dtype (checked once, on
+    every rank, before the first step that reads it).  The K-Means and weighted filters take fp32 shards only
+    (kmeans.py raises VatlqError on a 16-bit X).
     uncertainty: any accelerated name (THC*, WPU*, THC+WPU, HP, TPC, Entropy, MPE, Margin, None);
     representativeness: "None" or "Influence" (ActiveLearning.py:467-477); filter: "Coreset" (:609-614),
     "None" (top-k, :533-534), "Diversity" (:581-590), "K-Means" (:593-608) or "weighted" (:553-580; w_unc = cfg.VAL.W_UNC;
@@ -187,6 +191,10 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
     # (group=None means the default group to torch.distributed but "single GPU" to QueryPass.fuse)
     fuse_group = (group if group is not None else td.group.WORLD) if world > 1 else None
     n_unl = n - lab.size
+    # every rank must hold one embedding dtype: the all-gather of the filters needs one row size, and Influence's
+    # column sums are only the upcast's when every shard is read the same way (filter "None" reads no X)
+    if world > 1 and (representativeness == "Influence" or filter != "None"):
+        _agree_dtype(X_local, "distributed_query", group)
     score_local = qp.fuse(unl[lo:hi], thc_vs_wpu, labeled_ratio=lab.size / max(n, 1), group=fuse_group,
                           n_unlabeled_global=n_unl)
     if representativeness == "Influence" and n_unl > 1:                      # (:467-477, 517-526)
@@ -195,8 +203,6 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
     score = allgather_rows(score_local, n, world, group)
 
     def gather_X():
-        if world > 1:   # the all-gather needs one row size on every rank
-            _agree_dtype(X_local, "distributed_query", group)
         return allgather_rows(X_local, n, world, group)
     picks, _, st = select(score, unl, gather_X, k, filter, labeled=lab, moks=moks, lam=lam, rule=rule,
                           first_pick=first_pick, batch=batch, comm=comm.handle if comm is not None else None,

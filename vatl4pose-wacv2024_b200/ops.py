@@ -36,7 +36,7 @@ def _cuda(t: torch.Tensor, dtype, name: str) -> torch.Tensor:
 # heat-map element types and their VATLQ_* codes: 16-bit maps are read as they are, and every result equals the
 # fp32 path's on their exact upcast, bit for bit (include/vatlq.h)
 HEATMAP_DTYPES = {torch.float32: _lib.F32, torch.float16: _lib.F16, torch.bfloat16: _lib.BF16}
-# embedding element types of the core-set and pairwise-distance entries: the same contract, for X
+# embedding element types of the core-set, pairwise-distance and cosine row-sum entries: the same contract, for X
 EMBEDDING_DTYPES = HEATMAP_DTYPES
 
 
@@ -418,8 +418,11 @@ def heatmap_entropy(H: torch.Tensor) -> torch.Tensor:
 def cosine_rowsum(X: torch.Tensor, rows=None, group=None) -> torch.Tensor:
     """Row sums of the cosine-distance matrix of X[rows] (all rows when None): the Influence score
     before normalisation (ActiveLearning.py:471-475) / the Diversity score (:582-585), fp64 (m,).
-    `group`: ranks hold disjoint row sets of one pool; the column sums are all-reduced."""
-    X = _cuda(X, torch.float32, "X")
+    X (n,d) CUDA in one of EMBEDDING_DTYPES (vatlq_cosine_*_dt): a 16-bit X is read as it is and gives, bit for bit,
+    the row sums of its fp32 upcast.  `group`: ranks hold disjoint row sets of one pool; the column sums are
+    all-reduced."""
+    X = _embeddings(X, "X")
+    dt = EMBEDDING_DTYPES[X.dtype]
     n, d = X.shape
     dev = X.device
     r = None
@@ -434,16 +437,16 @@ def cosine_rowsum(X: torch.Tensor, rows=None, group=None) -> torch.Tensor:
     S = torch.empty(d, dtype=torch.float64, device=dev)
     out = torch.empty(m, dtype=torch.float64, device=dev)
     with torch.cuda.device(dev):
-        _lib.check(L.vatlq_cosine_colsum(_ptr(X), n, d, _ptr(r), m, _ptr(S), _ptr(ws), ws_bytes, _stream()),
-                   "vatlq_cosine_colsum")
+        _lib.check(L.vatlq_cosine_colsum_dt(_ptr(X), dt, n, d, _ptr(r), m, _ptr(S), _ptr(ws), ws_bytes, _stream()),
+                   "vatlq_cosine_colsum_dt")
         m_total = m
         if group is not None:
             torch.distributed.all_reduce(S, group=group)
             cnt = torch.tensor([m], dtype=torch.int64, device=dev)
             torch.distributed.all_reduce(cnt, group=group)
             m_total = int(cnt.item())
-        _lib.check(L.vatlq_cosine_rowsum(_ptr(X), n, d, _ptr(r), m, _ptr(S), float(m_total), _ptr(out), _stream()),
-                   "vatlq_cosine_rowsum")
+        _lib.check(L.vatlq_cosine_rowsum_dt(_ptr(X), dt, n, d, _ptr(r), m, _ptr(S), float(m_total), _ptr(out),
+                                            _stream()), "vatlq_cosine_rowsum_dt")
     return out
 
 

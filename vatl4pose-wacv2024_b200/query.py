@@ -64,7 +64,8 @@ def unlabelled_mask(n: int, labeled, device) -> torch.Tensor:
 def influence(X: torch.Tensor, unl: torch.Tensor, group=None) -> torch.Tensor:
     """Influence representativeness (ActiveLearning.py:467-475): row sums of the cosine-distance graph of the
     unlabelled rows, min-max normalised over them; fp64 (len(unl),), 0 on labelled rows.  X holds the rows `unl`
-    masks.  `group`: the ranks hold disjoint row ranges of one pool (column sums and min / max are all-reduced)."""
+    masks, in any of ops.EMBEDDING_DTYPES (a 16-bit X gives the bits of its fp32 upcast).  `group`: the ranks hold
+    disjoint row ranges of one pool (column sums and min / max are all-reduced)."""
     rows = torch.nonzero(unl, as_tuple=False).flatten()
     infl = torch.zeros(unl.numel(), dtype=torch.float64, device=unl.device)
     infl[rows] = ops.minmax_f64(ops.cosine_rowsum(X, rows=rows, group=group), group=group)
@@ -83,6 +84,8 @@ def select(score: torch.Tensor, unl: torch.Tensor, X, k: int, filter: str, *, la
     drops duplicate rows (np.unique(axis=0), which also sorts them), weighs each row 1 + w_unc * combine_weight *
     score and maps the chosen rows of that sorted matrix straight through the candidate ids (:553-580, kept as the
     reference has it); both clamp k to the rows they cluster, like the reference clamps query_size.
+    X may be fp32, fp16 or bf16 for Diversity and Coreset (read as it is, the picks of its fp32 upcast); K-Means and
+    weighted take fp32 only (kmeans.py raises VatlqError on a 16-bit X).
     `group`: the ranks hold the same X and share the K-Means assignment step.
     Returns (picks, k, stats): int64 ids on score's device in the reference's order, the k the filter used, and
     its CoresetStats or K-Means {"n_iter", "relocations"} (None for the other filters)."""
