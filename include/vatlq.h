@@ -336,10 +336,11 @@ int vatlq_oks(const float* kpts, const float* gt_kpts, const float* bbox_ann_xyx
  * sklearn.cluster.KMeans(n_clusters=query_size, random_state=318).fit_predict(embeddings[, sample_weight]) followed
  * by "per cluster, the member closest to its centre".  sklearn's algorithm (1.7.1 pinned by the reference:
  * _kmeans.py _kmeans_plusplus / _kmeans_single_lloyd, _k_means_lloyd.pyx, _k_means_common.pyx) in fp64 over the
- * fp32 embeddings; both GEMM-shaped steps run on the fp64 tensor cores.  The host layer (kmeans.py) draws the random
+ * embeddings; both GEMM-shaped steps run on the fp64 tensor cores.  The host layer (kmeans.py) draws the random
  * numbers from numpy's RandomState exactly as sklearn does and decides convergence from a few scalars.
- * X (n,d) fp32 row-major, 16-byte aligned, d % 4 == 0, n < 2^31; w fp64[n] sample weights or NULL (all 1).
- * One workspace of vatlq_kmeans_workspace_bytes(n,d,k) serves every call (they never overlap).
+ * X (n,d) row-major, d % 4 == 0, n < 2^31: fp32 (16-byte aligned for _pp and _assign) in the plain entries, fp32, fp16
+ * or bf16 in the *_dt entries (see below); w fp64[n] sample weights or NULL (all 1).
+ * One workspace of vatlq_kmeans_workspace_bytes(n,d,k) serves every call (they never overlap), in every dtype.
  *
  * Which bits matter: label decisions are robust to rounding, but the closest member of a TWO-member cluster is a
  * structural tie that the reference resolves by the rounding of its own arithmetic; the M step and the final
@@ -383,6 +384,31 @@ int vatlq_kmeans_rowdist(const float* X, int64_t n, int d, const double* C, cons
                          vatlq_stream_t stream);
 int vatlq_kmeans_pick(const double* dis, const int32_t* order, const int32_t* starts, int64_t k, int32_t* picks,
                       vatlq_stream_t stream);
+/* The seven calls that read X, on X in any VATLQ_* dtype (the fp32 entries are these calls with VATLQ_F32; the other
+ * arguments are theirs).  Every 16-bit value is widened exactly to fp32 at the load, and to fp64 where the fp32 code
+ * does that; the fp64 instruction sequence after the load is unchanged.  So for a 16-bit X every output (mean, the
+ * tolerance, center_ids, closest, centres, labels, the change count, sums, dis) equals, bit for bit, that of the same
+ * call on X's fp32 upcast, and the estimator built on them gives its labels, iteration count and picks.  A 16-bit X
+ * must be 8-byte aligned in every call; an fp32 X keeps the alignment rule of its plain entry.  An unknown dtype or a
+ * misaligned X returns VATLQ_EINVAL before any device work. */
+int vatlq_kmeans_mean_var_dt(const void* X, int dtype, int64_t n, int d, double* mean, double* out1, void* ws,
+                             size_t ws_bytes, vatlq_stream_t stream);
+int vatlq_kmeans_pp_dt(const void* X, int dtype, int64_t n, int d, const double* w, int64_t k, int64_t first_center,
+                       const double* rand_vals, int trials, int32_t* center_ids, double* closest, void* ws,
+                       size_t ws_bytes, vatlq_stream_t stream);
+int vatlq_kmeans_gather_dt(const void* X, int dtype, int d, const int32_t* ids, int64_t k, const double* mean,
+                           double* Cc, double* Cr, vatlq_stream_t stream);
+int vatlq_kmeans_assign_dt(const void* X, int dtype, int64_t n, int d, const double* C, int64_t k, int32_t* labels,
+                           const int32_t* labels_old, int32_t* changed, void* ws, size_t ws_bytes,
+                           vatlq_stream_t stream);
+int vatlq_kmeans_update_dt(const void* X, int dtype, int64_t n, int d, const double* w, const double* mean,
+                           const int32_t* labels, int64_t k, double* sums, double* wsum, int32_t* order,
+                           int32_t* starts, int32_t* n_empty, void* ws, size_t ws_bytes, vatlq_stream_t stream);
+int vatlq_kmeans_relocate_dt(const void* X, int dtype, int d, const double* w, const double* mean,
+                             const int32_t* labels, const int32_t* empty_ids, const int32_t* far_ids, int n_empty,
+                             double* sums, double* wsum, vatlq_stream_t stream);
+int vatlq_kmeans_rowdist_dt(const void* X, int dtype, int64_t n, int d, const double* C, const int32_t* labels,
+                            double* dis, vatlq_stream_t stream);
 
 /* fp64 tensor-core (mma.sync.m8n8k4.f64, DMMA) peak of the current device in FMA/s, measured with a saturating
  * register-only kernel (about 10 ms): the roofline denominator of the paired core-set pass, which is bound by the

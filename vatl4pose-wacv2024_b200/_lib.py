@@ -68,6 +68,13 @@ SIGNATURES = {
     "vatlq_kmeans_average": (_int, [_vp, _vp, _i64, _int, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "vatlq_kmeans_rowdist": (_int, [_vp, _i64, _int, _vp, _vp, _vp, _vp]),
     "vatlq_kmeans_pick": (_int, [_vp, _vp, _vp, _i64, _vp, _vp]),
+    "vatlq_kmeans_mean_var_dt": (_int, [_vp, _int, _i64, _int, _vp, _vp, _vp, _sz, _vp]),
+    "vatlq_kmeans_pp_dt": (_int, [_vp, _int, _i64, _int, _vp, _i64, _i64, _vp, _int, _vp, _vp, _vp, _sz, _vp]),
+    "vatlq_kmeans_gather_dt": (_int, [_vp, _int, _int, _vp, _i64, _vp, _vp, _vp, _vp]),
+    "vatlq_kmeans_assign_dt": (_int, [_vp, _int, _i64, _int, _vp, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "vatlq_kmeans_update_dt": (_int, [_vp, _int, _i64, _int, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "vatlq_kmeans_relocate_dt": (_int, [_vp, _int, _int, _vp, _vp, _vp, _vp, _vp, _int, _vp, _vp, _vp]),
+    "vatlq_kmeans_rowdist_dt": (_int, [_vp, _int, _i64, _int, _vp, _vp, _vp, _vp]),
     "vatlq_measure_fp64_mma": (_int, [_vp, _vp, _sz, _vp]),
     "vatlq_oks": (_int, [_vp, _vp, _vp, _i64, _vp, _vp]),
     "vatlq_profile_passes": (_int, [_int]),

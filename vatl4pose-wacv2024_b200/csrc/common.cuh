@@ -53,7 +53,10 @@ inline int sm_count() {
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 int fill_f64(double* p, long long n, double v, cudaStream_t stream);
-int vq_launch_norms(const float* X, int64_t n, int d, double* xx, cudaStream_t stream);   // canonical |x|^2 (coreset.cu)
+// canonical |x|^2 of every row (coreset.cu); a 16-bit X gives the bits of its fp32 upcast
+int vq_launch_norms(const float* X, int64_t n, int d, double* xx, cudaStream_t stream);
+int vq_launch_norms(const __half* X, int64_t n, int d, double* xx, cudaStream_t stream);
+int vq_launch_norms(const __nv_bfloat16* X, int64_t n, int d, double* xx, cudaStream_t stream);
 
 // ---------------------------------------------------------------- device helpers
 __device__ __forceinline__ float4 ldg_stream(const float4* p) {

@@ -2312,6 +2312,8 @@ static void prune_collect(const PruneState& P) {
 
 namespace vatlq {
 int vq_launch_norms(const float* X, int64_t n, int d, double* xx, cudaStream_t stream) { return launch_norms(X, n, d, xx, stream); }
+int vq_launch_norms(const __half* X, int64_t n, int d, double* xx, cudaStream_t stream) { return launch_norms(X, n, d, xx, stream); }
+int vq_launch_norms(const __nv_bfloat16* X, int64_t n, int d, double* xx, cudaStream_t stream) { return launch_norms(X, n, d, xx, stream); }
 }  // namespace vatlq
 
 // X of the core-set calls: check_x, plus 16-byte alignment when d = 2048 (the TMA passes copy whole rows with

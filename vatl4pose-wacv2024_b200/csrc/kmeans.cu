@@ -20,6 +20,9 @@
 // operation: X_mean = X.mean(axis=0) (sequential over rows), centre sums of (x - X_mean) * w in ascending row order
 // (= sklearn with one OpenMP thread; any thread count for clusters of <= 2 members), * (1 / weight), + X_mean, and
 // dis = ((X - centre) ** 2).sum(axis=1) in numpy's pairwise order.  DESIGN.md 4.7.
+// Every kernel that reads X is a template on its element type T (float, __half, __nv_bfloat16): a 16-bit feature is
+// widened exactly to fp32 where it is loaded and the fp64 instruction sequence after the load is the fp32 one, so a
+// 16-bit X gives, bit for bit, every result of its fp32 upcast.
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/block/block_scan.cuh>
 
@@ -37,17 +40,31 @@ __device__ __forceinline__ void cp_async16(void* smem, const void* gmem, bool va
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(smem)), "l"(gmem), "r"(sz) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+// four 16-bit features (8 bytes): the .ca form is the one that copies fewer than 16 bytes
+__device__ __forceinline__ void cp_async8(void* smem, const void* gmem, bool valid) {
+  const unsigned sz = valid ? 8u : 0u;       // src-size 0: the 8 bytes are zero-filled
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(smem_u32(smem)), "l"(gmem), "r"(sz) : "memory");
+}
+// a chunk of four X features, copied in X's own type
+template <typename T>
+__device__ __forceinline__ void cp_async_quad(T* smem, const T* gmem, bool valid) {
+  if constexpr (sizeof(T) == 4) cp_async16(smem, gmem, valid);
+  else cp_async8(smem, gmem, valid);
+}
 template <int N>
 __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
 }
 
 // ------------------------------------------------------------------------------------
-// Tile machine: S[i][j] = sum_k X[i][k] * C[j][k], X fp32 (n x d, converted on the fly), C fp64 (m x d).
+// Tile machine: S[i][j] = sum_k X[i][k] * C[j][k], X of type T (n x d, converted on the fly), C fp64 (m x d).
 // CTA tile BM rows x BN centres, WM x WN warps, each warp (BM/WM) x (BN/WN) as 8x8 DMMA tiles.  A k-block is 32
 // features = two sub-tiles of 16: lane (g = lane/4, q = lane%4) takes features 4q..4q+3 of a sub-tile for its
 // row g (one LDS.128 of X, two of C) and feeds them to four DMMAs — the k order inside a DMMA is free as long as
 // both operands agree.  Sub-tile rows: X 16 floats (64 B), C 16 + 2 doubles (144 B): both conflict-free.
+// A 16-bit X is staged in its own type (16 features = 32 B per sub-tile row, 8-byte cp.async chunks, one LDS.64 per
+// lane widened to a float4 in registers): lane (g, q) feeds the same four features to the same four DMMAs as in fp32,
+// so the accumulators hold the same bits.
 // MODE 0 (assign): running argmin_j (cn[j] - 2 S) over all centre chunks -> labels (+ count of changed labels)
 // MODE 1 (dist)  : out[i*BN + j] = max(0, (-2 S + cc[j]) + xx[i])   (sklearn _euclidean_distances, squared)
 // ------------------------------------------------------------------------------------
@@ -55,13 +72,14 @@ constexpr int kBK = 32;
 constexpr int kStages = 3;
 constexpr int kCS = 18;      // doubles per C sub-tile row
 
-template <int BM, int BN>
+template <typename T, int BM, int BN>
 struct GemmStage {
-  static constexpr size_t kBytes = (size_t)2 * BM * 16 * 4 + (size_t)2 * BN * kCS * 8;
+  static constexpr size_t kXBytes = (size_t)2 * BM * 16 * sizeof(T);
+  static constexpr size_t kBytes = kXBytes + (size_t)2 * BN * kCS * 8;
 };
 
 struct GemmArgs {
-  const float* X;
+  const void* X;         // n x d of the kernel's element type
   long long n;
   int d;
   const double* C;       // m x d
@@ -74,9 +92,11 @@ struct GemmArgs {
   double* out;           // MODE 1: n x BN
 };
 
-template <int BM, int BN, int WM, int WN, int MODE>
+template <typename T, int BM, int BN, int WM, int WN, int MODE>
 __global__ void __launch_bounds__(WM * WN * 32) km_gemm_kernel(GemmArgs a) {
   pdl_enter();
+  using Stage = GemmStage<T, BM, BN>;
+  const T* X = static_cast<const T*>(a.X);
   constexpr int kThreads = WM * WN * 32;
   constexpr int TM = BM / WM / 8, TN = BN / WN / 8;
   extern __shared__ __align__(16) unsigned char km_smem[];
@@ -88,21 +108,21 @@ __global__ void __launch_bounds__(WM * WN * 32) km_gemm_kernel(GemmArgs a) {
   const int chunks = (int)((a.m + BN - 1) / BN);
   const long long total = (long long)chunks * KT;
 
-  auto stage_A = [&](int s, int u) { return reinterpret_cast<float*>(km_smem + (size_t)s * GemmStage<BM, BN>::kBytes) + u * BM * 16; };
+  auto stage_A = [&](int s, int u) { return reinterpret_cast<T*>(km_smem + (size_t)s * Stage::kBytes) + u * BM * 16; };
   auto stage_C = [&](int s, int u) {
-    return reinterpret_cast<double*>(km_smem + (size_t)s * GemmStage<BM, BN>::kBytes + (size_t)2 * BM * 16 * 4) + u * BN * kCS;
+    return reinterpret_cast<double*>(km_smem + (size_t)s * Stage::kBytes + Stage::kXBytes) + u * BN * kCS;
   };
   auto load_stage = [&](long long it) {
     const int s = (int)(it % kStages);
     const int jc = (int)(it / KT), kt = (int)(it - (long long)jc * KT);
     const int k0 = kt * kBK;
-    // X: BM rows x 8 chunks of 4 floats
+    // X: BM rows x 8 chunks of 4 features
     for (int c = tid; c < BM * 8; c += kThreads) {
       const int r = c >> 3, ch = c & 7;
       const long long row = min(row0 + r, a.n - 1);
       const int col = k0 + ch * 4;
       const bool ok = col < a.d;
-      cp_async16(stage_A(s, ch >> 2) + r * 16 + (ch & 3) * 4, a.X + (size_t)row * a.d + (ok ? col : 0), ok);
+      cp_async_quad(stage_A(s, ch >> 2) + r * 16 + (ch & 3) * 4, X + (size_t)row * a.d + (ok ? col : 0), ok);
     }
     // C: BN rows x 16 chunks of 2 doubles
     for (int c = tid; c < BN * 16; c += kThreads) {
@@ -137,12 +157,12 @@ __global__ void __launch_bounds__(WM * WN * 32) km_gemm_kernel(GemmArgs a) {
     const int s = (int)(it % kStages);
 #pragma unroll
     for (int u = 0; u < 2; ++u) {
-      const float* As = stage_A(s, u);
+      const T* As = stage_A(s, u);
       const double* Cs = stage_C(s, u);
       float4 xa[TM];
       double cb[TN][4];
 #pragma unroll
-      for (int mi = 0; mi < TM; ++mi) xa[mi] = *reinterpret_cast<const float4*>(As + (wm * TM * 8 + mi * 8 + g) * 16 + 4 * q);
+      for (int mi = 0; mi < TM; ++mi) xa[mi] = load_quad(As + (wm * TM * 8 + mi * 8 + g) * 16 + 4 * q, 0);
 #pragma unroll
       for (int ni = 0; ni < TN; ++ni) {
         const double2* p = reinterpret_cast<const double2*>(Cs + (wn * TN * 8 + ni * 8 + g) * kCS + 4 * q);
@@ -241,12 +261,13 @@ __global__ void __launch_bounds__(WM * WN * 32) km_gemm_kernel(GemmArgs a) {
 
 // ------------------------------------------------------------------------------------ small kernels
 // seeds: Cc[t] = X[ids[t]] - X_mean (sklearn's centres live in the centred frame), Cr[t] = Cc[t] + X_mean
-__global__ void __launch_bounds__(256) km_gather_kernel(const float* __restrict__ X, int d, const int* __restrict__ ids,
+template <typename T>
+__global__ void __launch_bounds__(256) km_gather_kernel(const T* __restrict__ X, int d, const int* __restrict__ ids,
                                                         const double* __restrict__ mean, double* __restrict__ Cc, double* __restrict__ Cr) {
   const int t = blockIdx.x;
   const long long r = ids[t];
   for (int c = threadIdx.x; c < d; c += blockDim.x) {
-    const double v = __dsub_rn((double)X[(size_t)r * d + c], mean[c]);
+    const double v = __dsub_rn((double)to_f32(X[(size_t)r * d + c]), mean[c]);
     Cc[(size_t)t * d + c] = v;
     Cr[(size_t)t * d + c] = __dadd_rn(v, mean[c]);
   }
@@ -428,7 +449,8 @@ __global__ void km_pp_seed_kernel(PpState* st, int first) {
 }
 // candidate t of the step: clip(searchsorted(cum, rand_t * current_pot), n - 1) (side='left': first cum >= value;
 // rand_vals == NULL: the seed row already in the state), then its row as fp64 into the candidate tile + its norm
-__global__ void __launch_bounds__(256) km_candidates_kernel(const float* __restrict__ X, int d, long long n, const double* __restrict__ cum,
+template <typename T>
+__global__ void __launch_bounds__(256) km_candidates_kernel(const T* __restrict__ X, int d, long long n, const double* __restrict__ cum,
                                                             const double* __restrict__ rand_vals, PpState* st, int trials,
                                                             const double* __restrict__ xx, double* __restrict__ C, double* __restrict__ cc) {
   pdl_enter();
@@ -451,7 +473,7 @@ __global__ void __launch_bounds__(256) km_candidates_kernel(const float* __restr
   }
   __syncthreads();
   const long long r = s_row;
-  for (int c = threadIdx.x; c < d; c += blockDim.x) C[(size_t)t * d + c] = live ? (double)X[(size_t)r * d + c] : 0.0;
+  for (int c = threadIdx.x; c < d; c += blockDim.x) C[(size_t)t * d + c] = live ? (double)to_f32(X[(size_t)r * d + c]) : 0.0;
   if (threadIdx.x == 0) {
     cc[t] = live ? xx[r] : 0.0;
     if (rand_vals && live) st->cand[t] = (int)r;      // (dead blocks may see either cand[0]: they never use the row)
@@ -478,7 +500,8 @@ __global__ void __launch_bounds__(256) km_starts_kernel(const int* __restrict__ 
   starts[j] = (int)lo;
 }
 // centre sums in ascending row order: sums[j][c] = sum_i (x_i[c] - X_mean[c]) * w_i, wsum[j] = sum_i w_i; one CTA per cluster
-__global__ void __launch_bounds__(256) km_sums_kernel(const float* __restrict__ X, int d, const double* __restrict__ w, const double* __restrict__ mean,
+template <typename T>
+__global__ void __launch_bounds__(256) km_sums_kernel(const T* __restrict__ X, int d, const double* __restrict__ w, const double* __restrict__ mean,
                                                       const int* __restrict__ order, const int* __restrict__ starts, long long k,
                                                       double* __restrict__ sums, double* __restrict__ wsum, int* __restrict__ n_empty) {
   const long long j = blockIdx.x;
@@ -489,7 +512,7 @@ __global__ void __launch_bounds__(256) km_sums_kernel(const float* __restrict__ 
     for (int p = lo; p < hi; ++p) {
       const int i = order[p];
       const double wi = w ? w[i] : 1.0;
-      const float4 v = __ldg(reinterpret_cast<const float4*>(X + (size_t)i * d + c0));
+      const float4 v = ldg_quad(X + (size_t)i * d + c0, 0);
       s0 = __dadd_rn(s0, __dmul_rn(__dsub_rn((double)v.x, m0), wi));
       s1 = __dadd_rn(s1, __dmul_rn(__dsub_rn((double)v.y, m1), wi));
       s2 = __dadd_rn(s2, __dmul_rn(__dsub_rn((double)v.z, m2), wi));
@@ -506,7 +529,8 @@ __global__ void __launch_bounds__(256) km_sums_kernel(const float* __restrict__ 
   }
 }
 // _relocate_empty_clusters_dense: sequential over the empty clusters (a row's old cluster may repeat)
-__global__ void __launch_bounds__(256) km_relocate_kernel(const float* __restrict__ X, int d, const double* __restrict__ w,
+template <typename T>
+__global__ void __launch_bounds__(256) km_relocate_kernel(const T* __restrict__ X, int d, const double* __restrict__ w,
                                                           const double* __restrict__ mean, const int* __restrict__ labels, const int* __restrict__ empty_ids,
                                                           const int* __restrict__ far_ids, int n_empty, double* __restrict__ sums,
                                                           double* __restrict__ wsum) {
@@ -514,7 +538,7 @@ __global__ void __launch_bounds__(256) km_relocate_kernel(const float* __restric
     const int nw = empty_ids[e], far = far_ids[e], old = labels[far];
     const double wi = w ? w[far] : 1.0;
     for (int c = threadIdx.x; c < d; c += blockDim.x) {
-      const double xv = __dmul_rn(__dsub_rn((double)X[(size_t)far * d + c], mean[c]), wi);
+      const double xv = __dmul_rn(__dsub_rn((double)to_f32(X[(size_t)far * d + c]), mean[c]), wi);
       sums[(size_t)old * d + c] = __dsub_rn(sums[(size_t)old * d + c], xv);
       sums[(size_t)nw * d + c] = xv;
     }
@@ -569,11 +593,13 @@ __global__ void __launch_bounds__(256) km_average_kernel(const double* __restric
 // dis_i = ((x_i - C[label_i]) ** 2).sum() in numpy's pairwise order (numpy/_core/src/umath/loops_utils.h.src,
 // DOUBLE_pairwise_sum: < 8 sequential; <= 128: eight strided accumulators, fixed combine tree, sequential tail;
 // else split at n/2 rounded down to a multiple of 8).  One thread per row.
-__device__ __forceinline__ double km_sq(const float* __restrict__ x, const double* __restrict__ c, int i) {
-  const double t = __dsub_rn((double)x[i], c[i]);
+template <typename T>
+__device__ __forceinline__ double km_sq(const T* __restrict__ x, const double* __restrict__ c, int i) {
+  const double t = __dsub_rn((double)to_f32(x[i]), c[i]);
   return __dmul_rn(t, t);
 }
-__device__ __forceinline__ double km_pairwise_leaf(const float* __restrict__ x, const double* __restrict__ c, int n) {   // n <= 128
+template <typename T>
+__device__ __forceinline__ double km_pairwise_leaf(const T* __restrict__ x, const double* __restrict__ c, int n) {   // n <= 128
   if (n < 8) {
     double res = 0.0;
     for (int i = 0; i < n; ++i) res = __dadd_rn(res, km_sq(x, c, i));
@@ -592,7 +618,8 @@ __device__ __forceinline__ double km_pairwise_leaf(const float* __restrict__ x, 
   return res;
 }
 // the recursion "pairwise(a, n2) + pairwise(a + n2, n - n2)" unrolled onto an explicit stack (depth <= log2(n / 128) + 1)
-__device__ double km_pairwise(const float* __restrict__ x, const double* __restrict__ c, int n) {
+template <typename T>
+__device__ double km_pairwise(const T* __restrict__ x, const double* __restrict__ c, int n) {
   constexpr int kDepth = 24;
   int off[kDepth], len[kDepth];
   double acc[kDepth];
@@ -624,7 +651,8 @@ __device__ double km_pairwise(const float* __restrict__ x, const double* __restr
     ++sp;
   }
 }
-__global__ void __launch_bounds__(128) km_rowdist_kernel(const float* __restrict__ X, long long n, int d, const double* __restrict__ C,
+template <typename T>
+__global__ void __launch_bounds__(128) km_rowdist_kernel(const T* __restrict__ X, long long n, int d, const double* __restrict__ C,
                                                          const int* __restrict__ labels, double* __restrict__ dis) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -661,7 +689,8 @@ __global__ void __launch_bounds__(256) km_pick_kernel(const double* __restrict__
 
 // ---- X.mean(axis=0) exactly like numpy (out[c] += X[i][c] row after row, then / n): one thread per column,
 // eight rows of loads in flight
-__global__ void __launch_bounds__(128) km_colmean_kernel(const float* __restrict__ X, long long n, int d, double* __restrict__ mean) {
+template <typename T>
+__global__ void __launch_bounds__(128) km_colmean_kernel(const T* __restrict__ X, long long n, int d, double* __restrict__ mean) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= d) return;
   double s = 0.0;
@@ -669,16 +698,17 @@ __global__ void __launch_bounds__(128) km_colmean_kernel(const float* __restrict
   for (; i + 8 <= n; i += 8) {
     float v[8];
 #pragma unroll
-    for (int e = 0; e < 8; ++e) v[e] = __ldg(X + (size_t)(i + e) * d + c);
+    for (int e = 0; e < 8; ++e) v[e] = ldg_f32(X + (size_t)(i + e) * d + c);
 #pragma unroll
     for (int e = 0; e < 8; ++e) s = __dadd_rn(s, (double)v[e]);
   }
-  for (; i < n; ++i) s = __dadd_rn(s, (double)__ldg(X + (size_t)i * d + c));
+  for (; i < n; ++i) s = __dadd_rn(s, (double)ldg_f32(X + (size_t)i * d + c));
   mean[c] = __ddiv_rn(s, (double)n);
 }
 // ---- np.var(X, axis=0) (only feeds the convergence tolerance): fixed-order blocked sums of squared deviations
 constexpr int kVarRowBlocks = 256;
-__global__ void __launch_bounds__(256) km_colvar_kernel(const float* __restrict__ X, long long n, int d, const double* __restrict__ mean,
+template <typename T>
+__global__ void __launch_bounds__(256) km_colvar_kernel(const T* __restrict__ X, long long n, int d, const double* __restrict__ mean,
                                                         double* __restrict__ part) {
   const int c = blockIdx.x * 256 + threadIdx.x;
   const long long per = (n + gridDim.y - 1) / gridDim.y;
@@ -687,7 +717,7 @@ __global__ void __launch_bounds__(256) km_colvar_kernel(const float* __restrict_
   const double mu = mean[c];
   double s = 0.0;
   for (long long i = lo; i < hi; ++i) {
-    const double df = __dsub_rn((double)X[(size_t)i * d + c], mu);
+    const double df = __dsub_rn((double)to_f32(X[(size_t)i * d + c]), mu);
     s = fma(df, df, s);
   }
   part[(size_t)blockIdx.y * d + c] = s;
@@ -714,16 +744,16 @@ __global__ void __launch_bounds__(256) km_mean_kernel(const double* __restrict__
   }
 }
 
-template <int BM, int BN, int WM, int WN, int MODE>
+template <typename T, int BM, int BN, int WM, int WN, int MODE>
 static int launch_gemm(const GemmArgs& a, cudaStream_t stream, bool pdl = false) {
-  const size_t smem = kStages * GemmStage<BM, BN>::kBytes;
+  const size_t smem = kStages * GemmStage<T, BM, BN>::kBytes;
   static bool configured = false;
   if (!configured) {
-    VQ_CUDA(cudaFuncSetAttribute((km_gemm_kernel<BM, BN, WM, WN, MODE>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    VQ_CUDA(cudaFuncSetAttribute((km_gemm_kernel<T, BM, BN, WM, WN, MODE>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = true;
   }
   const unsigned grid = (unsigned)((a.n + BM - 1) / BM);
-  VQ_CUDA(launch_pdl(km_gemm_kernel<BM, BN, WM, WN, MODE>, dim3(grid), dim3(WM * WN * 32), smem, stream, pdl, a));
+  VQ_CUDA(launch_pdl(km_gemm_kernel<T, BM, BN, WM, WN, MODE>, dim3(grid), dim3(WM * WN * 32), smem, stream, pdl, a));
   g_launches.fetch_add(1);
   return 0;
 }
@@ -751,6 +781,18 @@ static size_t pp_ws_bytes(int64_t n, int d) {
 static size_t update_ws_bytes(int64_t n) { return align_up(sort_bytes(n), 256) + 3 * align_up((size_t)n * 4, 256); }
 static size_t var_ws_bytes(int d) { return (size_t)(kVarRowBlocks + 1) * d * 8; }
 
+// X of a *_dt entry, checked in the entry itself (the message names it): a known dtype code, and a 16-bit X 8-byte
+// aligned (its quad loads are 8 bytes wide).  An fp32 X keeps the checks its entry has always made.
+#define KM_REQUIRE_DTYPE(X, dtype)                                                              \
+  do {                                                                                          \
+    VQ_REQUIRE(dtype_size(dtype) != 0, "dtype must be VATLQ_F32, VATLQ_F16 or VATLQ_BF16");     \
+    VQ_REQUIRE((dtype) == VATLQ_F32 || quad_aligned(X, dtype), "a 16-bit X must be 8-byte aligned"); \
+  } while (0)
+
+// the element type of a with_dtype tag
+template <typename P>
+using km_elem_t = std::remove_const_t<std::remove_pointer_t<P>>;
+
 /* one scratch size that serves every vatlq_kmeans_* call (they never run concurrently on one workspace) */
 extern "C" size_t vatlq_kmeans_workspace_bytes(int64_t n, int d, int64_t k) {
   if (n <= 0 || d <= 0 || k <= 0) return 0;
@@ -758,36 +800,39 @@ extern "C" size_t vatlq_kmeans_workspace_bytes(int64_t n, int d, int64_t k) {
 }
 
 /* mean[d] = X.mean(axis=0) (numpy's order), out1[0] = np.mean(np.var(X, axis=0)) */
-extern "C" int vatlq_kmeans_mean_var(const float* X, int64_t n, int d, double* mean, double* out1, void* ws, size_t ws_bytes,
-                                     vatlq_stream_t stream_) {
+extern "C" int vatlq_kmeans_mean_var_dt(const void* X, int dtype, int64_t n, int d, double* mean, double* out1, void* ws,
+                                        size_t ws_bytes, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  KM_REQUIRE_DTYPE(X, dtype);
   VQ_REQUIRE(km_shape_ok(n, d) && X && mean && out1 && ws, "bad arguments");
   VQ_REQUIRE(ws_bytes >= var_ws_bytes(d), "workspace too small (vatlq_kmeans_workspace_bytes)");
   double* part = (double*)ws;
   double* var = part + (size_t)kVarRowBlocks * d;
-  km_colmean_kernel<<<(d + 127) / 128, 128, 0, stream>>>(X, n, d, mean);
-  VQ_LAUNCHED();
   const int rb = (int)std::min<long long>(kVarRowBlocks, n);
-  const dim3 grid((d + 255) / 256, rb);
-  km_colvar_kernel<<<grid, 256, 0, stream>>>(X, n, d, mean, part);
-  VQ_LAUNCHED();
+  const int rc = with_dtype(dtype, [&](auto tag) {
+    using T = km_elem_t<decltype(tag)>;
+    km_colmean_kernel<T><<<(d + 127) / 128, 128, 0, stream>>>((const T*)X, n, d, mean);
+    VQ_LAUNCHED();
+    km_colvar_kernel<T><<<dim3((d + 255) / 256, rb), 256, 0, stream>>>((const T*)X, n, d, mean, part);
+    VQ_LAUNCHED();
+    return 0;
+  });
+  if (rc) return rc;
   km_colfinal_kernel<<<(d + 255) / 256, 256, 0, stream>>>(part, rb, d, n, var);
   VQ_LAUNCHED();
   km_mean_kernel<<<1, 256, 0, stream>>>(var, d, out1);
   VQ_LAUNCHED();
   return 0;
 }
+extern "C" int vatlq_kmeans_mean_var(const float* X, int64_t n, int d, double* mean, double* out1, void* ws, size_t ws_bytes,
+                                     vatlq_stream_t stream) {
+  return vatlq_kmeans_mean_var_dt(X, VATLQ_F32, n, d, mean, out1, ws, ws_bytes, stream);
+}
 
-extern "C" int vatlq_kmeans_pp(const float* X, int64_t n, int d, const double* w, int64_t k, int64_t first_center,
-                               const double* rand_vals, int trials, int32_t* center_ids, double* closest, void* ws,
-                               size_t ws_bytes, vatlq_stream_t stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  VQ_REQUIRE(km_shape_ok(n, d) && k >= 1 && k <= n, "bad shape (1 <= k <= n < 2^31, d % 4 == 0)");
-  VQ_REQUIRE(trials >= 1 && trials <= 16, "1 <= n_local_trials <= 16 (2 + int(log k) stays below 16 for k < 1.2e6)");
-  VQ_REQUIRE(first_center >= 0 && first_center < n, "first centre out of range");
-  VQ_REQUIRE(X && center_ids && closest && ws && (k == 1 || rand_vals), "null pointer");
-  VQ_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15) == 0, "X must be 16-byte aligned");
-  VQ_REQUIRE(ws_bytes >= pp_ws_bytes(n, d), "workspace too small (vatlq_kmeans_workspace_bytes)");
+// the k-means++ chain of element type T (arguments checked by the entry)
+template <typename T>
+static int kmeans_pp(const T* X, int64_t n, int d, const double* w, int64_t k, int64_t first_center, const double* rand_vals,
+                     int trials, int32_t* center_ids, double* closest, void* ws, cudaStream_t stream) {
   char* p = (char*)ws;
   auto take = [&](size_t bytes) {
     char* r = p;
@@ -820,9 +865,9 @@ extern "C" int vatlq_kmeans_pp(const float* X, int64_t n, int d, const double* w
     const int tr = c == 0 ? 1 : trials;       // step 0: the first centre alone (closest = its distances)
     // (with rand_vals == NULL the state's seed row is used and no block writes the state).  Every kernel of the chain
     // is a programmatic dependent of the one before it (pdl_enter() at kernel entry keeps the data flow in stream order)
-    VQ_CUDA(launch_pdl(km_candidates_kernel, dim3(bn), dim3(256), 0, stream, c > 0, X, d, (long long)n, (const double*)cum,
+    VQ_CUDA(launch_pdl(km_candidates_kernel<T>, dim3(bn), dim3(256), 0, stream, c > 0, X, d, (long long)n, (const double*)cum,
                        c == 0 ? (const double*)nullptr : rand_vals + (size_t)(c - 1) * trials, st, tr, (const double*)xx, Cbuf, cc));
-    rc = narrow ? launch_gemm<128, 8, 4, 1, 1>(g, stream, true) : launch_gemm<128, 16, 4, 1, 1>(g, stream, true);
+    rc = narrow ? launch_gemm<T, 128, 8, 4, 1, 1>(g, stream, true) : launch_gemm<T, 128, 16, 4, 1, 1>(g, stream, true);
     if (rc) return rc;
     if (narrow)
       VQ_CUDA(launch_pdl(km_pot_partial_kernel<8>, dim3(pot_blocks), dim3(256), 0, stream, true, (const double*)D, (const double*)closest, w,
@@ -847,21 +892,53 @@ extern "C" int vatlq_kmeans_pp(const float* X, int64_t n, int d, const double* w
   return 0;
 }
 
-extern "C" int vatlq_kmeans_gather(const float* X, int d, const int32_t* ids, int64_t k, const double* mean, double* Cc, double* Cr,
-                                   vatlq_stream_t stream_) {
+extern "C" int vatlq_kmeans_pp_dt(const void* X, int dtype, int64_t n, int d, const double* w, int64_t k, int64_t first_center,
+                                  const double* rand_vals, int trials, int32_t* center_ids, double* closest, void* ws,
+                                  size_t ws_bytes, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  VQ_REQUIRE(X && ids && mean && Cc && Cr && k >= 1 && d > 0, "bad arguments");
-  km_gather_kernel<<<(unsigned)k, 256, 0, stream>>>(X, d, ids, mean, Cc, Cr);
-  VQ_LAUNCHED();
-  return 0;
+  KM_REQUIRE_DTYPE(X, dtype);
+  VQ_REQUIRE(km_shape_ok(n, d) && k >= 1 && k <= n, "bad shape (1 <= k <= n < 2^31, d % 4 == 0)");
+  VQ_REQUIRE(trials >= 1 && trials <= 16, "1 <= n_local_trials <= 16 (2 + int(log k) stays below 16 for k < 1.2e6)");
+  VQ_REQUIRE(first_center >= 0 && first_center < n, "first centre out of range");
+  VQ_REQUIRE(X && center_ids && closest && ws && (k == 1 || rand_vals), "null pointer");
+  VQ_REQUIRE(dtype != VATLQ_F32 || (reinterpret_cast<uintptr_t>(X) & 15) == 0, "X must be 16-byte aligned");
+  VQ_REQUIRE(ws_bytes >= pp_ws_bytes(n, d), "workspace too small (vatlq_kmeans_workspace_bytes)");
+  return with_dtype(dtype, [&](auto tag) {
+    using T = km_elem_t<decltype(tag)>;
+    return kmeans_pp((const T*)X, n, d, w, k, first_center, rand_vals, trials, center_ids, closest, ws, stream);
+  });
+}
+extern "C" int vatlq_kmeans_pp(const float* X, int64_t n, int d, const double* w, int64_t k, int64_t first_center,
+                               const double* rand_vals, int trials, int32_t* center_ids, double* closest, void* ws,
+                               size_t ws_bytes, vatlq_stream_t stream) {
+  return vatlq_kmeans_pp_dt(X, VATLQ_F32, n, d, w, k, first_center, rand_vals, trials, center_ids, closest, ws, ws_bytes, stream);
 }
 
-extern "C" int vatlq_kmeans_assign(const float* X, int64_t n, int d, const double* C, int64_t k, int32_t* labels,
-                                   const int32_t* labels_old, int32_t* changed, void* ws, size_t ws_bytes,
-                                   vatlq_stream_t stream_) {
+extern "C" int vatlq_kmeans_gather_dt(const void* X, int dtype, int d, const int32_t* ids, int64_t k, const double* mean, double* Cc,
+                                      double* Cr, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  KM_REQUIRE_DTYPE(X, dtype);
+  VQ_REQUIRE(X && ids && mean && Cc && Cr && k >= 1 && d > 0, "bad arguments");
+  return with_dtype(dtype, [&](auto tag) {
+    using T = km_elem_t<decltype(tag)>;
+    km_gather_kernel<T><<<(unsigned)k, 256, 0, stream>>>((const T*)X, d, ids, mean, Cc, Cr);
+    VQ_LAUNCHED();
+    return 0;
+  });
+}
+extern "C" int vatlq_kmeans_gather(const float* X, int d, const int32_t* ids, int64_t k, const double* mean, double* Cc, double* Cr,
+                                   vatlq_stream_t stream) {
+  return vatlq_kmeans_gather_dt(X, VATLQ_F32, d, ids, k, mean, Cc, Cr, stream);
+}
+
+extern "C" int vatlq_kmeans_assign_dt(const void* X, int dtype, int64_t n, int d, const double* C, int64_t k, int32_t* labels,
+                                      const int32_t* labels_old, int32_t* changed, void* ws, size_t ws_bytes,
+                                      vatlq_stream_t stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  KM_REQUIRE_DTYPE(X, dtype);
   VQ_REQUIRE(km_shape_ok(n, d) && k >= 1 && X && C && labels && ws, "bad arguments");
-  VQ_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15) == 0 && (reinterpret_cast<uintptr_t>(C) & 15) == 0, "X and C must be 16-byte aligned");
+  VQ_REQUIRE((dtype != VATLQ_F32 || (reinterpret_cast<uintptr_t>(X) & 15) == 0) && (reinterpret_cast<uintptr_t>(C) & 15) == 0,
+             "X and C must be 16-byte aligned");
   VQ_REQUIRE(ws_bytes >= align_up((size_t)k * 8, 256), "workspace too small (vatlq_kmeans_workspace_bytes)");
   double* cn = (double*)ws;
   km_cnorm_kernel<<<(unsigned)((k * 32 + 255) / 256), 256, 0, stream>>>(C, k, d, cn);
@@ -869,13 +946,19 @@ extern "C" int vatlq_kmeans_assign(const float* X, int64_t n, int d, const doubl
   if (changed) VQ_CUDA(cudaMemsetAsync(changed, 0, 4, stream));
   GemmArgs g{};
   g.X = X; g.n = n; g.d = d; g.C = C; g.m = k; g.cn = cn; g.labels = labels; g.labels_old = labels_old; g.changed = changed;
-  return launch_gemm<64, 64, 2, 2, 0>(g, stream);
+  return with_dtype(dtype, [&](auto tag) { return launch_gemm<km_elem_t<decltype(tag)>, 64, 64, 2, 2, 0>(g, stream); });
+}
+extern "C" int vatlq_kmeans_assign(const float* X, int64_t n, int d, const double* C, int64_t k, int32_t* labels,
+                                   const int32_t* labels_old, int32_t* changed, void* ws, size_t ws_bytes,
+                                   vatlq_stream_t stream) {
+  return vatlq_kmeans_assign_dt(X, VATLQ_F32, n, d, C, k, labels, labels_old, changed, ws, ws_bytes, stream);
 }
 
-extern "C" int vatlq_kmeans_update(const float* X, int64_t n, int d, const double* w, const double* mean, const int32_t* labels, int64_t k,
-                                   double* sums, double* wsum, int32_t* order, int32_t* starts, int32_t* n_empty, void* ws,
-                                   size_t ws_bytes, vatlq_stream_t stream_) {
+extern "C" int vatlq_kmeans_update_dt(const void* X, int dtype, int64_t n, int d, const double* w, const double* mean,
+                                      const int32_t* labels, int64_t k, double* sums, double* wsum, int32_t* order, int32_t* starts,
+                                      int32_t* n_empty, void* ws, size_t ws_bytes, vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  KM_REQUIRE_DTYPE(X, dtype);
   VQ_REQUIRE(km_shape_ok(n, d) && k >= 1 && X && mean && labels && sums && wsum && order && starts && n_empty && ws, "bad arguments");
   const size_t cb = sort_bytes(n);
   VQ_REQUIRE(ws_bytes >= update_ws_bytes(n), "workspace too small (vatlq_kmeans_workspace_bytes)");
@@ -897,19 +980,36 @@ extern "C" int vatlq_kmeans_update(const float* X, int64_t n, int d, const doubl
   km_starts_kernel<<<(unsigned)((k + 1 + 255) / 256), 256, 0, stream>>>(keys_out, n, k, starts);
   VQ_LAUNCHED();
   VQ_CUDA(cudaMemsetAsync(n_empty, 0, 4, stream));
-  km_sums_kernel<<<(unsigned)k, 256, 0, stream>>>(X, d, w, mean, order, starts, k, sums, wsum, n_empty);
-  VQ_LAUNCHED();
-  return 0;
+  return with_dtype(dtype, [&](auto tag) {
+    using T = km_elem_t<decltype(tag)>;
+    km_sums_kernel<T><<<(unsigned)k, 256, 0, stream>>>((const T*)X, d, w, mean, order, starts, k, sums, wsum, n_empty);
+    VQ_LAUNCHED();
+    return 0;
+  });
+}
+extern "C" int vatlq_kmeans_update(const float* X, int64_t n, int d, const double* w, const double* mean, const int32_t* labels, int64_t k,
+                                   double* sums, double* wsum, int32_t* order, int32_t* starts, int32_t* n_empty, void* ws,
+                                   size_t ws_bytes, vatlq_stream_t stream) {
+  return vatlq_kmeans_update_dt(X, VATLQ_F32, n, d, w, mean, labels, k, sums, wsum, order, starts, n_empty, ws, ws_bytes, stream);
 }
 
-extern "C" int vatlq_kmeans_relocate(const float* X, int d, const double* w, const double* mean, const int32_t* labels, const int32_t* empty_ids,
-                                     const int32_t* far_ids, int n_empty, double* sums, double* wsum, vatlq_stream_t stream_) {
+extern "C" int vatlq_kmeans_relocate_dt(const void* X, int dtype, int d, const double* w, const double* mean, const int32_t* labels,
+                                        const int32_t* empty_ids, const int32_t* far_ids, int n_empty, double* sums, double* wsum,
+                                        vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  KM_REQUIRE_DTYPE(X, dtype);
   VQ_REQUIRE(X && mean && labels && empty_ids && far_ids && sums && wsum && n_empty >= 0 && d > 0, "bad arguments");
   if (n_empty == 0) return 0;
-  km_relocate_kernel<<<1, 256, 0, stream>>>(X, d, w, mean, labels, empty_ids, far_ids, n_empty, sums, wsum);
-  VQ_LAUNCHED();
-  return 0;
+  return with_dtype(dtype, [&](auto tag) {
+    using T = km_elem_t<decltype(tag)>;
+    km_relocate_kernel<T><<<1, 256, 0, stream>>>((const T*)X, d, w, mean, labels, empty_ids, far_ids, n_empty, sums, wsum);
+    VQ_LAUNCHED();
+    return 0;
+  });
+}
+extern "C" int vatlq_kmeans_relocate(const float* X, int d, const double* w, const double* mean, const int32_t* labels, const int32_t* empty_ids,
+                                     const int32_t* far_ids, int n_empty, double* sums, double* wsum, vatlq_stream_t stream) {
+  return vatlq_kmeans_relocate_dt(X, VATLQ_F32, d, w, mean, labels, empty_ids, far_ids, n_empty, sums, wsum, stream);
 }
 
 extern "C" int vatlq_kmeans_average(const double* sums, const double* wsum, int64_t k, int d, int64_t argmax_weight, const double* mean,
@@ -921,13 +1021,21 @@ extern "C" int vatlq_kmeans_average(const double* sums, const double* wsum, int6
   return 0;
 }
 
-extern "C" int vatlq_kmeans_rowdist(const float* X, int64_t n, int d, const double* C, const int32_t* labels, double* dis,
-                                    vatlq_stream_t stream_) {
+extern "C" int vatlq_kmeans_rowdist_dt(const void* X, int dtype, int64_t n, int d, const double* C, const int32_t* labels, double* dis,
+                                       vatlq_stream_t stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  KM_REQUIRE_DTYPE(X, dtype);
   VQ_REQUIRE(km_shape_ok(n, d) && X && C && labels && dis, "bad arguments");
-  km_rowdist_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(X, n, d, C, labels, dis);
-  VQ_LAUNCHED();
-  return 0;
+  return with_dtype(dtype, [&](auto tag) {
+    using T = km_elem_t<decltype(tag)>;
+    km_rowdist_kernel<T><<<(unsigned)((n + 127) / 128), 128, 0, stream>>>((const T*)X, n, d, C, labels, dis);
+    VQ_LAUNCHED();
+    return 0;
+  });
+}
+extern "C" int vatlq_kmeans_rowdist(const float* X, int64_t n, int d, const double* C, const int32_t* labels, double* dis,
+                                    vatlq_stream_t stream) {
+  return vatlq_kmeans_rowdist_dt(X, VATLQ_F32, n, d, C, labels, dis, stream);
 }
 
 extern "C" int vatlq_kmeans_pick(const double* dis, const int32_t* order, const int32_t* starts, int64_t k, int32_t* picks,

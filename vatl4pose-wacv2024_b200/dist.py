@@ -155,11 +155,10 @@ def distributed_query(H_local, boxes_local, is_prev_local, is_next_local, X_loca
     """One query over a pool sharded across the ranks of `group` (one process per GPU).
     Every rank passes its slice of the pool and gets the same global pick list back.  Heat-map shards may be
     fp32, fp16 or bf16 (the same dtype on every rank; the picks equal those of the fp32 upcast), and so may the
-    embedding shards X_local for representativeness "Influence" and the Coreset and Diversity filters: Influence
-    reads each rank's shard as it is, the filters gather the shards and select on them as they are, and the
-    scores and picks equal those of the fp32 upcast.  Every rank must hold X_local in one dtype (checked once, on
-    every rank, before the first step that reads it).  The K-Means and weighted filters take fp32 shards only
-    (kmeans.py raises VatlqError on a 16-bit X).
+    embedding shards X_local for representativeness "Influence" and every filter: Influence reads each rank's
+    shard as it is, the filters gather the shards and select on them as they are, and the scores and picks equal
+    those of the fp32 upcast.  Every rank must hold X_local in one dtype (checked once, on every rank, before the
+    first step that reads it).
     uncertainty: any accelerated name (THC*, WPU*, THC+WPU, HP, TPC, Entropy, MPE, Margin, None);
     representativeness: "None" or "Influence" (ActiveLearning.py:467-477); filter: "Coreset" (:609-614),
     "None" (top-k, :533-534), "Diversity" (:581-590), "K-Means" (:593-608) or "weighted" (:553-580; w_unc = cfg.VAL.W_UNC;

@@ -84,8 +84,7 @@ def select(score: torch.Tensor, unl: torch.Tensor, X, k: int, filter: str, *, la
     drops duplicate rows (np.unique(axis=0), which also sorts them), weighs each row 1 + w_unc * combine_weight *
     score and maps the chosen rows of that sorted matrix straight through the candidate ids (:553-580, kept as the
     reference has it); both clamp k to the rows they cluster, like the reference clamps query_size.
-    X may be fp32, fp16 or bf16 for Diversity and Coreset (read as it is, the picks of its fp32 upcast); K-Means and
-    weighted take fp32 only (kmeans.py raises VatlqError on a 16-bit X).
+    X may be fp32, fp16 or bf16 for every filter: it is read as it is and the picks equal those of its fp32 upcast.
     `group`: the ranks hold the same X and share the K-Means assignment step.
     Returns (picks, k, stats): int64 ids on score's device in the reference's order, the k the filter used, and
     its CoresetStats or K-Means {"n_iter", "relocations"} (None for the other filters)."""
